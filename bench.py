@@ -7,6 +7,7 @@ default 16 steps are exactly the 1024-spp BASELINE frame).  Metric: Msamples/s (
 
   python bench.py [--gpus N] [--steps K] [--warmup W]           this repo's CUDA path
   python bench.py --impl reference [...]                        the reference CPU renderer
+  python bench.py [...] --dump-outputs DIR                      also write the frame of the timed steps as DIR/*.npy
 
 N > 1 is launched by torchrun, one process per GPU; the frame is tile-sharded (tile t -> rank
 t mod N), every rank renders ONLY its tiles into a compact buffer (1/N of the frame,
@@ -59,7 +60,12 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--out-png", default="")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the frame the timed steps rendered as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm renders a timing-dependent sample)")
+    return args
 
 
 class ClockSampler:
@@ -223,6 +229,25 @@ def scene_bytes(d) -> int:
     return n
 
 
+DUMP_PIXELS = 1 << 20   # 32 bytes a pixel (two float32 RGB planes and the index): 32 MB at most
+
+
+def dump_outputs(out_dir: str, planes: dict) -> None:
+    """--dump-outputs: each (H, W, 3) plane of the frame as out_dir/<name>.npy, float32, flattened to (pixels, 3).  A
+    frame of more than DUMP_PIXELS pixels is sampled: the same fixed, seeded set of pixels in every plane and in every
+    run, their ascending flat indices in pixel_index.npy, so that two builds can be compared value for value."""
+    import numpy as np
+
+    planes = {k: v for k, v in planes.items() if v is not None}   # a tile-sharded multi-GPU frame comes back as RGB8 only
+    h, w = next(iter(planes.values())).shape[:2]
+    n = h * w
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    for name, plane in planes.items():
+        np.save(os.path.join(out_dir, name + ".npy"), plane.reshape(n, -1)[idx].astype(np.float32))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -254,6 +279,8 @@ def run_b200(args):
     # N > 1, sample-sharded (frames with too few tiles) and N = 1: a full-frame int64 buffer (a torch tensor bound with
     # rt_bind_accum), summed over ranks with one int64 reduce.
     compact = world > 1 and plan.mode == sharding.RT_SHARD_TILES
+    if args.dump_outputs and world > 1 and not compact:   # every rank decides the same, before any rendering
+        raise SystemExit("--dump-outputs: a sample-sharded multi-GPU run does not bring its frame to one host")
     tile = 16
     accum = g8 = g8_all = None
     cap = 0
@@ -331,17 +358,20 @@ def run_b200(args):
     total_samples = width * height * spp_step * args.steps
     value = total_samples / (ms * 1e-3) * 1e-6
 
-    frame_out = None
-    if rank == 0 and args.out_png:
+    # the frame of the timed steps as a caller receives it (before the counted pass below overwrites the sums)
+    frame_lin = frame_b8 = None
+    if rank == 0 and (args.out_png or args.dump_outputs):
         if compact:
-            frame_out = ctx.untile(torch.stack(g8_all).data_ptr(), cap * 3, 3, world, width, height, tile)
+            frame_b8 = ctx.untile(torch.stack(g8_all).data_ptr(), cap * 3, 3, world, width, height, tile)
         elif world == 1:
-            frame_out = ctx.download(spp_step * args.steps, linear=False, rgb8=True)
+            frame_lin, frame_b8 = ctx.download(spp_step * args.steps, linear=True, rgb8=True)
 
-    if frame_out is not None:
+    if frame_b8 is not None and args.out_png:
         from raytracingoneweekendapplication_b200.host_png import write_png
 
-        write_png(args.out_png, frame_out)
+        write_png(args.out_png, frame_b8)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"frame_linear": frame_lin, "frame_rgb8": frame_b8})
 
     # ---- per-launch algorithmic work (one counted pass of the same step, untimed) ---------------
     ctx.render(width, height, spp_step, max_depth=depth, seed=1, stats=True, **shard)   # blocking: fills counters

@@ -30,8 +30,8 @@ def _run(cmd, cwd=None):
     subprocess.check_call(cmd, cwd=cwd)
 
 
-def build_cuda(force: bool = False, verbose_ptxas: bool = False, alt_kernels: bool = False) -> str:
-    out = os.path.join(PKG, "librt_b200.so")
+def build_cuda(force: bool = False, verbose_ptxas: bool = False, alt_kernels: bool = False, out: str | None = None) -> str:
+    out = out or os.path.join(PKG, "librt_b200.so")
     csrc = os.path.join(PKG, "csrc")
     srcs = [os.path.join(csrc, f) for f in os.listdir(csrc)] + [os.path.join(ROOT, "include", "rt_b200.h")]
     if force or _newer(out, srcs):

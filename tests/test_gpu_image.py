@@ -164,24 +164,46 @@ def test_full_4k_frame_properties(ctx, scene_of):
     assert img[:200, 1200:2200, :3].mean() > img[:200, :400, :3].mean()   # the ceiling light is up there
 
 
-def test_both_kernel_versions_render_the_same_bits(built, scene_of):
+def test_both_kernel_versions_render_the_same_bits(built, tmp_path_factory):
     """render_kernel (v1, fixed ownership), render_kernel_v2 (warp streams), render_kernel_v3 (two
     path contexts per lane, rt_kernel_v3.cuh) and the wavefront pipeline (rt_wavefront.cuh)
     schedule the same samples completely differently; fixed-point sums make the frames
     bit-identical.  The three alternatives lose to v2 on every BASELINE scene and are compiled only with
-    -DRT_B200_ALT_KERNELS (`python -m raytracingoneweekendapplication_b200.build --alt`): the default library refuses them."""
+    -DRT_B200_ALT_KERNELS (`python -m raytracingoneweekendapplication_b200.build --alt`): the default library refuses them,
+    so the comparison runs in a child process on such a library, built into a temporary directory (RT_B200_LIB)."""
+    import os
+    import subprocess
+    import sys
+
+    from raytracingoneweekendapplication_b200 import build, capi
+
+    os.environ["RT_B200_KERNEL"] = "v1"
+    try:
+        with pytest.raises(capi.RtError) as e:
+            capi.Context(0).close()
+    finally:
+        os.environ.pop("RT_B200_KERNEL", None)
+    assert e.value.code == capi.RT_ERR_UNSUPPORTED and "RT_B200_ALT_KERNELS" in str(e.value)
+    lib = build.build_cuda(alt_kernels=True, out=str(tmp_path_factory.mktemp("alt_kernels") / "librt_b200.so"))
+    r = subprocess.run([sys.executable, "-c", "import sys; sys.path.insert(0, 'tests'); import test_gpu_image as t; "
+                        "t.kernel_versions_render_the_same_bits()"], cwd=helpers.ROOT, env=dict(os.environ, RT_B200_LIB=lib),
+                       capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stdout + r.stderr
+
+
+def kernel_versions_render_the_same_bits():
+    """The body of test_both_kernel_versions_render_the_same_bits, in a process whose library has the alternatives."""
     import os
 
     from raytracingoneweekendapplication_b200 import capi
 
-    os.environ["RT_B200_KERNEL"] = "v1"
-    try:
-        capi.Context(0).close()
-    except capi.RtError as e:
-        assert e.code == capi.RT_ERR_UNSUPPORTED and "RT_B200_ALT_KERNELS" in str(e)
-        pytest.skip("the alternative kernels are not compiled into the default library")
-    finally:
-        os.environ.pop("RT_B200_KERNEL", None)
+    scenes = {}
+
+    def scene_of(name):
+        if name not in scenes:
+            scenes[name] = capi.Scene(name)
+        return scenes[name]
+
     frames = []
     for version in ("v1", "v2", "wf", "v3"):
         os.environ["RT_B200_KERNEL"] = version
