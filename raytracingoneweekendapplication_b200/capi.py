@@ -13,11 +13,11 @@ from typing import Optional
 import numpy as np
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
-RT_B200_ABI_VERSION = 3
+RT_B200_ABI_VERSION = 4
 RT_ACCUM_FRAC_BITS = 28
 
 RT_OK, RT_ERR_INVALID, RT_ERR_CUDA, RT_ERR_NOMEM, RT_ERR_STATE, RT_ERR_UNSUPPORTED, RT_ERR_KERNEL = range(7)
-RT_PRIM_SPHERE, RT_PRIM_QUAD, RT_PRIM_TRIANGLE = range(3)
+RT_PRIM_SPHERE, RT_PRIM_QUAD, RT_PRIM_TRIANGLE, RT_PRIM_MESH = range(4)
 (RT_MAT_LAMBERTIAN, RT_MAT_METAL, RT_MAT_DIELECTRIC, RT_MAT_DIFFUSE_LIGHT, RT_MAT_EMISSIVE_LIGHT, RT_MAT_ISOTROPIC,
  RT_MAT_SPECULAR) = range(7)
 RT_TEX_SOLID, RT_TEX_CHECKER, RT_TEX_CHECKER_TRIANGLE, RT_TEX_IMAGE, RT_TEX_NOISE = range(5)
@@ -43,6 +43,12 @@ class rt_quad(C.Structure):
 class rt_triangle(C.Structure):
     _fields_ = [("p0", d3), ("p1", d3), ("p2", d3), ("uv0", C.c_float * 2), ("uv1", C.c_float * 2), ("uv2", C.c_float * 2),
                 ("material", C.c_int32), ("xform", C.c_int32)]
+
+
+class rt_mesh(C.Structure):
+    _fields_ = [("positions", C.POINTER(C.c_float)), ("indices", C.POINTER(C.c_uint32)), ("uvs", C.POINTER(C.c_float)),
+                ("uv_indices", C.POINTER(C.c_uint32)), ("n_vertices", C.c_int32), ("n_triangles", C.c_int32), ("n_uvs", C.c_int32),
+                ("material", C.c_int32), ("xform", C.c_int32), ("pad_", C.c_int32)]
 
 
 class rt_prim_ref(C.Structure):
@@ -97,7 +103,12 @@ class rt_scene_desc(C.Structure):
         ("perlins", C.POINTER(rt_perlin)), ("n_perlins", C.c_int32),
         ("lights", C.POINTER(rt_point_light)), ("n_lights", C.c_int32),
         ("camera", rt_camera),
+        ("meshes", C.POINTER(rt_mesh)), ("n_meshes", C.c_int32),
     ]
+
+
+# size of an ABI-3 rt_scene_desc (everything before `meshes`), which rt_upload_scene still accepts with abi_version 3
+RT_SCENE_DESC_V3_SIZE = rt_scene_desc.meshes.offset
 
 
 class rt_render_params(C.Structure):
@@ -141,7 +152,7 @@ EXPORTED_SYMBOLS = [
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
-               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref]
+               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref, rt_mesh]
 
 _lib = None
 _scenes = None
@@ -228,6 +239,8 @@ def load_scenes() -> C.CDLL:
     s.rtsc_scene_name.restype = C.c_char_p
     s.rtsc_build.argtypes = [C.c_char_p, C.c_uint, C.c_char_p]
     s.rtsc_build.restype = C.c_void_p
+    s.rtsc_set_indexed_meshes.argtypes = [C.c_int]
+    s.rtsc_set_indexed_meshes.restype = C.c_int
     s.rtsc_desc.argtypes = [C.c_void_p]
     s.rtsc_desc.restype = C.POINTER(rt_scene_desc)
     s.rtsc_frame.argtypes = [C.c_void_p] + [C.POINTER(C.c_int)] * 4
@@ -247,16 +260,33 @@ def load_scenes() -> C.CDLL:
     return s
 
 
-class Scene:
-    """A BASELINE scene built by the C++ host mirror (scenes/scenes.h) and flattened."""
+class indexed_meshes:
+    """`with indexed_meshes(True):` the scene builder loads OBJ files as indexed meshes (rt_mesh) instead of
+    triangle soups -- for Scene and for the camera::render entry points (rtsc_render_png, rtsc_render_resumable)."""
 
-    def __init__(self, name: str, seed: int = 1, asset_dir: Optional[str] = None):
+    def __init__(self, on: bool = True):
+        self.on = on
+
+    def __enter__(self):
+        self._was = load_scenes().rtsc_set_indexed_meshes(int(self.on))
+        return self
+
+    def __exit__(self, *exc):
+        load_scenes().rtsc_set_indexed_meshes(self._was)
+
+
+class Scene:
+    """A BASELINE scene built by the C++ host mirror (scenes/scenes.h) and flattened.  indexed=True loads its OBJ
+    files as indexed meshes (rt_mesh) instead of rt_triangle records: same triangles, same image."""
+
+    def __init__(self, name: str, seed: int = 1, asset_dir: Optional[str] = None, indexed: bool = False):
         from .assets import ensure_assets
 
         self.name = name
         self._s = load_scenes()
         asset_dir = ensure_assets(asset_dir)
-        self._h = self._s.rtsc_build(name.encode(), seed, asset_dir.encode())
+        with indexed_meshes(indexed):
+            self._h = self._s.rtsc_build(name.encode(), seed, asset_dir.encode())
         if not self._h:
             raise ValueError(f"unknown scene {name!r}")
         self.desc_ptr = self._s.rtsc_desc(self._h)
@@ -281,13 +311,16 @@ class Scene:
 
 
 class ObjScene(Scene):
-    """An OBJ file loaded by the host mirror's mesh::loadObj (fast path or the reference's structure)."""
+    """An OBJ file loaded by the host mirror's mesh::loadObj: the fast path (one triangle_soup), with indexed=True
+    the fast path into one indexed mesh (rt_mesh), or with per_triangle=True the reference's structure."""
 
-    def __init__(self, path: str, per_triangle: bool = False, with_media: bool = False, scale: float = 1.0):
+    def __init__(self, path: str, per_triangle: bool = False, with_media: bool = False, scale: float = 1.0, indexed: bool = False):
+        if per_triangle and indexed:
+            raise ValueError("per_triangle and indexed are two different loaders")
         self.name = path
         self._s = load_scenes()
         ms = (C.c_double * 2)()
-        self._h = self._s.rtsc_load_obj(path.encode(), int(per_triangle), int(with_media), scale, ms)
+        self._h = self._s.rtsc_load_obj(path.encode(), 2 if indexed else int(per_triangle), int(with_media), scale, ms)
         if not self._h:
             raise ValueError(f"cannot load {path!r}")
         self.load_ms, self.flatten_ms = ms[0], ms[1]

@@ -6,6 +6,8 @@
 // arrays are copied to the device as they are and seven kernels turn them into the arena the
 // render kernel reads —
 //
+//   prim_map_kernel  (scenes with indexed meshes only) primitive -> (world ref, triangle of the mesh):
+//                    a cub scan over the per-ref primitive counts, then a binary search per primitive
 //   bounds_kernel    per primitive: bake its transform (double), conservative FP32 box, scene bounds
 //   morton_kernel    63-bit Morton code of the box centre (21 bits per axis)
 //   cub radix sort   (code, primitive) pairs
@@ -34,6 +36,7 @@
 
 #include <chrono>
 #include <cstdlib>
+#include <unordered_map>
 #include <vector>
 
 #include "bvh_build.h"
@@ -59,7 +62,8 @@ struct Targets {  // arena blocks the device path fills (world part of each type
 struct Scratch {
     const rt_prim_ref* world;
     Sources src;
-    int n;
+    int n;                                 // primitives: world refs with every mesh ref expanded to its triangles
+    uint2* prim_map;                       // per primitive: (world ref, triangle of the mesh); null without meshes
     float4 *box_lo, *box_hi;               // per primitive in INPUT order; lo.w = type bits
     unsigned long long *key_in, *key_out;  // Morton codes
     uint32_t *val_in, *val_out;            // primitive index
@@ -87,12 +91,53 @@ __global__ void init_kernel(Scratch W) {
     if (threadIdx.x < 8) W.counters[threadIdx.x] = 0u;
 }
 
+// primitives of each world ref (a mesh ref stands for its triangles)
+__global__ void __launch_bounds__(256) ref_count_kernel(Scratch W, int n_world, uint32_t* count) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_world) return;
+    const rt_prim_ref r = W.world[i];
+    count[i] = r.type == RT_PRIM_MESH ? (uint32_t)W.src.meshes[r.index].n_triangles : 1u;
+}
+// primitive p lies in the last world ref whose first primitive is <= p (refs of empty meshes share
+// their first with the next ref and are skipped by taking the last)
+__global__ void __launch_bounds__(256) prim_map_kernel(Scratch W, const uint32_t* ref_first, int n_world) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= W.n) return;
+    int lo = 0, hi = n_world - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ref_first[mid] <= (uint32_t)p) lo = mid;
+        else hi = mid - 1;
+    }
+    W.prim_map[p] = make_uint2((unsigned)lo, (unsigned)p - ref_first[lo]);
+}
+
+// the world ref primitive i comes from, and which triangle of it when it is a mesh ref
+template <bool MESH>
+__device__ __forceinline__ rt_prim_ref world_ref(const Scratch& W, unsigned i, unsigned* local) {
+    if (!MESH) {
+        *local = 0;
+        return W.world[i];
+    }
+    const uint2 m = W.prim_map[i];
+    *local = m.y;
+    return W.world[m.x];
+}
+template <bool MESH>
+__device__ __forceinline__ BakedPrim fetch_prim(const Scratch& W, unsigned i) {
+    unsigned k;
+    const rt_prim_ref r = world_ref<MESH>(W, i, &k);
+    if (MESH && r.type == RT_PRIM_MESH) return rtprep::bake_mesh_triangle(W.src, r.index, k, (int)i);
+    return rtprep::bake_prim(W.src, r, (int)i);
+}
+
+template <bool MESH>
 __global__ void __launch_bounds__(256) bounds_kernel(Scratch W) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     float c[3] = {0, 0, 0};
     const bool live = i < W.n;
     if (live) {
-        const BakedPrim b = rtprep::bake_prim(W.src, W.world[i], i);
+        const BakedPrim b = fetch_prim<MESH>(W, (unsigned)i);
         float lo[3], hi[3];
         rtprep::prim_bounds(b, lo, hi);
         W.box_lo[i] = make_float4(lo[0], lo[1], lo[2], __uint_as_float(b.dev_type));
@@ -339,11 +384,12 @@ __global__ void __launch_bounds__(256) clusters_kernel(Scratch W, unsigned max_c
 __device__ __forceinline__ float4 f4(rtprep::F4 v) { return make_float4(v.x, v.y, v.z, v.w); }
 __device__ __forceinline__ int4 i4(rtprep::I4 v) { return make_int4(v.x, v.y, v.z, v.w); }
 
+template <bool MESH>
 __global__ void __launch_bounds__(256) prims_kernel(Scratch W, Targets T) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= W.n) return;
     const unsigned s = W.val_out[k];
-    const BakedPrim b = rtprep::bake_prim(W.src, W.world[s], (int)s);
+    const BakedPrim b = fetch_prim<MESH>(W, s);
     const size_t r = W.rank_at[k];
     if (b.dev_type == rtprep::PREP_TRI) {
         const rtprep::TriRec v = rtprep::make_triangle(b);
@@ -355,7 +401,10 @@ __global__ void __launch_bounds__(256) prims_kernel(Scratch W, Targets T) {
         for (int q = 0; q < 3; q++) T.quad[3 * r + q] = f4(v.q[q]);
         for (int q = 0; q < 12; q++) T.quad_d[12 * r + q] = v.d[q];
         int4 sh = i4(v.sh);
-        if (W.quad_light) sh.w = W.quad_light[W.world[s].index];
+        if (W.quad_light) {
+            unsigned local;
+            sh.w = W.quad_light[world_ref<MESH>(W, s, &local).index];
+        }
         T.quad_sh[r] = sh;
     } else if (b.dev_type == rtprep::PREP_SPHERE) {
         const rtprep::SphereRec v = rtprep::make_sphere(b);
@@ -383,22 +432,67 @@ struct ScratchPlan {
     }
 };
 
+// One array behind the meshes (positions, indices, uvs or uv_indices), copied once however many meshes share it.
+struct MeshArray {
+    const void* host;
+    size_t bytes, off;
+};
+
 struct Layout {
     size_t world, spheres, quads, triangles, xforms;
     size_t box_lo, box_hi, key_in, key_out, val_in, val_out, flag, scan, rank_at, left, right, parent_int, parent_leaf, range_first,
         nbox_lo, nbox_hi, visit, bounds, counters, cub_temp, clusters, cost, quad_light;
+    size_t meshes, ref_count, ref_first, prim_map;
+    std::vector<MeshArray> mesh_arrays;
+    std::vector<int> mesh_slots;  // per mesh: positions, indices, uvs, uv_indices -> mesh_arrays (-1: none)
+    size_t largest_input;         // biggest single host array copied in (decides whether the pinned ring is worth it)
     size_t cub_temp_bytes, total;
 };
 
-inline Layout plan_scratch(const rt_scene_desc* sc) {
+// `n` primitives: the world refs with every mesh ref expanded (validate_scene counted them)
+inline Layout plan_scratch(const rt_scene_desc* sc, int n_prims) {
     Layout L{};
     ScratchPlan p;
-    const size_t n = (size_t)sc->n_world;
-    L.world = p.add(n * sizeof(rt_prim_ref));
+    const size_t n = (size_t)n_prims, n_world = (size_t)sc->n_world;
+    L.world = p.add(n_world * sizeof(rt_prim_ref));
     L.spheres = p.add((size_t)sc->n_spheres * sizeof(rt_sphere));
     L.quads = p.add((size_t)sc->n_quads * sizeof(rt_quad));
     L.triangles = p.add((size_t)sc->n_triangles * sizeof(rt_triangle));
     L.xforms = p.add((size_t)sc->n_xforms * sizeof(rt_xform));
+    L.largest_input = std::max({(size_t)sc->n_spheres * sizeof(rt_sphere), (size_t)sc->n_quads * sizeof(rt_quad),
+                                (size_t)sc->n_triangles * sizeof(rt_triangle)});
+    const bool meshes = sc->n_meshes > 0;
+    L.meshes = p.add((size_t)sc->n_meshes * sizeof(rt_mesh));
+    if (meshes) {
+        std::unordered_map<const void*, int> seen;
+        auto slot = [&](const void* host, size_t bytes) {
+            if (!host || !bytes) return -1;
+            auto it = seen.find(host);
+            if (it != seen.end()) {
+                MeshArray& a = L.mesh_arrays[(size_t)it->second];
+                a.bytes = std::max(a.bytes, bytes);
+                return it->second;
+            }
+            seen.emplace(host, (int)L.mesh_arrays.size());
+            L.mesh_arrays.push_back(MeshArray{host, bytes, 0});
+            return (int)L.mesh_arrays.size() - 1;
+        };
+        for (int i = 0; i < sc->n_meshes; i++) {
+            const rt_mesh& m = sc->meshes[i];
+            const size_t t3 = (size_t)m.n_triangles * 3 * sizeof(uint32_t);
+            L.mesh_slots.push_back(slot(m.positions, (size_t)m.n_vertices * 3 * sizeof(float)));
+            L.mesh_slots.push_back(slot(m.indices, t3));
+            L.mesh_slots.push_back(slot(m.uvs, (size_t)m.n_uvs * 2 * sizeof(float)));
+            L.mesh_slots.push_back(slot(m.uv_indices, t3));
+        }
+        for (MeshArray& a : L.mesh_arrays) {
+            a.off = p.add(a.bytes);
+            L.largest_input = std::max(L.largest_input, a.bytes);
+        }
+    }
+    L.ref_count = p.add(meshes ? n_world * 4 : 0);
+    L.ref_first = p.add(meshes ? n_world * 4 : 0);
+    L.prim_map = p.add(meshes ? n * 8 : 0);
     L.box_lo = p.add(n * 16); L.box_hi = p.add(n * 16);
     L.key_in = p.add(n * 8); L.key_out = p.add(n * 8);
     L.val_in = p.add(n * 4); L.val_out = p.add(n * 4);
@@ -410,7 +504,7 @@ inline Layout plan_scratch(const rt_scene_desc* sc) {
     size_t sort_bytes = 0, scan_bytes = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
                                     (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, 0, 63);
-    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n);
+    cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)std::max(n, n_world));
     L.cub_temp_bytes = sort_bytes > scan_bytes ? sort_bytes : scan_bytes;
     L.cub_temp = p.add(L.cub_temp_bytes);
     L.clusters = p.add((size_t)kMaxClusters * sizeof(Cluster));
@@ -482,18 +576,21 @@ inline cudaError_t copy_in(void* dst, const void* src, size_t bytes, cudaStream_
 
 struct BuildResult {
     unsigned nodes = 0, leaves = 0, depth = 0;
+    size_t bytes_in = 0;     // host -> device bytes: the raw arrays, the mesh table, the SAH top levels
     int root = 0;            // index of the root node in the node array
     unsigned top_nodes = 0;  // nodes of the SAH top tree appended after the n - 1 radix-tree slots (0: pure LBVH)
     unsigned rebuilt_clusters = 0;
     float ms_copy_in = 0, ms_build = 0, ms_emit = 0, ms_top = 0;
 };
 
-// Copies the raw arrays of `sc` into `scratch` and runs the build on `stream`.  `T` points into
-// the scene arena.  Returns a cudaError_t-compatible code (0 = success).
-inline cudaError_t build_on_device(const rt_scene_desc* sc, unsigned char* scratch, const Layout& L, const Targets& T,
+// Copies the raw arrays of `sc` into `scratch` and runs the build of its `n` primitives (world refs
+// with the mesh refs expanded) on `stream`.  `T` points into the scene arena.  Returns a
+// cudaError_t-compatible code (0 = success).  The mesh indices must have been checked.
+inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char* scratch, const Layout& L, const Targets& T,
                                    cudaStream_t stream, CopyRing& ring, int device, bool hybrid_top, const int* quad_light,
                                    BuildResult& out) {
-    const int n = sc->n_world;
+    const int n_world = sc->n_world;
+    const bool meshes = sc->n_meshes > 0;
     Scratch W{};
     auto at = [&](size_t off) { return scratch + off; };
     cudaError_t e;
@@ -501,19 +598,39 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, unsigned char* scrat
     for (auto& v : ev) if ((e = cudaEventCreate(&v)) != cudaSuccess) return e;
     cudaEventRecord(ev[0], stream);
 #define RT_COPY_IN(field, ptr, count, type)                                                                                   \
-    if ((count) > 0 && (e = copy_in(at(L.field), ptr, (size_t)(count) * sizeof(type), stream, ring, device)) != cudaSuccess) return e;
-    RT_COPY_IN(world, sc->world, n, rt_prim_ref)
+    if ((count) > 0) {                                                                                                        \
+        if ((e = copy_in(at(L.field), ptr, (size_t)(count) * sizeof(type), stream, ring, device)) != cudaSuccess) return e;  \
+        out.bytes_in += (size_t)(count) * sizeof(type);                                                                       \
+    }
+    RT_COPY_IN(world, sc->world, n_world, rt_prim_ref)
     RT_COPY_IN(spheres, sc->spheres, sc->n_spheres, rt_sphere)
     RT_COPY_IN(quads, sc->quads, sc->n_quads, rt_quad)
     RT_COPY_IN(triangles, sc->triangles, sc->n_triangles, rt_triangle)
     RT_COPY_IN(xforms, sc->xforms, sc->n_xforms, rt_xform)
     if (quad_light) { RT_COPY_IN(quad_light, quad_light, sc->n_quads, int) }
+    if (meshes) {
+        // each distinct mesh array once, then the mesh table with its pointers moved to those copies
+        for (const MeshArray& a : L.mesh_arrays) {
+            if ((e = copy_in(at(a.off), a.host, a.bytes, stream, ring, device)) != cudaSuccess) return e;
+            out.bytes_in += a.bytes;
+        }
+        std::vector<rt_mesh> table(sc->meshes, sc->meshes + sc->n_meshes);
+        auto dev = [&](int slot) -> const void* { return slot < 0 ? nullptr : at(L.mesh_arrays[(size_t)slot].off); };
+        for (size_t i = 0; i < table.size(); i++) {
+            table[i].positions = (const float*)dev(L.mesh_slots[4 * i]);
+            table[i].indices = (const uint32_t*)dev(L.mesh_slots[4 * i + 1]);
+            table[i].uvs = (const float*)dev(L.mesh_slots[4 * i + 2]);
+            table[i].uv_indices = (const uint32_t*)dev(L.mesh_slots[4 * i + 3]);
+        }
+        RT_COPY_IN(meshes, table.data(), sc->n_meshes, rt_mesh)
+    }
 #undef RT_COPY_IN
     cudaEventRecord(ev[1], stream);
     W.world = (const rt_prim_ref*)at(L.world);
     W.src = Sources{(const rt_sphere*)at(L.spheres), (const rt_quad*)at(L.quads), (const rt_triangle*)at(L.triangles),
-                    (const rt_xform*)at(L.xforms)};
+                    (const rt_xform*)at(L.xforms), (const rt_mesh*)at(L.meshes)};
     W.n = n;
+    W.prim_map = meshes ? (uint2*)at(L.prim_map) : nullptr;
     W.box_lo = (float4*)at(L.box_lo); W.box_hi = (float4*)at(L.box_hi);
     W.key_in = (unsigned long long*)at(L.key_in); W.key_out = (unsigned long long*)at(L.key_out);
     W.val_in = (uint32_t*)at(L.val_in); W.val_out = (uint32_t*)at(L.val_out);
@@ -529,9 +646,19 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, unsigned char* scrat
 
     const int tpb = 256, gn = (n + tpb - 1) / tpb, gi = (n - 1 + tpb - 1) / tpb;
     init_kernel<<<1, 32, 0, stream>>>(W);
-    bounds_kernel<<<gn, tpb, 0, stream>>>(W);
-    morton_kernel<<<gn, tpb, 0, stream>>>(W);
     size_t tb = W.cub_temp_bytes;
+    if (meshes) {
+        uint32_t* count = (uint32_t*)at(L.ref_count);
+        uint32_t* first = (uint32_t*)at(L.ref_first);
+        ref_count_kernel<<<(n_world + tpb - 1) / tpb, tpb, 0, stream>>>(W, n_world, count);
+        if ((e = cub::DeviceScan::ExclusiveSum(W.cub_temp, tb, count, first, n_world, stream)) != cudaSuccess) return e;
+        prim_map_kernel<<<gn, tpb, 0, stream>>>(W, first, n_world);
+        bounds_kernel<true><<<gn, tpb, 0, stream>>>(W);
+    } else {
+        bounds_kernel<false><<<gn, tpb, 0, stream>>>(W);
+    }
+    morton_kernel<<<gn, tpb, 0, stream>>>(W);
+    tb = W.cub_temp_bytes;
     if ((e = cub::DeviceRadixSort::SortPairs(W.cub_temp, tb, W.key_in, W.key_out, W.val_in, W.val_out, n, 0, 63, stream)) != cudaSuccess) return e;
     karras_kernel<<<gi, tpb, 0, stream>>>(W);
     fit_kernel<<<gn, tpb, 0, stream>>>(W);
@@ -554,7 +681,8 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, unsigned char* scrat
     }
     cudaEventRecord(ev[2], stream);
     nodes_kernel<<<gi, tpb, 0, stream>>>(W, T);
-    prims_kernel<<<gn, tpb, 0, stream>>>(W, T);
+    if (meshes) prims_kernel<true><<<gn, tpb, 0, stream>>>(W, T);
+    else prims_kernel<false><<<gn, tpb, 0, stream>>>(W, T);
     cudaEventRecord(ev[3], stream);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     unsigned c[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -606,6 +734,7 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, unsigned char* scrat
                 // on `stream` and waited for: a plain cudaMemcpy from pageable memory returns once the data is staged, and
                 // the render kernels run on a non-blocking stream that the legacy stream does not order against
                 if ((e = cudaMemcpyAsync(T.nodes + 4 * (size_t)base, top.nodes.data(), top.nodes.size() * sizeof(rtbvh::Node), cudaMemcpyHostToDevice, stream)) != cudaSuccess) return e;
+                out.bytes_in += top.nodes.size() * sizeof(rtbvh::Node);
                 if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return e;
                 out.root = top.root + base;
                 out.top_nodes = (unsigned)top.nodes.size();

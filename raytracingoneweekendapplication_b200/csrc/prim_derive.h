@@ -85,12 +85,13 @@ struct BakedPrim {
 };
 
 // The typed source arrays of a scene description (host pointers on the host path, device copies
-// on the device path).
+// on the device path; on the device path the mesh table points at device copies of the mesh arrays).
 struct Sources {
     const rt_sphere* spheres;
     const rt_quad* quads;
     const rt_triangle* triangles;
     const rt_xform* xforms;
+    const rt_mesh* meshes;
 };
 
 RT_HD inline BakedPrim bake_prim(const Sources& src, rt_prim_ref r, int prim_id) {
@@ -128,6 +129,37 @@ RT_HD inline BakedPrim bake_prim(const Sources& src, rt_prim_ref r, int prim_id)
         b.xform = t.xform;
         b.uv[0] = t.uv0[0]; b.uv[1] = t.uv0[1]; b.uv[2] = t.uv1[0]; b.uv[3] = t.uv1[1]; b.uv[4] = t.uv2[0]; b.uv[5] = t.uv2[1];
         b.dev_type = PREP_TRI;
+    }
+    return b;
+}
+
+// Triangle k of mesh `mesh` (indices already checked): the float positions widened to double, then
+// transformed -- the same BakedPrim as an rt_triangle that holds the widened values.
+RT_HD inline BakedPrim bake_mesh_triangle(const Sources& src, int mesh, uint32_t k, int prim_id) {
+    const rt_mesh& m = src.meshes[mesh];
+    const rt_xform* x = m.xform >= 0 ? &src.xforms[m.xform] : nullptr;
+    const uint32_t* vi = m.indices + 3 * (size_t)k;
+    const uint32_t* ti = m.uv_indices ? m.uv_indices + 3 * (size_t)k : vi;
+    auto corner = [&](uint32_t v) {
+        const float* p = m.positions + 3 * (size_t)v;
+        return D3{(double)p[0], (double)p[1], (double)p[2]};
+    };
+    BakedPrim b;
+    b.dev_type = PREP_TRI;
+    b.prim_id = prim_id;
+    b.radius = 0.0;
+    b.a = xf_point(x, corner(vi[0]));
+    b.b = xf_point(x, corner(vi[1]));
+    b.c = xf_point(x, corner(vi[2]));
+    b.material = m.material;
+    b.xform = m.xform;
+    if (m.uvs) {
+        for (int c = 0; c < 3; c++) {
+            b.uv[2 * c] = m.uvs[2 * (size_t)ti[c]];
+            b.uv[2 * c + 1] = m.uvs[2 * (size_t)ti[c] + 1];
+        }
+    } else {  // triangle.h:24-26
+        b.uv[0] = 0.0f; b.uv[1] = 0.0f; b.uv[2] = 1.0f; b.uv[3] = 0.0f; b.uv[4] = 0.0f; b.uv[5] = 1.0f;
     }
     return b;
 }

@@ -164,6 +164,15 @@ extern "C" int rt_visible_devices(void) {
 
 extern "C" int rt_upload_scene(rt_ctx* ctx, const rt_scene_desc* sc) {
     RT_NEED(ctx);
+    // an ABI-3 description ends where `meshes` begins: read no byte past its struct_size, upload it as a scene without meshes
+    rt_scene_desc v3;
+    if (sc && sc->abi_version == 3 && sc->struct_size == offsetof(rt_scene_desc, meshes)) {
+        std::memset(&v3, 0, sizeof v3);
+        std::memcpy(&v3, sc, offsetof(rt_scene_desc, meshes));
+        v3.struct_size = sizeof v3;
+        v3.abi_version = RT_B200_ABI_VERSION;
+        sc = &v3;
+    }
     ctx->rendered = false;
     if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], dev_upload_scene(ctx->dev[0], sc));
     // replicated scene: one host thread per device (the host BVH build is repeated per device -- milliseconds for

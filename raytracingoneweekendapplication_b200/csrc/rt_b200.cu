@@ -732,6 +732,7 @@ struct DevCtx {
     // scene-upload path: 0 auto (device from kDeviceBuildAuto primitives up), 1 host SAH, 2 device (LBVH + SAH top levels), 3 device, pure LBVH
     int bvh_builder = 0;
     size_t world_type_count[4] = {0, 0, 0, 0};  // primitives of each device type in the world list (validate_scene)
+    int n_prims = 0;  // primitives of the world list with every mesh ref expanded to its triangles (validate_scene)
     rtlbvh::CopyRing copy_ring;        // pinned staging of the device path's raw-input copy
     unsigned char* scratch = nullptr;  // work space of the device build, reused across uploads
     size_t scratch_cap = 0;
@@ -946,6 +947,26 @@ bool texture_needs_uv(const rt_scene_desc* sc, int tex, int depth = 0) {
     return false;
 }
 
+// the first of n triangles with a corner index >= bound, or -1; big index buffers are split over the host cores
+int first_bad_triangle(const uint32_t* idx, int n, uint32_t bound) {
+    const int workers = n < (1 << 18) ? 1 : (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    std::vector<int> bad((size_t)workers, -1);
+    auto run = [&](int w) {
+        const int a = (int)((long long)n * w / workers), b = (int)((long long)n * (w + 1) / workers);
+        for (int t = a; t < b; t++) {
+            const uint32_t* c = idx + 3 * (size_t)t;
+            if ((c[0] >= bound) | (c[1] >= bound) | (c[2] >= bound)) { bad[(size_t)w] = t; return; }
+        }
+    };
+    std::vector<std::thread> pool;
+    for (int w = 1; w < workers; w++) pool.emplace_back(run, w);
+    run(0);
+    for (auto& t : pool) t.join();
+    for (int b : bad)
+        if (b >= 0) return b;
+    return -1;
+}
+
 }  // namespace
 
 // shallow: what must hold before the arrays may be read at all (the fingerprint of an unchanged scene is taken next);
@@ -958,18 +979,43 @@ static int validate_scene(DevCtx* ctx, const rt_scene_desc* sc, bool shallow) {
     auto neg = [](int n) { return n < 0; };
     if (neg(sc->n_world) || neg(sc->n_boundary_refs) || neg(sc->n_spheres) || neg(sc->n_quads) || neg(sc->n_triangles) ||
         neg(sc->n_media) || neg(sc->n_xforms) || neg(sc->n_materials) || neg(sc->n_textures) || neg(sc->n_images) ||
-        neg(sc->n_perlins) || neg(sc->n_lights))
+        neg(sc->n_perlins) || neg(sc->n_lights) || neg(sc->n_meshes))
         return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: negative count");
     if ((long long)sc->n_world + sc->n_boundary_refs >= (1 << 25)) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_upload_scene: more than 2^25 primitives");
     // every array with a non-zero count must be there: nothing below dereferences a null pointer
     if ((sc->n_world && !sc->world) || (sc->n_boundary_refs && !sc->boundary_refs) || (sc->n_spheres && !sc->spheres) || (sc->n_quads && !sc->quads) ||
         (sc->n_triangles && !sc->triangles) || (sc->n_media && !sc->media) || (sc->n_xforms && !sc->xforms) || (sc->n_materials && !sc->materials) ||
-        (sc->n_textures && !sc->textures) || (sc->n_images && !sc->images) || (sc->n_perlins && !sc->perlins) || (sc->n_lights && !sc->lights))
+        (sc->n_textures && !sc->textures) || (sc->n_images && !sc->images) || (sc->n_perlins && !sc->perlins) || (sc->n_lights && !sc->lights) ||
+        (sc->n_meshes && !sc->meshes))
         return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: an array with a non-zero count is null");
+    for (int i = 0; i < sc->n_meshes; i++) {
+        const rt_mesh& m = sc->meshes[i];
+        if (neg(m.n_vertices) || neg(m.n_triangles) || neg(m.n_uvs)) return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: negative count", i);
+        if ((m.n_vertices && !m.positions) || (m.n_triangles && !m.indices) || (m.n_uvs && !m.uvs) || (m.uv_indices && !m.uvs))
+            return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: an array with a non-zero count is null (or uv_indices without uvs)", i);
+        if (m.uvs && !m.uv_indices && m.n_uvs != m.n_vertices)
+            return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: without uv_indices n_uvs (%d) must equal n_vertices (%d)", i, m.n_uvs, m.n_vertices);
+        if (m.material < 0 || m.material >= sc->n_materials) return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: material out of range", i);
+        if (m.xform < -1 || m.xform >= sc->n_xforms) return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: xform out of range", i);
+    }
+    // the primitive count: a mesh ref stands for its triangles (a bad ref counts one here and is refused by the full pass)
+    long long n_prims = sc->n_world;
+    if (sc->n_meshes > 0) {
+        n_prims = 0;
+        for (int i = 0; i < sc->n_world; i++) {
+            const rt_prim_ref r = sc->world[i];
+            n_prims += (r.type == RT_PRIM_MESH && r.index >= 0 && r.index < sc->n_meshes) ? sc->meshes[r.index].n_triangles : 1;
+        }
+    }
+    if (n_prims + sc->n_boundary_refs >= (1 << 25))
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_upload_scene: more than 2^25 primitives (%lld with the meshes expanded)", n_prims + sc->n_boundary_refs);
+    ctx->n_prims = (int)n_prims;
     // the free-flight uniforms of medium m come from Philox stream RS_MEDIUM + m / 4, which shares its counter word with
     // the bounce number shifted by 8: more media than this would run into the bounce bits
     if (sc->n_media > 4 * (256 - (int)RS_MEDIUM)) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_upload_scene: at most %d media", 4 * (256 - (int)RS_MEDIUM));
+    if (shallow) return RT_OK;
     auto check_ref = [&](const rt_prim_ref& r, bool boundary) -> const char* {
+        if (r.type == RT_PRIM_MESH && !boundary) return r.index < 0 || r.index >= sc->n_meshes ? "mesh index out of range" : nullptr;
         int n = r.type == RT_PRIM_SPHERE ? sc->n_spheres : r.type == RT_PRIM_QUAD ? sc->n_quads : r.type == RT_PRIM_TRIANGLE ? sc->n_triangles : -1;
         if (n < 0) return "unknown primitive type";
         if (r.index < 0 || r.index >= n) return "primitive index out of range";
@@ -993,6 +1039,10 @@ static int validate_scene(DevCtx* ctx, const rt_scene_desc* sc, bool shallow) {
             for (int i = a; i < b; i++) {
                 const rt_prim_ref r = sc->world[i];
                 if (const char* m = check_ref(r, false)) { p.bad = i; p.msg = m; return; }
+                if (r.type == RT_PRIM_MESH) {
+                    p.count[PT_TRI] += (size_t)sc->meshes[r.index].n_triangles;
+                    continue;
+                }
                 uint32_t t = r.type == RT_PRIM_QUAD ? PT_QUAD : (r.type == RT_PRIM_TRIANGLE ? PT_TRI : PT_SPHERE);
                 if (r.type == RT_PRIM_SPHERE) {
                     const double* v = sc->spheres[r.index].center_vec;
@@ -1015,8 +1065,19 @@ static int validate_scene(DevCtx* ctx, const rt_scene_desc* sc, bool shallow) {
             for (int k = 0; k < 4; k++) ctx->world_type_count[k] += p.count[k];
         }
     }
-    for (int i = 0; i < sc->n_boundary_refs; i++)
+    for (int i = 0; i < sc->n_boundary_refs; i++) {
+        if (sc->boundary_refs[i].type == RT_PRIM_MESH) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_upload_scene: boundary_refs[%d]: a mesh cannot bound a medium", i);
         if (const char* m = check_ref(sc->boundary_refs[i], true)) return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: boundary_refs[%d]: %s", i, m);
+    }
+    // every mesh index, before anything gathers through it (host or device path)
+    for (int i = 0; i < sc->n_meshes; i++) {
+        const rt_mesh& m = sc->meshes[i];
+        int tri = -1;
+        if ((tri = first_bad_triangle(m.indices, m.n_triangles, (uint32_t)m.n_vertices)) >= 0)
+            return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: triangle %d: position index out of range (n_vertices %d)", i, tri, m.n_vertices);
+        if (m.uv_indices && (tri = first_bad_triangle(m.uv_indices, m.n_triangles, (uint32_t)m.n_uvs)) >= 0)
+            return fail(ctx, RT_ERR_INVALID, "rt_upload_scene: meshes[%d]: triangle %d: uv index out of range (n_uvs %d)", i, tri, m.n_uvs);
+    }
     for (int i = 0; i < sc->n_media; i++) {
         const rt_medium& m = sc->media[i];
         if (m.boundary_first < 0 || m.boundary_count < 0 || m.boundary_first + m.boundary_count > sc->n_boundary_refs)
@@ -1066,7 +1127,7 @@ static uint64_t hash_bytes(uint64_t h, const void* data, size_t bytes) {
 static uint64_t scene_key(const DevCtx* ctx, const rt_scene_desc* sc) {
     uint64_t h = 0x1234567887654321ull;
     const int32_t counts[16] = {sc->n_world, sc->n_boundary_refs, sc->n_spheres, sc->n_quads, sc->n_triangles, sc->n_media, sc->n_xforms, sc->n_materials,
-                                sc->n_textures, sc->n_images, sc->n_perlins, sc->n_lights, ctx->bvh_builder, ctx->bvh_width, RT_B200_ABI_VERSION, 0};
+                                sc->n_textures, sc->n_images, sc->n_perlins, sc->n_lights, ctx->bvh_builder, ctx->bvh_width, RT_B200_ABI_VERSION, sc->n_meshes};
     h = hash_bytes(h, counts, sizeof counts);
     h = hash_bytes(h, &sc->camera, sizeof sc->camera);
     h = hash_bytes(h, sc->world, (size_t)sc->n_world * sizeof(rt_prim_ref));
@@ -1080,6 +1141,15 @@ static uint64_t scene_key(const DevCtx* ctx, const rt_scene_desc* sc) {
     h = hash_bytes(h, sc->textures, (size_t)sc->n_textures * sizeof(rt_texture));
     h = hash_bytes(h, sc->perlins, (size_t)sc->n_perlins * sizeof(rt_perlin));
     h = hash_bytes(h, sc->lights, (size_t)sc->n_lights * sizeof(rt_point_light));
+    for (int i = 0; i < sc->n_meshes; i++) {
+        const rt_mesh& m = sc->meshes[i];
+        const int32_t f[6] = {m.n_vertices, m.n_triangles, m.n_uvs, m.material, m.xform, (m.uvs ? 1 : 0) | (m.uv_indices ? 2 : 0)};
+        h = hash_bytes(h, f, sizeof f);
+        h = hash_bytes(h, m.positions, (size_t)m.n_vertices * 3 * sizeof(float));
+        h = hash_bytes(h, m.indices, (size_t)m.n_triangles * 3 * sizeof(uint32_t));
+        if (m.uvs) h = hash_bytes(h, m.uvs, (size_t)m.n_uvs * 2 * sizeof(float));
+        if (m.uv_indices) h = hash_bytes(h, m.uv_indices, (size_t)m.n_triangles * 3 * sizeof(uint32_t));
+    }
     for (int i = 0; i < sc->n_images; i++) {
         const int32_t wh[2] = {sc->images[i].width, sc->images[i].height};
         h = hash_bytes(h, wh, sizeof wh);
@@ -1186,7 +1256,8 @@ static bool box_slabs(const rtprep::BakedPrim* q, float4 out[4]) {
 
 static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_build, bool* too_deep) {
     auto t_begin = std::chrono::steady_clock::now();
-    const rtprep::Sources src{sc->spheres, sc->quads, sc->triangles, sc->xforms};
+    const rtprep::Sources src{sc->spheres, sc->quads, sc->triangles, sc->xforms, sc->meshes};
+    const int n_prims = ctx->n_prims;      // the world list with every mesh ref expanded: canonical ids 0 .. n_prims - 1
     size_t world_count[4] = {0, 0, 0, 0};  // device path: primitives of each device type the kernels will write
 
     // ---- bake instance transforms, build per-primitive bounds -----------------------
@@ -1198,12 +1269,19 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         for (int i = 0; i < sc->n_boundary_refs; i++) baked.push_back(rtprep::bake_prim(src, sc->boundary_refs[i], -1));
     } else {
         for (int k = 0; k < 4; k++) world_count[k] = 0;
-        baked.reserve((size_t)sc->n_world + sc->n_boundary_refs);
-        for (int i = 0; i < sc->n_world; i++) baked.push_back(rtprep::bake_prim(src, sc->world[i], i));
+        baked.reserve((size_t)n_prims + sc->n_boundary_refs);
+        for (int i = 0; i < sc->n_world; i++) {
+            const rt_prim_ref r = sc->world[i];
+            if (r.type != RT_PRIM_MESH) {
+                baked.push_back(rtprep::bake_prim(src, r, (int)baked.size()));
+                continue;
+            }
+            for (int k = 0; k < sc->meshes[r.index].n_triangles; k++) baked.push_back(rtprep::bake_mesh_triangle(src, r.index, (uint32_t)k, (int)baked.size()));
+        }
         for (int i = 0; i < sc->n_boundary_refs; i++) baked.push_back(rtprep::bake_prim(src, sc->boundary_refs[i], -1));
 
-        std::vector<rtbvh::Prim> prims((size_t)sc->n_world);
-        for (int i = 0; i < sc->n_world; i++) {
+        std::vector<rtbvh::Prim> prims((size_t)n_prims);
+        for (int i = 0; i < n_prims; i++) {
             rtbvh::Prim& p = prims[i];
             rtprep::prim_bounds(baked[i], p.box.lo, p.box.hi);
             for (int k = 0; k < 3; k++) p.centroid[k] = 0.5f * (p.box.lo[k] + p.box.hi[k]);
@@ -1218,7 +1296,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         if (const char* e = getenv("RT_B200_ALL_AXES")) tune.all_axes_max = (uint32_t)atoll(e);
         rtbvh::build_bvh(prims, bvh, tune);
     }
-    const size_t first_boundary = device_build ? 0 : (size_t)sc->n_world;
+    const size_t first_boundary = device_build ? 0 : (size_t)n_prims;
 
     // ---- device arrays in leaf order, boundaries appended ------------------------------
     std::vector<float4> sph, msph, quad, tri, tri_sh;
@@ -1400,9 +1478,9 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
 
     // ---- the wide quantised tree, collapsed from the SAH BVH2 (host-built scenes) -----------------
     rtwide::Built wide;
-    if (!device_build && ctx->bvh_width != 2 && sc->n_world > 0) {
+    if (!device_build && ctx->bvh_width != 2 && n_prims > 0) {
         float wlo[3] = {FLT_MAX, FLT_MAX, FLT_MAX}, whi[3] = {-FLT_MAX, -FLT_MAX, -FLT_MAX};
-        for (int i = 0; i < sc->n_world; i++) {
+        for (int i = 0; i < n_prims; i++) {
             float lo[3], hi[3];
             rtprep::prim_bounds(baked[i], lo, hi);
             for (int k = 0; k < 3; k++) {
@@ -1440,7 +1518,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         blocks.push_back(b);
     };
     // device path: n - 1 radix-tree slots + room for the SAH top tree over at most kMaxClusters clusters
-    const size_t node_skip = device_build ? ((size_t)(sc->n_world - 1) + rtlbvh::kMaxClusters) * 64 : 0;
+    const size_t node_skip = device_build ? ((size_t)(n_prims - 1) + rtlbvh::kMaxClusters) * 64 : 0;
 #define UP(vec, field) add_block(vec.data(), vec.size() * sizeof(vec[0]), 0, (const void**)&S.field);
 #define UPW(vec, field, type, rec_bytes) add_block(vec.data(), vec.size() * sizeof(vec[0]), world_count[type] * (size_t)(rec_bytes), (const void**)&S.field);
     add_block(nodes.data(), device_build ? 0 : nodes.size() * sizeof(float4), node_skip, (const void**)&S.nodes);
@@ -1493,12 +1571,18 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         ctx->staged_bytes = plan.size;
         ctx->stats.upload_bytes = plan.size;
     } else {
-        for (int i = 0; i < sc->n_images; i++)
-            CU(ctx, cudaMemcpyAsync(ctx->arena + img_off[i], ctx->staging + img_stage[i], (size_t)sc->images[i].width * sc->images[i].height * 3,
-                                    cudaMemcpyHostToDevice, ctx->stream));
+        size_t staged = 0;
+        for (int i = 0; i < sc->n_images; i++) {
+            const size_t bytes = (size_t)sc->images[i].width * sc->images[i].height * 3;
+            CU(ctx, cudaMemcpyAsync(ctx->arena + img_off[i], ctx->staging + img_stage[i], bytes, cudaMemcpyHostToDevice, ctx->stream));
+            staged += bytes;
+        }
         for (const Block& b : blocks)
-            if (b.bytes) CU(ctx, cudaMemcpyAsync(ctx->arena + b.off + b.skip, ctx->staging + b.stage_off, b.bytes, cudaMemcpyHostToDevice, ctx->stream));
-        const rtlbvh::Layout L = rtlbvh::plan_scratch(sc);
+            if (b.bytes) {
+                CU(ctx, cudaMemcpyAsync(ctx->arena + b.off + b.skip, ctx->staging + b.stage_off, b.bytes, cudaMemcpyHostToDevice, ctx->stream));
+                staged += b.bytes;
+            }
+        const rtlbvh::Layout L = rtlbvh::plan_scratch(sc, n_prims);
         if (L.total > ctx->scratch_cap) {
             if (ctx->scratch) cudaFree(ctx->scratch);
             ctx->scratch = nullptr;
@@ -1513,16 +1597,16 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         T.sph_d = (double*)S.sph_d; T.msph_d = (double*)S.msph_d; T.quad_d = (double*)S.quad_d; T.tri_d = (double*)S.tri_d;
         T.sph_sh = (int4*)S.sph_sh; T.msph_sh = (int4*)S.msph_sh; T.quad_sh = (int4*)S.quad_sh;
         rtlbvh::BuildResult br;
-        if ((size_t)sc->n_triangles * sizeof(rt_triangle) >= 4 * rtlbvh::kCopyChunk || (size_t)sc->n_quads * sizeof(rt_quad) >= 4 * rtlbvh::kCopyChunk ||
-            (size_t)sc->n_spheres * sizeof(rt_sphere) >= 4 * rtlbvh::kCopyChunk)
-            CU(ctx, ctx->copy_ring.init());
-        CU(ctx, rtlbvh::build_on_device(sc, ctx->scratch, L, T, ctx->stream, ctx->copy_ring, ctx->device, ctx->bvh_builder != 3,
+        if (L.largest_input >= 4 * rtlbvh::kCopyChunk) CU(ctx, ctx->copy_ring.init());
+        CU(ctx, rtlbvh::build_on_device(sc, n_prims, ctx->scratch, L, T, ctx->stream, ctx->copy_ring, ctx->device, ctx->bvh_builder != 3,
                                         quad_light.empty() ? nullptr : quad_light.data(), br));
         n_nodes = br.nodes;
         depth = br.depth;
         leaves = br.leaves;
         root = br.root;
-        device_nodes = sc->n_world - 1 + (int)br.top_nodes;
+        device_nodes = n_prims - 1 + (int)br.top_nodes;
+        // what crossed to the device: the raw arrays (and top levels) plus the staged tables and images
+        ctx->stats.upload_bytes = br.bytes_in + staged;
         ctx->stats.device_build_ms = br.ms_build + br.ms_emit;
         ctx->stats.device_top_ms = br.ms_top;
         ctx->stats.device_copy_in_ms = br.ms_copy_in;
@@ -1541,7 +1625,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     ctx->stats.bvh_on_device = device_build ? 1 : 0;
     S.root = root;
     S.n_nodes = device_build ? device_nodes : (int)bvh.nodes.size();
-    S.n_world = sc->n_world;
+    S.n_world = n_prims;
     S.n_media = sc->n_media;
     S.n_lights = sc->n_lights;
     S.n_nee_lights = (int)nee_lights.size();
@@ -1587,8 +1671,14 @@ static int dev_upload_scene(DevCtx* ctx, const rt_scene_desc* sc) {
     // an asynchronous render may still be reading the arena -- on the caller's stream, not necessarily ours
     rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    // the same scene again (same bytes, same builder settings): the staged arena is still in pinned memory -- copy it, done
-    const uint64_t key = getenv("RT_B200_NO_SCENE_CACHE") ? 0 : scene_key(ctx, sc);
+    // which path: host (bake + binned SAH on the CPU) or device (csrc/bvh_device.cuh)
+    const int n_prims = ctx->n_prims;
+    const bool device_build = n_prims >= kDeviceBuildMin && (ctx->bvh_builder >= 2 || (ctx->bvh_builder == 0 && n_prims >= kDeviceBuildAuto));
+    // the same scene again (same bytes, same builder settings): the staged arena is still in pinned memory -- copy it, done.
+    // Only the host path leaves its whole arena staged, so only a host-path scene is fingerprinted (hashing a
+    // device-path scene would cost more than its upload)
+    const bool cache = !getenv("RT_B200_NO_SCENE_CACHE");
+    uint64_t key = cache && !device_build ? scene_key(ctx, sc) : 0;
     if (key && ctx->has_scene && ctx->staged_key == key && ctx->staged_bytes > 0) {
         CU(ctx, cudaMemcpyAsync(ctx->arena, ctx->staging, ctx->staged_bytes, cudaMemcpyHostToDevice, ctx->stream));
         CU(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1603,12 +1693,13 @@ static int dev_upload_scene(DevCtx* ctx, const rt_scene_desc* sc) {
     rc = validate_scene(ctx, sc, /*shallow=*/false);
     if (rc != RT_OK) return rc;
     free_scene(ctx);
-    // which path: host (bake + binned SAH on the CPU) or device (csrc/bvh_device.cuh)
-    const bool device_build = sc->n_world >= kDeviceBuildMin && (ctx->bvh_builder >= 2 || (ctx->bvh_builder == 0 && sc->n_world >= kDeviceBuildAuto));
     ctx->stats.device_build_ms = ctx->stats.device_copy_in_ms = ctx->stats.device_top_ms = 0;
     bool too_deep = false;
     rc = upload_scene_impl(ctx, sc, device_build, &too_deep);
-    if (rc == RT_OK && too_deep) rc = upload_scene_impl(ctx, sc, false, &too_deep);  // degenerate input: the SAH tree is shallow
+    if (rc == RT_OK && too_deep) {
+        rc = upload_scene_impl(ctx, sc, false, &too_deep);  // degenerate input: the SAH tree is shallow
+        if (cache) key = scene_key(ctx, sc);
+    }
     if (rc == RT_OK && ctx->staged_bytes > 0) ctx->staged_key = key;  // host path: the whole arena sits in the pinned staging buffer
     if (rc == RT_OK) ctx->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     return rc;
@@ -2459,7 +2550,8 @@ static int dev_get_stats(DevCtx* ctx, rt_stats* out) {
 extern "C" size_t rt_struct_size(int which) {
     static const size_t sizes[] = {sizeof(rt_scene_desc), sizeof(rt_render_params), sizeof(rt_stats), sizeof(rt_sphere), sizeof(rt_quad),
                                    sizeof(rt_triangle), sizeof(rt_medium), sizeof(rt_material), sizeof(rt_texture), sizeof(rt_image),
-                                   sizeof(rt_perlin), sizeof(rt_point_light), sizeof(rt_camera), sizeof(rt_xform), sizeof(rt_prim_ref)};
+                                   sizeof(rt_perlin), sizeof(rt_point_light), sizeof(rt_camera), sizeof(rt_xform), sizeof(rt_prim_ref),
+                                   sizeof(rt_mesh)};
     return (which >= 0 && which < (int)(sizeof(sizes) / sizeof(sizes[0]))) ? sizes[which] : 0;
 }
 

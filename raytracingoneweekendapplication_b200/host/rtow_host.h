@@ -319,6 +319,21 @@ struct xform3 {
     double t[3] = {0, 0, 0};
 };
 
+// The arrays of one indexed triangle mesh (rt_mesh), shared by the hittable that holds them and the
+// flattened scenes that point at them.
+struct mesh_arrays {
+    pod_vector<float> positions;      // 3 per vertex
+    pod_vector<uint32_t> indices;     // 3 per triangle
+    pod_vector<float> uvs;            // 2 per texture coordinate; empty: every triangle gets (0,0), (1,0), (0,1)
+    pod_vector<uint32_t> uv_indices;  // 3 per triangle; empty: the position indices
+    size_t triangles() const { return indices.size() / 3; }
+    // corner c of triangle k, widened to double (what an rt_triangle of the same face holds)
+    void corner(size_t k, int c, double out[3]) const {
+        const float* p = positions.data() + 3 * (size_t)indices[3 * k + c];
+        for (int d = 0; d < 3; d++) out[d] = p[d];
+    }
+};
+
 // Owns the POD arrays of one flattened scene and hands out an rt_scene_desc view.
 struct flat_scene {
     pod_vector<rt_prim_ref> world, boundary_refs;
@@ -333,6 +348,8 @@ struct flat_scene {
     std::vector<std::vector<uint8_t>> image_bytes;
     std::vector<rt_perlin> perlins;
     std::vector<rt_point_light> lights;
+    std::vector<rt_mesh> meshes;
+    std::vector<std::shared_ptr<const mesh_arrays>> mesh_data;  // keeps the arrays behind `meshes` alive (not copied)
     rt_camera camera{};
 
     rt_scene_desc desc() const {
@@ -352,6 +369,7 @@ struct flat_scene {
         d.images = images.data();          d.n_images = (int32_t)images.size();
         d.perlins = perlins.data();        d.n_perlins = (int32_t)perlins.size();
         d.lights = lights.data();          d.n_lights = (int32_t)lights.size();
+        d.meshes = meshes.data();          d.n_meshes = (int32_t)meshes.size();
         d.camera = camera;
         return d;
     }
@@ -376,6 +394,14 @@ struct flat_scene {
         }
         add(perlins.data(), perlins.size() * sizeof(rt_perlin));
         add(lights.data(), lights.size() * sizeof(rt_point_light));
+        for (const rt_mesh& m : meshes) {
+            const int32_t f[6] = {m.n_vertices, m.n_triangles, m.n_uvs, m.material, m.xform, (m.uvs ? 1 : 0) | (m.uv_indices ? 2 : 0)};
+            add(f, sizeof f);
+            add(m.positions, (size_t)m.n_vertices * 3 * sizeof(float));
+            add(m.indices, (size_t)m.n_triangles * 3 * sizeof(uint32_t));
+            if (m.uvs) add(m.uvs, (size_t)m.n_uvs * 2 * sizeof(float));
+            if (m.uv_indices) add(m.uv_indices, (size_t)m.n_triangles * 3 * sizeof(uint32_t));
+        }
         add(&camera, sizeof camera);
         return h;
     }
@@ -466,6 +492,48 @@ class flattener {
                 ref[i] = rt_prim_ref{RT_PRIM_TRIANGLE, (int32_t)(first + i)};
             }
         });
+    }
+
+    // An indexed mesh: one rt_mesh and ONE world ref (its triangles take consecutive canonical ids, as a soup's
+    // would).  Inside a medium boundary, where meshes are not accepted, it becomes that many rt_triangles.
+    void add_mesh(const std::shared_ptr<const mesh_arrays>& a, const shared_ptr<material>& m) {
+        const size_t n = a->triangles();
+        if (n == 0) return;
+        if (boundary_depth > 0) {
+            pod_vector<rt_triangle> tris(n);
+            for (size_t k = 0; k < n; k++) {
+                rt_triangle& t = tris[k];
+                std::memset(&t, 0, sizeof t);
+                a->corner(k, 0, t.p0); a->corner(k, 1, t.p1); a->corner(k, 2, t.p2);
+                float* uv[3] = {t.uv0, t.uv1, t.uv2};
+                for (int c = 0; c < 3; c++) {
+                    if (a->uvs.empty()) {  // triangle.h:24-26
+                        uv[c][0] = c == 1 ? 1.0f : 0.0f;
+                        uv[c][1] = c == 2 ? 1.0f : 0.0f;
+                    } else {
+                        const uint32_t i = (a->uv_indices.empty() ? a->indices : a->uv_indices)[3 * k + c];
+                        uv[c][0] = a->uvs[2 * (size_t)i];
+                        uv[c][1] = a->uvs[2 * (size_t)i + 1];
+                    }
+                }
+            }
+            add_triangles(tris, m);
+            return;
+        }
+        rt_mesh r;
+        std::memset(&r, 0, sizeof r);
+        r.positions = a->positions.data();
+        r.indices = a->indices.data();
+        r.uvs = a->uvs.empty() ? nullptr : a->uvs.data();
+        r.uv_indices = a->uv_indices.empty() ? nullptr : a->uv_indices.data();
+        r.n_vertices = (int32_t)(a->positions.size() / 3);
+        r.n_triangles = (int32_t)n;
+        r.n_uvs = (int32_t)(a->uvs.size() / 2);
+        r.material = material_id(m);
+        r.xform = current_xform();
+        fs.meshes.push_back(r);
+        fs.mesh_data.push_back(a);
+        add_ref(RT_PRIM_MESH, (int)fs.meshes.size() - 1);
     }
 
     // --- participating media (constant_medium.h:8-61) -------------------------------
@@ -1026,6 +1094,34 @@ class triangle_soup : public hittable {
     double lo[3] = {infinity, infinity, infinity}, hi[3] = {-infinity, -infinity, -infinity};
 };
 
+// The same faces as a triangle_soup, as an indexed mesh (rt_mesh): shared float vertices and 12 bytes of
+// indices per triangle instead of 104 bytes of doubles.  Flattens to ONE rt_mesh and one world ref; the
+// device records derived from it are bit-identical to the soup's, so is the image.
+class indexed_mesh : public hittable {
+  public:
+    indexed_mesh(std::shared_ptr<const rtb200::mesh_arrays> arrays, std::shared_ptr<material> m, const double l[3], const double h[3])
+        : data(std::move(arrays)), mat(std::move(m)) {
+        for (int k = 0; k < 3; k++) { lo[k] = l[k]; hi[k] = h[k]; }
+    }
+    const rtb200::mesh_arrays& arrays() const { return *data; }
+    aabb bounding_box() const override {
+        if (data->triangles() == 0) return aabb();
+        return aabb(vec3(lo[0], lo[1], lo[2]), vec3(hi[0], hi[1], hi[2]));
+    }
+    void flatten(rtb200::flattener& f) const override { f.add_mesh(data, mat); }
+    size_t list_items() const override { return data->triangles(); }
+    aabb list_item_box(size_t k) const override {  // what triangle::set_bbox gives the k-th face
+        double p[3][3];
+        for (int c = 0; c < 3; c++) data->corner(k, c, p[c]);
+        return aabb(vec3(std::min({p[0][0], p[1][0], p[2][0]}), std::min({p[0][1], p[1][1], p[2][1]}), std::min({p[0][2], p[1][2], p[2][2]})),
+                    vec3(std::max({p[0][0], p[1][0], p[2][0]}), std::max({p[0][1], p[1][1], p[2][1]}), std::max({p[0][2], p[1][2], p[2][2]})));
+    }
+  private:
+    std::shared_ptr<const rtb200::mesh_arrays> data;
+    std::shared_ptr<material> mat;
+    double lo[3] = {infinity, infinity, infinity}, hi[3] = {-infinity, -infinity, -infinity};
+};
+
 class translate : public hittable {
   public:
     translate(shared_ptr<hittable> obj, const vec3& off) : object(obj), offset(off) { bbox = object->bounding_box() + offset; }
@@ -1204,6 +1300,13 @@ class mesh {
     // stringstream per line and one shared_ptr<triangle> per face.  Both give the same flattened
     // scene, byte for byte (tests/test_obj_fast_path.py).
     static bool& per_triangle_objects() {
+        static bool flag = false;
+        return flag;
+    }
+    // With the fast path: true makes the faces ONE indexed_mesh (rt_mesh: each vertex transformed once, stored
+    // as float, 12 bytes of indices per triangle) instead of a triangle_soup -- same faces, same order, same
+    // skip rules and UVs (Q5), same device records and image.  Default false.
+    static bool& indexed_meshes() {
         static bool flag = false;
         return flag;
     }
@@ -1408,6 +1511,7 @@ class mesh {
         // the reference indexes vertices[] unchecked (undefined behaviour); such faces are refused here
         if (listed != total) std::cerr << "Skipping " << (listed - total) << " triangles with a vertex index outside the file." << std::endl;
         if (total == 0) return true;
+        if (indexed_meshes()) return emitIndexed(pieces, positions, texcoords, total, world, mat, transform);
         auto soup = make_shared<triangle_soup>(mat);
         rt_triangle* out = soup->grow(total);
         const size_t m0 = mesh_matrices.size();
@@ -1444,6 +1548,65 @@ class mesh {
         });
         for (const obj_piece& pc : pieces) soup->merge_bounds(pc.lo, pc.hi);
         world.add(soup);
+        return true;
+    }
+
+    // loadObjFast's faces as one indexed_mesh.  Every vertex goes through the float mat4 once (the soup
+    // transforms it once per face that uses it: the same operation, the same floats).  Texture coordinates
+    // keep their own indices; a corner whose `vt` index is missing or out of range points at a (0,0)
+    // appended after the file's own, which is the UV the soup gives it.
+    bool emitIndexed(std::vector<obj_piece>& pieces, const std::vector<glm::vec3>& positions, const std::vector<glm::vec2>& texcoords,
+                     size_t total, hittable_list& world, const shared_ptr<lambertian>& mat, const glm::mat4& transform) {
+        auto for_pieces = [&](auto&& fn) { rtb200::parallel_parts(pieces.size(), [&fn](size_t i, size_t) { fn(i); }); };
+        const size_t nv = positions.size(), nt = texcoords.size();
+        auto a = std::make_shared<rtb200::mesh_arrays>();
+        std::vector<glm::vec4> moved(nv);
+        a->positions.resize(3 * nv);
+        rtb200::parallel_parts(rtb200::host_parts(nv, 1 << 16), [&](size_t part, size_t parts) {
+            for (size_t v = nv * part / parts, e = nv * (part + 1) / parts; v < e; v++) {
+                moved[v] = transform * glm::vec4(positions[v], 1.0f);  // mesh.h:105-117
+                a->positions[3 * v] = moved[v].x; a->positions[3 * v + 1] = moved[v].y; a->positions[3 * v + 2] = moved[v].z;
+            }
+        });
+        a->uvs.resize(2 * (nt + 1));
+        for (size_t t = 0; t < nt; t++) { a->uvs[2 * t] = texcoords[t].x; a->uvs[2 * t + 1] = texcoords[t].y; }
+        a->uvs[2 * nt] = 0.0f;
+        a->uvs[2 * nt + 1] = 0.0f;
+        a->indices.resize(3 * total);
+        a->uv_indices.resize(3 * total);
+        const size_t m0 = mesh_matrices.size();
+        mesh_matrices.resize(m0 + total);
+        const int nvi = (int)nv;
+        for_pieces([&](size_t i) {
+            obj_piece& pc = pieces[i];
+            size_t w = pc.first_triangle;
+            auto emit = [&](const int* r, int a0, int b0, int c0) {
+                const int v[3] = {r[1 + a0], r[1 + b0], r[1 + c0]};
+                for (int k = 0; k < 3; k++)
+                    if (v[k] < 0 || v[k] >= nvi) return;
+                glm::mat4 m(1.0f);
+                for (int k = 0; k < 3; k++) {
+                    a->indices[3 * w + k] = (uint32_t)v[k];
+                    const int t = r[5 + k];  // always the face's FIRST three texcoord indices (SURVEY Q5)
+                    a->uv_indices[3 * w + k] = (t >= 0 && t < (int)nt) ? (uint32_t)t : (uint32_t)nt;
+                    m[k] = moved[(size_t)v[k]];
+                    const double p[3] = {moved[(size_t)v[k]].x, moved[(size_t)v[k]].y, moved[(size_t)v[k]].z};
+                    for (int d = 0; d < 3; d++) { pc.lo[d] = std::min(pc.lo[d], p[d]); pc.hi[d] = std::max(pc.hi[d], p[d]); }
+                }
+                m[3] = glm::vec4(0, 0, 0, 1);
+                mesh_matrices[m0 + w] = m;
+                w++;
+            };
+            for (size_t k = 0; k + 8 <= pc.face.size(); k += 8) {
+                const int* r = &pc.face[k];
+                emit(r, 0, 1, 2);
+                if (r[0] == 4) emit(r, 0, 2, 3);
+            }
+        });
+        double lo[3] = {infinity, infinity, infinity}, hi[3] = {-infinity, -infinity, -infinity};
+        for (const obj_piece& pc : pieces)
+            for (int k = 0; k < 3; k++) { lo[k] = std::min(lo[k], pc.lo[k]); hi[k] = std::max(hi[k], pc.hi[k]); }
+        world.add(make_shared<indexed_mesh>(std::move(a), mat, lo, hi));
         return true;
     }
 

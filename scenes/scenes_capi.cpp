@@ -34,6 +34,14 @@ const char* rtsc_scene_name(int i) {
     return (i >= 0 && i < n) ? names[i] : nullptr;
 }
 
+// mesh::indexed_meshes() for the scenes built from here on (rtsc_build, rtsc_render_png, rtsc_render_resumable):
+// 1 loads their OBJ files as indexed meshes (rt_mesh), 0 (default) as triangle soups.  Returns the previous setting.
+int rtsc_set_indexed_meshes(int on) {
+    const bool was = mesh::indexed_meshes();
+    mesh::indexed_meshes() = on != 0;
+    return was ? 1 : 0;
+}
+
 // Builds scene `name` with construction seed `seed`; returns NULL for an unknown name.
 rtsc_scene* rtsc_build(const char* name, unsigned seed, const char* asset_dir) {
     rtsc_scene* s = new rtsc_scene();
@@ -104,24 +112,26 @@ int rtsc_render_resumable(const char* name, unsigned seed, const char* asset_dir
     return 0;
 }
 
-// mesh::loadObj on its own (SURVEY 8f rank 2).  per_triangle = 1 selects the reference's structure
+// mesh::loadObj on its own (SURVEY 8f rank 2).  loader = 1 selects the reference's structure
 // (one shared_ptr<triangle> per face, mesh.h:22-121), 0 the fast path (parallel parse, one
-// triangle_soup).  with_media adds three constant_medium spheres next to the mesh and wraps the list
+// triangle_soup), 2 the fast path into one indexed_mesh (rt_mesh).  with_media adds three constant_medium spheres next to the mesh and wraps the list
 // in a bvh_node, which makes the flattened media multiplicities depend on the replayed median split
 // (Q15).  `ms` receives {load, bvh_node + flatten} in milliseconds.
-rtsc_scene* rtsc_load_obj(const char* path, int per_triangle, int with_media, float scale, double* ms) {
+rtsc_scene* rtsc_load_obj(const char* path, int loader, int with_media, float scale, double* ms) {
     using clk = std::chrono::steady_clock;
     rtsc_scene* s = new rtsc_scene();
     hittable_list world;
     auto mat = make_shared<lambertian>(color(0.5, 0.4, 0.3));
     mesh m;
-    const bool saved = mesh::per_triangle_objects();
-    mesh::per_triangle_objects() = per_triangle != 0;
+    const bool saved = mesh::per_triangle_objects(), saved_indexed = mesh::indexed_meshes();
+    mesh::per_triangle_objects() = loader == 1;
+    mesh::indexed_meshes() = loader == 2;  // 0 is the soup, whatever rtsc_set_indexed_meshes says
     auto t0 = clk::now();
     glm::mat4 xf = glm::scale(glm::translate(glm::mat4(1.0f), glm::vec3(0.25f, -0.5f, 1.0f)), glm::vec3(scale));
     bool ok = m.loadObj(path, world, mat, xf);
     auto t1 = clk::now();
     mesh::per_triangle_objects() = saved;
+    mesh::indexed_meshes() = saved_indexed;
     if (!ok) { delete s; return nullptr; }
     std::vector<point_light> lights;
     if (with_media) {
