@@ -121,7 +121,7 @@ class Builder {
         // if that one offers no split); ranges of <= kAllAxes primitives get the full 3-axis search.
         // Building is on the scene-upload path (host time is end-to-end time).  The limit was 256 at
         // first ("the top of the tree is where a single axis is almost always the SAH winner"): measured,
-        // the full search at the top is worth +3.3 % on C5 (tools/axes_ab.sh), and scenes big enough
+        // the full search at the top is worth +3.3 % on C5 (an A/B over Tuning::all_axes_max), and scenes big enough
         // for it to cost build time go to the device builder anyway.
         int order_axes[3] = {0, 1, 2};
         std::sort(order_axes, order_axes + 3, [&](int x, int y) { return cb.hi[x] - cb.lo[x] > cb.hi[y] - cb.lo[y]; });

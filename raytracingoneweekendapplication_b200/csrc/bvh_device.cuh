@@ -696,8 +696,7 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char
     out.root = 0;
     out.top_nodes = 0;
     // ---- SAH top levels over the cut of the radix tree ------------------------------------------
-    unsigned max_count = std::max<unsigned>((unsigned)kClusterMax, (unsigned)(2ull * (unsigned long long)n / (kMaxClusters / 2)));
-    if (const char* ev_c = getenv("RT_B200_CLUSTER")) max_count = std::max(2, atoi(ev_c));  // tuning experiments
+    const unsigned max_count = std::max<unsigned>((unsigned)kClusterMax, (unsigned)(2ull * (unsigned long long)n / (kMaxClusters / 2)));
     if (hybrid_top && (unsigned)n > 4 * max_count) {
         auto t0 = std::chrono::steady_clock::now();
         Cluster* d_clusters = (Cluster*)at(L.clusters);

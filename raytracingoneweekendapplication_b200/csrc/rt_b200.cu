@@ -1,15 +1,21 @@
 // rt_b200.cu — the C ABI of include/rt_b200.h: scene upload (flatten -> bake -> SAH BVH ->
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
-// Kernel inventory (all hand-written, no library kernels):
-//   render_kernel<STATS>   persistent megakernel: raygen -> traverse -> media -> shade ->
-//                          accumulate, with path regeneration (a lane whose path ended
-//                          starts its next sample in the same loop iteration) and 64-bit
-//                          fixed-point accumulation
+// Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT>
+//                          the persistent megakernel that renders: raygen -> traverse -> media ->
+//                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
+//                          fixed-point accumulation.  Instances: plain / LITE / STATS for the binary
+//                          and both wide trees, NEE (binary tree), and the feature instances of kInstances
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
+//   untile_kernel, tile_pack_kernel, add_sums_kernel   shard frames: compact tiles <-> full frame, sums
+//   pair_nodes_kernel      device-built BVH2 nodes -> the paired layout the traversal reads
 //   probe_*_kernel         per-function known-answer probes
-//   fma_peak_kernel        FP32 roofline denominator
+//   fma_peak_kernel, l1_peak_kernel   FP32 and L1 roofline denominators
+//   rtlbvh::*              the device BVH builder (bvh_device.cuh)
+// With -DRT_B200_ALT_KERNELS only: render_kernel (v1), render_kernel_v3 and the wavefront pipeline
+// (rtwf::wf_*), the measured alternatives to render_kernel_v2 (RT_B200_KERNEL=v1 | v3 | wf).
 #include <cuda_runtime.h>
 
 #include <chrono>
@@ -100,24 +106,14 @@ constexpr float kSampleClamp = 1048576.0f;   // 2^20: keeps 2^16 saturated sampl
 #ifndef RT_WIDE_MIN_BLOCKS
 #define RT_WIDE_MIN_BLOCKS RT_MIN_BLOCKS  // blocks per SM the wide instances are compiled for (register budget)
 #endif
-#ifndef RT_SMEM_STACK
-#define RT_SMEM_STACK 0  // binary kernel: this many traversal-stack entries per lane live in shared memory ([entry][thread]), the rest in local memory
-#endif
-#ifndef RT_STEPS_PER_VOTE
-#define RT_STEPS_PER_VOTE 1
-#endif
 #ifndef RT_V2_THREADS
 #define RT_V2_THREADS 256  // threads per block of render_kernel_v2 (tuning experiments: 224 x 3 trades warps for registers)
-#endif
-#ifndef RT_DESCEND_DIV
-#define RT_DESCEND_DIV 0
 #endif
 // STATS only: histograms of the shape of a ray's traversal, written behind the Stats block --
 // node steps before the first leaf [0,64), between two leaf visits [64,128), after the last
 // leaf (or of a ray that reaches none) [128,192), and leaf visits per ray [192,208)
 constexpr int kTravHistBins = 208;
 constexpr int kTravThreshold = RT_TRAV_THRESHOLD;
-constexpr int kDescendDiv = RT_DESCEND_DIV;
 enum : int { LANE_IDLE = 0, LANE_TRAVERSE = 1, LANE_SHADE = 2 };
 
 // WIDTH: which acceleration structure the instance traverses -- 2: the binary tree of 64-byte nodes
@@ -127,25 +123,6 @@ template <int WIDTH>
 struct TravSel { using Trav = TravW<WIDTH>; using RayConst = RayConstW; };
 template <>
 struct TravSel<2> { using Trav = rtdev::Trav; using RayConst = rtdev::RayConst; };
-
-#ifndef RT_PARK_STATE
-#define RT_PARK_STATE 0  // measured: -2.3 % on C5 (DESIGN.md section 3b item 7); stays off
-#endif
-// One 64-bit RED into the frame.  RT_FRAME_HINT 1: with an L2 evict_first policy -- the frame (265 MB at 4K) streams through
-// the 126 MB L2 once per pass and would otherwise push out the lines that are re-used: the local-memory stacks and spills
-// (119 MB allocated at 32 warps per SM) and the scene.
-#ifndef RT_FRAME_HINT
-#define RT_FRAME_HINT 0  // measured: -0.5 % on C5, -3 % on C3 (profiles/r2_frame_hint_ab.txt); stays off
-#endif
-__device__ __forceinline__ void frame_add(unsigned long long* a, unsigned long long v) {
-#if RT_FRAME_HINT
-    unsigned long long policy;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
-    asm volatile("red.global.add.L2::cache_hint.u64 [%0], %1, %2;" ::"l"(a), "l"(v), "l"(policy) : "memory");
-#else
-    atomicAdd(a, v);
-#endif
-}
 
 // FEAT: which rarely needed code the instance carries (like LITE: code that never runs still costs registers and spills).
 //   FEAT_MEDIA          the scene has a constant_medium (without: C1, C2, C4 -- +2 %, +1.9 %, +3.4 %)
@@ -167,10 +144,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     const unsigned lt_mask = (1u << lane) - 1u;
     Stats st;
     if (STATS) memset(&st, 0, sizeof st);
-#if RT_PERLIN_SMEM
-    stage_perlin(S);
-    __syncthreads();
-#endif
 
     // warp-uniform pool of (pixel, sample) pairs
     unsigned pool_pos = 0, pool_size = 0;
@@ -179,12 +152,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     // when the sample starts and read when it ends -- no register is held across the whole path for it
     __shared__ uint32_t lane_slot[RT_V2_THREADS];
     unsigned slot_base = 0;
-#if RT_PARK_STATE
-    // tuning experiment: the path state only the shade phase uses (radiance, throughput, pixel, sample, bounce) lives in
-    // shared memory [word][thread] between shade phases, so that it holds no registers (and causes no spills) across
-    // the traversal loops
-    __shared__ uint32_t park[9][RT_V2_THREADS];
-#endif
     bool exhausted = A.max_depth <= 0;  // ray_color(depth <= 0) is black before anything is traced
 
     int state = LANE_IDLE;
@@ -199,12 +166,10 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     uint32_t bounce = 0, origin_prim = PRIM_NONE;
     float nee_pdf = 0.0f;  // NEE: > 0 when the previous vertex sampled the listed emitters directly: the density of the direction it scattered into
     typename TravSel<WIDTH>::Trav tr;
-    StackEntry stack_mem[WIDTH == 2 ? STACK_SIZE - RT_SMEM_STACK : 1];
+    StackEntry stack_mem[WIDTH == 2 ? STACK_SIZE : 1];
     extern __shared__ uint2 wide_stack_mem[];
     auto stack = [&]() {
-        if constexpr (WIDTH == 2 && RT_SMEM_STACK == 0) return &stack_mem[0];
-        else if constexpr (WIDTH == 2)
-            return HybridStack<RT_SMEM_STACK, RT_V2_THREADS>{(uint32_t)__cvta_generic_to_shared(wide_stack_mem) + threadIdx.x * 8u, &stack_mem[0]};
+        if constexpr (WIDTH == 2) return &stack_mem[0];
         else return SmemStack<RT_V2_THREADS>::make(wide_stack_mem);
     }();
     tr.clear();
@@ -251,13 +216,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     L = v3(0, 0, 0);
                     T = v3(1, 1, 1);
                     bounce = 0;
-#if RT_PARK_STATE
-                    park[0][threadIdx.x] = park[1][threadIdx.x] = park[2][threadIdx.x] = 0u;
-                    park[3][threadIdx.x] = park[4][threadIdx.x] = park[5][threadIdx.x] = 0x3F800000u;
-                    park[6][threadIdx.x] = rng.pixel;
-                    park[7][threadIdx.x] = rng.sample;
-                    park[8][threadIdx.x] = 0u;
-#endif
                     origin_prim = PRIM_NONE;
                     nee_pdf = 0.0f;
                     tr.init(S, kInf);
@@ -276,19 +234,16 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
             rc.set(ray);
             while (true) {
                 // descend: every traversing lane that holds an interior node takes one step per
-                // iteration; lanes that reached a leaf wait, but only until the descending ones
-                // are a minority (1/kDescendDiv of the traversing lanes) -- those simply keep
-                // descending in the next round while the others intersect their leaves
+                // iteration; lanes that reached a leaf wait until no lane of the warp descends
                 while (true) {
                     // a lane that is not traversing holds LINK_DONE (negative), so the link alone says who
                     // descends; the vote goes straight to a predicate (two instructions fewer per step: +1.2 % on C5)
                     const bool descending = tr.wants_node();
-                    if (!STATS && kDescendDiv == 0) {
+                    if (!STATS) {
                         if (!__any_sync(0xffffffffu, descending)) break;
                     }
-                    const unsigned dmask = (STATS || kDescendDiv > 0) ? __ballot_sync(0xffffffffu, descending) : 1u;
+                    const unsigned dmask = STATS ? __ballot_sync(0xffffffffu, descending) : 1u;
                     if (dmask == 0u) break;
-                    if (kDescendDiv > 0 && kDescendDiv * __popc(dmask) <= __popc(__ballot_sync(0xffffffffu, state == LANE_TRAVERSE))) break;
                     if (STATS) {
                         const unsigned tmask = __ballot_sync(0xffffffffu, state == LANE_TRAVERSE);
                         if (lane == 0) { st.desc_iters++; st.desc_lanes += __popc(dmask); st.desc_trav_lanes += __popc(tmask); }
@@ -302,11 +257,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                                 atomicAdd(hist + 192 + min(n_leaf, 15u), 1ull);
                             }
                         }
-                        // RT_STEPS_PER_VOTE > 1: further steps of the lanes that still descend without asking the warp in between (the
-                        // vote, the reconvergence and the loop branch are 10 of a binary step's 75 instructions)
-#pragma unroll
-                        for (int extra = 1; extra < RT_STEPS_PER_VOTE; extra++)
-                            if (!STATS && tr.wants_node()) tr.template node_step<STATS>(S, ray, rc, 0.001f, stack, &st);
                     }
                 }
                 if (STATS) {
@@ -339,13 +289,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
             if (lane == 0) { st.shade_iters++; st.shade_lanes += __popc(smask); }
         }
         if (state == LANE_SHADE) {
-#if RT_PARK_STATE
-            L = v3(__uint_as_float(park[0][threadIdx.x]), __uint_as_float(park[1][threadIdx.x]), __uint_as_float(park[2][threadIdx.x]));
-            T = v3(__uint_as_float(park[3][threadIdx.x]), __uint_as_float(park[4][threadIdx.x]), __uint_as_float(park[5][threadIdx.x]));
-            rng.pixel = park[6][threadIdx.x];
-            rng.sample = park[7][threadIdx.x];
-            bounce = park[8][threadIdx.x];
-#endif
             Hit hit = tr.hit;
             int medium = -1;
             if ((FEAT & FEAT_MEDIA) && S.n_media > 0) medium = media_hit<STATS, (FEAT & FEAT_MEDIA_GENERAL) != 0>(S, ray, 0.001f, hit.t, rng, bounce, &st);
@@ -409,20 +352,15 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
             if (done) {
                 unsigned long long* a = accum + 4ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel);
                 if (isfinite(L.x) && isfinite(L.y) && isfinite(L.z)) {
-                    frame_add(a + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
-                    frame_add(a + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
-                    frame_add(a + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
+                    atomicAdd(a + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
+                    atomicAdd(a + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
+                    atomicAdd(a + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
                 } else {
                     atomicAdd(a + 3, 1ull);
                     if (STATS) st.nonfinite++;
                 }
                 state = LANE_IDLE;
             } else {
-#if RT_PARK_STATE
-                park[0][threadIdx.x] = __float_as_uint(L.x); park[1][threadIdx.x] = __float_as_uint(L.y); park[2][threadIdx.x] = __float_as_uint(L.z);
-                park[3][threadIdx.x] = __float_as_uint(T.x); park[4][threadIdx.x] = __float_as_uint(T.y); park[5][threadIdx.x] = __float_as_uint(T.z);
-                park[8][threadIdx.x] = bounce;
-#endif
                 tr.init(S, kInf);
                 state = tr.done() ? LANE_SHADE : LANE_TRAVERSE;
                 if (STATS) { st.rays++; seg_steps = n_leaf = 0; }
@@ -686,7 +624,7 @@ struct DevCtx {
     AccumLayout acc;                        // layout of `accum`
     unsigned char* frame_scratch = nullptr;  // full-frame copies of compact data (checkpoints, single-shard downloads)
     size_t frame_scratch_cap = 0;
-    unsigned long long* counters = nullptr;  // [0] work counter, [1] overflow flag
+    unsigned long long* counters = nullptr;  // [0] work counter, [1..3] unused
     Stats* dstats = nullptr;
     rt_stats stats{};
     int cam_w = 0, cam_h = 0;  // frame the device camera block was computed for
@@ -819,7 +757,7 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     CU(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     CU(ctx, cudaEventCreate(&ctx->ev0));
     CU(ctx, cudaEventCreate(&ctx->ev1));
-    CU(ctx, cudaMalloc(&ctx->counters, 12 * sizeof(unsigned long long)));  // {work counter, guard flag, -, -} x (plain, overlap lane 0, lane 1)
+    CU(ctx, cudaMalloc(&ctx->counters, 12 * sizeof(unsigned long long)));  // {work counter, -, -, -} x (plain, overlap lane 0, lane 1)
     CU(ctx, cudaMalloc(&ctx->dstats, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long)));
     // local-memory traversal stacks live in L1: prefer L1 over shared memory (the wide instances
     // get their carve-out per launch, from the depth of the uploaded tree)
@@ -829,21 +767,6 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     cudaFuncSetAttribute(render_kernel_v2<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     cudaFuncSetAttribute(render_kernel_v2<false, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     for (int k = 0; k < kNumInstances; k++) cudaFuncSetAttribute((const void*)kInstances[k].kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-#if RT_PARK_STATE  // measurement build: 9 words per thread of parked path state, RT_MIN_BLOCKS blocks per SM
-    {
-        const int pct = (int)((100 * RT_MIN_BLOCKS * (10 * RT_V2_THREADS * 4 + 2048) + 233471) / 233472);
-        cudaFuncSetAttribute(render_kernel_v2<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        cudaFuncSetAttribute(render_kernel_v2<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        cudaFuncSetAttribute(render_kernel_v2<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        cudaFuncSetAttribute(render_kernel_v2<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        cudaFuncSetAttribute(render_kernel_v2<false, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-    }
-#endif
-#if RT_PERLIN_SMEM  // measurement build: room for three blocks' tables
-    cudaFuncSetAttribute(render_kernel_v2<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 10);
-    cudaFuncSetAttribute(render_kernel_v2<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 10);
-    cudaFuncSetAttribute(render_kernel_v2<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 10);
-#endif
     if (const char* bv = getenv("RT_B200_BVH"))
         ctx->bvh_builder = strcmp(bv, "host") == 0 ? 1 : (strcmp(bv, "device") == 0 ? 2 : (strcmp(bv, "lbvh") == 0 ? 3 : 0));
     if (const char* wv = getenv("RT_B200_BVH_WIDTH")) {
@@ -1289,12 +1212,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
             p.index = (uint32_t)i;
             p.cost = baked[i].dev_type == PT_SPHERE ? 1.0f : (baked[i].dev_type == PT_MSPHERE ? 1.2f : 1.3f);
         }
-        rtbvh::Tuning tune;  // RT_B200_MAX_LEAF / RT_B200_TRAV_COST: tuning experiments only
-        if (const char* e = getenv("RT_B200_MAX_LEAF")) tune.max_leaf = std::max(1, std::min(8, atoi(e)));
-        if (const char* e = getenv("RT_B200_TRAV_COST")) tune.trav_cost = (float)atof(e);
-        if (const char* e = getenv("RT_B200_SHORTCUT_MIN")) tune.shortcut_min = (size_t)atoll(e);
-        if (const char* e = getenv("RT_B200_ALL_AXES")) tune.all_axes_max = (uint32_t)atoll(e);
-        rtbvh::build_bvh(prims, bvh, tune);
+        rtbvh::build_bvh(prims, bvh);
     }
     const size_t first_boundary = device_build ? 0 : (size_t)n_prims;
 
@@ -1472,9 +1390,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     std::vector<float4> nodes(bvh.nodes.size() * 4);
     static_assert(sizeof(rtbvh::Node) == 64, "node layout");
     std::memcpy(nodes.data(), bvh.nodes.data(), bvh.nodes.size() * 64);
-#if RT_NODE_PAIRED
     for (size_t i = 0; i < bvh.nodes.size(); i++) pair_node(&nodes[4 * i]);
-#endif
 
     // ---- the wide quantised tree, collapsed from the SAH BVH2 (host-built scenes) -----------------
     rtwide::Built wide;
@@ -1489,12 +1405,8 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
                 whi[k] = std::max(whi[k], hi[k] + e);
             }
         }
-        rtwide::CollapseTuning wt;  // RT_B200_WIDE_*: tuning experiments only
-        if (const char* e = getenv("RT_B200_WIDE_NODE_COST")) wt.node_cost = (float)atof(e);
-        if (const char* e = getenv("RT_B200_WIDE_GRID_STEPS")) wt.grid_steps = (float)atof(e);
-        if (const char* e = getenv("RT_B200_WIDE_SCALE_AWARE")) wt.scale_aware = atoi(e) != 0;
-        if (ctx->bvh_width == 8) rtwide::build_wide<8>(bvh, true, wlo, whi, wide, wt);
-        else rtwide::build_wide<4>(bvh, true, wlo, whi, wide, wt);
+        if (ctx->bvh_width == 8) rtwide::build_wide<8>(bvh, true, wlo, whi, wide);
+        else rtwide::build_wide<4>(bvh, true, wlo, whi, wide);
         if (wide.depth > (uint32_t)kWideMaxDepth) wide = rtwide::Built();  // degenerate tree: keep the binary one
     }
 
@@ -1614,13 +1526,11 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
             *too_deep = true;
             return RT_OK;
         }
-#if RT_NODE_PAIRED
         if (device_nodes > 0) {
             pair_nodes_kernel<<<(device_nodes + 255) / 256, 256, 0, ctx->stream>>>((float4*)S.nodes, device_nodes);
             CU(ctx, cudaGetLastError());
             CU(ctx, cudaStreamSynchronize(ctx->stream));
         }
-#endif
     }
     ctx->stats.bvh_on_device = device_build ? 1 : 0;
     S.root = root;
@@ -1904,8 +1814,8 @@ static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int
     return RT_OK;
 }
 
-// Finish what an RT_FLAG_ASYNC render left pending: wait for the stream it ran on, read the device time, the
-// guard counters and (STATS) the counters.  Everything that touches the frame or the scene calls this first.
+// Finish what an RT_FLAG_ASYNC render left pending: wait for the stream it ran on, read the device time and
+// (STATS) the counters.  Everything that touches the frame or the scene calls this first.
 static int dev_wait_lanes(DevCtx* ctx, float* ms_per_pass) {
     float ms_max = 0.0f;
     bool had = false;
@@ -1940,10 +1850,6 @@ static int dev_wait(DevCtx* ctx) {
     float ms = 0;
     CU(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     ctx->stats.render_ms = ms;
-    unsigned long long c[2] = {0, 0};
-    CU(ctx, cudaMemcpyAsync(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    if (c[1]) return fail(ctx, RT_ERR_KERNEL, "traversal stack overflow (BVH deeper than %d)", STACK_SIZE);
     if (ov_ms >= 0.0f) ctx->stats.render_ms = ov_ms;
     if (ctx->pending_stats) {
         Stats h;
@@ -2053,7 +1959,6 @@ static int launch_wavefront(DevCtx* ctx, const RenderArgs& A, cudaStream_t strea
         CU(ctx, cudaStreamSynchronize(stream));
         if (h[3] == 0) break;  // nothing appended by the last shade: every path ended and the stream is dry
     }
-    CU(ctx, cudaMemcpyAsync(ctx->counters + 1, P.ctr + 1, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, stream));
     ctx->stats.kernel_launches = launches;
     return RT_OK;
 }
@@ -2079,7 +1984,7 @@ static RenderKernel v2_kernel(int variant, int width) {
     return width == 8 ? v2_instance<8>(variant) : (width == 4 ? v2_instance<4>(variant) : v2_instance<2>(variant));
 }
 // dynamic shared memory of a wide instance: the traversal stacks, [entry][thread]
-static size_t v2_smem(const DevCtx* ctx, int width) { return width <= 2 ? (size_t)RT_SMEM_STACK * RT_V2_THREADS * 8 : (size_t)std::max(ctx->wide_depth, 1) * RT_V2_THREADS * sizeof(uint2); }
+static size_t v2_smem(const DevCtx* ctx, int width) { return width <= 2 ? 0 : (size_t)std::max(ctx->wide_depth, 1) * RT_V2_THREADS * sizeof(uint2); }
 
 // blocks per SM the kernel instance runs with (the grid is persistent: SMs x this)
 static int v2_blocks_per_sm(DevCtx* ctx, int variant, int width, int* out) {
@@ -2098,16 +2003,7 @@ static int v2_blocks_per_sm(DevCtx* ctx, int variant, int width, int* out) {
 static int launch_v2(DevCtx* ctx, int variant, int width, int grid, const RenderArgs& A, cudaStream_t stream, unsigned long long* counters = nullptr) {
     if (!counters) counters = ctx->counters;
     width = v2_effective_width(variant, width);
-    size_t smem = v2_smem(ctx, width);
-    // RT_B200_DUMMY_SMEM: unused dynamic shared memory per block, to measure what giving up
-    // that much L1 would cost (tuning experiment, binary kernel only)
-    if (width == 2)
-        if (const char* e = getenv("RT_B200_DUMMY_SMEM")) {
-            smem = (size_t)atoi(e);
-            const int pct = (int)std::min<size_t>(100, (100 * 3 * (smem + 1024) + 233471) / 233472);
-            cudaFuncSetAttribute((const void*)v2_kernel(variant, 2), cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        }
-    v2_kernel(variant, width)<<<grid, RT_V2_THREADS, smem, stream>>>(ctx->scene, A, ctx->accum, counters, ctx->dstats);
+    v2_kernel(variant, width)<<<grid, RT_V2_THREADS, v2_smem(ctx, width), stream>>>(ctx->scene, A, ctx->accum, counters, ctx->dstats);
     return RT_OK;
 }
 
@@ -2214,10 +2110,8 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     const unsigned long long resident_warps = (unsigned long long)grid * (ctx->kernel_version == 2 ? RT_V2_THREADS / 32 : 8);
     int n_seg = 1;
     if (A.n_local_samples > 0 && pixel_blocks > 0) {
-        // >= kItemsPerWarp items per resident warp: the end-of-kernel tail is one item long
-        unsigned long long per_warp = 64;
-        if (const char* e = getenv("RT_B200_ITEMS_PER_WARP")) per_warp = (unsigned long long)std::max(1, atoi(e));  // tuning experiments
-        unsigned long long want = (resident_warps * per_warp + pixel_blocks - 1) / pixel_blocks;
+        // >= 64 items per resident warp: the end-of-kernel tail is one item long
+        unsigned long long want = (resident_warps * 64 + pixel_blocks - 1) / pixel_blocks;
         if (want < 1) want = 1;
         if (want > (unsigned long long)A.n_local_samples) want = A.n_local_samples;
         n_seg = (int)want;
@@ -2518,7 +2412,6 @@ static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* p
     alloc((void**)&d_n, n * 12, normal);
     alloc((void**)&d_p, n * 12, point);
     alloc((void**)&d_uv, n * 8, uv);
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), ctx->stream);
     if (e == cudaSuccess) {
         dim3 block(8, 8), grid((width + 7) / 8, (height + 7) / 8);
         aov_kernel<<<grid, block, 0, ctx->stream>>>(ctx->scene, ctx->camera_d, width, height, d_id, d_t, d_n, d_p, d_uv);
@@ -2535,9 +2428,6 @@ static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* p
     fetch(uv, d_uv, n * 8);
     cudaFree(d_id); cudaFree(d_t); cudaFree(d_n); cudaFree(d_p); cudaFree(d_uv);
     if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_render_aov: %s", cudaGetErrorString(e));
-    unsigned long long c[2] = {0, 0};
-    CU(ctx, cudaMemcpy(c, ctx->counters, sizeof c, cudaMemcpyDeviceToHost));
-    if (c[1]) return fail(ctx, RT_ERR_KERNEL, "traversal stack overflow (BVH deeper than %d)", STACK_SIZE);
     return RT_OK;
 }
 
@@ -2619,7 +2509,6 @@ static int run_probe(DevCtx* ctx, const char* name, const std::vector<std::pair<
     }
     for (size_t i = 0; i < outputs.size() && e == cudaSuccess; i++)
         if (outputs[i].first) e = cudaMalloc(&dout[i], std::max<size_t>(outputs[i].second, 16));
-    if (e == cudaSuccess) e = cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), ctx->stream);
     if (e == cudaSuccess) {
         launch(din, dout);
         e = cudaGetLastError();

@@ -151,30 +151,7 @@ __device__ __forceinline__ V3 fma3(float s, V3 a, V3 b) { return V3{fmaf(s, a.x,
 __device__ __forceinline__ V3 normalize(V3 a) { return rsqrtf(dot(a, a)) * a; }
 
 __device__ __forceinline__ float4 ldg4(const float4* p) { return __ldg(p); }
-// node / primitive loads with an L1 eviction priority (tuning experiment, -DRT_NODE_HINT=1 evict_last, 2 evict_first;
-// -DRT_PRIM_HINT likewise): the working set of C5 (nodes 140 KB + primitives 420 KB + shading records) is larger than L1
-#ifndef RT_PREFETCH_FAR
-#define RT_PREFETCH_FAR 0
-#endif
-#ifndef RT_NODE_HINT
-#define RT_NODE_HINT 0
-#endif
-#ifndef RT_PRIM_HINT
-#define RT_PRIM_HINT 0
-#endif
-template <int HINT>
-__device__ __forceinline__ float4 ldg4_hint(const float4* p) {
-    if (HINT == 0) return __ldg(p);
-    float4 v;
-    if (HINT == 1) asm("ld.global.nc.L1::evict_last.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    else if (HINT == 2) asm("ld.global.nc.L1::evict_first.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    else asm("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    return v;
-}
 
-#ifndef RT_NODE_PAIRED
-#define RT_NODE_PAIRED 1
-#endif
 // a * s + t on both halves in one instruction (FFMA2, new with sm_100; the scalars are broadcast operands)
 __device__ __forceinline__ float2 ffma2(float2 a, float s, float t) {
     unsigned long long ra = (unsigned long long)__float_as_uint(a.x) | ((unsigned long long)__float_as_uint(a.y) << 32);
@@ -196,10 +173,8 @@ __device__ __forceinline__ float2 ffma2(float2 a, float s, float t) {
 // ---------------------------------------------------------------------------------
 constexpr uint32_t RS_CAMERA = 0, RS_DEFOCUS = 1, RS_SCATTER = 16, RS_NEE = 24, RS_MEDIUM = 32;
 
-#ifndef RT_PHILOX_ATTR
-#define RT_PHILOX_ATTR __forceinline__  // out of line costs 10 % on C5 (call ABI spills); measured
-#endif
-__device__ RT_PHILOX_ATTR uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+// inlined: out of line it costs 10 % on C5 (call ABI spills)
+__device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
 #pragma unroll
     for (int r = 0; r < 10; r++) {
         uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
@@ -349,7 +324,7 @@ __device__ __forceinline__ void hit_prim(const DevScene& S, uint32_t type, uint3
         const double* cd;
         const bool moving = MSPH && type == PT_MSPHERE;
         if (!moving) {
-            s = ldg4_hint<RT_PRIM_HINT>(S.sph + idx);
+            s = ldg4(S.sph + idx);
             cd = S.sph_d + 4 * (size_t)idx;
         } else {
             const float4* m = S.msph + 2 * (size_t)idx;
@@ -363,7 +338,7 @@ __device__ __forceinline__ void hit_prim(const DevScene& S, uint32_t type, uint3
         if (STATS) st->quad_tests++;
         if (prim == origin_prim) return;  // a ray leaving a planar primitive cannot hit it again
         const float4* q = S.quad + 3 * (size_t)idx;
-        hit_quad(ldg4_hint<RT_PRIM_HINT>(q), ldg4_hint<RT_PRIM_HINT>(q + 1), ldg4_hint<RT_PRIM_HINT>(q + 2), ray, tmin, prim, hit);
+        hit_quad(ldg4(q), ldg4(q + 1), ldg4(q + 2), ray, tmin, prim, hit);
     } else if (!LITE && type == PT_TRI) {
         if (STATS) st->tri_tests++;
         if (prim == origin_prim) return;
@@ -402,32 +377,6 @@ __device__ __forceinline__ StackEntry pack_entry(int link, float t) {
     return ((unsigned long long)__float_as_uint(t) << 32) | (unsigned)link;
 }
 
-// Where a lane's stack lives.  A plain pointer = a local-memory array (every lane's entry at its own
-// depth is its own 32-byte sector: ncu measured 1.4-1.9 of 32 bytes used per sector).  HybridStack =
-// the first K entries in shared memory laid out [entry][thread] (the 32 lanes of a warp always hit 32
-// different banks, whatever depth each is at), deeper entries in the local array.
-__device__ __forceinline__ StackEntry stack_ld(const StackEntry* s, int i) { return s[i]; }
-__device__ __forceinline__ void stack_st(StackEntry* s, int i, StackEntry v) { s[i] = v; }
-template <int K, int STRIDE>
-struct HybridStack {
-    uint32_t addr;      // shared-window address of this thread's column
-    StackEntry* local;  // entries K and up
-};
-template <int K, int STRIDE>
-__device__ __forceinline__ StackEntry stack_ld(HybridStack<K, STRIDE> s, int i) {
-    if (i < K) {
-        StackEntry v;
-        asm volatile("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(s.addr + (uint32_t)i * (STRIDE * 8u)));
-        return v;
-    }
-    return s.local[i - K];
-}
-template <int K, int STRIDE>
-__device__ __forceinline__ void stack_st(HybridStack<K, STRIDE> s, int i, StackEntry v) {
-    if (i < K) asm volatile("st.shared.u64 [%0], %1;" ::"r"(s.addr + (uint32_t)i * (STRIDE * 8u)), "l"(v) : "memory");
-    else s.local[i - K] = v;
-}
-
 struct Trav {
     Hit hit;
     int cur;  // >= 0 interior node, < 0 leaf, LINK_DONE finished (also < 0)
@@ -446,12 +395,11 @@ struct Trav {
     __device__ __forceinline__ bool wants_node() const { return cur >= 0; }
 
     // pop, skipping subtrees that start beyond the closest hit so far
-    template <class Stack>
-    __device__ __forceinline__ void pop(Stack stack) {
+    __device__ __forceinline__ void pop(const StackEntry* stack) {
         cur = LINK_DONE;
         while (sp > 0) {
             sp--;
-            const StackEntry e = stack_ld(stack, sp);
+            const StackEntry e = stack[sp];
             if (__uint_as_float((unsigned)(e >> 32)) <= hit.t) {
                 cur = (int)(unsigned)e;
                 break;
@@ -462,13 +410,11 @@ struct Trav {
     // One 64-byte node = two child boxes (aabb.h:61-85 twice).  The choice of the next link is
     // select-based: the four outcomes (both / left / right / none) share one instruction stream,
     // the push is a predicated store, and only the (rare) "none" case branches into pop().
-    template <bool STATS, class Stack>
-    __device__ __forceinline__ void interior(const DevScene& S, const RayConst& rc, float tmin, Stack stack, Stats* st,
-                                             int* overflow) {
+    template <bool STATS>
+    __device__ __forceinline__ void interior(const DevScene& S, const RayConst& rc, float tmin, StackEntry* stack, Stats* st) {
         const float4* n = S.nodes + 4 * (size_t)cur;
-        float4 a = ldg4_hint<RT_NODE_HINT>(n), b = ldg4_hint<RT_NODE_HINT>(n + 1), c = ldg4_hint<RT_NODE_HINT>(n + 2), e = ldg4_hint<RT_NODE_HINT>(n + 3);
+        float4 a = ldg4(n), b = ldg4(n + 1), c = ldg4(n + 2), e = ldg4(n + 3);
         if (STATS) { st->node_visits++; st->box_tests += 2; }
-#if RT_NODE_PAIRED
         // paired layout (pair_nodes): the same plane of the left and the right box sit side by side, so one
         // FFMA2 (fma.rn.f32x2, sm_100) moves both to ray space -- 6 instructions instead of 12, same values
         const float2 x0 = ffma2(make_float2(a.x, a.y), rc.idx, -rc.ox), y0 = ffma2(make_float2(a.z, a.w), rc.idy, -rc.oy);
@@ -477,15 +423,6 @@ struct Trav {
         const float lx0 = x0.x, rx0 = x0.y, ly0 = y0.x, ry0 = y0.y, lz0 = z0.x, rz0 = z0.y;
         const float lx1 = x1.x, rx1 = x1.y, ly1 = y1.x, ry1 = y1.y, lz1 = z1.x, rz1 = z1.y;
         const int linkl = __float_as_int(e.x), linkr = __float_as_int(e.y);
-#else
-        float lx0 = fmaf(a.x, rc.idx, -rc.ox), lx1 = fmaf(b.x, rc.idx, -rc.ox);
-        float ly0 = fmaf(a.y, rc.idy, -rc.oy), ly1 = fmaf(b.y, rc.idy, -rc.oy);
-        float lz0 = fmaf(a.z, rc.idz, -rc.oz), lz1 = fmaf(b.z, rc.idz, -rc.oz);
-        float rx0 = fmaf(c.x, rc.idx, -rc.ox), rx1 = fmaf(e.x, rc.idx, -rc.ox);
-        float ry0 = fmaf(c.y, rc.idy, -rc.oy), ry1 = fmaf(e.y, rc.idy, -rc.oy);
-        float rz0 = fmaf(c.z, rc.idz, -rc.oz), rz1 = fmaf(e.z, rc.idz, -rc.oz);
-        const int linkl = __float_as_int(a.w), linkr = __float_as_int(b.w);
-#endif
         float ln = fmaxf(fmaxf(fminf(lx0, lx1), fminf(ly0, ly1)), fmaxf(fminf(lz0, lz1), tmin));
         float lf = fminf(fminf(fmaxf(lx0, lx1), fmaxf(ly0, ly1)), fminf(fmaxf(lz0, lz1), hit.t));
         float rn = fmaxf(fmaxf(fminf(rx0, rx1), fminf(ry0, ry1)), fmaxf(fminf(rz0, rz1), tmin));
@@ -498,46 +435,38 @@ struct Trav {
         const float far_t = right_first ? ln : rn;
         if (hl && hr) {
             // no bounds check here: a ray's stack never holds more entries than the tree has levels, and
-            // rt_upload_scene refuses (host path) or rebuilds on the host (device path) a tree with
-            // STACK_SIZE levels or more.  The masked index + overflow flag this replaces cost 2.5 % on C5.
-            stack_st(stack, sp, pack_entry(far_l, far_t));
+            // rt_upload_scene guarantees fewer than STACK_SIZE levels when the tree is uploaded -- it refuses
+            // (host path) or rebuilds on the host (device path) a deeper tree.  A device-side check costs 2.5 % on C5.
+            stack[sp] = pack_entry(far_l, far_t);
             sp++;
-#if RT_PREFETCH_FAR == 1  // tuning experiment: the pushed subtree's root node on its way to L1 while the near one is walked
-            if (far_l >= 0) asm volatile("prefetch.global.L1 [%0];" ::"l"(S.nodes + 4 * (size_t)far_l));
-#elif RT_PREFETCH_FAR == 2
-            if (far_l >= 0) {
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(S.nodes + 4 * (size_t)far_l));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(S.nodes + 4 * (size_t)far_l + 2));
-            }
-#endif
         }
         if (hl || hr) cur = near_l;
         else pop(stack);
     }
 
-    template <bool STATS, bool LITE = false, bool MSPH = true, class Stack>
+    template <bool STATS, bool LITE = false, bool MSPH = true>
     __device__ __forceinline__ void leaf(const DevScene& S, const Ray& ray, const RayConst& rc, float tmin, uint32_t origin_prim,
-                                         Stack stack, Stats* st) {
+                                         StackEntry* stack, Stats* st) {
         uint32_t v = ~(uint32_t)cur;
         uint32_t type = v >> 28, cnt = ((v >> 25) & 7u) + 1u, first = v & 0x1ffffffu;
         for (uint32_t i = 0; i < cnt; i++) hit_prim<STATS, LITE, MSPH>(S, type, first + i, ray, rc.inv_a, tmin, origin_prim, hit, st);
         pop(stack);
     }
 
-    template <bool STATS, class Stack>
-    __device__ __forceinline__ void node_step(const DevScene& S, const Ray&, const RayConst& rc, float tmin, Stack stack, Stats* st) {
-        interior<STATS>(S, rc, tmin, stack, st, nullptr);
+    template <bool STATS>
+    __device__ __forceinline__ void node_step(const DevScene& S, const Ray&, const RayConst& rc, float tmin, StackEntry* stack, Stats* st) {
+        interior<STATS>(S, rc, tmin, stack, st);
     }
-    template <bool STATS, bool LITE, bool MSPH = true, class Stack>
+    template <bool STATS, bool LITE, bool MSPH = true>
     __device__ __forceinline__ void leaf_step(const DevScene& S, const Ray& ray, const RayConst& rc, float tmin, uint32_t origin_prim,
-                                              Stack stack, Stats* st) {
+                                              StackEntry* stack, Stats* st) {
         leaf<STATS, LITE, MSPH>(S, ray, rc, tmin, origin_prim, stack, st);
     }
 };
 
 template <bool STATS>
 __device__ __forceinline__ void traverse(const DevScene& S, const Ray& ray, float tmin, float tmax, uint32_t origin_prim,
-                                         Hit& hit, Stats* st, int* overflow) {
+                                         Hit& hit, Stats* st) {
     RayConst rc;
     rc.set(ray);
     if (STATS) st->rays++;
@@ -546,7 +475,7 @@ __device__ __forceinline__ void traverse(const DevScene& S, const Ray& ray, floa
     tr.init(S, tmax);
     StackEntry* const sp_ = stack;
     while (!tr.done()) {
-        if (tr.cur >= 0) tr.interior<STATS>(S, rc, tmin, sp_, st, overflow);
+        if (tr.cur >= 0) tr.interior<STATS>(S, rc, tmin, sp_, st);
         else tr.leaf<STATS>(S, ray, rc, tmin, origin_prim, sp_, st);
     }
     hit = tr.hit;
@@ -671,30 +600,9 @@ __device__ __forceinline__ int media_hit(const DevScene& S, const Ray& ray, floa
 // floorf of a float is a float, and px - floorf(px) needs no more bits than px has, so the lattice cell and the
 // fractional position are the same numbers a double-precision split of the same (FP32) point would give -- without the
 // FP64 conversions the first version spent on it (3.3 % of C5's time at 2.4 lanes for ONE marble sphere).
-#ifndef RT_PERLIN_SMEM
-#define RT_PERLIN_SMEM 0  // measurement only (north_star: "Perlin permutation tables are staged in shared memory"): the tables of
-                          // perlin 0 (4864 B per block) copied to shared memory when render_kernel_v2 starts.  Measured against
-                          // the global/L1 path in profiles/r2_perlin_smem_ab.txt; the default stays 0.
-#endif
-#if RT_PERLIN_SMEM
-__shared__ float4 sh_perlin_vec[256];
-__shared__ unsigned char sh_perlin_perm[768];
-__device__ __forceinline__ void stage_perlin(const DevScene& S) {
-    if (S.perlin_vec == nullptr) return;
-    for (unsigned i = threadIdx.x; i < 256u; i += blockDim.x) sh_perlin_vec[i] = S.perlin_vec[i];
-    for (unsigned i = threadIdx.x; i < 768u; i += blockDim.x) sh_perlin_perm[i] = S.perlin_perm[i];
-}
-#endif
 __device__ __forceinline__ float perlin_noise(const DevScene& S, int pidx, float px, float py, float pz) {
-#if RT_PERLIN_SMEM
-    const float4* vec = pidx == 0 ? sh_perlin_vec : S.perlin_vec + 256 * (size_t)pidx;
-    const unsigned char* perm = pidx == 0 ? sh_perlin_perm : S.perlin_perm + 768 * (size_t)pidx;
-#define RT_PERLIN_LD(p) (*(p))
-#else
     const float4* vec = S.perlin_vec + 256 * (size_t)pidx;
     const unsigned char* perm = S.perlin_perm + 768 * (size_t)pidx;
-#define RT_PERLIN_LD(p) __ldg(p)
-#endif
     const float fx = floorf(px), fy = floorf(py), fz = floorf(pz);
     const float u = px - fx, v = py - fy, w = pz - fz;
     // the lattice index modulo 256 (perlin.h:25-27 `& 255`): beyond 2^31 the float is a multiple of 256 anyway
@@ -707,8 +615,8 @@ __device__ __forceinline__ float perlin_noise(const DevScene& S, int pidx, float
         for (int dj = 0; dj < 2; dj++)
 #pragma unroll
             for (int dk = 0; dk < 2; dk++) {
-                int h = RT_PERLIN_LD(perm + ((i + di) & 255)) ^ RT_PERLIN_LD(perm + 256 + ((j + dj) & 255)) ^ RT_PERLIN_LD(perm + 512 + ((k + dk) & 255));
-                float4 g = RT_PERLIN_LD(vec + h);
+                int h = __ldg(perm + ((i + di) & 255)) ^ __ldg(perm + 256 + ((j + dj) & 255)) ^ __ldg(perm + 512 + ((k + dk) & 255));
+                float4 g = __ldg(vec + h);
                 float wx = u - di, wy = v - dj, wz = w - dk;
                 accum += (di ? uu : 1.0f - uu) * (dj ? vv : 1.0f - vv) * (dk ? ww : 1.0f - ww) * (g.x * wx + g.y * wy + g.z * wz);
             }
@@ -1192,8 +1100,7 @@ __device__ __forceinline__ void traverse_wide(const DevScene& S, const Ray& ray,
 template <int WIDTH>
 __device__ __forceinline__ void traverse_sel(const DevScene& S, const Ray& ray, float tmin, float tmax, uint32_t origin_prim, Hit& hit) {
     if constexpr (WIDTH == 2) {
-        int ov = 0;
-        traverse<false>(S, ray, tmin, tmax, origin_prim, hit, nullptr, &ov);
+        traverse<false>(S, ray, tmin, tmax, origin_prim, hit, nullptr);
     } else {
         traverse_wide<WIDTH, false>(S, ray, tmin, tmax, origin_prim, hit, nullptr);
     }

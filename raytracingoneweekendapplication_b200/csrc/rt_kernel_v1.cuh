@@ -11,7 +11,6 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Dev
     const unsigned lane = threadIdx.x & 31u;
     Stats st;
     if (STATS) memset(&st, 0, sizeof st);
-    int overflow = 0;
     unsigned long long dropped = 0;
 
     while (true) {
@@ -64,7 +63,7 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Dev
             }
             // ---- one bounce: Camera.txt:203-238 ------------------------------------
             Hit hit;
-            traverse<STATS>(S, ray, 0.001f, __int_as_float(0x7f800000), origin_prim, hit, &st, &overflow);
+            traverse<STATS>(S, ray, 0.001f, __int_as_float(0x7f800000), origin_prim, hit, &st);
             int medium = -1;
             if (S.n_media > 0) medium = media_hit<STATS>(S, ray, 0.001f, hit.t, rng, bounce, &st);
 
@@ -128,7 +127,6 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Dev
         dropped = 0;
         __syncwarp();
     }
-    if (overflow) atomicAdd(&counters[1], 1ull);
     if (STATS) {
         unsigned long long* g = reinterpret_cast<unsigned long long*>(gstats);
         const unsigned long long* l = reinterpret_cast<const unsigned long long*>(&st);

@@ -84,7 +84,6 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) render_kernel_v3(const __g
     uint32_t* const park = &park_all[threadIdx.x >> 5][0][lane];
     Stats st;
     if (STATS) memset(&st, 0, sizeof st);
-    int overflow = 0;
 
     // warp-uniform pool of (pixel, sample) pairs
     unsigned pool_pos = 0, pool_size = 0;
@@ -291,7 +290,7 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) render_kernel_v3(const __g
                     const unsigned lmask = __ballot_sync(0xffffffffu, c.state == LANE_TRAVERSE && tr.cur < 0);
                     if (__popc(lmask) >= kLeafTrigger) break;
                     if (STATS && lane == 0) { st.desc_iters++; st.desc_lanes += __popc(dmask); st.desc_trav_lanes += __popc(dmask | lmask); }
-                    if (descending) tr.interior<STATS>(S, rc, 0.001f, stack, &st, &overflow);
+                    if (descending) tr.interior<STATS>(S, rc, 0.001f, stack, &st);
                 }
                 if (STATS) {
                     const unsigned lm = __ballot_sync(0xffffffffu, c.state == LANE_TRAVERSE && tr.cur < 0 && !tr.done());
@@ -325,7 +324,6 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) render_kernel_v3(const __g
             c.sp = tr.sp;
         }
     }
-    if (overflow) atomicAdd(&counters[1], 1ull);
     if (STATS) {
         unsigned long long* g = reinterpret_cast<unsigned long long*>(gstats);
         const unsigned long long* l = reinterpret_cast<const unsigned long long*>(&st);

@@ -33,7 +33,7 @@ struct Pool {
     uint2* id;       // pixel, sample
     float4* hit;     // t, as_float(prim), u, v
     uint32_t* list[2];
-    // ctr[0] next index of the sample stream, [1] stack overflow flag, [2] n_active (current),
+    // ctr[0] next index of the sample stream, [1] unused, [2] n_active (current),
     // [3] n_active (next), [4] extend cursor, [5] current list (0/1)
     unsigned long long* ctr;
     uint32_t capacity;
@@ -124,7 +124,6 @@ __global__ void __launch_bounds__(256, 4) wf_extend(const __grid_constant__ DevS
     const uint32_t* list = P.list[P.ctr[5] & 1ull];
     Stats st;
     if (STATS) memset(&st, 0, sizeof st);
-    int overflow = 0;
     bool queue_empty = n == 0;
     bool active = false;
     uint32_t slot = 0, origin_prim = PRIM_NONE;
@@ -171,7 +170,7 @@ __global__ void __launch_bounds__(256, 4) wf_extend(const __grid_constant__ DevS
             while (true) {
                 const bool descending = active && tr.cur >= 0;
                 if (__ballot_sync(0xffffffffu, descending) == 0u) break;
-                if (descending) tr.interior<STATS>(S, rc, 0.001f, stack, &st, &overflow);
+                if (descending) tr.interior<STATS>(S, rc, 0.001f, stack, &st);
             }
             if (active) {
                 if (!tr.done()) tr.leaf<STATS>(S, ray, rc, 0.001f, origin_prim, stack, &st);
@@ -185,7 +184,6 @@ __global__ void __launch_bounds__(256, 4) wf_extend(const __grid_constant__ DevS
             if (!queue_empty && 32 - __popc(act) >= RT_WF_REFILL) break;
         }
     }
-    if (overflow) atomicAdd(&P.ctr[1], 1ull);
     if (STATS) {
         unsigned long long* g = reinterpret_cast<unsigned long long*>(gstats);
         const unsigned long long* l = reinterpret_cast<const unsigned long long*>(&st);
