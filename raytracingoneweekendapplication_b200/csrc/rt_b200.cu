@@ -135,6 +135,20 @@ struct TravSel<2> { using Trav = rtdev::Trav; using RayConst = rtdev::RayConst; 
 // The plain binary-tree instances are compiled for the masks of kInstances; a scene runs the first one that covers it.
 enum : int { FEAT_MEDIA = 1, FEAT_MEDIA_GENERAL = 2, FEAT_SPECULAR = 4, FEAT_MSPHERE = 8, FEAT_TRI = 16, FEAT_LIGHTS = 32,
              FEAT_DEFOCUS = 64, FEAT_ALL = 127 };
+// One 16-byte slot of local memory per lane, moved with one vector store and one vector load.  The accesses are
+// volatile PTX, so the value stays in the slot between them instead of occupying registers or scattered scalar spills.
+struct LocalSlot {
+    float4 mem;
+    __device__ __forceinline__ void store(float4 v) {
+        asm volatile("st.local.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(__cvta_generic_to_local(&mem)), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w));
+    }
+    __device__ __forceinline__ float4 load() {
+        float4 v;
+        asm volatile("ld.local.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(__cvta_generic_to_local(&mem)));
+        return v;
+    }
+};
+
 template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
@@ -162,7 +176,10 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     Ray ray;
     ray.o = ray.d = v3(0, 0, 0);
     ray.time = 0;
-    V3 L = v3(0, 0, 0), T = v3(1, 1, 1);
+    // the path's radiance L and throughput T live in local memory between shade phases: written where a sample starts
+    // and at the end of each shade phase, read once in the shade phase, after the surface has been shaded.  Held in
+    // registers, they were spilled by the compiler around the traversal phase and the out-of-line calls of the shade phase.
+    LocalSlot radiance, throughput;
     uint32_t bounce = 0, origin_prim = PRIM_NONE;
     float nee_pdf = 0.0f;  // NEE: > 0 when the previous vertex sampled the listed emitters directly: the density of the direction it scattered into
     typename TravSel<WIDTH>::Trav tr;
@@ -213,8 +230,8 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     rng.sample = (uint32_t)(A.spp_begin + A.sample_offset + (seg_s0 + (int)(e >> 5)) * A.sample_stride);
                     if (A.compact) lane_slot[threadIdx.x] = slot_base + ((e >> 3) & 3u) * (unsigned)A.tile_size + (e & 7u);
                     ray = camera_ray<NO_DEFOCUS>(S, px, py, rng);
-                    L = v3(0, 0, 0);
-                    T = v3(1, 1, 1);
+                    radiance.store(make_float4(0, 0, 0, 0));
+                    throughput.store(make_float4(1, 1, 1, 0));
                     bounce = 0;
                     origin_prim = PRIM_NONE;
                     nee_pdf = 0.0f;
@@ -289,11 +306,18 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
             if (lane == 0) { st.shade_iters++; st.shade_lanes += __popc(smask); }
         }
         if (state == LANE_SHADE) {
+            V3 L, T;
+            auto load_path = [&] {
+                const float4 l4 = radiance.load(), t4 = throughput.load();
+                L = v3(l4.x, l4.y, l4.z);
+                T = v3(t4.x, t4.y, t4.z);
+            };
             Hit hit = tr.hit;
             int medium = -1;
             if ((FEAT & FEAT_MEDIA) && S.n_media > 0) medium = media_hit<STATS, (FEAT & FEAT_MEDIA_GENERAL) != 0>(S, ray, 0.001f, hit.t, rng, bounce, &st);
             bool done = false;
             if (medium < 0 && hit.prim == PRIM_NONE) {
+                load_path();
                 L = L + T * v3(S.background);
                 done = true;
             } else {
@@ -314,11 +338,10 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     origin_prim = hit.prim;
                 }
                 const DevMaterial& m = S.mats[sf.material];
-                float4 u4 = make_float4(0, 0, 0, 0);
-                if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) u4 = rng.draw(bounce, RS_SCATTER);
                 V3 att, emitted;
                 Ray next;
-                const bool scattered = shade_surface<(FEAT & FEAT_SPECULAR) != 0>(S, m, ray, sf, u4, emitted, att, next);
+                const bool scattered = shade_surface<(FEAT & FEAT_SPECULAR) != 0>(S, m, ray, sf, [&] { return rng.draw(bounce, RS_SCATTER); },
+                                                                                  emitted, att, next);
                 // NEE: a listed emitter reached from a vertex that also sampled the emitters directly shares the
                 // estimate with that sample (balance heuristic)
                 if (NEE && nee_pdf > 0.0f && medium < 0 && sf.nee_light > 0) {
@@ -327,6 +350,7 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     const float p_light = light_density(S, sf.t * sf.t * d2, fmaxf(cos_y, 1e-20f));
                     emitted = (nee_pdf / (nee_pdf + p_light)) * emitted;
                 }
+                load_path();
                 L = L + T * emitted;
                 if (!scattered) {
                     done = true;
@@ -360,7 +384,13 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     if (STATS) st.nonfinite++;
                 }
                 state = LANE_IDLE;
+                // an idle lane's traversal state is never read, but unless it is set here the previous ray's hit and
+                // links stay live through the whole shade phase
+                tr.init(S, kInf);
+                tr.clear();
             } else {
+                radiance.store(make_float4(L.x, L.y, L.z, 0.0f));
+                throughput.store(make_float4(T.x, T.y, T.z, 0.0f));
                 tr.init(S, kInf);
                 state = tr.done() ? LANE_SHADE : LANE_TRAVERSE;
                 if (STATS) { st.rays++; seg_steps = n_leaf = 0; }

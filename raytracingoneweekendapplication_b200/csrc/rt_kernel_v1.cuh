@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Dev
                 if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) u4 = rng.draw(bounce, RS_SCATTER);
                 V3 att, emitted;
                 Ray next;
-                const bool scattered = shade_surface(S, m, ray, sf, u4, emitted, att, next);
+                const bool scattered = shade_surface(S, m, ray, sf, [&] { return u4; }, emitted, att, next);
                 L = L + T * emitted;
                 if (!scattered) {
                     done = true;

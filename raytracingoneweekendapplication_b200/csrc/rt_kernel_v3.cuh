@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(256, RT_MIN_BLOCKS) render_kernel_v3(const __g
                     if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) u4 = rng.draw(c.bounce, RS_SCATTER);
                     V3 att, emitted;
                     Ray next;
-                    const bool scattered = shade_surface(S, m, c.ray, sf, u4, emitted, att, next);
+                    const bool scattered = shade_surface(S, m, c.ray, sf, [&] { return u4; }, emitted, att, next);
                     c.L = c.L + c.T * emitted;
                     if (!scattered) {
                         done = true;

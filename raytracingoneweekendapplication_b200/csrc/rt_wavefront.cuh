@@ -253,7 +253,7 @@ __global__ void __launch_bounds__(256, 3) wf_shade(const __grid_constant__ DevSc
                 if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) u4 = rng.draw(bounce, RS_SCATTER);
                 V3 att, emitted;
                 Ray next;
-                const bool scattered = shade_surface(S, m, ray, sf, u4, emitted, att, next);
+                const bool scattered = shade_surface(S, m, ray, sf, [&] { return u4; }, emitted, att, next);
                 L = L + T * emitted;
                 if (!scattered) {
                     done = true;
