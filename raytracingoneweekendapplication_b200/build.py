@@ -30,15 +30,13 @@ def _run(cmd, cwd=None):
     subprocess.check_call(cmd, cwd=cwd)
 
 
-def build_cuda(force: bool = False, verbose_ptxas: bool = False, alt_kernels: bool = False, out: str | None = None) -> str:
-    out = out or os.path.join(PKG, "librt_b200.so")
+def build_cuda(force: bool = False, verbose_ptxas: bool = False) -> str:
+    out = os.path.join(PKG, "librt_b200.so")
     csrc = os.path.join(PKG, "csrc")
     srcs = [os.path.join(csrc, f) for f in os.listdir(csrc)] + [os.path.join(ROOT, "include", "rt_b200.h")]
     if force or _newer(out, srcs):
         nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
         cmd = [nvcc, *NVCC_FLAGS, "-I" + os.path.join(ROOT, "include"), "-o", out, os.path.join(csrc, "rt_b200.cu"), "-ldl"]
-        if alt_kernels:   # the measured alternatives to render_kernel_v2 (v1, v3, wavefront): RT_B200_KERNEL=v1|v3|wf
-            cmd[1:1] = ["-DRT_B200_ALT_KERNELS"]
         if verbose_ptxas:
             cmd[1:1] = ["-Xptxas", "-v"]
         _run(cmd)
@@ -88,8 +86,8 @@ def build_oracle() -> None:
     _run(["make", "-C", os.path.join(ROOT, "oracle"), "all"])
 
 
-def build_all(force: bool = False, alt_kernels: bool = False) -> None:
-    build_cuda(force or alt_kernels, alt_kernels=alt_kernels)
+def build_all(force: bool = False) -> None:
+    build_cuda(force)
     build_host(force)
     build_oracle()
     from .assets import ensure_assets
@@ -99,4 +97,4 @@ def build_all(force: bool = False, alt_kernels: bool = False) -> None:
 
 
 if __name__ == "__main__":
-    build_all(force="--force" in sys.argv, alt_kernels="--alt" in sys.argv)
+    build_all(force="--force" in sys.argv)

@@ -14,8 +14,6 @@
 //   probe_*_kernel         per-function known-answer probes
 //   fma_peak_kernel, l1_peak_kernel   FP32 and L1 roofline denominators
 //   rtlbvh::*              the device BVH builder (bvh_device.cuh)
-// With -DRT_B200_ALT_KERNELS only: render_kernel (v1), render_kernel_v3 and the wavefront pipeline
-// (rtwf::wf_*), the measured alternatives to render_kernel_v2 (RT_B200_KERNEL=v1 | v3 | wf).
 #include <cuda_runtime.h>
 
 #include <chrono>
@@ -35,13 +33,6 @@
 #include "rt_b200.h"
 #include "rt_device.cuh"
 #include "rt_wide.cuh"
-#ifdef RT_B200_ALT_KERNELS
-// The measured alternatives to render_kernel_v2 (DESIGN.md section 3): the first megakernel (v1), the
-// two-contexts-per-lane kernel (v3) and the wavefront pipeline.  All three lose to v2 on every
-// BASELINE scene; they are compiled only with -DRT_B200_ALT_KERNELS (build.py --alt) and selected
-// with RT_B200_KERNEL=v1|v3|wf.
-#include "rt_wavefront.cuh"
-#endif
 
 using namespace rtdev;
 
@@ -69,10 +60,6 @@ struct RenderArgs {
 
 constexpr float kAccumScale = 268435456.0f;  // 2^RT_ACCUM_FRAC_BITS
 constexpr float kSampleClamp = 1048576.0f;   // 2^20: keeps 2^16 saturated samples inside 64 bits
-
-#ifdef RT_B200_ALT_KERNELS
-#include "rt_kernel_v1.cuh"
-#endif
 
 // ---------------------------------------------------------------------------------
 // render_kernel_v2 — the production megakernel.
@@ -408,10 +395,6 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     }
 }
 
-#ifdef RT_B200_ALT_KERNELS
-#include "rt_kernel_v3.cuh"
-#endif
-
 // The compiled feature instances of the plain binary-tree kernel (see FEAT_* above); variant 5 + k of the dispatch below.
 typedef void (*RenderKernel)(const DevScene, const RenderArgs, unsigned long long*, unsigned long long*, Stats*);
 struct FeatInstance {
@@ -660,13 +643,6 @@ struct DevCtx {
     int cam_w = 0, cam_h = 0;  // frame the device camera block was computed for
     CameraD camera_d{};        // the same camera in double (deterministic pixel-centre rays of the AOV)
     int sm_count = 0;
-    int kernel_version = 2;  // 2 = render_kernel_v2; with -DRT_B200_ALT_KERNELS RT_B200_KERNEL=v1 | v3 | wf select the measured alternatives
-#ifdef RT_B200_ALT_KERNELS
-    rtwf::Pool pool{};       // wavefront path pool (allocated on first use)
-    void* pool_mem = nullptr;
-    int wf_blocks_per_sm[2] = {0, 0};
-#endif
-    int blocks_per_sm[2] = {0, 0};
     // acceleration structure the render kernels traverse: 2 = binary tree, 8 / 4 = wide quantised tree
     // (host-built scenes only; a device-built scene keeps the binary tree).  rt_set_bvh_width / RT_B200_BVH_WIDTH
     // asynchronous frame hand-out (rt_download_begin / rt_untile_begin / rt_frame_end): the device-to-host copy runs on
@@ -739,11 +715,6 @@ static void release_buffers(DevCtx* ctx) {
     ctx->copy_ring.release();
     ctx->scratch = nullptr;
     ctx->scratch_cap = 0;
-#ifdef RT_B200_ALT_KERNELS
-    if (ctx->pool_mem) cudaFree(ctx->pool_mem);
-    ctx->pool_mem = nullptr;
-    ctx->pool = rtwf::Pool{};
-#endif
     if (ctx->staging) cudaFreeHost(ctx->staging);
     if (ctx->out_lin) cudaFree(ctx->out_lin);
     if (ctx->out_rgb8) cudaFree(ctx->out_rgb8);
@@ -804,44 +775,14 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
         if (w != 2 && w != 4 && w != 8) return fail(ctx, RT_ERR_INVALID, "RT_B200_BVH_WIDTH=%s: 2, 4 or 8", wv);
         ctx->bvh_width = w;
     }
-    cudaFuncAttributes fa;
-#ifdef RT_B200_ALT_KERNELS
-    if (const char* kv = getenv("RT_B200_KERNEL"))
-        ctx->kernel_version = strcmp(kv, "v1") == 0 ? 1 : (strcmp(kv, "wf") == 0 ? 3 : (strcmp(kv, "v3") == 0 ? 4 : 2));
-    cudaFuncSetAttribute(render_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(render_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    // v3 parks one path context per lane in shared memory: 23.5 KB per block, three blocks per SM
-    cudaFuncSetAttribute(render_kernel_v3<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 40);
-    cudaFuncSetAttribute(render_kernel_v3<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 40);
-    cudaFuncSetAttribute(render_kernel_v3<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 40);
-    cudaFuncSetAttribute(rtwf::wf_extend<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(rtwf::wf_extend<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(rtwf::wf_shade<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(rtwf::wf_shade<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->wf_blocks_per_sm[0], rtwf::wf_extend<false>, 256, 0));
-    CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->wf_blocks_per_sm[1], rtwf::wf_shade<false>, 256, 0));
-    if (ctx->kernel_version == 1) {
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[0], render_kernel<false>, 256, 0));
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[1], render_kernel<true>, 256, 0));
-        CU(ctx, cudaFuncGetAttributes(&fa, render_kernel<false>));
-    } else if (ctx->kernel_version == 4) {
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[0], render_kernel_v3<false, false>, 256, 0));
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[1], render_kernel_v3<true, false>, 256, 0));
-        CU(ctx, cudaFuncGetAttributes(&fa, render_kernel_v3<false, false>));
-    } else
-#else
     if (const char* kv = getenv("RT_B200_KERNEL"))
         if (strcmp(kv, "v2") != 0)
-            return fail(ctx, RT_ERR_UNSUPPORTED, "RT_B200_KERNEL=%s: the alternative kernels are compiled only with -DRT_B200_ALT_KERNELS (build.py --alt)", kv);
-#endif
-    {
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[0], render_kernel_v2<false, false>, RT_V2_THREADS, 0));
-        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->blocks_per_sm[1], render_kernel_v2<true, false>, RT_V2_THREADS, 0));
-        CU(ctx, cudaFuncGetAttributes(&fa, render_kernel_v2<false, false>));
-    }
+            return fail(ctx, RT_ERR_UNSUPPORTED, "RT_B200_KERNEL=%s: render_kernel_v2 is the only render kernel; the alternatives were removed (DESIGN.md section 3)", kv);
+    cudaFuncAttributes fa;
+    CU(ctx, cudaFuncGetAttributes(&fa, render_kernel_v2<false, false>));
     ctx->stats.regs_per_thread = fa.numRegs;
     ctx->stats.local_bytes_per_thread = (uint32_t)fa.localSizeBytes;
-    ctx->stats.threads_per_block = ctx->kernel_version == 2 ? RT_V2_THREADS : 256;
+    ctx->stats.threads_per_block = RT_V2_THREADS;
     return RT_OK;
 }
 
@@ -1928,72 +1869,6 @@ static int dev_sync(DevCtx* ctx) {
     return RT_OK;
 }
 
-// ---------------------------------------------------------------------------------
-// wavefront driver (RT_B200_KERNEL=wf): generate once, then (swap, extend, shade) per bounce
-// of the pool until the sample stream is exhausted and no path is alive
-// ---------------------------------------------------------------------------------
-#ifdef RT_B200_ALT_KERNELS
-static int launch_wavefront(DevCtx* ctx, const RenderArgs& A, cudaStream_t stream, bool stats, unsigned long long pixel_blocks) {
-    rtwf::Stream W;
-    std::memset(&W, 0, sizeof W);
-    W.width = A.width; W.height = A.height; W.max_depth = A.max_depth; W.spp_begin = A.spp_begin;
-    W.n_local_samples = A.n_local_samples; W.sample_stride = A.sample_stride; W.sample_offset = A.sample_offset;
-    W.tiles_x = A.tiles_x; W.tile_size = A.tile_size; W.tile_stride = A.tile_stride; W.tile_offset = A.tile_offset;
-    W.blocks_per_tile_x = A.blocks_per_tile_x; W.blocks_per_tile_y = A.blocks_per_tile_y;
-    W.total = pixel_blocks * 32ull * (unsigned long long)A.n_local_samples;
-    W.k0 = A.k0; W.k1 = A.k1;
-
-    const uint32_t want_cap = 1u << 20;  // 1 Mi paths in flight: 3.4 waves of 148 x 2048 threads
-    if (!ctx->pool_mem) {
-        const size_t per_path = 5 * sizeof(float4) + sizeof(uint2) + 2 * sizeof(uint32_t);
-        const size_t bytes = (size_t)want_cap * per_path + 256;
-        if (cudaMalloc(&ctx->pool_mem, bytes) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render: cannot allocate the wavefront path pool (%zu bytes)", bytes);
-        unsigned char* p = (unsigned char*)ctx->pool_mem;
-        rtwf::Pool& P = ctx->pool;
-        P.ctr = (unsigned long long*)p; p += 256;
-        P.ray_o = (float4*)p; p += (size_t)want_cap * sizeof(float4);
-        P.ray_d = (float4*)p; p += (size_t)want_cap * sizeof(float4);
-        P.thr = (float4*)p; p += (size_t)want_cap * sizeof(float4);
-        P.rad = (float4*)p; p += (size_t)want_cap * sizeof(float4);
-        P.hit = (float4*)p; p += (size_t)want_cap * sizeof(float4);
-        P.id = (uint2*)p; p += (size_t)want_cap * sizeof(uint2);
-        P.list[0] = (uint32_t*)p; p += (size_t)want_cap * sizeof(uint32_t);
-        P.list[1] = (uint32_t*)p;
-        P.capacity = want_cap;
-    }
-    rtwf::Pool P = ctx->pool;
-    unsigned long long live = std::min<unsigned long long>(W.total, want_cap);
-    P.capacity = (uint32_t)((live + 255) / 256 * 256);
-    if (P.capacity > want_cap) P.capacity = want_cap;
-    if (P.capacity == 0) return RT_OK;
-    CU(ctx, cudaMemsetAsync(P.ctr, 0, 64, stream));
-    rtwf::wf_generate<<<P.capacity / 256, 256, 0, stream>>>(ctx->scene, W, P);
-    uint32_t launches = 1;
-    const int grid_e = ctx->sm_count * std::max(1, ctx->wf_blocks_per_sm[0]);
-    const int grid_s = ctx->sm_count * std::max(1, ctx->wf_blocks_per_sm[1]);
-    unsigned long long h[8];
-    for (int batch = 0; batch < (1 << 20); batch++) {
-        for (int it = 0; it < 16; it++) {
-            rtwf::wf_swap<<<1, 1, 0, stream>>>(P);
-            if (stats) {
-                rtwf::wf_extend<true><<<grid_e, 256, 0, stream>>>(ctx->scene, P, ctx->dstats);
-                rtwf::wf_shade<true><<<grid_s, 256, 0, stream>>>(ctx->scene, W, P, ctx->accum, ctx->dstats);
-            } else {
-                rtwf::wf_extend<false><<<grid_e, 256, 0, stream>>>(ctx->scene, P, ctx->dstats);
-                rtwf::wf_shade<false><<<grid_s, 256, 0, stream>>>(ctx->scene, W, P, ctx->accum, ctx->dstats);
-            }
-            launches += 3;
-        }
-        CU(ctx, cudaGetLastError());
-        CU(ctx, cudaMemcpyAsync(h, P.ctr, sizeof h, cudaMemcpyDeviceToHost, stream));
-        CU(ctx, cudaStreamSynchronize(stream));
-        if (h[3] == 0) break;  // nothing appended by the last shade: every path ended and the stream is dry
-    }
-    ctx->stats.kernel_launches = launches;
-    return RT_OK;
-}
-#endif
-
 // The instances of render_kernel_v2: variant 0 plain (everything), 1 LITE, 2 STATS, 3 NEE + LITE, 4 NEE; width 2, 4, 8
 // (3, 4: binary tree only).  Variants 5 + k: the binary-tree instance kInstances[k], compiled for one feature mask.
 template <int WIDTH>
@@ -2057,7 +1932,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     // the host; it needs the frame the passes before it render into, unchanged
     // (the camera of this frame size must be set up already: the first pass onto a restored checkpoint is a plain one)
     const bool overlap = (p->flags & RT_FLAG_OVERLAP) && (p->flags & RT_FLAG_ASYNC) && (p->flags & RT_FLAG_ACCUMULATE) &&
-                         !(p->flags & RT_FLAG_STATS) && ctx->kernel_version == 2 && ctx->accum != nullptr &&
+                         !(p->flags & RT_FLAG_STATS) && ctx->accum != nullptr &&
                          ctx->cam_w == p->width && ctx->cam_h == p->height;
     // a pending asynchronous render (possibly on another stream) shares the work counter, the guard flags and the
     // stats block with this one: finish it first
@@ -2103,7 +1978,6 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     L.height = p->height;
     if (p->flags & RT_FLAG_COMPACT_TILES) {
         if (mode != RT_SHARD_TILES) return fail(ctx, RT_ERR_INVALID, "rt_render: RT_FLAG_COMPACT_TILES needs tile sharding (shard_mode RT_SHARD_TILES)");
-        if (ctx->kernel_version != 2) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: compact tile buffers are implemented by render_kernel_v2 only");
         L.compact = true;
         L.rank = rank;
         L.count = count;
@@ -2115,7 +1989,6 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     rc = ensure_accum(ctx, L);
     if (rc != RT_OK) return rc;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
-    int bps = ctx->blocks_per_sm[stats ? 1 : 0];
     // which instance of render_kernel_v2 runs: LITE = no triangles, no point lights, no defocus blur in this scene (see hit_prim)
     const bool lite = ctx->scene_lite && !getenv("RT_B200_NO_LITE");
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
@@ -2129,15 +2002,14 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
                 variant = 5 + k;
                 break;
             }
-    if (ctx->kernel_version == 2) {
-        rc = v2_blocks_per_sm(ctx, variant, width, &bps);
-        if (rc != RT_OK) return rc;
-    }
+    int bps = 0;
+    rc = v2_blocks_per_sm(ctx, variant, width, &bps);
+    if (rc != RT_OK) return rc;
     const int grid = ctx->sm_count * (bps > 0 ? bps : 1);
     // segment length: enough work items to keep every resident warp busy ~64 times over,
     // but never shorter than 1 sample (fixed-point sums make the split result-neutral)
     const unsigned long long pixel_blocks = (unsigned long long)A.n_local_tiles * A.blocks_per_tile_x * A.blocks_per_tile_y;
-    const unsigned long long resident_warps = (unsigned long long)grid * (ctx->kernel_version == 2 ? RT_V2_THREADS / 32 : 8);
+    const unsigned long long resident_warps = (unsigned long long)grid * (RT_V2_THREADS / 32);
     int n_seg = 1;
     if (A.n_local_samples > 0 && pixel_blocks > 0) {
         // >= 64 items per resident warp: the end-of-kernel tail is one item long
@@ -2207,28 +2079,12 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     CU(ctx, cudaEventRecord(ctx->ev0, stream));
     ctx->stats.kernel_launches = 0;
     if (A.n_items > 0) {
-#ifdef RT_B200_ALT_KERNELS
-        if (ctx->kernel_version == 3) {
-            rc = launch_wavefront(ctx, A, stream, stats, pixel_blocks);
-            if (rc != RT_OK) return rc;
-        } else if (ctx->kernel_version == 1) {
-            if (stats) render_kernel<true><<<grid, 256, 0, stream>>>(ctx->scene, A, ctx->accum, ctx->counters, ctx->dstats);
-            else render_kernel<false><<<grid, 256, 0, stream>>>(ctx->scene, A, ctx->accum, ctx->counters, ctx->dstats);
-        } else if (ctx->kernel_version == 4) {
-            const bool lite = ctx->scene_lite && !getenv("RT_B200_NO_LITE");
-            if (stats) render_kernel_v3<true, false><<<grid, 256, 0, stream>>>(ctx->scene, A, ctx->accum, ctx->counters, ctx->dstats);
-            else if (lite) render_kernel_v3<false, true><<<grid, 256, 0, stream>>>(ctx->scene, A, ctx->accum, ctx->counters, ctx->dstats);
-            else render_kernel_v3<false, false><<<grid, 256, 0, stream>>>(ctx->scene, A, ctx->accum, ctx->counters, ctx->dstats);
-        } else
-#endif
-        {
-            A.nee_emitters = want_nee;
-            A.shadow_point_lights = want_shadow;
-            rc = launch_v2(ctx, variant, width, grid, A, stream);
-            if (rc != RT_OK) return rc;
-        }
+        A.nee_emitters = want_nee;
+        A.shadow_point_lights = want_shadow;
+        rc = launch_v2(ctx, variant, width, grid, A, stream);
+        if (rc != RT_OK) return rc;
         CU(ctx, cudaGetLastError());
-        if (ctx->kernel_version != 3) ctx->stats.kernel_launches = 1;
+        ctx->stats.kernel_launches = 1;
     }
     ctx->stats.blocks = grid;
     ctx->stats.samples = pass_samples();

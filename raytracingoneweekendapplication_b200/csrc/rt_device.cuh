@@ -467,19 +467,16 @@ struct Trav {
     }
 };
 
-template <bool STATS>
-__device__ __forceinline__ void traverse(const DevScene& S, const Ray& ray, float tmin, float tmax, uint32_t origin_prim,
-                                         Hit& hit, Stats* st) {
+__device__ __forceinline__ void traverse(const DevScene& S, const Ray& ray, float tmin, float tmax, uint32_t origin_prim, Hit& hit) {
     RayConst rc;
     rc.set(ray);
-    if (STATS) st->rays++;
     Trav tr;
     StackEntry stack[STACK_SIZE];
     tr.init(S, tmax);
     StackEntry* const sp_ = stack;
     while (!tr.done()) {
-        if (tr.cur >= 0) tr.interior<STATS>(S, rc, tmin, sp_, st);
-        else tr.leaf<STATS>(S, ray, rc, tmin, origin_prim, sp_, st);
+        if (tr.cur >= 0) tr.interior<false>(S, rc, tmin, sp_, nullptr);
+        else tr.leaf<false>(S, ray, rc, tmin, origin_prim, sp_, nullptr);
     }
     hit = tr.hit;
 }
@@ -538,7 +535,7 @@ __device__ __noinline__ float2 boundary_pair_box(const float4* __restrict__ bx, 
 // one if it lies beyond t1 + 1e-4 (sphere.h:44-49).
 // GENERAL = false: every boundary of the scene is one static sphere (both media of C5); the out-of-line box / generic
 // paths are then not even call sites -- they cost the caller registers and spills where they never run (C5 +3.7 %).
-template <bool STATS, bool GENERAL = true>
+template <bool STATS, bool GENERAL>
 __device__ __forceinline__ int media_hit(const DevScene& S, const Ray& ray, float tmin, float& t_hit, const Rng& rng,
                                          uint32_t bounce, Stats* st) {
     int which = -1;
@@ -1122,7 +1119,7 @@ __device__ __forceinline__ void traverse_wide(const DevScene& S, const Ray& ray,
 template <int WIDTH>
 __device__ __forceinline__ void traverse_sel(const DevScene& S, const Ray& ray, float tmin, float tmax, uint32_t origin_prim, Hit& hit) {
     if constexpr (WIDTH == 2) {
-        traverse<false>(S, ray, tmin, tmax, origin_prim, hit, nullptr);
+        traverse(S, ray, tmin, tmax, origin_prim, hit);
     } else {
         traverse_wide<WIDTH, false>(S, ray, tmin, tmax, origin_prim, hit, nullptr);
     }
@@ -1195,7 +1192,7 @@ __device__ __noinline__ V3 point_lighting_shadowed(const DevScene& S, V3 p, V3 n
 // Camera.txt:177-200 get_ray.  Directions are built relative to the camera centre
 // (dir00 = pixel00_loc - center, evaluated in double on the host) so that FP32 keeps
 // sub-pixel accuracy when the camera sits hundreds of units from the origin.
-template <bool LITE = false>
+template <bool LITE>
 __device__ __forceinline__ Ray camera_ray(const DevScene& S, int i, int j, const Rng& rng) {
     float4 u = rng.draw(0, RS_CAMERA);
     float fx = (float)i + (u.x - 0.5f), fy = (float)j + (u.y - 0.5f);

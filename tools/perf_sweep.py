@@ -7,7 +7,7 @@ from raytracingoneweekendapplication_b200 import capi
 cases = [a.split(":") for a in sys.argv[1:] if ":" in a] or [["final", "1920", "1080", "16"], ["cornell", "600", "600", "32"],
                                                              ["book1", "800", "450", "16"], ["mesh", "1920", "1080", "8"],
                                                              ["cornell_smoke", "600", "600", "32"]]
-variants = [a for a in sys.argv[1:] if ":" not in a] or ["v1", "v2"]
+variants = [a for a in sys.argv[1:] if ":" not in a] or ["v2"]
 for name, w, h, spp in cases:
     w, h, spp = int(w), int(h), int(spp)
     sc = capi.Scene(name)
