@@ -38,6 +38,8 @@ int main(int argc, char** argv) {
     if (argc > 6) cam.samples_per_pixel = std::atoi(argv[6]);
     // additions: --checkpoint FILE [--every N] [--stop-after N] [--linear FILE.exr|.pfm] [--nee 0|1]
     //            --devices all | 0,1,2,...   split the frame over several GPUs of this box (one context, tiles gathered over NVLink)
+    //            --noise X [--noise-every N]  stop once the relative frame noise is <= X, checked every N samples (default 256)
+    //            --variance FILE.exr|.pfm     also write the per-pixel sample variance
     for (int i = 7; i + 1 < argc; i += 2) {
         std::string k = argv[i];
         if (k == "--checkpoint") cam.checkpoint_path = argv[i + 1];
@@ -45,6 +47,9 @@ int main(int argc, char** argv) {
         else if (k == "--stop-after") cam.stop_after_spp = std::atoi(argv[i + 1]);
         else if (k == "--linear") cam.linear_name = argv[i + 1];
         else if (k == "--nee") cam.next_event_estimation = std::atoi(argv[i + 1]) != 0;
+        else if (k == "--noise") cam.noise_target = std::atof(argv[i + 1]);
+        else if (k == "--noise-every") cam.noise_check_every_spp = std::atoi(argv[i + 1]);
+        else if (k == "--variance") cam.variance_name = argv[i + 1];
         else if (k == "--shadowed-point-lights") cam.shadowed_point_lights = std::atoi(argv[i + 1]) != 0;
         else if (k == "--devices") {
             std::string v = argv[i + 1];
@@ -67,5 +72,7 @@ int main(int argc, char** argv) {
     cam.image_name = out.c_str();
     std::cout << "Rendering Image: " << cam.image_name << std::endl;
     cam.render(world, lights);
+    if (cam.noise_target > 0 || !cam.variance_name.empty())
+        std::cout << "Samples per pixel: " << cam.last_spp_done << ", relative noise " << cam.last_noise << std::endl;
     return 0;
 }

@@ -264,6 +264,12 @@ typedef enum rt_shard_mode {
                                  or anything that waits (rt_sync, rt_download, rt_resolve_tiles, ...) before using the
                                  frame.  Ignored (a plain asynchronous pass) without both other flags and with
                                  RT_FLAG_STATS.  rt_stats.render_ms is then the average per overlapped pass. */
+#define RT_FLAG_MOMENTS 128u  /* also accumulate per-pixel second moments (exact integer sums of the squared samples) into a
+                                 moments buffer of the context (48 bytes per pixel, the layout of the sums).  A pass
+                                 without RT_FLAG_ACCUMULATE starts them; an accumulating pass with the flag needs a frame
+                                 whose moments describe its sums (RT_ERR_STATE otherwise), and one without it leaves the
+                                 frame without moments.  Runs the general kernel instances (plain / NEE); with RT_FLAG_STATS
+                                 it is RT_ERR_UNSUPPORTED.  The image is the same as without the flag. */
 
 typedef struct rt_render_params {
     uint32_t struct_size;
@@ -423,6 +429,30 @@ int rt_bind_accum(rt_ctx* ctx, void* device_ptr, size_t bytes, int32_t width, in
  * uninterrupted render of the same total. */
 int rt_accum_download(rt_ctx* ctx, uint64_t* host, size_t bytes);
 int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height);
+
+/* Per-pixel noise of a frame rendered with RT_FLAG_MOMENTS.  A sample's value x in channel c is the integer its
+ * radiance word adds (2^-28 units, clamped to [0, 2^20]); the moments hold S2 = sum x^2 exactly as two 48-bit limbs,
+ * m[6p + 2c] = sum (x^2 mod 2^48), m[6p + 2c + 1] = sum (x^2 >> 48).  Like the sums they are bit-identical for any
+ * device count, shard mode, pass split, overlap or resume.  A frame without valid moments is RT_ERR_STATE. */
+/* Unbiased per-sample variance of every pixel and channel, s^2 = (n*S2 - S1^2) / (n*(n-1)) * 2^-56 with n = total_spp
+ * (the rt_download divisor; dropped non-finite samples count as 0, as in the mean).  width*height*3 floats, row-major,
+ * like rgb_linear: the same quantity as the `var` of the golden fixtures.  total_spp >= 2.  n*S2 - S1^2 is exact;
+ * n*S2 saturates at 2^128 - 1, which only samples saturated at the 2^20 clamp at 65536 spp can reach.
+ * Multi-device contexts: tile-sharded frames without a restored checkpoint (else RT_ERR_UNSUPPORTED). */
+int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* variance);
+
+/* Raw moments for checkpoints: width*height*6 uint64 (per channel: sum of the low and of the high 48 bits of x^2),
+ * always the full frame like rt_accum_download.  rt_moments_upload restores the moments of the frame that
+ * rt_accum_upload restored just before (RT_ERR_STATE otherwise).  Single-device contexts. */
+int rt_moments_download(rt_ctx* ctx, uint64_t* host, size_t bytes);
+int rt_moments_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height);
+
+/* Frame noise: the mean linear radiance over pixels and channels, and the RMS over pixels and channels of the
+ * standard error of the pixel mean, sqrt(mean(s^2 / n)).  Reduced on the device as exact integer sums, so the result is
+ * a pure function of the sums and moments: sum S1, and sum q with q = round(s^2 / n * 2^32) in double arithmetic
+ * (saturating at 2^64 - 1), then divided once on the host.  Covers the pixels the context holds (a compact shard: its
+ * own tiles).  Multi-device contexts: as rt_download_variance. */
+int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double* rms_std_error);
 
 /* Compact tile buffers across processes (one process per GPU, e.g. under torchrun; single-device contexts):
  *   rt_shard_pixels   slots of the compact buffer of shard (rank, count): its tiles x tile_size^2 (edge tiles padded)

@@ -24,6 +24,7 @@ RT_TEX_SOLID, RT_TEX_CHECKER, RT_TEX_CHECKER_TRIANGLE, RT_TEX_IMAGE, RT_TEX_NOIS
 RT_SHARD_AUTO, RT_SHARD_TILES, RT_SHARD_SAMPLES = range(3)
 RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_STATS, RT_FLAG_NEE, RT_FLAG_SHADOWED_POINT_LIGHTS, RT_FLAG_COMPACT_TILES = 1, 2, 4, 8, 16, 32
 RT_FLAG_OVERLAP = 64
+RT_FLAG_MOMENTS = 128
 
 d3 = C.c_double * 3
 
@@ -149,6 +150,7 @@ EXPORTED_SYMBOLS = [
     "rt_probe_hit", "rt_struct_size", "rt_accum_download", "rt_accum_upload", "rt_set_bvh_builder",
     "rt_set_bvh_width", "rt_device_count", "rt_shard_pixels", "rt_resolve_tiles", "rt_untile",
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
+    "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
@@ -210,6 +212,10 @@ def load() -> C.CDLL:
     lib.rt_frame_end.argtypes = [vp, C.POINTER(vp), C.POINTER(vp)]
     lib.rt_accum_download.argtypes = [vp, vp, C.c_size_t]
     lib.rt_accum_upload.argtypes = [vp, vp, C.c_size_t, i32, i32]
+    lib.rt_download_variance.argtypes = [vp, i32, vp]
+    lib.rt_moments_download.argtypes = [vp, vp, C.c_size_t]
+    lib.rt_moments_upload.argtypes = [vp, vp, C.c_size_t, i32, i32]
+    lib.rt_frame_noise.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double)]
     lib.rt_measure_l1_peak.argtypes = [vp, C.POINTER(C.c_double)]
     lib.rt_probe_texture.argtypes = [vp, i32, i32, vp, vp]
@@ -381,7 +387,8 @@ class Context:
     def render(self, width: int, height: int, spp: int, max_depth: int = 50, seed: int = 1, spp_begin: int = 0,
                accumulate: bool = False, stats: bool = False, shard_rank: int = 0, shard_count: int = 1,
                shard_mode: int = RT_SHARD_AUTO, tile_size: int = 0, stream: Optional[int] = None, blocking: bool = True,
-               nee: bool = False, shadowed_point_lights: bool = False, compact: bool = False, overlap: bool = False) -> None:
+               nee: bool = False, shadowed_point_lights: bool = False, compact: bool = False, overlap: bool = False,
+               moments: bool = False) -> None:
         p = rt_render_params()
         p.struct_size = C.sizeof(rt_render_params)
         p.width, p.height, p.samples_per_pixel, p.max_depth = width, height, spp, max_depth
@@ -389,7 +396,7 @@ class Context:
         p.shard_mode, p.shard_rank, p.shard_count = shard_mode, shard_rank, shard_count
         p.flags = ((RT_FLAG_ACCUMULATE if accumulate else 0) | (RT_FLAG_STATS if stats else 0) | (0 if blocking else RT_FLAG_ASYNC) |
                    (RT_FLAG_NEE if nee else 0) | (RT_FLAG_SHADOWED_POINT_LIGHTS if shadowed_point_lights else 0) |
-                   (RT_FLAG_COMPACT_TILES if compact else 0) | (RT_FLAG_OVERLAP if overlap else 0))
+                   (RT_FLAG_COMPACT_TILES if compact else 0) | (RT_FLAG_OVERLAP if overlap else 0) | (RT_FLAG_MOMENTS if moments else 0))
         p.stream = stream
         self._check(self.lib.rt_render(self._h, C.byref(p)))
         self.width, self.height = width, height
@@ -480,6 +487,29 @@ class Context:
         h, w = sums.shape[0], sums.shape[1]
         self._check(self.lib.rt_accum_upload(self._h, sums.ctypes.data, sums.nbytes, w, h))
         self.width, self.height = w, h
+
+    def download_variance(self, total_spp: int) -> np.ndarray:
+        """Unbiased per-sample variance (H, W, 3) float32 of a frame rendered with moments=True."""
+        out = np.empty((self.height, self.width, 3), dtype=np.float32)
+        self._check(self.lib.rt_download_variance(self._h, total_spp, out.ctypes.data))
+        return out
+
+    def moments_download(self) -> np.ndarray:
+        """The raw second moments (H, W, 6) uint64: per channel the sums of the low and the high 48 bits of x^2."""
+        out = np.empty((self.height, self.width, 6), dtype=np.uint64)
+        self._check(self.lib.rt_moments_download(self._h, out.ctypes.data, out.nbytes))
+        return out
+
+    def moments_upload(self, m: np.ndarray) -> None:
+        """Restore the moments of the frame accum_upload() restored just before."""
+        m = np.ascontiguousarray(m, dtype=np.uint64)
+        self._check(self.lib.rt_moments_upload(self._h, m.ctypes.data, m.nbytes, m.shape[1], m.shape[0]))
+
+    def frame_noise(self, total_spp: int):
+        """(mean linear radiance, RMS standard error of the pixel mean) of a frame rendered with moments=True."""
+        mean, rms = C.c_double(), C.c_double()
+        self._check(self.lib.rt_frame_noise(self._h, total_spp, C.byref(mean), C.byref(rms)))
+        return mean.value, rms.value
 
     def stats(self) -> dict:
         st = rt_stats()

@@ -469,6 +469,7 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
         cudaSetDevice(d->device);
         if (d->accum && !d->accum_external) CUX(ctx, cudaMemsetAsync(d->accum, 0, d->accum_bytes, d->stream));
         CUX(ctx, cudaStreamSynchronize(d->stream));
+        d->moments_valid = false;  // moments are not restored across devices (rt_moments_upload is single-device)
     }
     cudaSetDevice(d0->device);
     if (ctx->base_sums) cudaFree(ctx->base_sums);
@@ -479,6 +480,74 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
     CUX(ctx, cudaMemcpyAsync(ctx->base_sums, host, need, cudaMemcpyHostToDevice, d0->stream));
     CUX(ctx, cudaStreamSynchronize(d0->stream));
     return RT_OK;
+}
+
+// ---- second moments (RT_FLAG_MOMENTS) ------------------------------------------------------------------------------
+// A multi-device frame has per-device variance only when each pixel lives on one device: tiles, no restored checkpoint.
+static int multi_moments_frame(rt_ctx* ctx, const char* what) {
+    if (!ctx->rendered) return failx(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
+    if (!(ctx->dev[0]->acc.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size()))
+        return failx(ctx, RT_ERR_UNSUPPORTED, "%s: a multi-device context resolves tile-sharded frames without a restored checkpoint only", what);
+    return RT_OK;
+}
+
+extern "C" int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* variance) {
+    RT_NEED(ctx);
+    const int n = (int)ctx->dev.size();
+    if (n == 1) return fwd(ctx, ctx->dev[0], dev_download_variance(ctx->dev[0], total_spp, variance));
+    if (!variance) return RT_ERR_INVALID;
+    if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
+    int rc = multi_moments_frame(ctx, "rt_download_variance");
+    if (rc != RT_OK) return rc;
+    // like the linear radiance of rt_download: resolved where the tiles were rendered, 12 bytes per pixel gathered
+    std::vector<const void*> src((size_t)n);
+    std::vector<size_t> bytes((size_t)n);
+    size_t stride = 0;
+    for (int d = 0; d < n; d++) {
+        DevCtx* dc = ctx->dev[d];
+        rc = moments_ready(dc, "rt_download_variance");
+        if (rc == RT_OK) rc = dev_variance_into(dc, total_spp);
+        if (rc != RT_OK) return fwd(ctx, dc, rc);
+        src[d] = dc->out_lin;
+        bytes[d] = dc->acc.slots() * 12;
+        stride = std::max(stride, (bytes[d] + 255) & ~(size_t)255);
+    }
+    rc = gather_to_dev0(ctx, src, bytes, stride);
+    if (rc != RT_OK) return rc;
+    return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 12, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, variance));
+}
+
+extern "C" int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double* rms_std_error) {
+    RT_NEED(ctx);
+    if (!mean_radiance || !rms_std_error) return RT_ERR_INVALID;
+    if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_frame_noise: total_spp must be at least 2");
+    if (ctx->dev.size() > 1) {
+        int rc = multi_moments_frame(ctx, "rt_frame_noise");
+        if (rc != RT_OK) return rc;
+    }
+    // integer partials of every device added on the host: the same words whatever the device count
+    uint64_t sum[12] = {0}, pixels = 0;
+    for (DevCtx* d : ctx->dev) {
+        uint64_t part[12], px = 0;
+        int rc = dev_noise_partials(d, total_spp, part, &px);
+        if (rc != RT_OK) return fwd(ctx, d, rc);
+        for (int k = 0; k < 12; k++) sum[k] += part[k];
+        pixels += px;
+    }
+    noise_from_partials(sum, pixels, total_spp, mean_radiance, rms_std_error);
+    return RT_OK;
+}
+
+extern "C" int rt_moments_download(rt_ctx* ctx, uint64_t* host, size_t bytes) {
+    RT_NEED(ctx);
+    if (ctx->dev.size() != 1) return failx(ctx, RT_ERR_UNSUPPORTED, "rt_moments_download: single-device contexts only");
+    return fwd(ctx, ctx->dev[0], dev_moments_download(ctx->dev[0], host, bytes));
+}
+
+extern "C" int rt_moments_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height) {
+    RT_NEED(ctx);
+    if (ctx->dev.size() != 1) return failx(ctx, RT_ERR_UNSUPPORTED, "rt_moments_upload: single-device contexts only");
+    return fwd(ctx, ctx->dev[0], dev_moments_upload(ctx->dev[0], host, bytes, width, height));
 }
 
 extern "C" int rt_resolve_tiles(rt_ctx* ctx, int32_t total_spp, float* dev_rgb_linear, uint8_t* dev_rgb8, size_t capacity_pixels) {

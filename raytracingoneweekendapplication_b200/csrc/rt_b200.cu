@@ -2,13 +2,15 @@
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
 // Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
-//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT>
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
 //                          fixed-point accumulation.  Instances: plain / LITE / STATS for the binary
-//                          and both wide trees, NEE (binary tree), and the feature instances of kInstances
+//                          and both wide trees, NEE (binary tree), the feature instances of kInstances,
+//                          and the MOMENTS twins of plain / LITE / NEE / NEE + LITE (binary tree)
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
+//   variance_kernel, noise_kernel   sums + second moments -> per-pixel sample variance, frame noise partials
 //   untile_kernel, tile_pack_kernel, add_sums_kernel   shard frames: compact tiles <-> full frame, sums
 //   pair_nodes_kernel      device-built BVH2 nodes -> the paired layout the traversal reads
 //   probe_*_kernel         per-function known-answer probes
@@ -51,15 +53,33 @@ struct RenderArgs {
     int tile_stride, tile_offset;      // global tile = tile_offset + k * tile_stride
     int n_local_tiles;
     int blocks_per_tile_x, blocks_per_tile_y;  // 8x4 pixel blocks per tile
+    uint32_t moments_lo;     // MOMENTS instances: the moments buffer, its two 32-bit halves in the struct's two alignment
+                             // holes (here and after shadow_point_lights), so that no offset of a field or a kernel parameter moves
     unsigned long long n_items;
     uint32_t k0, k1;
     int compact;             // RT_FLAG_COMPACT_TILES: `accum` holds only this shard's tiles, tile-major: slot = local_tile * tile_size^2 + y_in_tile * tile_size + x_in_tile
     int nee_emitters;        // NEE instance: sample the listed quad emitters (RT_FLAG_NEE)
     int shadow_point_lights; // NEE instance: shadow rays for the point lights (RT_FLAG_SHADOWED_POINT_LIGHTS)
+    uint32_t moments_hi;
+    __host__ __device__ unsigned long long* moments() const { return (unsigned long long*)(((uint64_t)moments_hi << 32) | moments_lo); }
+    void set_moments(unsigned long long* p) { moments_lo = (uint32_t)(uintptr_t)p; moments_hi = (uint32_t)((uint64_t)(uintptr_t)p >> 32); }
 };
+static_assert(sizeof(RenderArgs) == 104 && offsetof(RenderArgs, n_items) == 72, "the moments pointer fills alignment holes only");
 
 constexpr float kAccumScale = 268435456.0f;  // 2^RT_ACCUM_FRAC_BITS
 constexpr float kSampleClamp = 1048576.0f;   // 2^20: keeps 2^16 saturated samples inside 64 bits
+
+// RT_FLAG_MOMENTS: the second moment of a sample.  x is the exact integer added to a radiance word (x <= 2^48 after the
+// clamp), so x^2 <= 2^96 is exact in 128 bits; it is added as two 48-bit limbs, m[0] += x^2 mod 2^48 and
+// m[1] += x^2 >> 48, each < 2^48 except m[1] = 2^48 for a sample saturated at kSampleClamp.  With at most 2^16 samples
+// per pixel a limb word stays below 2^64 however the samples are split -- save for 2^16 samples that ALL saturate,
+// the edge the radiance words share (kSampleClamp).  A zero limb (every black sample) costs no atomic.
+__device__ __forceinline__ void add_square(unsigned long long* m, unsigned long long x) {
+    const unsigned long long lo = x * x, hi = __umul64hi(x, x);
+    const unsigned long long l0 = lo & ((1ull << 48) - 1ull), l1 = (lo >> 48) | (hi << 16);
+    if (l0) atomicAdd(m, l0);
+    if (l1) atomicAdd(m + 1, l1);
+}
 
 // ---------------------------------------------------------------------------------
 // render_kernel_v2 — the production megakernel.
@@ -136,7 +156,8 @@ struct LocalSlot {
     }
 };
 
-template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL>
+// MOMENTS: also add the second moments of every finished sample to A.moments() (6 words per slot, see add_square)
+template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
                                                         unsigned long long* __restrict__ counters, Stats* __restrict__ gstats) {
@@ -366,6 +387,12 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     atomicAdd(a + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
                     atomicAdd(a + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
                     atomicAdd(a + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
+                    if constexpr (MOMENTS) {
+                        unsigned long long* m = A.moments() + 6ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel);
+                        add_square(m + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
+                        add_square(m + 2, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
+                        add_square(m + 4, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
+                    }
                 } else {
                     atomicAdd(a + 3, 1ull);
                     if (STATS) st.nonfinite++;
@@ -412,6 +439,16 @@ static const FeatInstance kInstances[] = {
 };
 #undef RT_INSTANCE
 constexpr int kNumInstances = (int)(sizeof(kInstances) / sizeof(kInstances[0]));
+// the RT_FLAG_MOMENTS instances: plain, LITE, NEE + LITE, NEE (variants 0, 1, 3, 4 of the dispatch below), binary tree only
+constexpr int kMomentsVariant = 64;
+static RenderKernel v2_moments_kernel(int variant) {
+    switch (variant) {
+        case 1: return render_kernel_v2<false, true, false, 2, FEAT_ALL, true>;
+        case 3: return render_kernel_v2<false, true, true, 2, FEAT_ALL, true>;
+        case 4: return render_kernel_v2<false, false, true, 2, FEAT_ALL, true>;
+        default: return render_kernel_v2<false, false, false, 2, FEAT_ALL, true>;
+    }
+}
 
 // one ray through whichever acceleration structure the scene was uploaded with (test kernels)
 __device__ __forceinline__ void traverse_uploaded(const DevScene& S, const Ray& ray, float tmin, float tmax, Hit& hit) {
@@ -490,6 +527,84 @@ __global__ void resolve_kernel(const unsigned long long* __restrict__ accum, int
             rgb8[3ull * px + c] = (unsigned char)(int)(255.999f * g);
         }
     }
+}
+
+// RT_FLAG_MOMENTS resolve.  With n = total_spp, S1 the radiance word and S2 = m0 + m1 * 2^48 its moments (both in the
+// 2^-28 units of x), D = n * S2 - S1^2 is computed exactly in 128 bits.  It is >= 0 by Cauchy-Schwarz (dropped samples
+// count as x = 0 of the n).  n * S2 can reach 2^128 only when samples saturate at kSampleClamp at 65536 spp: the
+// product then saturates at 2^128 - 1 instead of wrapping, and D is a lower bound.
+struct U128 {
+    unsigned long long lo, hi;
+};
+__device__ __forceinline__ U128 moments_d(unsigned long long s1, unsigned long long m0, unsigned long long m1, unsigned long long n) {
+    const unsigned long long s2_lo = m0 + (m1 << 48);
+    const unsigned long long s2_hi = (m1 >> 16) + (s2_lo < m0 ? 1ull : 0ull);
+    U128 ns2;
+    ns2.lo = n * s2_lo;
+    const unsigned long long c = __umul64hi(n, s2_lo);
+    ns2.hi = n * s2_hi + c;
+    if (__umul64hi(n, s2_hi) != 0 || ns2.hi < c) ns2.lo = ns2.hi = ~0ull;  // saturate
+    const unsigned long long q_lo = s1 * s1, q_hi = __umul64hi(s1, s1);
+    U128 d;
+    if (ns2.hi < q_hi || (ns2.hi == q_hi && ns2.lo < q_lo)) {
+        d.lo = d.hi = 0;  // only a total_spp below the true sample count gets here
+        return d;
+    }
+    d.lo = ns2.lo - q_lo;
+    d.hi = ns2.hi - q_hi - (ns2.lo < q_lo ? 1ull : 0ull);
+    return d;
+}
+// a 128-bit integer rounded once to the nearest double (ties to even): the top 64 bits with a sticky bit for the rest
+__device__ __forceinline__ double u128_to_double(U128 v) {
+    if (v.hi == 0) return __ull2double_rn(v.lo);
+    const int sh = 64 - __clzll((long long)v.hi);  // 1..64
+    const unsigned long long top = sh == 64 ? v.hi : (v.hi << (64 - sh)) | (v.lo >> sh);
+    const unsigned long long sticky = (sh == 64 ? v.lo : (v.lo << (64 - sh))) != 0 ? 1ull : 0ull;
+    return ldexp(__ull2double_rn(top | sticky), sh);
+}
+// unbiased per-sample variance s^2 = D / (n (n - 1)) * 2^-56, rounded once to double, divided, rounded once to float
+__global__ void variance_kernel(const unsigned long long* __restrict__ accum, const unsigned long long* __restrict__ moments, int n_slots,
+                                int n, float* __restrict__ var) {
+    const int px = blockIdx.x * blockDim.x + threadIdx.x;
+    if (px >= n_slots) return;
+    const double nn1 = (double)n * (double)(n - 1);
+    for (int c = 0; c < 3; c++) {
+        const U128 d = moments_d(accum[4ull * px + c], moments[6ull * px + 2 * c], moments[6ull * px + 2 * c + 1], (unsigned long long)n);
+        var[3ull * px + c] = (float)__dmul_rn(__ddiv_rn(u128_to_double(d), nn1), 0x1p-56);
+    }
+}
+// rt_frame_noise partials, exact integer sums over the slots: out[2c], out[2c + 1] += the low / high 32 bits of S1 of
+// channel c; out[6 + 2c], out[7 + 2c] += the low / high 32 bits of q = round(s^2 / n * 2^kNoiseFracBits) of channel c,
+// q saturating at 2^64 - 1.  A word adds at most 2^31 values below 2^32: no overflow for any frame rt_render accepts.
+constexpr int kNoiseFracBits = 32;
+__global__ void noise_kernel(const unsigned long long* __restrict__ accum, const unsigned long long* __restrict__ moments, int n_slots, int n,
+                             unsigned long long* __restrict__ out) {
+    __shared__ unsigned long long part[12];
+    if (threadIdx.x < 12) part[threadIdx.x] = 0;
+    __syncthreads();
+    const int px = blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long w[12];
+    for (int k = 0; k < 12; k++) w[k] = 0;
+    if (px < n_slots) {
+        const double nn2 = (double)n * (double)n * (double)(n - 1);
+        for (int c = 0; c < 3; c++) {
+            const unsigned long long s1 = accum[4ull * px + c];
+            const U128 d = moments_d(s1, moments[6ull * px + 2 * c], moments[6ull * px + 2 * c + 1], (unsigned long long)n);
+            const double q = __dmul_rn(__ddiv_rn(u128_to_double(d), nn2), 0x1p-24);  // s^2 / n in 2^-kNoiseFracBits units
+            const unsigned long long qi = q >= 0x1p64 ? ~0ull : __double2ull_rn(q);
+            w[2 * c] = s1 & 0xffffffffull;
+            w[2 * c + 1] = s1 >> 32;
+            w[6 + 2 * c] = qi & 0xffffffffull;
+            w[7 + 2 * c] = qi >> 32;
+        }
+    }
+    for (int k = 0; k < 12; k++) {
+        unsigned long long v = w[k];
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
+        if ((threadIdx.x & 31u) == 0 && v) atomicAdd(&part[k], v);
+    }
+    __syncthreads();
+    if (threadIdx.x < 12 && part[threadIdx.x]) atomicAdd(out + threadIdx.x, part[threadIdx.x]);
 }
 
 __global__ void probe_texture_kernel(const __grid_constant__ DevScene S, int tex, int n, const float* __restrict__ uvp,
@@ -609,6 +724,15 @@ struct AccumLayout {
         return tiles > (size_t)rank ? (tiles - rank + count - 1) / count : 0;
     }
     size_t slots() const { return compact ? local_tiles() * tile * tile : (size_t)width * height; }
+    // pixels of the frame the slots hold (a compact buffer's partial edge tiles have slots outside the frame)
+    size_t pixels() const {
+        if (!compact) return (size_t)width * height;
+        const int tiles_x = (width + tile - 1) / tile, n_tiles = tiles_x * ((height + tile - 1) / tile);
+        size_t px = 0;
+        for (int t = rank; t < n_tiles; t += count)
+            px += (size_t)std::min(tile, width - (t % tiles_x) * tile) * std::min(tile, height - (t / tiles_x) * tile);
+        return px;
+    }
 };
 
 struct DevCtx {
@@ -635,6 +759,15 @@ struct DevCtx {
     size_t accum_bytes = 0, accum_cap = 0;
     bool accum_external = false;
     AccumLayout acc;                        // layout of `accum`
+    // RT_FLAG_MOMENTS: 6 words per slot of `acc` (add_square), allocated by the first moments render; valid when they
+    // describe the same samples as the sums (set by a non-accumulating moments pass or rt_moments_upload, cleared by
+    // an accumulating pass without the flag, a pass that replaces the frame without it, a layout change, rt_bind_accum
+    // and rt_accum_upload)
+    unsigned long long* moments = nullptr;
+    size_t moments_cap = 0;
+    bool moments_valid = false;
+    bool sums_uploaded = false;              // the frame is an rt_accum_upload, not rendered onto since (rt_moments_upload)
+    unsigned long long* noise_sums = nullptr;  // rt_frame_noise: the 12 partial words of noise_kernel
     unsigned char* frame_scratch = nullptr;  // full-frame copies of compact data (checkpoints, single-shard downloads)
     size_t frame_scratch_cap = 0;
     unsigned long long* counters = nullptr;  // [0] work counter, [1..3] unused
@@ -768,6 +901,7 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     cudaFuncSetAttribute(render_kernel_v2<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     cudaFuncSetAttribute(render_kernel_v2<false, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     for (int k = 0; k < kNumInstances; k++) cudaFuncSetAttribute((const void*)kInstances[k].kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+    for (int v : {0, 1, 3, 4}) cudaFuncSetAttribute((const void*)v2_moments_kernel(v), cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     if (const char* bv = getenv("RT_B200_BVH"))
         ctx->bvh_builder = strcmp(bv, "host") == 0 ? 1 : (strcmp(bv, "device") == 0 ? 2 : (strcmp(bv, "lbvh") == 0 ? 3 : 0));
     if (const char* wv = getenv("RT_B200_BVH_WIDTH")) {
@@ -793,6 +927,8 @@ static void dev_destroy(DevCtx* ctx) {
     free_scene(ctx);
     release_buffers(ctx);
     if (ctx->accum && !ctx->accum_external) cudaFree(ctx->accum);
+    if (ctx->moments) cudaFree(ctx->moments);
+    if (ctx->noise_sums) cudaFree(ctx->noise_sums);
     if (ctx->counters) cudaFree(ctx->counters);
     if (ctx->dstats) cudaFree(ctx->dstats);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
@@ -1621,6 +1757,7 @@ static int ensure_accum(DevCtx* ctx, const AccumLayout& L) {
         return RT_OK;
     }
     if (ctx->accum && ctx->acc == L) return RT_OK;
+    ctx->moments_valid = false;
     if (!ctx->accum || need > ctx->accum_cap) {
         if (ctx->accum) cudaFree(ctx->accum);
         ctx->accum = nullptr;
@@ -1635,6 +1772,18 @@ static int ensure_accum(DevCtx* ctx, const AccumLayout& L) {
     return RT_OK;
 }
 
+// the moments buffer of RT_FLAG_MOMENTS: 48 bytes per slot, same layout as `accum` (its contents are set by the caller)
+static int ensure_moments(DevCtx* ctx, size_t slots) {
+    const size_t need = std::max<size_t>(slots, 1) * 6 * sizeof(unsigned long long);
+    if (ctx->moments && need <= ctx->moments_cap) return RT_OK;
+    if (ctx->moments) cudaFree(ctx->moments);
+    ctx->moments = nullptr;
+    ctx->moments_cap = 0;
+    if (cudaMalloc(&ctx->moments, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes for the moments buffer", need);
+    ctx->moments_cap = need;
+    return RT_OK;
+}
+
 static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t width, int32_t height) {
     if (!ctx) return RT_ERR_INVALID;
     CU(ctx, cudaSetDevice(ctx->device));
@@ -1646,6 +1795,7 @@ static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t w
     ctx->accum_external = false;
     ctx->acc = AccumLayout();
     ctx->accum_bytes = ctx->accum_cap = 0;
+    ctx->moments_valid = ctx->sums_uploaded = false;
     if (!device_ptr) return RT_OK;
     size_t need = (size_t)width * height * 4 * sizeof(unsigned long long);
     if (width <= 0 || height <= 0 || bytes < need) return fail(ctx, RT_ERR_INVALID, "rt_bind_accum: need %zu bytes for %dx%d, got %zu", need, width, height, bytes);
@@ -1668,7 +1818,7 @@ static int dev_accum_buffer(DevCtx* ctx, void** device_ptr, size_t* bytes) {
 // Scatter the compact tile buffers of `count` shards (shard r starts at shards + r * stride bytes) into a full
 // row-major frame of `bpp`-byte pixels: pixel (x, y) lies in tile t = (y / tile) * tiles_x + x / tile, which is local
 // tile t / count of shard t mod count.  only_rank >= 0: take that shard's tiles from `shards` directly (stride
-// unused) and leave the other pixels as they are.  bpp: 3 (RGB8), 12 (float RGB) or 32 (the uint64 sums).
+// unused) and leave the other pixels as they are.  bpp: 3 (RGB8), 12 (float RGB), 32 (the uint64 sums) or 48 (the moments).
 template <int BPP>
 __global__ void untile_kernel(const unsigned char* __restrict__ shards, size_t stride, int count, int only_rank, int width, int height,
                               int tile, unsigned char* __restrict__ dst) {
@@ -1690,6 +1840,12 @@ __global__ void untile_kernel(const unsigned char* __restrict__ shards, size_t s
         const float* sf = reinterpret_cast<const float*>(src);
         float* df = reinterpret_cast<float*>(out);
         df[0] = sf[0]; df[1] = sf[1]; df[2] = sf[2];
+    } else if (BPP == 48) {
+        const uint4* s4 = reinterpret_cast<const uint4*>(src);
+        uint4* d4 = reinterpret_cast<uint4*>(out);
+        d4[0] = s4[0];
+        d4[1] = s4[1];
+        d4[2] = s4[2];
     } else {
         out[0] = src[0]; out[1] = src[1]; out[2] = src[2];
     }
@@ -1721,6 +1877,7 @@ static cudaError_t launch_untile(int bpp, const void* shards, size_t stride, int
     unsigned char* d = (unsigned char*)dst;
     if (bpp == 32) untile_kernel<32><<<grid, block, 0, stream>>>(s, stride, count, only_rank, width, height, tile, d);
     else if (bpp == 12) untile_kernel<12><<<grid, block, 0, stream>>>(s, stride, count, only_rank, width, height, tile, d);
+    else if (bpp == 48) untile_kernel<48><<<grid, block, 0, stream>>>(s, stride, count, only_rank, width, height, tile, d);
     else untile_kernel<3><<<grid, block, 0, stream>>>(s, stride, count, only_rank, width, height, tile, d);
     return cudaGetLastError();
 }
@@ -1782,6 +1939,8 @@ static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int
     // start before the sums have landed)
     CU(ctx, cudaMemcpyAsync(ctx->accum, host, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->moments_valid = false;  // until rt_moments_upload restores the moments of the same samples
+    ctx->sums_uploaded = true;
     return RT_OK;
 }
 
@@ -1871,6 +2030,7 @@ static int dev_sync(DevCtx* ctx) {
 
 // The instances of render_kernel_v2: variant 0 plain (everything), 1 LITE, 2 STATS, 3 NEE + LITE, 4 NEE; width 2, 4, 8
 // (3, 4: binary tree only).  Variants 5 + k: the binary-tree instance kInstances[k], compiled for one feature mask.
+// kMomentsVariant | v (v = 0, 1, 3, 4): the RT_FLAG_MOMENTS twin of variant v, binary tree only.
 template <int WIDTH>
 static RenderKernel v2_instance(int variant) {
     switch (variant) {
@@ -1883,6 +2043,7 @@ static RenderKernel v2_instance(int variant) {
 // then both go through it): two fat kernels less per width in the shipped library
 static int v2_effective_width(int variant, int width) { return variant >= 3 ? 2 : width; }
 static RenderKernel v2_kernel(int variant, int width) {
+    if (variant & kMomentsVariant) return v2_moments_kernel(variant & ~kMomentsVariant);
     if (variant == 3) return render_kernel_v2<false, true, true, 2>;
     if (variant == 4) return render_kernel_v2<false, false, true, 2>;
     if (variant >= 5 && variant < 5 + kNumInstances) return kInstances[variant - 5].kernel;
@@ -1926,6 +2087,11 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     const int count = p->shard_count <= 1 ? 1 : p->shard_count;
     const int rank = count == 1 ? 0 : p->shard_rank;
     if (rank < 0 || rank >= count) return fail(ctx, RT_ERR_INVALID, "rt_render: shard_rank %d outside [0,%d)", rank, count);
+    const bool moments = (p->flags & RT_FLAG_MOMENTS) != 0;
+    if (moments && (p->flags & RT_FLAG_STATS)) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_MOMENTS has no RT_FLAG_STATS instance");
+    if (moments && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->moments_valid)
+        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_MOMENTS | RT_FLAG_ACCUMULATE onto a frame whose sums have no moments "
+                                       "(start it with a non-accumulating moments pass, or restore both with rt_accum_upload + rt_moments_upload)");
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
     // RT_FLAG_OVERLAP: this pass goes to one of the two lane streams with its own work counter and waits for nothing on
@@ -1988,12 +2154,20 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE onto a buffer of another frame size or tile layout");
     rc = ensure_accum(ctx, L);
     if (rc != RT_OK) return rc;
+    if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) {
+        rc = ensure_moments(ctx, L.slots());
+        if (rc != RT_OK) return rc;
+    }
+    A.set_moments(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
+    ctx->moments_valid = moments;  // an accumulating moments pass was checked above; any pass without the flag invalidates them
+    ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
     // which instance of render_kernel_v2 runs: LITE = no triangles, no point lights, no defocus blur in this scene (see hit_prim)
     const bool lite = ctx->scene_lite && !getenv("RT_B200_NO_LITE");
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
     int variant = (want_nee || want_shadow) ? (lite ? 3 : 4) : (stats ? 2 : (lite ? 1 : 0));
+    if (moments) variant |= kMomentsVariant;  // the general binary-tree twins: no per-scene moments instances
     const int width = ctx->scene.wide_width ? ctx->scene.wide_width : 2;
     // the first compiled instance that covers the scene's features (RT_B200_GENERAL_INSTANCE=1: always a general one)
     if (variant <= 1 && width == 2 && !getenv("RT_B200_GENERAL_INSTANCE"))
@@ -2073,6 +2247,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         return RT_OK;
     }
     if (!(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->accum, 0, L.slots() * 32, stream));
+    if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->moments, 0, L.slots() * 48, stream));
     CU(ctx, cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), stream));
     if (stats) CU(ctx, cudaMemsetAsync(ctx->dstats, 0, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long), stream));
     const bool async = (p->flags & RT_FLAG_ASYNC) != 0;
@@ -2276,6 +2451,109 @@ static int dev_download(DevCtx* ctx, int32_t total_spp, float* rgb_linear, uint8
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_download: %s", cudaGetErrorString(e));
+    return RT_OK;
+}
+
+// ---- second moments (RT_FLAG_MOMENTS) ------------------------------------------------------------------------------
+static int moments_ready(DevCtx* ctx, const char* what) {
+    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
+    if (!ctx->moments_valid) return fail(ctx, RT_ERR_STATE, "%s: the frame has no moments (render it with RT_FLAG_MOMENTS)", what);
+    return dev_wait(ctx);
+}
+
+// variance_kernel over the slots of the frame into out_lin (the buffer of the linear radiance of rt_download)
+static int dev_variance_into(DevCtx* ctx, int32_t total_spp) {
+    const size_t n = ctx->acc.slots();
+    int rc = ensure_out(ctx, n);
+    if (rc != RT_OK) return rc;
+    if (n) variance_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, ctx->moments, (int)n, total_spp, ctx->out_lin);
+    CU(ctx, cudaGetLastError());
+    return RT_OK;
+}
+
+static int dev_download_variance(DevCtx* ctx, int32_t total_spp, float* variance) {
+    if (!ctx || !variance) return RT_ERR_INVALID;
+    if (total_spp < 2) return fail(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
+    int rc = moments_ready(ctx, "rt_download_variance");
+    if (rc == RT_OK) rc = dev_variance_into(ctx, total_spp);
+    if (rc != RT_OK) return rc;
+    const size_t full = (size_t)ctx->acc.width * ctx->acc.height * 12;
+    const void* src = ctx->out_lin;
+    if (ctx->acc.compact) {
+        // one shard of a frame: its tiles go to their places in a zeroed full frame
+        const AccumLayout& L = ctx->acc;
+        rc = ensure_scratch_out(ctx, full);
+        if (rc != RT_OK) return rc;
+        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
+        CU(ctx, launch_untile(12, ctx->out_lin, 0, L.count, L.rank, L.width, L.height, L.tile, ctx->frame_scratch, ctx->stream));
+        src = ctx->frame_scratch;
+    }
+    CU(ctx, cudaMemcpyAsync(variance, src, full, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+// the 12 integer partials of noise_kernel over the slots of this device, and the frame pixels they cover
+static int dev_noise_partials(DevCtx* ctx, int32_t total_spp, uint64_t* partials, uint64_t* pixels) {
+    int rc = moments_ready(ctx, "rt_frame_noise");
+    if (rc != RT_OK) return rc;
+    if (!ctx->noise_sums) CU(ctx, cudaMalloc(&ctx->noise_sums, 12 * sizeof(unsigned long long)));
+    CU(ctx, cudaMemsetAsync(ctx->noise_sums, 0, 12 * sizeof(unsigned long long), ctx->stream));
+    const size_t n = ctx->acc.slots();
+    if (n) noise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, ctx->moments, (int)n, total_spp, ctx->noise_sums);
+    CU(ctx, cudaGetLastError());
+    CU(ctx, cudaMemcpyAsync(partials, ctx->noise_sums, 12 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    *pixels = ctx->acc.pixels();
+    return RT_OK;
+}
+
+// the partials -> (mean linear radiance, RMS standard error of the pixel mean), the one division of rt_frame_noise
+static void noise_from_partials(const uint64_t* w, uint64_t pixels, int32_t total_spp, double* mean, double* rms) {
+    unsigned __int128 s1 = 0, q = 0;
+    for (int c = 0; c < 3; c++) {
+        s1 += (unsigned __int128)w[2 * c] + ((unsigned __int128)w[2 * c + 1] << 32);
+        q += (unsigned __int128)w[6 + 2 * c] + ((unsigned __int128)w[7 + 2 * c] << 32);
+    }
+    const double values = 3.0 * (double)pixels;
+    *mean = pixels ? (double)s1 / ((double)kAccumScale * (double)total_spp * values) : 0.0;
+    *rms = pixels ? std::sqrt(std::ldexp((double)q, -kNoiseFracBits) / values) : 0.0;
+}
+
+static int dev_moments_download(DevCtx* ctx, uint64_t* host, size_t bytes) {
+    if (!ctx || !host) return RT_ERR_INVALID;
+    const size_t full = (size_t)ctx->acc.width * ctx->acc.height * 48;
+    if (ctx->accum && bytes != full) return fail(ctx, RT_ERR_INVALID, "rt_moments_download: a %dx%d frame is %zu bytes, got %zu", ctx->acc.width, ctx->acc.height, full, bytes);
+    int rc = moments_ready(ctx, "rt_moments_download");
+    if (rc != RT_OK) return rc;
+    const unsigned long long* src = ctx->moments;
+    if (ctx->acc.compact) {
+        rc = ensure_scratch_out(ctx, full);
+        if (rc != RT_OK) return rc;
+        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
+        CU(ctx, launch_untile(48, ctx->moments, 0, ctx->acc.count, ctx->acc.rank, ctx->acc.width, ctx->acc.height, ctx->acc.tile, ctx->frame_scratch, ctx->stream));
+        src = (const unsigned long long*)ctx->frame_scratch;
+    }
+    CU(ctx, cudaMemcpyAsync(host, src, full, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
+// the moments of the sums rt_accum_upload restored just before (same full frame)
+static int dev_moments_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height) {
+    if (!ctx || !host) return RT_ERR_INVALID;
+    if (width <= 0 || height <= 0 || (long long)width * height >= (1ll << 31)) return fail(ctx, RT_ERR_INVALID, "rt_moments_upload: bad frame size %dx%d", width, height);
+    const size_t need = (size_t)width * height * 48;
+    if (bytes != need) return fail(ctx, RT_ERR_INVALID, "rt_moments_upload: a %dx%d frame is %zu bytes, got %zu", width, height, need, bytes);
+    if (!ctx->sums_uploaded || ctx->acc.compact || ctx->acc.width != width || ctx->acc.height != height)
+        return fail(ctx, RT_ERR_STATE, "rt_moments_upload: follows rt_accum_upload of the same %dx%d frame", width, height);
+    CU(ctx, cudaSetDevice(ctx->device));
+    int rc = dev_wait(ctx);
+    if (rc == RT_OK) rc = ensure_moments(ctx, (size_t)width * height);
+    if (rc != RT_OK) return rc;
+    CU(ctx, cudaMemcpyAsync(ctx->moments, host, need, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->moments_valid = true;
     return RT_OK;
 }
 

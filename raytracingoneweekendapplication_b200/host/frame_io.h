@@ -100,7 +100,7 @@ inline bool write_exr(const char* path, int w, int h, const float* rgb) {
 // ---- checkpoint ------------------------------------------------------------------------
 struct checkpoint_header {
     char magic[8];         // "RTB2CKPT"
-    uint32_t version;      // 1
+    uint32_t version;      // 1: the sums; 2: the sums, then the second moments (RT_FLAG_MOMENTS, width * height * 6 uint64)
     int32_t width, height;
     int32_t spp_done;      // samples [0, spp_done) of every pixel are in the sums
     int32_t max_depth;
@@ -116,30 +116,35 @@ inline uint64_t fnv1a(const void* data, size_t n, uint64_t h = 14695981039346656
     return h;
 }
 
-inline bool write_checkpoint(const char* path, const checkpoint_header& hd, const uint64_t* sums) {
+inline bool write_checkpoint(const char* path, const checkpoint_header& hd, const uint64_t* sums, const uint64_t* moments = nullptr) {
     // write-then-rename so that an interruption DURING the save leaves the previous checkpoint intact
     std::string tmp = std::string(path) + ".tmp";
     std::FILE* f = std::fopen(tmp.c_str(), "wb");
     if (!f) return false;
     const size_t n = (size_t)hd.width * hd.height * 4;
     bool ok = std::fwrite(&hd, sizeof hd, 1, f) == 1 && std::fwrite(sums, 8, n, f) == n;
+    if (hd.version == 2) ok = ok && moments && std::fwrite(moments, 8, n / 4 * 6, f) == n / 4 * 6;
     ok = (std::fclose(f) == 0) && ok;
     if (!ok) { std::remove(tmp.c_str()); return false; }
     return std::rename(tmp.c_str(), path) == 0;
 }
 
-inline bool read_checkpoint(const char* path, checkpoint_header& hd, std::vector<uint64_t>& sums) {
+inline bool read_checkpoint(const char* path, checkpoint_header& hd, std::vector<uint64_t>& sums, std::vector<uint64_t>* moments = nullptr) {
     std::FILE* f = std::fopen(path, "rb");
     if (!f) return false;
-    bool ok = std::fread(&hd, sizeof hd, 1, f) == 1 && std::memcmp(hd.magic, "RTB2CKPT", 8) == 0 && hd.version == 1 &&
+    bool ok = std::fread(&hd, sizeof hd, 1, f) == 1 && std::memcmp(hd.magic, "RTB2CKPT", 8) == 0 && (hd.version == 1 || hd.version == 2) &&
               hd.width > 0 && hd.height > 0 && hd.spp_done >= 0 && (long long)hd.width * hd.height < (1ll << 31);
     if (ok) {
-        // the file must be exactly header + width * height * 32 bytes BEFORE anything is allocated from its header
-        const size_t n = (size_t)hd.width * hd.height * 4;
-        ok = std::fseek(f, 0, SEEK_END) == 0 && (unsigned long long)std::ftell(f) == sizeof hd + 8ull * n && std::fseek(f, (long)sizeof hd, SEEK_SET) == 0;
+        // the file must be exactly header + width * height * (32 | 80) bytes BEFORE anything is allocated from its header
+        const size_t n = (size_t)hd.width * hd.height * 4, nm = hd.version == 2 ? (size_t)hd.width * hd.height * 6 : 0;
+        ok = std::fseek(f, 0, SEEK_END) == 0 && (unsigned long long)std::ftell(f) == sizeof hd + 8ull * (n + nm) && std::fseek(f, (long)sizeof hd, SEEK_SET) == 0;
         if (ok) {
             sums.resize(n);
             ok = std::fread(sums.data(), 8, n, f) == n;
+        }
+        if (ok && moments) {
+            moments->resize(nm);
+            ok = std::fread(moments->data(), 8, nm, f) == nm;
         }
     }
     std::fclose(f);

@@ -1724,6 +1724,18 @@ class camera {
     int last_spp_done = 0;     // samples per pixel in the frame when render() returned
     int last_spp_resumed = 0;  // of which came from the checkpoint
     std::vector<float> last_linear;
+    // per-pixel noise (RT_FLAG_MOMENTS; on only when one of the first two is set -- otherwise flags, passes and
+    // checkpoint files are as without them):
+    //   noise_target     > 0: stop once rms_std_error / mean_radiance of rt_frame_noise <= this, samples_per_pixel
+    //                    being the cap
+    //   noise_check_every_spp  the noise is checked only when the frame holds a multiple of this many samples, so the
+    //                    stopping sample count is a function of the scene and settings alone, on any device list
+    //   variance_name    "x.exr" / "x.pfm": also write the per-pixel sample variance (rt_download_variance)
+    //   last_noise       rms_std_error / mean_radiance when render() returned (0 without moments)
+    double noise_target = 0;
+    int noise_check_every_spp = 256;
+    std::string variance_name;
+    double last_noise = 0;
 
     int image_height() const {
         int h = int(image_width / aspect_ratio);  // Camera.txt:137-138
@@ -1767,7 +1779,8 @@ class camera {
         rtb200::checkpoint_header ck;
         std::memset(&ck, 0, sizeof ck);
         std::memcpy(ck.magic, "RTB2CKPT", 8);
-        ck.version = 1;
+        const bool moments = noise_target > 0 || !variance_name.empty();
+        ck.version = moments ? 2 : 1;  // 2: the second moments follow the sums
         ck.width = p.width; ck.height = p.height; ck.max_depth = max_depth; ck.seed = seed;
         ck.scene_hash = checkpoint_path.empty() ? 0 : fs.hash();
         const uint32_t estimator_flags = (next_event_estimation ? RT_FLAG_NEE : 0u) | (shadowed_point_lights ? RT_FLAG_SHADOWED_POINT_LIGHTS : 0u);
@@ -1778,13 +1791,24 @@ class camera {
             if (ctx) rt_destroy(ctx);
             std::exit(2);
         }
-        std::vector<uint64_t> sums;
+        if (moments && devs.size() > 1) {
+            if (!checkpoint_path.empty()) {
+                std::cerr << "rt_b200: a noise target or variance output with a checkpoint needs one device (moments are downloaded from one context device)" << std::endl;
+                rt_destroy(ctx);
+                std::exit(2);
+            }
+            p.shard_mode = RT_SHARD_TILES;  // a multi-device context resolves the noise of tile-sharded frames
+        }
+        std::vector<uint64_t> sums, msums;
         if (!checkpoint_path.empty()) {
             rtb200::checkpoint_header old;
-            if (rtb200::read_checkpoint(checkpoint_path.c_str(), old, sums)) {
-                if (old.width == ck.width && old.height == ck.height && old.max_depth == ck.max_depth && old.seed == ck.seed &&
+            if (rtb200::read_checkpoint(checkpoint_path.c_str(), old, sums, &msums)) {
+                if (moments && old.version != 2) {
+                    std::cerr << "Ignoring " << checkpoint_path << ": it holds no second moments (version 1), which a noise target or variance output needs" << std::endl;
+                } else if (old.width == ck.width && old.height == ck.height && old.max_depth == ck.max_depth && old.seed == ck.seed &&
                     old.scene_hash == ck.scene_hash && old.flags == ck.flags && old.spp_done <= samples_per_pixel) {
                     if (rt_accum_upload(ctx, sums.data(), sums.size() * 8, p.width, p.height) != RT_OK) fail("rt_accum_upload");
+                    if (moments && rt_moments_upload(ctx, msums.data(), msums.size() * 8, p.width, p.height) != RT_OK) fail("rt_moments_upload");
                     done = old.spp_done;
                     std::cerr << "Resuming " << image_name << " at sample " << done << " from " << checkpoint_path << std::endl;
                 } else {
@@ -1796,38 +1820,53 @@ class camera {
         auto save_checkpoint = [&](int spp_done) {
             sums.resize((size_t)p.width * p.height * 4);
             if (rt_accum_download(ctx, sums.data(), sums.size() * 8) != RT_OK) fail("rt_accum_download");
+            if (moments) {
+                msums.resize((size_t)p.width * p.height * 6);
+                if (rt_moments_download(ctx, msums.data(), msums.size() * 8) != RT_OK) fail("rt_moments_download");
+            }
             ck.spp_done = spp_done;
-            if (!rtb200::write_checkpoint(checkpoint_path.c_str(), ck, sums.data()))
+            if (!rtb200::write_checkpoint(checkpoint_path.c_str(), ck, sums.data(), msums.data()))
                 std::cerr << "\nrt_b200: cannot write checkpoint " << checkpoint_path << std::endl;
         };
         // progressive passes so the reference's progress line (Camera.txt:102-106) still ticks
         const int target = stop_after_spp > 0 ? std::min(stop_after_spp, samples_per_pixel) : samples_per_pixel;
         const int pass_spp = std::max(1, std::min(samples_per_pixel, 64));
         int since_save = 0, passes = 0;
-        bool fresh = done == 0;
-        while (done < target) {
+        bool fresh = done == 0, converged = false;
+        const int check_every = std::max(1, noise_check_every_spp);
+        auto frame_noise = [&]() {
+            double mean = 0, rms = 0;
+            if (rt_frame_noise(ctx, done, &mean, &rms) != RT_OK) fail("rt_frame_noise");
+            return mean > 0 ? rms / mean : 0.0;
+        };
+        while (done < target && !converged) {
             int n = std::min(pass_spp, target - done);
             if (!checkpoint_path.empty() && checkpoint_every_spp > 0) n = std::min(n, std::max(1, checkpoint_every_spp - since_save));
+            if (noise_target > 0) n = std::min(n, check_every - done % check_every);
             p.samples_per_pixel = n;
             p.spp_begin = done;
             // passes after the first are enqueued without waiting and overlap their drains (RT_FLAG_OVERLAP: the last,
             // longest paths of one pass run while the next fills the freed SMs; integer sums, same frame).  Every eighth
             // pass is waited for, so that the progress line below stays within eight passes of the truth; checkpoints
             // and the download wait for everything by themselves.
-            p.flags = (fresh ? 0 : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC | RT_FLAG_OVERLAP)) | estimator_flags;
+            p.flags = (fresh ? 0 : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC | RT_FLAG_OVERLAP)) | estimator_flags | (moments ? RT_FLAG_MOMENTS : 0u);
             fresh = false;
             if (rt_render(ctx, &p) != RT_OK) fail("rt_render");
             if (++passes % 8 == 0 && rt_sync(ctx) != RT_OK) fail("rt_sync");
             done += n;
             since_save += n;
-            if (!checkpoint_path.empty() && checkpoint_every_spp > 0 && since_save >= checkpoint_every_spp && done < samples_per_pixel) {
+            if (noise_target > 0 && done % check_every == 0 && done >= 2 && frame_noise() <= noise_target) {
+                converged = true;
+                std::cout << "\nNoise target " << noise_target << " reached at " << done << " samples per pixel" << std::endl;
+            }
+            if (!checkpoint_path.empty() && checkpoint_every_spp > 0 && since_save >= checkpoint_every_spp && done < samples_per_pixel && !converged) {
                 save_checkpoint(done);
                 since_save = 0;
             }
             std::cerr << "\rPercent Rendered: " << (100 * done / samples_per_pixel) << "% " << std::flush;
         }
         if (!checkpoint_path.empty()) {
-            if (done < samples_per_pixel) save_checkpoint(done);  // stopped early: keep what we have
+            if (done < samples_per_pixel && !converged) save_checkpoint(done);  // stopped early: keep what we have
             else std::remove(checkpoint_path.c_str());              // finished: nothing left to resume
         }
         last_spp_done = done;
@@ -1836,6 +1875,12 @@ class camera {
         if (want_linear) last_linear.assign((size_t)p.width * p.height * 3, 0.0f);
         if (done > 0) {
             if (rt_download(ctx, done, want_linear ? last_linear.data() : nullptr, last_rgb8.data()) != RT_OK) fail("rt_download");
+        }
+        last_noise = moments && done >= 2 ? frame_noise() : 0.0;
+        std::vector<float> variance;
+        if (!variance_name.empty() && done >= 2) {
+            variance.assign((size_t)p.width * p.height * 3, 0.0f);
+            if (rt_download_variance(ctx, done, variance.data()) != RT_OK) fail("rt_download_variance");
         }
         rt_get_stats(ctx, &last_stats);
         rt_destroy(ctx);
@@ -1846,6 +1891,12 @@ class camera {
             bool ok = pfm ? rtb200::write_pfm(linear_name.c_str(), p.width, p.height, last_linear.data())
                           : rtb200::write_exr(linear_name.c_str(), p.width, p.height, last_linear.data());
             if (!ok) std::cerr << "rt_b200: cannot write " << linear_name << std::endl;
+        }
+        if (!variance.empty()) {
+            const bool pfm = variance_name.size() >= 4 && variance_name.compare(variance_name.size() - 4, 4, ".pfm") == 0;
+            bool ok = pfm ? rtb200::write_pfm(variance_name.c_str(), p.width, p.height, variance.data())
+                          : rtb200::write_exr(variance_name.c_str(), p.width, p.height, variance.data());
+            if (!ok) std::cerr << "rt_b200: cannot write " << variance_name << std::endl;
         }
     }
 };
