@@ -40,6 +40,7 @@ int main(int argc, char** argv) {
     //            --devices all | 0,1,2,...   split the frame over several GPUs of this box (one context, tiles gathered over NVLink)
     //            --noise X [--noise-every N]  stop once the relative frame noise is <= X, checked every N samples (default 256)
     //            --variance FILE.exr|.pfm     also write the per-pixel sample variance
+    //            --turntable N                N views around lookat in one batch, written to <stem>_000<ext> ...
     for (int i = 7; i + 1 < argc; i += 2) {
         std::string k = argv[i];
         if (k == "--checkpoint") cam.checkpoint_path = argv[i + 1];
@@ -50,6 +51,7 @@ int main(int argc, char** argv) {
         else if (k == "--noise") cam.noise_target = std::atof(argv[i + 1]);
         else if (k == "--noise-every") cam.noise_check_every_spp = std::atoi(argv[i + 1]);
         else if (k == "--variance") cam.variance_name = argv[i + 1];
+        else if (k == "--turntable") cam.turntable_frames = std::atoi(argv[i + 1]);
         else if (k == "--shadowed-point-lights") cam.shadowed_point_lights = std::atoi(argv[i + 1]) != 0;
         else if (k == "--devices") {
             std::string v = argv[i + 1];

@@ -395,6 +395,29 @@ int rt_join(rt_ctx* ctx, void* stream);
  * samples per pixel accumulated over all shards and passes. */
 int rt_download(rt_ctx* ctx, int32_t total_spp, float* rgb_linear, uint8_t* rgb8);
 
+/* Multi-view batches: n_views cameras of the uploaded scene rendered in one pass (one kernel launch), for turntables,
+ * fly-throughs and multi-view datasets, without an rt_upload_scene per view.
+ *
+ * rt_render_views renders into a views frame of the context (n_views x height x width, view-major, 32 B per pixel like
+ * the sums of rt_render).  View v is bit-identical to rt_render of the scene uploaded with cameras[v] and the same params
+ * and seed (seeds[v] when seeds != NULL).  cameras[v].background must equal the uploaded camera's (RT_ERR_INVALID
+ * otherwise), as must n_views >= 1 and cameras != NULL.
+ *   - flags: RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_NEE and RT_FLAG_SHADOWED_POINT_LIGHTS; params->stream is honoured.
+ *     RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, shard_count > 1 and multi-device contexts are
+ *     RT_ERR_UNSUPPORTED, and so is a frame of n_views x width x height >= 2^31 slots.
+ *   - the views frame is a buffer of its own: a views render does not touch the frame, moments or bound buffer of
+ *     rt_render, and rt_render does not touch the views frame.
+ *   - an RT_FLAG_ACCUMULATE pass must continue a views frame of the same (n_views, width, height), cameras and seeds
+ *     (RT_ERR_STATE otherwise).
+ *   - rt_stats: samples = n_views * width * height * samples_per_pixel, kernel_launches = 1, render_ms as for rt_render.
+ * rt_download_views copies views [first, first + count) of the views frame to the host: count * height * width * 3 floats
+ * / bytes, each view laid out like rt_download's planes.  Either pointer may be NULL.  RT_ERR_STATE before any views
+ * render, RT_ERR_INVALID for a range outside the frame. */
+int rt_render_views(rt_ctx* ctx, const rt_render_params* params,
+                    const rt_camera* cameras, const uint64_t* seeds, int32_t n_views);
+int rt_download_views(rt_ctx* ctx, int32_t total_spp, int32_t first, int32_t count,
+                      float* rgb_linear, uint8_t* rgb8);
+
 /* Deterministic primary-hit AOV for parity tests: casts the pixel-centre ray
  * ray(center, pixel00 + i*du + j*dv - center, time 0) over (0.001, inf) through
  * the same traversal/intersection code as rt_render, which decides WHICH primitive

@@ -151,6 +151,7 @@ EXPORTED_SYMBOLS = [
     "rt_set_bvh_width", "rt_device_count", "rt_shard_pixels", "rt_resolve_tiles", "rt_untile",
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
     "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
+    "rt_render_views", "rt_download_views",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
@@ -216,6 +217,8 @@ def load() -> C.CDLL:
     lib.rt_moments_download.argtypes = [vp, vp, C.c_size_t]
     lib.rt_moments_upload.argtypes = [vp, vp, C.c_size_t, i32, i32]
     lib.rt_frame_noise.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    lib.rt_render_views.argtypes = [vp, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.POINTER(C.c_uint64), i32]
+    lib.rt_download_views.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double)]
     lib.rt_measure_l1_peak.argtypes = [vp, C.POINTER(C.c_double)]
     lib.rt_probe_texture.argtypes = [vp, i32, i32, vp, vp]
@@ -256,6 +259,9 @@ def load_scenes() -> C.CDLL:
     s.rtsc_render_png.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p]
     s.rtsc_render_resumable.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_char_p,
                                         C.c_int, C.c_int, C.c_char_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    s.rtsc_render_turntable.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_int,
+                                        C.c_int, C.c_int]
+    s.rtsc_turntable_camera.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.POINTER(rt_camera)]
     s.rtsc_write_exr.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
     s.rtsc_write_pfm.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
     s.rtsc_load_obj.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_double)]
@@ -400,6 +406,44 @@ class Context:
         p.stream = stream
         self._check(self.lib.rt_render(self._h, C.byref(p)))
         self.width, self.height = width, height
+
+    def render_views(self, cameras, width: int, height: int, spp: int, max_depth: int = 50, seed: int = 1, seeds=None,
+                     spp_begin: int = 0, accumulate: bool = False, blocking: bool = True, nee: bool = False,
+                     shadowed_point_lights: bool = False, tile_size: int = 0, stream: Optional[int] = None) -> None:
+        """Render the uploaded scene from every rt_camera of `cameras` in one pass (rt_render_views), into the context's
+        views frame.  View v equals render() of the scene uploaded with cameras[v], seeded with seeds[v] (or `seed`)."""
+        cams = list(cameras)
+        arr = (rt_camera * max(1, len(cams)))(*cams)
+        seed_arr = None
+        if seeds is not None:
+            seeds = list(seeds)
+            if len(seeds) != len(cams):
+                raise ValueError(f"{len(seeds)} seeds for {len(cams)} cameras")
+            seed_arr = (C.c_uint64 * max(1, len(seeds)))(*seeds)
+        p = rt_render_params()
+        p.struct_size = C.sizeof(rt_render_params)
+        p.width, p.height, p.samples_per_pixel, p.max_depth = width, height, spp, max_depth
+        p.spp_begin, p.seed, p.tile_size = spp_begin, seed, tile_size
+        p.flags = ((RT_FLAG_ACCUMULATE if accumulate else 0) | (0 if blocking else RT_FLAG_ASYNC) | (RT_FLAG_NEE if nee else 0) |
+                   (RT_FLAG_SHADOWED_POINT_LIGHTS if shadowed_point_lights else 0))
+        p.stream = stream
+        self._check(self.lib.rt_render_views(self._h, C.byref(p), arr if cams else None, seed_arr, len(cams)))
+        self.views_shape = (len(cams), height, width)
+
+    def download_views(self, total_spp: int, first: int = 0, count: Optional[int] = None, linear: bool = True, rgb8: bool = False):
+        """Views [first, first + count) of the views frame as (count, H, W, 3) arrays: float32 radiance and / or RGB8,
+        each view laid out like download()."""
+        n, h, w = getattr(self, "views_shape", (0, 0, 0))
+        if count is None:
+            count = n - first
+        shape = (max(count, 0), h, w, 3)
+        lin = np.empty(shape, dtype=np.float32) if linear else None
+        b8 = np.empty(shape, dtype=np.uint8) if rgb8 else None
+        self._check(self.lib.rt_download_views(self._h, total_spp, first, count, lin.ctypes.data if linear else None,
+                                               b8.ctypes.data if rgb8 else None))
+        if linear and rgb8:
+            return lin, b8
+        return lin if linear else b8
 
     def sync(self) -> None:
         self._check(self.lib.rt_sync(self._h))

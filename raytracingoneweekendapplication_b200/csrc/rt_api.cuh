@@ -267,6 +267,18 @@ extern "C" int rt_render(rt_ctx* ctx, const rt_render_params* p) {
     return RT_OK;
 }
 
+// ---- multi-view batches: single-device contexts ------------------------------------------------------------------------
+extern "C" int rt_render_views(rt_ctx* ctx, const rt_render_params* params, const rt_camera* cameras, const uint64_t* seeds, int32_t n_views) {
+    RT_NEED(ctx);
+    if (ctx->dev.size() != 1) return failx(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: single-device contexts only");
+    return fwd(ctx, ctx->dev[0], dev_render_views(ctx->dev[0], params, cameras, seeds, n_views));
+}
+extern "C" int rt_download_views(rt_ctx* ctx, int32_t total_spp, int32_t first, int32_t count, float* rgb_linear, uint8_t* rgb8) {
+    RT_NEED(ctx);
+    if (ctx->dev.size() != 1) return failx(ctx, RT_ERR_UNSUPPORTED, "rt_download_views: single-device contexts only");
+    return fwd(ctx, ctx->dev[0], dev_download_views(ctx->dev[0], total_spp, first, count, rgb_linear, rgb8));
+}
+
 extern "C" int rt_join(rt_ctx* ctx, void* stream) {
     RT_NEED(ctx);
     if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], dev_join(ctx->dev[0], (cudaStream_t)stream));

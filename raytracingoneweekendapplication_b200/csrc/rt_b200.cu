@@ -2,12 +2,13 @@
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
 // Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
-//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS>
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
 //                          fixed-point accumulation.  Instances: plain / LITE / STATS for the binary
 //                          and both wide trees, NEE (binary tree), the feature instances of kInstances,
-//                          and the MOMENTS twins of plain / LITE / NEE / NEE + LITE (binary tree)
+//                          and the MOMENTS and the VIEWS (rt_render_views) twins of plain / LITE / NEE /
+//                          NEE + LITE (binary tree)
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
 //   variance_kernel, noise_kernel   sums + second moments -> per-pixel sample variance, frame noise partials
@@ -53,18 +54,21 @@ struct RenderArgs {
     int tile_stride, tile_offset;      // global tile = tile_offset + k * tile_stride
     int n_local_tiles;
     int blocks_per_tile_x, blocks_per_tile_y;  // 8x4 pixel blocks per tile
-    uint32_t moments_lo;     // MOMENTS instances: the moments buffer, its two 32-bit halves in the struct's two alignment
-                             // holes (here and after shadow_point_lights), so that no offset of a field or a kernel parameter moves
+    uint32_t side_lo;        // the side pointer, its two 32-bit halves in the struct's two alignment holes (here and after
+                             // shadow_point_lights), so that no offset of a field or a kernel parameter moves.  It serves the
+                             // instances that need it, which are never the same: MOMENTS, the moments buffer (unsigned long
+                             // long); VIEWS, the view table (ViewRecord)
     unsigned long long n_items;
     uint32_t k0, k1;
     int compact;             // RT_FLAG_COMPACT_TILES: `accum` holds only this shard's tiles, tile-major: slot = local_tile * tile_size^2 + y_in_tile * tile_size + x_in_tile
     int nee_emitters;        // NEE instance: sample the listed quad emitters (RT_FLAG_NEE)
     int shadow_point_lights; // NEE instance: shadow rays for the point lights (RT_FLAG_SHADOWED_POINT_LIGHTS)
-    uint32_t moments_hi;
-    __host__ __device__ unsigned long long* moments() const { return (unsigned long long*)(((uint64_t)moments_hi << 32) | moments_lo); }
-    void set_moments(unsigned long long* p) { moments_lo = (uint32_t)(uintptr_t)p; moments_hi = (uint32_t)((uint64_t)(uintptr_t)p >> 32); }
+    uint32_t side_hi;
+    template <class T>
+    __host__ __device__ T* side() const { return (T*)(((uint64_t)side_hi << 32) | side_lo); }
+    void set_side(const void* p) { side_lo = (uint32_t)(uintptr_t)p; side_hi = (uint32_t)((uint64_t)(uintptr_t)p >> 32); }
 };
-static_assert(sizeof(RenderArgs) == 104 && offsetof(RenderArgs, n_items) == 72, "the moments pointer fills alignment holes only");
+static_assert(sizeof(RenderArgs) == 104 && offsetof(RenderArgs, n_items) == 72, "the side pointer fills alignment holes only");
 
 constexpr float kAccumScale = 268435456.0f;  // 2^RT_ACCUM_FRAC_BITS
 constexpr float kSampleClamp = 1048576.0f;   // 2^20: keeps 2^16 saturated samples inside 64 bits
@@ -156,8 +160,12 @@ struct LocalSlot {
     }
 };
 
-// MOMENTS: also add the second moments of every finished sample to A.moments() (6 words per slot, see add_square)
-template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false>
+// MOMENTS: also add the second moments of every finished sample to A.side() (6 words per slot, see add_square)
+// VIEWS: a multi-view batch (rt_render_views).  The local tiles run over views x tiles of one view's frame, view-major
+// (item / items_per_view = tile / (tiles_x * tiles_y) is the view); each lane takes camera and Philox key from its view's
+// record in A.side() and accumulates into slot view * width * height + pixel of `accum`, kept in lane_slot like a
+// compact tile slot.  Never with STATS, MOMENTS, compact tiles or shards.
+template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false, bool VIEWS = false>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
                                                         unsigned long long* __restrict__ counters, Stats* __restrict__ gstats) {
@@ -173,7 +181,7 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     // compact tile buffers: where a lane's current sample goes.  One word of shared memory per lane, written
     // when the sample starts and read when it ends -- no register is held across the whole path for it
     __shared__ uint32_t lane_slot[RT_V2_THREADS];
-    unsigned slot_base = 0;
+    unsigned slot_base = 0;  // compact tiles: the slot of the pool's pixel block; VIEWS (never compact): the pool's view
     bool exhausted = A.max_depth <= 0;  // ray_color(depth <= 0) is black before anything is traced
 
     int state = LANE_IDLE;
@@ -221,14 +229,20 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                 const unsigned long long blk = item / (unsigned long long)A.n_segments;
                 const unsigned blocks_per_tile = (unsigned)(A.blocks_per_tile_x * A.blocks_per_tile_y);
                 const unsigned local_tile = (unsigned)(blk / blocks_per_tile), in_tile = (unsigned)(blk % blocks_per_tile);
-                const unsigned tile = A.tile_offset + local_tile * A.tile_stride;
+                unsigned tile = A.tile_offset + local_tile * A.tile_stride;
+                if constexpr (VIEWS) {
+                    const unsigned tiles_per_view = (unsigned)(A.tiles_x * A.tiles_y);
+                    slot_base = tile / tiles_per_view;
+                    tile -= slot_base * tiles_per_view;
+                }
                 blk_x0 = (int)(tile % A.tiles_x) * A.tile_size + (int)(in_tile % A.blocks_per_tile_x) * 8;
                 blk_y0 = (int)(tile / A.tiles_x) * A.tile_size + (int)(in_tile / A.blocks_per_tile_x) * 4;
                 seg_s0 = (int)seg * A.seg_len;
                 pool_size = 32u * (unsigned)min(A.seg_len, A.n_local_samples - seg_s0);
                 pool_pos = 0;
-                slot_base = (local_tile * (unsigned)A.tile_size + (in_tile / (unsigned)A.blocks_per_tile_x) * 4u) * (unsigned)A.tile_size +
-                            (in_tile % (unsigned)A.blocks_per_tile_x) * 8u;
+                if constexpr (!VIEWS)
+                    slot_base = (local_tile * (unsigned)A.tile_size + (in_tile / (unsigned)A.blocks_per_tile_x) * 4u) * (unsigned)A.tile_size +
+                                (in_tile % (unsigned)A.blocks_per_tile_x) * 8u;
             }
             const unsigned e = pool_pos + __popc(needy & lt_mask);
             if (state == LANE_IDLE && e < pool_size) {
@@ -237,7 +251,15 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                     rng.pixel = (uint32_t)(py * A.width + px);
                     rng.sample = (uint32_t)(A.spp_begin + A.sample_offset + (seg_s0 + (int)(e >> 5)) * A.sample_stride);
                     if (A.compact) lane_slot[threadIdx.x] = slot_base + ((e >> 3) & 3u) * (unsigned)A.tile_size + (e & 7u);
-                    ray = camera_ray<NO_DEFOCUS>(S, px, py, rng);
+                    if constexpr (VIEWS) {
+                        const ViewRecord& V = A.side<const ViewRecord>()[slot_base];
+                        lane_slot[threadIdx.x] = slot_base * (unsigned)(A.width * A.height) + rng.pixel;
+                        rng.k0 = V.k0;
+                        rng.k1 = V.k1;
+                        ray = camera_ray<NO_DEFOCUS>(V, px, py, rng);
+                    } else {
+                        ray = camera_ray<NO_DEFOCUS>(S, px, py, rng);
+                    }
                     radiance.store(make_float4(0, 0, 0, 0));
                     throughput.store(make_float4(1, 1, 1, 0));
                     bounce = 0;
@@ -382,13 +404,13 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                 }
             }
             if (done) {
-                unsigned long long* a = accum + 4ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel);
+                unsigned long long* a = accum + 4ull * ((VIEWS || A.compact) ? lane_slot[threadIdx.x] : rng.pixel);
                 if (isfinite(L.x) && isfinite(L.y) && isfinite(L.z)) {
                     atomicAdd(a + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
                     atomicAdd(a + 1, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
                     atomicAdd(a + 2, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
                     if constexpr (MOMENTS) {
-                        unsigned long long* m = A.moments() + 6ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel);
+                        unsigned long long* m = A.side<unsigned long long>() + 6ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel);
                         add_square(m + 0, __float2ull_rn(fminf(fmaxf(L.x, 0.0f), kSampleClamp) * kAccumScale));
                         add_square(m + 2, __float2ull_rn(fminf(fmaxf(L.y, 0.0f), kSampleClamp) * kAccumScale));
                         add_square(m + 4, __float2ull_rn(fminf(fmaxf(L.z, 0.0f), kSampleClamp) * kAccumScale));
@@ -447,6 +469,16 @@ static RenderKernel v2_moments_kernel(int variant) {
         case 3: return render_kernel_v2<false, true, true, 2, FEAT_ALL, true>;
         case 4: return render_kernel_v2<false, false, true, 2, FEAT_ALL, true>;
         default: return render_kernel_v2<false, false, false, 2, FEAT_ALL, true>;
+    }
+}
+// the multi-view (rt_render_views) instances: the same four general binary-tree variants, no per-scene views instances
+constexpr int kViewsVariant = 128;
+static RenderKernel v2_views_kernel(int variant) {
+    switch (variant) {
+        case 1: return render_kernel_v2<false, true, false, 2, FEAT_ALL, false, true>;
+        case 3: return render_kernel_v2<false, true, true, 2, FEAT_ALL, false, true>;
+        case 4: return render_kernel_v2<false, false, true, 2, FEAT_ALL, false, true>;
+        default: return render_kernel_v2<false, false, false, 2, FEAT_ALL, false, true>;
     }
 }
 
@@ -753,6 +785,7 @@ struct DevCtx {
     DevScene scene{};
     bool has_scene = false;
     bool scene_lite = false;  // no triangles, no point lights, no defocus: the LITE kernel instance applies
+    bool geom_lite = false;   // no triangles, no point lights: LITE up to the camera (rt_render_views checks its views)
     rt_camera camera{};
     // accumulation
     unsigned long long* accum = nullptr;
@@ -768,6 +801,15 @@ struct DevCtx {
     bool moments_valid = false;
     bool sums_uploaded = false;              // the frame is an rt_accum_upload, not rendered onto since (rt_moments_upload)
     unsigned long long* noise_sums = nullptr;  // rt_frame_noise: the 12 partial words of noise_kernel
+    // rt_render_views: the views frame (views_n x views_h x views_w slots of 32 B, view-major; no other call touches it),
+    // the view table on the device, and what an accumulating views pass must match: the frame's shape and a
+    // fingerprint of the cameras and seeds (views_n == 0: no views render yet)
+    unsigned long long* views_accum = nullptr;
+    size_t views_cap = 0;
+    ViewRecord* view_table = nullptr;
+    size_t view_table_cap = 0;
+    int views_n = 0, views_w = 0, views_h = 0;
+    uint64_t views_key = 0;
     unsigned char* frame_scratch = nullptr;  // full-frame copies of compact data (checkpoints, single-shard downloads)
     size_t frame_scratch_cap = 0;
     unsigned long long* counters = nullptr;  // [0] work counter, [1..3] unused
@@ -902,6 +944,7 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     cudaFuncSetAttribute(render_kernel_v2<false, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     for (int k = 0; k < kNumInstances; k++) cudaFuncSetAttribute((const void*)kInstances[k].kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     for (int v : {0, 1, 3, 4}) cudaFuncSetAttribute((const void*)v2_moments_kernel(v), cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+    for (int v : {0, 1, 3, 4}) cudaFuncSetAttribute((const void*)v2_views_kernel(v), cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     if (const char* bv = getenv("RT_B200_BVH"))
         ctx->bvh_builder = strcmp(bv, "host") == 0 ? 1 : (strcmp(bv, "device") == 0 ? 2 : (strcmp(bv, "lbvh") == 0 ? 3 : 0));
     if (const char* wv = getenv("RT_B200_BVH_WIDTH")) {
@@ -929,6 +972,8 @@ static void dev_destroy(DevCtx* ctx) {
     if (ctx->accum && !ctx->accum_external) cudaFree(ctx->accum);
     if (ctx->moments) cudaFree(ctx->moments);
     if (ctx->noise_sums) cudaFree(ctx->noise_sums);
+    if (ctx->views_accum) cudaFree(ctx->views_accum);
+    if (ctx->view_table) cudaFree(ctx->view_table);
     if (ctx->counters) cudaFree(ctx->counters);
     if (ctx->dstats) cudaFree(ctx->dstats);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
@@ -1188,9 +1233,16 @@ static uint64_t scene_key(const DevCtx* ctx, const rt_scene_desc* sc) {
     return h ? h : 1;
 }
 
-// Camera.txt:136-175 in double; stores the FP32 camera block for a width x height frame.
-static void setup_camera(DevCtx* ctx, int width, int height) {
-    const rt_camera& c = ctx->camera;
+// Camera.txt:136-175 in double for a width x height frame: the FP32 camera block the render kernels read (fields named
+// as in DevScene and ViewRecord) and the same vectors in double for the AOV.  A pure function of (camera, width,
+// height): rt_render and every view of rt_render_views get the same floats from the same operations in the same order,
+// which is what makes a view bit-identical to a single render with that camera.
+struct CameraBlock {
+    float center[3], dir00[3], du[3], dv[3], disk_u[3], disk_v[3];
+    int defocus;
+    CameraD d;
+};
+static CameraBlock camera_block(const rt_camera& c, int width, int height) {
     const double pi = 3.1415926535897932385;
     D3 lookfrom = d3(c.lookfrom), lookat = d3(c.lookat), vup = d3(c.vup);
     double theta = c.vfov * pi / 180.0;
@@ -1208,21 +1260,45 @@ static void setup_camera(DevCtx* ctx, int width, int height) {
     D3 dir00 = (-c.focus_dist) * w - 0.5 * viewport_u - 0.5 * viewport_v + 0.5 * (du + dv);
     double defocus_radius = c.focus_dist * std::tan((c.defocus_angle / 2) * pi / 180.0);
     D3 disk_u = defocus_radius * u, disk_v = defocus_radius * v;
-    DevScene& S = ctx->scene;
+    CameraBlock B;
     auto put = [](float* dst, D3 s) { dst[0] = (float)s.x; dst[1] = (float)s.y; dst[2] = (float)s.z; };
-    put(S.center, lookfrom);
-    put(S.dir00, dir00);
-    put(S.du, du);
-    put(S.dv, dv);
-    put(S.disk_u, disk_u);
-    put(S.disk_v, disk_v);
-    put(S.background, d3(c.background));
-    S.defocus = c.defocus_angle > 0 ? 1 : 0;
+    put(B.center, lookfrom);
+    put(B.dir00, dir00);
+    put(B.du, du);
+    put(B.dv, dv);
+    put(B.disk_u, disk_u);
+    put(B.disk_v, disk_v);
+    B.defocus = c.defocus_angle > 0 ? 1 : 0;
     auto putd = [](double* dst, D3 s) { dst[0] = s.x; dst[1] = s.y; dst[2] = s.z; };
-    putd(ctx->camera_d.center, lookfrom);
-    putd(ctx->camera_d.dir00, dir00);
-    putd(ctx->camera_d.du, du);
-    putd(ctx->camera_d.dv, dv);
+    putd(B.d.center, lookfrom);
+    putd(B.d.dir00, dir00);
+    putd(B.d.du, du);
+    putd(B.d.dv, dv);
+    return B;
+}
+
+// copies the camera fields of a CameraBlock into a DevScene or a ViewRecord
+template <class Cam>
+static void put_camera(Cam& dst, const CameraBlock& B) {
+    std::memcpy(dst.center, B.center, sizeof B.center);
+    std::memcpy(dst.dir00, B.dir00, sizeof B.dir00);
+    std::memcpy(dst.du, B.du, sizeof B.du);
+    std::memcpy(dst.dv, B.dv, sizeof B.dv);
+    std::memcpy(dst.disk_u, B.disk_u, sizeof B.disk_u);
+    std::memcpy(dst.disk_v, B.disk_v, sizeof B.disk_v);
+    dst.defocus = B.defocus;
+}
+
+static void put_background(DevScene& S, const rt_camera& c) {
+    for (int k = 0; k < 3; k++) S.background[k] = (float)c.background[k];
+}
+
+// the uploaded camera's block for a width x height frame, into the scene the kernels get
+static void setup_camera(DevCtx* ctx, int width, int height) {
+    const CameraBlock B = camera_block(ctx->camera, width, height);
+    put_camera(ctx->scene, B);
+    put_background(ctx->scene, ctx->camera);
+    ctx->camera_d = B.d;
     ctx->cam_w = width;
     ctx->cam_h = height;
 }
@@ -1667,7 +1743,8 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     if (!tri.empty() || world_count[PT_TRI] > 0) ctx->scene_feat |= FEAT_TRI;
     if (sc->n_lights > 0) ctx->scene_feat |= FEAT_LIGHTS;
     if (sc->camera.defocus_angle > 0) ctx->scene_feat |= FEAT_DEFOCUS;
-    ctx->scene_lite = tri.empty() && world_count[PT_TRI] == 0 && sc->n_lights == 0 && !(sc->camera.defocus_angle > 0);
+    ctx->geom_lite = tri.empty() && world_count[PT_TRI] == 0 && sc->n_lights == 0;
+    ctx->scene_lite = ctx->geom_lite && !(sc->camera.defocus_angle > 0);
     ctx->cam_w = ctx->cam_h = 0;
     ctx->has_scene = true;
     ctx->stats.bvh_nodes = n_nodes;
@@ -2030,7 +2107,8 @@ static int dev_sync(DevCtx* ctx) {
 
 // The instances of render_kernel_v2: variant 0 plain (everything), 1 LITE, 2 STATS, 3 NEE + LITE, 4 NEE; width 2, 4, 8
 // (3, 4: binary tree only).  Variants 5 + k: the binary-tree instance kInstances[k], compiled for one feature mask.
-// kMomentsVariant | v (v = 0, 1, 3, 4): the RT_FLAG_MOMENTS twin of variant v, binary tree only.
+// kMomentsVariant | v (v = 0, 1, 3, 4): the RT_FLAG_MOMENTS twin of variant v, binary tree only; kViewsVariant | v: the
+// rt_render_views twin.
 template <int WIDTH>
 static RenderKernel v2_instance(int variant) {
     switch (variant) {
@@ -2044,6 +2122,7 @@ static RenderKernel v2_instance(int variant) {
 static int v2_effective_width(int variant, int width) { return variant >= 3 ? 2 : width; }
 static RenderKernel v2_kernel(int variant, int width) {
     if (variant & kMomentsVariant) return v2_moments_kernel(variant & ~kMomentsVariant);
+    if (variant & kViewsVariant) return v2_views_kernel(variant & ~kViewsVariant);
     if (variant == 3) return render_kernel_v2<false, true, true, 2>;
     if (variant == 4) return render_kernel_v2<false, false, true, 2>;
     if (variant >= 5 && variant < 5 + kNumInstances) return kInstances[variant - 5].kernel;
@@ -2158,7 +2237,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         rc = ensure_moments(ctx, L.slots());
         if (rc != RT_OK) return rc;
     }
-    A.set_moments(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
+    A.set_side(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
     ctx->moments_valid = moments;  // an accumulating moments pass was checked above; any pass without the flag invalidates them
     ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
@@ -2268,6 +2347,142 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     ctx->pending_stats = stats;
     ctx->pending_stream = stream;
     if (async) return RT_OK;
+    return dev_wait(ctx);
+}
+
+// ---- multi-view batches (rt_render_views) ---------------------------------------------------------------------------
+// n_views cameras of the uploaded scene in one launch of a VIEWS instance, into the views frame of the context.  View v
+// runs the arithmetic of a single render with cameras[v] (camera_block, camera_ray) under the key of its seed, so it is
+// bit-identical to that render: a sample is a pure function of (scene, camera, pixel, sample index, depth, key), and the
+// sums are order-independent integers.
+static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_camera* cameras, const uint64_t* seeds, int32_t n_views) {
+    if (!ctx) return RT_ERR_INVALID;
+    if (!p || p->struct_size != sizeof(rt_render_params)) return fail(ctx, RT_ERR_INVALID, "rt_render_views: bad params struct");
+    if (!ctx->has_scene) return fail(ctx, RT_ERR_STATE, "rt_render_views: no scene uploaded");
+    if (n_views < 1 || !cameras) return fail(ctx, RT_ERR_INVALID, "rt_render_views: needs n_views >= 1 cameras (got %d%s)", n_views, cameras ? "" : ", NULL");
+    if (p->width <= 0 || p->height <= 0 || p->samples_per_pixel <= 0 || p->max_depth < 0 || p->spp_begin < 0)
+        return fail(ctx, RT_ERR_INVALID, "rt_render_views: width/height/samples must be positive");
+    const uint32_t unsupported = RT_FLAG_STATS | RT_FLAG_MOMENTS | RT_FLAG_COMPACT_TILES | RT_FLAG_OVERLAP;
+    if ((p->flags & unsupported) || p->shard_count > 1)
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP and shards are not "
+                                             "supported for multi-view batches (flags 0x%x, shard_count %d)", p->flags & unsupported, p->shard_count);
+    if ((long long)p->spp_begin + p->samples_per_pixel > 65536)
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: samples %d + %d exceed 65536 per pixel, the capacity of the 64-bit fixed-point sums",
+                    p->spp_begin, p->samples_per_pixel);
+    if ((long long)n_views * p->width * p->height >= (1ll << 31))
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: %d views of %dx%d are 2^31 slots or more", n_views, p->width, p->height);
+    const int tile_size = p->tile_size > 0 ? p->tile_size : 16;
+    if (tile_size % 8 != 0) return fail(ctx, RT_ERR_INVALID, "rt_render_views: tile_size must be a multiple of 8");
+    bool defocus = false;
+    for (int v = 0; v < n_views; v++) {
+        if (std::memcmp(cameras[v].background, ctx->camera.background, sizeof ctx->camera.background) != 0)
+            return fail(ctx, RT_ERR_INVALID, "rt_render_views: the background of camera %d differs from the uploaded camera's (the scene keeps one background)", v);
+        defocus = defocus || cameras[v].defocus_angle > 0;
+    }
+    // the views, their seeds and the frame shape: what an accumulating pass must continue
+    uint64_t key = 0x5eed5eed00000000ull ^ (uint64_t)n_views;
+    const int32_t shape[3] = {n_views, p->width, p->height};
+    key = hash_bytes(key, shape, sizeof shape);
+    key = hash_bytes(key, cameras, (size_t)n_views * sizeof(rt_camera));
+    std::vector<ViewRecord> table((size_t)n_views);
+    for (int v = 0; v < n_views; v++) {
+        const uint64_t seed = seeds ? seeds[v] : p->seed;
+        key = hash_bytes(key, &seed, sizeof seed);
+        ViewRecord& R = table[v];
+        std::memset(&R, 0, sizeof R);
+        put_camera(R, camera_block(cameras[v], p->width, p->height));
+        R.k0 = (uint32_t)(seed & 0xffffffffu);
+        R.k1 = (uint32_t)(seed >> 32);
+    }
+    const bool accumulate = (p->flags & RT_FLAG_ACCUMULATE) != 0;
+    if (accumulate && !(ctx->views_n > 0 && ctx->views_n == n_views && ctx->views_w == p->width && ctx->views_h == p->height && ctx->views_key == key))
+        return fail(ctx, RT_ERR_STATE, "rt_render_views: RT_FLAG_ACCUMULATE onto a views frame of other views, size, cameras or seeds%s",
+                    ctx->views_n > 0 ? "" : " (no views render yet)");
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
+    // a pending asynchronous render shares the work counter and the events with this one; it may also still read the table
+    int rc = dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    const size_t slots = (size_t)n_views * p->width * p->height;
+    if (!ctx->views_accum || slots * 32 > ctx->views_cap) {
+        if (ctx->views_accum) cudaFree(ctx->views_accum);
+        ctx->views_accum = nullptr;
+        ctx->views_cap = 0;
+        ctx->views_n = 0;
+        if (cudaMalloc(&ctx->views_accum, slots * 32) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate %zu bytes for the views frame", slots * 32);
+        ctx->views_cap = slots * 32;
+    }
+    if ((size_t)n_views * sizeof(ViewRecord) > ctx->view_table_cap) {
+        if (ctx->view_table) cudaFree(ctx->view_table);
+        ctx->view_table = nullptr;
+        ctx->view_table_cap = 0;
+        if (cudaMalloc(&ctx->view_table, (size_t)n_views * sizeof(ViewRecord)) != cudaSuccess)
+            return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate the table of %d views", n_views);
+        ctx->view_table_cap = (size_t)n_views * sizeof(ViewRecord);
+    }
+    // the single-frame path's background, whether or not rt_render has set up the camera since the upload
+    put_background(ctx->scene, ctx->camera);
+
+    RenderArgs A;
+    std::memset(&A, 0, sizeof A);
+    A.width = p->width;
+    A.height = p->height;
+    A.max_depth = p->max_depth;
+    A.spp_begin = p->spp_begin;
+    A.tile_size = tile_size;
+    A.tiles_x = (p->width + tile_size - 1) / tile_size;
+    A.tiles_y = (p->height + tile_size - 1) / tile_size;
+    A.blocks_per_tile_x = tile_size / 8;
+    A.blocks_per_tile_y = tile_size / 4;
+    // the local tiles are views x tiles, view-major; no shards
+    A.tile_stride = 1;
+    A.tile_offset = 0;
+    A.n_local_tiles = n_views * A.tiles_x * A.tiles_y;
+    A.sample_stride = 1;
+    A.sample_offset = 0;
+    A.n_local_samples = p->samples_per_pixel;
+    A.set_side(ctx->view_table);
+    // LITE only when no view needs the defocus code the LITE instance leaves out
+    const bool lite = ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE");
+    const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
+    const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
+    const int variant = kViewsVariant | ((want_nee || want_shadow) ? (lite ? 3 : 4) : (lite ? 1 : 0));
+    int bps = 0;
+    rc = v2_blocks_per_sm(ctx, variant, 2, &bps);
+    if (rc != RT_OK) return rc;
+    const int grid = ctx->sm_count * (bps > 0 ? bps : 1);
+    // segment length as in dev_render, over the pixel blocks of all views
+    const unsigned long long pixel_blocks = (unsigned long long)A.n_local_tiles * A.blocks_per_tile_x * A.blocks_per_tile_y;
+    const unsigned long long resident_warps = (unsigned long long)grid * (RT_V2_THREADS / 32);
+    unsigned long long want = (resident_warps * 64 + pixel_blocks - 1) / pixel_blocks;
+    if (want < 1) want = 1;
+    if (want > (unsigned long long)A.n_local_samples) want = A.n_local_samples;
+    const int n_seg = (int)want;
+    A.seg_len = (A.n_local_samples + n_seg - 1) / n_seg;
+    A.n_segments = (A.n_local_samples + A.seg_len - 1) / A.seg_len;
+    A.n_items = pixel_blocks * (unsigned long long)A.n_segments;
+    A.nee_emitters = want_nee;
+    A.shadow_point_lights = want_shadow;
+
+    CU(ctx, cudaMemcpyAsync(ctx->view_table, table.data(), table.size() * sizeof(ViewRecord), cudaMemcpyHostToDevice, stream));
+    if (!accumulate) CU(ctx, cudaMemsetAsync(ctx->views_accum, 0, slots * 32, stream));
+    CU(ctx, cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), stream));
+    CU(ctx, cudaEventRecord(ctx->ev0, stream));
+    v2_kernel(variant, 2)<<<grid, RT_V2_THREADS, 0, stream>>>(ctx->scene, A, ctx->views_accum, ctx->counters, ctx->dstats);
+    CU(ctx, cudaGetLastError());
+    CU(ctx, cudaEventRecord(ctx->ev1, stream));
+    ctx->views_n = n_views;
+    ctx->views_w = p->width;
+    ctx->views_h = p->height;
+    ctx->views_key = key;
+    ctx->stats.kernel_launches = 1;
+    ctx->stats.blocks = grid;
+    ctx->stats.samples = (uint64_t)slots * (uint64_t)p->samples_per_pixel;
+    ctx->pending_async = true;
+    ctx->pending_stats = false;
+    ctx->pending_stream = stream;
+    // `table` may go with an asynchronous pass still queued: a copy from pageable memory has been staged when it returns
+    if (p->flags & RT_FLAG_ASYNC) return RT_OK;
     return dev_wait(ctx);
 }
 
@@ -2451,6 +2666,32 @@ static int dev_download(DevCtx* ctx, int32_t total_spp, float* rgb_linear, uint8
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_download: %s", cudaGetErrorString(e));
+    return RT_OK;
+}
+
+// views [first, first + count) of the views frame, each resolved like rt_download's planes
+static int dev_download_views(DevCtx* ctx, int32_t total_spp, int32_t first, int32_t count, float* rgb_linear, uint8_t* rgb8) {
+    if (!ctx) return RT_ERR_INVALID;
+    if (ctx->views_n <= 0) return fail(ctx, RT_ERR_STATE, "rt_download_views: no views rendered yet");
+    if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_download_views: total_spp must be positive");
+    if (first < 0 || count < 1 || (long long)first + count > ctx->views_n)
+        return fail(ctx, RT_ERR_INVALID, "rt_download_views: views [%d, %d + %d) outside the frame's %d views", first, first, count, ctx->views_n);
+    int rc = dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    if (!rgb_linear && !rgb8) return RT_OK;
+    const size_t per_view = (size_t)ctx->views_w * ctx->views_h, n = per_view * count;
+    rc = ensure_out(ctx, n);
+    if (rc != RT_OK) return rc;
+    // an outstanding rt_download_begin may still be copying out of the output buffers
+    if (ctx->copy_stream) CU(ctx, cudaStreamSynchronize(ctx->copy_stream));
+    const double inv = 1.0 / ((double)kAccumScale * (double)total_spp);
+    resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->views_accum + 4 * per_view * first, (int)n, inv,
+                                                                          rgb_linear ? ctx->out_lin : nullptr, rgb8 ? ctx->out_rgb8 : nullptr);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess && rgb_linear) e = cudaMemcpyAsync(rgb_linear, ctx->out_lin, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && rgb8) e = cudaMemcpyAsync(rgb8, ctx->out_rgb8, n * 3, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_download_views: %s", cudaGetErrorString(e));
     return RT_OK;
 }
 

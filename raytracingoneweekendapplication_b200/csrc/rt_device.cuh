@@ -120,6 +120,15 @@ struct DevScene {
     int defocus;
 };
 
+// One camera of a multi-view batch (rt_render_views): the camera block of DevScene for that view's camera and frame,
+// and the Philox key of its seed.  96 B.
+struct ViewRecord {
+    float center[3], dir00[3], du[3], dv[3], disk_u[3], disk_v[3];
+    int defocus;
+    uint32_t k0, k1;
+    uint32_t pad[3];
+};
+
 struct Stats {
     unsigned long long rays, node_visits, box_tests, sphere_tests, quad_tests, tri_tests, medium_queries,
         boundary_tests, fp64_sphere, nonfinite, samples;
@@ -1191,9 +1200,11 @@ __device__ __noinline__ V3 point_lighting_shadowed(const DevScene& S, V3 p, V3 n
 
 // Camera.txt:177-200 get_ray.  Directions are built relative to the camera centre
 // (dir00 = pixel00_loc - center, evaluated in double on the host) so that FP32 keeps
-// sub-pixel accuracy when the camera sits hundreds of units from the origin.
-template <bool LITE>
-__device__ __forceinline__ Ray camera_ray(const DevScene& S, int i, int j, const Rng& rng) {
+// sub-pixel accuracy when the camera sits hundreds of units from the origin.  `Cam` is anything with the camera fields
+// of DevScene (center, dir00, du, dv, disk_u, disk_v, defocus): the scene itself, or one view of a multi-view batch,
+// so both go through the same arithmetic.
+template <bool LITE, class Cam>
+__device__ __forceinline__ Ray camera_ray(const Cam& S, int i, int j, const Rng& rng) {
     float4 u = rng.draw(0, RS_CAMERA);
     float fx = (float)i + (u.x - 0.5f), fy = (float)j + (u.y - 0.5f);
     V3 dir = fma3(fx, v3(S.du), fma3(fy, v3(S.dv), v3(S.dir00)));

@@ -1736,6 +1736,11 @@ class camera {
     int noise_check_every_spp = 256;
     std::string variance_name;
     double last_noise = 0;
+    // turntable (rt_render_views): turntable_frames > 1 renders that many views of the scene in one batch, frame k from
+    // lookfrom rotated about the axis through lookat along vup by 2 pi k / turntable_frames (turntable_camera), every
+    // frame with `seed`; frame k is written to <stem>_<k:03d><ext> and last_rgb8 holds all frames, frame-major.  Not
+    // combined with a checkpoint, a noise target, variance output or several devices.  0 or 1: off.
+    int turntable_frames = 0;
 
     int image_height() const {
         int h = int(image_width / aspect_ratio);  // Camera.txt:137-138
@@ -1747,6 +1752,33 @@ class camera {
             c.lookfrom[k] = lookfrom[k]; c.lookat[k] = lookat[k]; c.vup[k] = vup[k]; c.background[k] = background[k];
         }
         c.vfov = vfov; c.defocus_angle = defocus_angle; c.focus_dist = focus_dist;
+    }
+
+    // The rt_camera of turntable frame k (of turntable_frames), in double; frame 0 is the camera itself.
+    rt_camera turntable_camera(int k) const {
+        rt_camera c;
+        export_camera(c);
+        const int n = std::max(1, turntable_frames);
+        if (k % n == 0) return c;
+        const double pi = 3.1415926535897932385, angle = 2.0 * pi * (double)k / (double)n;
+        double a[3] = {vup[0], vup[1], vup[2]};
+        const double len = std::sqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
+        for (double& x : a) x /= len;
+        const double r[3] = {c.lookfrom[0] - c.lookat[0], c.lookfrom[1] - c.lookat[1], c.lookfrom[2] - c.lookat[2]};
+        // Rodrigues: r cos + (a x r) sin + a (a . r)(1 - cos)
+        const double cs = std::cos(angle), sn = std::sin(angle), ad = a[0] * r[0] + a[1] * r[1] + a[2] * r[2];
+        const double ax[3] = {a[1] * r[2] - a[2] * r[1], a[2] * r[0] - a[0] * r[2], a[0] * r[1] - a[1] * r[0]};
+        for (int i = 0; i < 3; i++) c.lookfrom[i] = c.lookat[i] + (r[i] * cs + ax[i] * sn + a[i] * ad * (1.0 - cs));
+        return c;
+    }
+
+    // <stem>_<k:03d><ext> of a turntable frame (the extension is what follows the last '.' of the file name)
+    static std::string frame_name(const std::string& name, int k) {
+        const size_t slash = name.find_last_of("/\\"), dot = name.find_last_of('.');
+        const bool ext = dot != std::string::npos && (slash == std::string::npos || dot > slash);
+        char num[16];
+        std::snprintf(num, sizeof num, "_%03d", k);
+        return ext ? name.substr(0, dot) + num + name.substr(dot) : name + num;
     }
 
     // Same signature as Camera.txt:54.  Fails loudly (message + exit code 2) when the
@@ -1764,8 +1796,16 @@ class camera {
             if (ctx) rt_destroy(ctx);
             std::exit(2);
         };
+        if (turntable_frames > 1 && (!checkpoint_path.empty() || noise_target > 0 || !variance_name.empty() || devs.size() > 1)) {
+            std::cerr << "rt_b200: a turntable renders on one device without a checkpoint, a noise target or variance output" << std::endl;
+            std::exit(2);
+        }
         if (rt_create(&ctx, devs.data(), (int)devs.size()) != RT_OK) fail("rt_create");
         if (rt_upload_scene(ctx, &d) != RT_OK) fail("rt_upload_scene");
+        if (turntable_frames > 1) {
+            render_turntable(ctx, fail);
+            return;
+        }
 
         rt_render_params p;
         std::memset(&p, 0, sizeof p);
@@ -1897,6 +1937,60 @@ class camera {
             bool ok = pfm ? rtb200::write_pfm(variance_name.c_str(), p.width, p.height, variance.data())
                           : rtb200::write_exr(variance_name.c_str(), p.width, p.height, variance.data());
             if (!ok) std::cerr << "rt_b200: cannot write " << variance_name << std::endl;
+        }
+    }
+
+  private:
+    // turntable_frames views of the uploaded scene in one batch (rt_render_views), progressive passes of up to 64
+    // samples like render(); frame k is bit-identical to render() with turntable_camera(k)
+    template <class Fail>
+    void render_turntable(rt_ctx* ctx, Fail& fail) {
+        const int n = turntable_frames, w = image_width, h = image_height();
+        std::vector<rt_camera> cams((size_t)n);
+        for (int k = 0; k < n; k++) cams[k] = turntable_camera(k);
+        rt_render_params p;
+        std::memset(&p, 0, sizeof p);
+        p.struct_size = sizeof p;
+        p.width = w;
+        p.height = h;
+        p.max_depth = max_depth;
+        p.seed = seed;
+        const uint32_t estimator_flags = (next_event_estimation ? RT_FLAG_NEE : 0u) | (shadowed_point_lights ? RT_FLAG_SHADOWED_POINT_LIGHTS : 0u);
+        const int target = stop_after_spp > 0 ? std::min(stop_after_spp, samples_per_pixel) : samples_per_pixel;
+        const int pass_spp = std::max(1, std::min(samples_per_pixel, 64));
+        int done = 0, passes = 0;
+        while (done < target) {
+            const int k = std::min(pass_spp, target - done);
+            p.samples_per_pixel = k;
+            p.spp_begin = done;
+            // passes after the first are enqueued without waiting; every eighth is waited for (the progress line)
+            p.flags = (done == 0 ? 0u : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC)) | estimator_flags;
+            if (rt_render_views(ctx, &p, cams.data(), nullptr, n) != RT_OK) fail("rt_render_views");
+            if (++passes % 8 == 0 && rt_sync(ctx) != RT_OK) fail("rt_sync");
+            done += k;
+            std::cerr << "\rPercent Rendered: " << (100 * done / samples_per_pixel) << "% " << std::flush;
+        }
+        last_spp_done = done;
+        last_spp_resumed = 0;
+        last_noise = 0;
+        const size_t frame = (size_t)w * h * 3;
+        last_rgb8.assign(frame * n, 0);
+        const bool want_linear = !linear_name.empty();
+        if (want_linear) last_linear.assign(frame * n, 0.0f);
+        if (done > 0 && rt_download_views(ctx, done, 0, n, want_linear ? last_linear.data() : nullptr, last_rgb8.data()) != RT_OK)
+            fail("rt_download_views");
+        rt_get_stats(ctx, &last_stats);
+        rt_destroy(ctx);
+        std::cout << "\nDone rendering " << n << " turntable frames of " << image_name << std::endl;
+        for (int k = 0; k < n; k++) {
+            if (write_image) rtb200::write_png_rgb8(frame_name(image_name, k).c_str(), w, h, last_rgb8.data() + frame * k);
+            if (want_linear) {
+                const std::string name = frame_name(linear_name, k);
+                const bool pfm = name.size() >= 4 && name.compare(name.size() - 4, 4, ".pfm") == 0;
+                bool ok = pfm ? rtb200::write_pfm(name.c_str(), w, h, last_linear.data() + frame * k)
+                              : rtb200::write_exr(name.c_str(), w, h, last_linear.data() + frame * k);
+                if (!ok) std::cerr << "rt_b200: cannot write " << name << std::endl;
+            }
         }
     }
 };

@@ -112,6 +112,40 @@ int rtsc_render_resumable(const char* name, unsigned seed, const char* asset_dir
     return 0;
 }
 
+// camera::render as a turntable of `frames` views (camera::turntable_frames, one rt_render_views batch): frame k is
+// written to <stem>_<k:03d><ext> of out_png.  nee / shadowed: the estimator flags.
+int rtsc_render_turntable(const char* name, unsigned seed, const char* asset_dir, int width, int height, int spp, int depth,
+                          const char* out_png, int frames, int nee, int shadowed) {
+    scene_config cfg;
+    if (asset_dir) cfg.asset_dir = asset_dir;
+    hittable_list world;
+    camera cam;
+    std::vector<point_light> lights;
+    if (!build_scene(name, seed, world, cam, lights, cfg)) return 1;
+    if (width > 0 && height > 0) { cam.image_width = width; cam.aspect_ratio = double(width) / double(height); }
+    if (spp > 0) cam.samples_per_pixel = spp;
+    if (depth > 0) cam.max_depth = depth;
+    cam.image_name = out_png;
+    cam.turntable_frames = frames;
+    cam.next_event_estimation = nee != 0;
+    cam.shadowed_point_lights = shadowed != 0;
+    cam.render(world, lights);
+    return 0;
+}
+
+// The rt_camera of turntable frame k of `frames` for a BASELINE scene, as camera::turntable_camera computes it.
+int rtsc_turntable_camera(const char* name, unsigned seed, const char* asset_dir, int frames, int k, rt_camera* out) {
+    scene_config cfg;
+    if (asset_dir) cfg.asset_dir = asset_dir;
+    hittable_list world;
+    camera cam;
+    std::vector<point_light> lights;
+    if (!out || !build_scene(name, seed, world, cam, lights, cfg)) return 1;
+    cam.turntable_frames = frames;
+    *out = cam.turntable_camera(k);
+    return 0;
+}
+
 // mesh::loadObj on its own (SURVEY 8f rank 2).  loader = 1 selects the reference's structure
 // (one shared_ptr<triangle> per face, mesh.h:22-121), 0 the fast path (parallel parse, one
 // triangle_soup), 2 the fast path into one indexed_mesh (rt_mesh).  with_media adds three constant_medium spheres next to the mesh and wraps the list
