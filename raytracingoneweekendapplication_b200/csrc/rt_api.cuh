@@ -230,10 +230,8 @@ extern "C" int rt_render(rt_ctx* ctx, const rt_render_params* p) {
     const int ucount = p->shard_count <= 1 ? 1 : p->shard_count, urank = ucount == 1 ? 0 : p->shard_rank;
     if (urank < 0 || urank >= ucount) return failx(ctx, RT_ERR_INVALID, "rt_render: shard_rank %d outside [0,%d)", urank, ucount);
     const int count = ucount * n;
-    const int tile = p->tile_size > 0 ? p->tile_size : 16;
-    const long long n_tiles = (long long)((p->width + tile - 1) / tile) * ((p->height + tile - 1) / tile);
-    int mode = p->shard_mode;
-    if (mode == RT_SHARD_AUTO) mode = (n_tiles / count >= 256) ? RT_SHARD_TILES : RT_SHARD_SAMPLES;
+    const int tile = tile_size_of(p);
+    const int mode = shard_mode_of(p->width, p->height, tile, count, p->shard_mode);
     if (mode != RT_SHARD_TILES && mode != RT_SHARD_SAMPLES) return failx(ctx, RT_ERR_INVALID, "rt_render: unknown shard_mode %d", p->shard_mode);
     const bool compact = mode == RT_SHARD_TILES && is_pow2(tile);
     rt_render_params q = *p;

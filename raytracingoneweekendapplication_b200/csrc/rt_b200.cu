@@ -5,10 +5,7 @@
 //   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
-//                          fixed-point accumulation.  Instances: plain / LITE / STATS for the binary
-//                          and both wide trees, NEE (binary tree), the feature instances of kInstances,
-//                          and the MOMENTS and the VIEWS (rt_render_views) twins of plain / LITE / NEE /
-//                          NEE + LITE (binary tree)
+//                          fixed-point accumulation.  Its compiled instances are the rows of kV2Instances
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
 //   variance_kernel, noise_kernel   sums + second moments -> per-pixel sample variance, frame noise partials
@@ -143,7 +140,7 @@ struct TravSel<2> { using Trav = rtdev::Trav; using RayConst = rtdev::RayConst; 
 //   FEAT_TRI / FEAT_LIGHTS / FEAT_DEFOCUS   triangles / point lights / defocus blur: what LITE = true removes together;
 //                       a LITE = false instance carries only those of the three its mask names (C1: defocus only,
 //                       C4: triangles and point lights)
-// The plain binary-tree instances are compiled for the masks of kInstances; a scene runs the first one that covers it.
+// The plain binary-tree kernel is compiled for the masks listed in kV2Instances; a scene runs the first one that covers it.
 enum : int { FEAT_MEDIA = 1, FEAT_MEDIA_GENERAL = 2, FEAT_SPECULAR = 4, FEAT_MSPHERE = 8, FEAT_TRI = 16, FEAT_LIGHTS = 32,
              FEAT_DEFOCUS = 64, FEAT_ALL = 127 };
 // One 16-byte slot of local memory per lane, moved with one vector store and one vector load.  The accesses are
@@ -444,42 +441,60 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
     }
 }
 
-// The compiled feature instances of the plain binary-tree kernel (see FEAT_* above); variant 5 + k of the dispatch below.
+// Every compiled instance of render_kernel_v2, by its template parameters.  A request runs the first entry that covers it
+// (v2_select), so the order is the preference: the per-scene feature instances of the plain binary-tree kernel (see FEAT_*
+// above), then the general ones, LITE before plain.  NEE, MOMENTS and VIEWS exist for the binary tree only (every scene
+// has one; shadow rays and paths then both go through it), and only as general instances.
 typedef void (*RenderKernel)(const DevScene, const RenderArgs, unsigned long long*, unsigned long long*, Stats*);
-struct FeatInstance {
-    bool lite;  // the scene must be LITE (no triangles, point lights, defocus) for lite = true
-    int feat;   // FEAT_* bits the instance carries
+struct V2Instance {
+    bool stats, lite, nee, moments, views;  // lite: the scene must be LITE (no triangles, point lights, defocus)
+    int width;
+    int feat;  // FEAT_* bits the instance carries
     RenderKernel kernel;
 };
-#define RT_INSTANCE(lite, feat) {lite, feat, render_kernel_v2<false, lite, false, 2, (feat)>}
-static const FeatInstance kInstances[] = {
-    RT_INSTANCE(true, 0),                                                   // C2: quads, nothing else
-    RT_INSTANCE(true, FEAT_MEDIA | FEAT_MSPHERE),                           // C5: media bounded by spheres, a moving sphere
-    RT_INSTANCE(true, FEAT_MEDIA | FEAT_MEDIA_GENERAL),                     // C3: media bounded by boxes
-    RT_INSTANCE(false, FEAT_DEFOCUS),                                       // C1: defocus blur, nothing else
-    RT_INSTANCE(false, FEAT_TRI | FEAT_LIGHTS),                             // C4: triangles and point lights
+#define RT_V2(S, L, N, M, V, W, F) {S, L, N, M, V, W, F, render_kernel_v2<S, L, N, W, F, M, V>}
+static const V2Instance kV2Instances[] = {
+    RT_V2(false, true, false, false, false, 2, 0),                                  // C2: quads, nothing else
+    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MSPHERE),          // C5: media bounded by spheres, a moving sphere
+    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MEDIA_GENERAL),    // C3: media bounded by boxes
+    RT_V2(false, false, false, false, false, 2, FEAT_DEFOCUS),                      // C1: defocus blur, nothing else
+    RT_V2(false, false, false, false, false, 2, FEAT_TRI | FEAT_LIGHTS),            // C4: triangles and point lights
+    RT_V2(false, true, false, false, false, 2, FEAT_ALL),                           // LITE
+    RT_V2(false, false, false, false, false, 2, FEAT_ALL),                          // plain
+    RT_V2(true, false, false, false, false, 2, FEAT_ALL),                           // STATS
+    RT_V2(false, true, false, false, false, 4, FEAT_ALL),
+    RT_V2(false, false, false, false, false, 4, FEAT_ALL),
+    RT_V2(true, false, false, false, false, 4, FEAT_ALL),
+    RT_V2(false, true, false, false, false, 8, FEAT_ALL),
+    RT_V2(false, false, false, false, false, 8, FEAT_ALL),
+    RT_V2(true, false, false, false, false, 8, FEAT_ALL),
+    RT_V2(false, true, true, false, false, 2, FEAT_ALL),                            // NEE + LITE
+    RT_V2(false, false, true, false, false, 2, FEAT_ALL),                           // NEE
+    RT_V2(false, true, false, true, false, 2, FEAT_ALL),                            // MOMENTS twins
+    RT_V2(false, false, false, true, false, 2, FEAT_ALL),
+    RT_V2(false, true, true, true, false, 2, FEAT_ALL),
+    RT_V2(false, false, true, true, false, 2, FEAT_ALL),
+    RT_V2(false, true, false, false, true, 2, FEAT_ALL),                            // VIEWS twins (rt_render_views)
+    RT_V2(false, false, false, false, true, 2, FEAT_ALL),
+    RT_V2(false, true, true, false, true, 2, FEAT_ALL),
+    RT_V2(false, false, true, false, true, 2, FEAT_ALL),
 };
-#undef RT_INSTANCE
-constexpr int kNumInstances = (int)(sizeof(kInstances) / sizeof(kInstances[0]));
-// the RT_FLAG_MOMENTS instances: plain, LITE, NEE + LITE, NEE (variants 0, 1, 3, 4 of the dispatch below), binary tree only
-constexpr int kMomentsVariant = 64;
-static RenderKernel v2_moments_kernel(int variant) {
-    switch (variant) {
-        case 1: return render_kernel_v2<false, true, false, 2, FEAT_ALL, true>;
-        case 3: return render_kernel_v2<false, true, true, 2, FEAT_ALL, true>;
-        case 4: return render_kernel_v2<false, false, true, 2, FEAT_ALL, true>;
-        default: return render_kernel_v2<false, false, false, 2, FEAT_ALL, true>;
-    }
-}
-// the multi-view (rt_render_views) instances: the same four general binary-tree variants, no per-scene views instances
-constexpr int kViewsVariant = 128;
-static RenderKernel v2_views_kernel(int variant) {
-    switch (variant) {
-        case 1: return render_kernel_v2<false, true, false, 2, FEAT_ALL, false, true>;
-        case 3: return render_kernel_v2<false, true, true, 2, FEAT_ALL, false, true>;
-        case 4: return render_kernel_v2<false, false, true, 2, FEAT_ALL, false, true>;
-        default: return render_kernel_v2<false, false, false, 2, FEAT_ALL, false, true>;
-    }
+#undef RT_V2
+
+// What a pass asks of the kernel: nee = NEE or shadowed point lights; lite = the scene (and every view) allows LITE;
+// width = the uploaded tree; feat = the FEAT_* bits the scene needs (FEAT_ALL: a general instance)
+struct V2Key {
+    bool stats, lite, nee, moments, views;
+    int width;
+    int feat;
+};
+static const V2Instance* v2_select(const V2Key& k) {
+    const int width = (k.nee || k.moments || k.views) ? 2 : k.width;  // binary tree only
+    for (const V2Instance& e : kV2Instances)
+        if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.width == width &&
+            (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
+            return &e;
+    return nullptr;
 }
 
 // one ray through whichever acceleration structure the scene was uploaded with (test kernels)
@@ -937,14 +952,8 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     CU(ctx, cudaMalloc(&ctx->dstats, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long)));
     // local-memory traversal stacks live in L1: prefer L1 over shared memory (the wide instances
     // get their carve-out per launch, from the depth of the uploaded tree)
-    cudaFuncSetAttribute(render_kernel_v2<false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(render_kernel_v2<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(render_kernel_v2<true, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(render_kernel_v2<false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    cudaFuncSetAttribute(render_kernel_v2<false, false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    for (int k = 0; k < kNumInstances; k++) cudaFuncSetAttribute((const void*)kInstances[k].kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    for (int v : {0, 1, 3, 4}) cudaFuncSetAttribute((const void*)v2_moments_kernel(v), cudaFuncAttributePreferredSharedMemoryCarveout, 0);
-    for (int v : {0, 1, 3, 4}) cudaFuncSetAttribute((const void*)v2_views_kernel(v), cudaFuncAttributePreferredSharedMemoryCarveout, 0);
+    for (const V2Instance& e : kV2Instances)
+        if (e.width == 2) cudaFuncSetAttribute((const void*)e.kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     if (const char* bv = getenv("RT_B200_BVH"))
         ctx->bvh_builder = strcmp(bv, "host") == 0 ? 1 : (strcmp(bv, "device") == 0 ? 2 : (strcmp(bv, "lbvh") == 0 ? 3 : 0));
     if (const char* wv = getenv("RT_B200_BVH_WIDTH")) {
@@ -2105,63 +2114,129 @@ static int dev_sync(DevCtx* ctx) {
     return RT_OK;
 }
 
-// The instances of render_kernel_v2: variant 0 plain (everything), 1 LITE, 2 STATS, 3 NEE + LITE, 4 NEE; width 2, 4, 8
-// (3, 4: binary tree only).  Variants 5 + k: the binary-tree instance kInstances[k], compiled for one feature mask.
-// kMomentsVariant | v (v = 0, 1, 3, 4): the RT_FLAG_MOMENTS twin of variant v, binary tree only; kViewsVariant | v: the
-// rt_render_views twin.
-template <int WIDTH>
-static RenderKernel v2_instance(int variant) {
-    switch (variant) {
-        case 1: return render_kernel_v2<false, true, false, WIDTH>;
-        case 2: return render_kernel_v2<true, false, false, WIDTH>;
-        default: return render_kernel_v2<false, false, false, WIDTH>;
-    }
-}
-// the opt-in NEE instances exist for the binary tree only (every scene has one; shadow rays and paths
-// then both go through it): two fat kernels less per width in the shipped library
-static int v2_effective_width(int variant, int width) { return variant >= 3 ? 2 : width; }
-static RenderKernel v2_kernel(int variant, int width) {
-    if (variant & kMomentsVariant) return v2_moments_kernel(variant & ~kMomentsVariant);
-    if (variant & kViewsVariant) return v2_views_kernel(variant & ~kViewsVariant);
-    if (variant == 3) return render_kernel_v2<false, true, true, 2>;
-    if (variant == 4) return render_kernel_v2<false, false, true, 2>;
-    if (variant >= 5 && variant < 5 + kNumInstances) return kInstances[variant - 5].kernel;
-    return width == 8 ? v2_instance<8>(variant) : (width == 4 ? v2_instance<4>(variant) : v2_instance<2>(variant));
-}
 // dynamic shared memory of a wide instance: the traversal stacks, [entry][thread]
 static size_t v2_smem(const DevCtx* ctx, int width) { return width <= 2 ? 0 : (size_t)std::max(ctx->wide_depth, 1) * RT_V2_THREADS * sizeof(uint2); }
 
-// blocks per SM the kernel instance runs with (the grid is persistent: SMs x this)
-static int v2_blocks_per_sm(DevCtx* ctx, int variant, int width, int* out) {
-    width = v2_effective_width(variant, width);
-    RenderKernel k = v2_kernel(variant, width);
-    const size_t smem = v2_smem(ctx, width);
+// the persistent grid of the instance: SMs x the blocks per SM it runs with
+static int v2_grid(DevCtx* ctx, const V2Instance* e, int* grid) {
+    if (!e) return fail(ctx, RT_ERR_UNSUPPORTED, "no compiled instance of render_kernel_v2 for this pass");
+    const size_t smem = v2_smem(ctx, e->width);
     if (smem) {
         // carve out what RT_MIN_BLOCKS blocks need (plus the 1 KB the system reserves per block), the rest stays L1
         const int pct = (int)std::min<size_t>(100, (100 * RT_WIDE_MIN_BLOCKS * (smem + 1024) + 233471) / 233472);
-        CU(ctx, cudaFuncSetAttribute((const void*)k, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
+        CU(ctx, cudaFuncSetAttribute((const void*)e->kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
     }
-    CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(out, (const void*)k, RT_V2_THREADS, smem));
+    int bps = 0;
+    CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void*)e->kernel, RT_V2_THREADS, smem));
+    *grid = ctx->sm_count * (bps > 0 ? bps : 1);
     return RT_OK;
 }
 
-static int launch_v2(DevCtx* ctx, int variant, int width, int grid, const RenderArgs& A, cudaStream_t stream, unsigned long long* counters = nullptr) {
-    if (!counters) counters = ctx->counters;
-    width = v2_effective_width(variant, width);
-    v2_kernel(variant, width)<<<grid, RT_V2_THREADS, v2_smem(ctx, width), stream>>>(ctx->scene, A, ctx->accum, counters, ctx->dstats);
+static int launch_v2(DevCtx* ctx, const V2Instance& e, int grid, const RenderArgs& A, unsigned long long* accum,
+                     unsigned long long* counters, cudaStream_t stream) {
+    e.kernel<<<grid, RT_V2_THREADS, v2_smem(ctx, e.width), stream>>>(ctx->scene, A, accum, counters, ctx->dstats);
+    CU(ctx, cudaGetLastError());
     return RT_OK;
+}
+
+// the checks of rt_render_params that rt_render and rt_render_views share; `entry` names the entry point in the messages
+static int check_render_params(DevCtx* ctx, const rt_render_params* p, const char* entry) {
+    if (!p || p->struct_size != sizeof(rt_render_params)) return fail(ctx, RT_ERR_INVALID, "%s: bad params struct", entry);
+    if (!ctx->has_scene) return fail(ctx, RT_ERR_STATE, "%s: no scene uploaded", entry);
+    if (p->width <= 0 || p->height <= 0 || p->samples_per_pixel <= 0 || p->max_depth < 0 || p->spp_begin < 0)
+        return fail(ctx, RT_ERR_INVALID, "%s: width/height/samples must be positive", entry);
+    // a sample is clamped to 2^20 (kSampleClamp) and stored in 2^-28 units: 2^16 saturated samples fill a 64-bit sum
+    if ((long long)p->spp_begin + p->samples_per_pixel > 65536)
+        return fail(ctx, RT_ERR_UNSUPPORTED, "%s: samples %d + %d exceed 65536 per pixel, the capacity of the 64-bit fixed-point sums",
+                    entry, p->spp_begin, p->samples_per_pixel);
+    if (p->tile_size > 0 && p->tile_size % 8 != 0) return fail(ctx, RT_ERR_INVALID, "%s: tile_size must be a multiple of 8", entry);
+    return RT_OK;
+}
+
+static int tile_size_of(const rt_render_params* p) { return p->tile_size > 0 ? p->tile_size : 16; }
+
+// The shard mode a render of `count` shards runs: a single shard renders all tiles; RT_SHARD_AUTO shards tiles when every
+// shard gets 256 or more of them, samples otherwise (sharding.py plans the same).  Any other mode is returned as given.
+static int shard_mode_of(int width, int height, int tile, int count, int mode) {
+    if (count == 1) return RT_SHARD_TILES;
+    if (mode != RT_SHARD_AUTO) return mode;
+    const long long n_tiles = (long long)((width + tile - 1) / tile) * ((height + tile - 1) / tile);
+    return n_tiles / count >= 256 ? RT_SHARD_TILES : RT_SHARD_SAMPLES;
+}
+
+// The geometry of a pass: the tiles of the frame, the tiles or samples of shard `rank` of `count` (mode RT_SHARD_TILES or
+// RT_SHARD_SAMPLES), and the (pixel block, sample segment) work items for a grid of `grid` blocks.  A batch of n_views
+// frames (rt_render_views) is one shard whose local tiles are views x tiles, view-major.
+static void plan_pass(RenderArgs& A, const rt_render_params* p, int mode, int rank, int count, int n_views, int grid) {
+    std::memset(&A, 0, sizeof A);
+    A.width = p->width;
+    A.height = p->height;
+    A.max_depth = p->max_depth;
+    A.spp_begin = p->spp_begin;
+    A.tile_size = tile_size_of(p);
+    A.tiles_x = (p->width + A.tile_size - 1) / A.tile_size;
+    A.tiles_y = (p->height + A.tile_size - 1) / A.tile_size;
+    A.blocks_per_tile_x = A.tile_size / 8;
+    A.blocks_per_tile_y = A.tile_size / 4;
+    const int n_tiles = n_views * A.tiles_x * A.tiles_y;
+    if (mode == RT_SHARD_TILES) {
+        A.tile_stride = count;
+        A.tile_offset = rank;
+        A.n_local_tiles = (n_tiles - rank + count - 1) / count;
+        A.sample_stride = 1;
+        A.sample_offset = 0;
+        A.n_local_samples = p->samples_per_pixel;
+    } else {
+        A.tile_stride = 1;
+        A.tile_offset = 0;
+        A.n_local_tiles = n_tiles;
+        A.sample_stride = count;
+        A.sample_offset = rank;
+        A.n_local_samples = (p->samples_per_pixel - rank + count - 1) / count;  // 0 for a shard past the last sample
+    }
+    // segment length: enough work items to keep every resident warp busy ~64 times over,
+    // but never shorter than 1 sample (fixed-point sums make the split result-neutral)
+    const unsigned long long pixel_blocks = (unsigned long long)A.n_local_tiles * A.blocks_per_tile_x * A.blocks_per_tile_y;
+    const unsigned long long resident_warps = (unsigned long long)grid * (RT_V2_THREADS / 32);
+    int n_seg = 1;
+    if (A.n_local_samples > 0 && pixel_blocks > 0) {
+        // >= 64 items per resident warp: the end-of-kernel tail is one item long
+        unsigned long long want = (resident_warps * 64 + pixel_blocks - 1) / pixel_blocks;
+        if (want < 1) want = 1;
+        if (want > (unsigned long long)A.n_local_samples) want = A.n_local_samples;
+        n_seg = (int)want;
+    }
+    A.seg_len = A.n_local_samples > 0 ? (A.n_local_samples + n_seg - 1) / n_seg : 1;
+    A.n_segments = A.n_local_samples > 0 ? (A.n_local_samples + A.seg_len - 1) / A.seg_len : 0;
+    A.n_items = pixel_blocks * (unsigned long long)A.n_segments;
+}
+
+// The tail of a pass on `stream`, after the caller has queued its clears: reset the work counter, launch between ev0 and
+// ev1 (nothing to launch for a shard without samples), account the pass and leave it pending, or wait for it
+static int enqueue_pass(DevCtx* ctx, const V2Instance& e, int grid, const RenderArgs& A, unsigned long long* accum,
+                        cudaStream_t stream, uint64_t samples, bool stats, bool async) {
+    CU(ctx, cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), stream));
+    CU(ctx, cudaEventRecord(ctx->ev0, stream));
+    ctx->stats.kernel_launches = 0;
+    if (A.n_items > 0) {
+        int rc = launch_v2(ctx, e, grid, A, accum, ctx->counters, stream);
+        if (rc != RT_OK) return rc;
+        ctx->stats.kernel_launches = 1;
+    }
+    ctx->stats.blocks = grid;
+    ctx->stats.samples = samples;
+    CU(ctx, cudaEventRecord(ctx->ev1, stream));
+    ctx->pending_async = true;
+    ctx->pending_stats = stats;
+    ctx->pending_stream = stream;
+    if (async) return RT_OK;
+    return dev_wait(ctx);
 }
 
 static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     if (!ctx) return RT_ERR_INVALID;
-    if (!p || p->struct_size != sizeof(rt_render_params)) return fail(ctx, RT_ERR_INVALID, "rt_render: bad params struct");
-    if (!ctx->has_scene) return fail(ctx, RT_ERR_STATE, "rt_render: no scene uploaded");
-    if (p->width <= 0 || p->height <= 0 || p->samples_per_pixel <= 0 || p->max_depth < 0 || p->spp_begin < 0)
-        return fail(ctx, RT_ERR_INVALID, "rt_render: width/height/samples must be positive");
-    // a sample is clamped to 2^20 (kSampleClamp) and stored in 2^-28 units: 2^16 saturated samples fill a 64-bit sum
-    if ((long long)p->spp_begin + p->samples_per_pixel > 65536)
-        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: samples %d + %d exceed 65536 per pixel, the capacity of the 64-bit fixed-point sums",
-                    p->spp_begin, p->samples_per_pixel);
+    int rc = check_render_params(ctx, p, "rt_render");
+    if (rc != RT_OK) return rc;
     if ((long long)p->width * p->height >= (1ll << 31)) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: frame too large");
     const int count = p->shard_count <= 1 ? 1 : p->shard_count;
     const int rank = count == 1 ? 0 : p->shard_rank;
@@ -2181,43 +2256,12 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
                          ctx->cam_w == p->width && ctx->cam_h == p->height;
     // a pending asynchronous render (possibly on another stream) shares the work counter, the guard flags and the
     // stats block with this one: finish it first
-    int rc = overlap ? RT_OK : dev_wait(ctx);
+    rc = overlap ? RT_OK : dev_wait(ctx);
     if (rc != RT_OK) return rc;
     if (ctx->cam_w != p->width || ctx->cam_h != p->height) setup_camera(ctx, p->width, p->height);
 
-    RenderArgs A;
-    std::memset(&A, 0, sizeof A);
-    A.width = p->width;
-    A.height = p->height;
-    A.max_depth = p->max_depth;
-    A.spp_begin = p->spp_begin;
-    A.tile_size = p->tile_size > 0 ? p->tile_size : 16;
-    if (A.tile_size % 8 != 0) return fail(ctx, RT_ERR_INVALID, "rt_render: tile_size must be a multiple of 8");
-    A.tiles_x = (p->width + A.tile_size - 1) / A.tile_size;
-    A.tiles_y = (p->height + A.tile_size - 1) / A.tile_size;
-    A.blocks_per_tile_x = A.tile_size / 8;
-    A.blocks_per_tile_y = A.tile_size / 4;
-    const int n_tiles = A.tiles_x * A.tiles_y;
-    int mode = p->shard_mode;
-    if (mode == RT_SHARD_AUTO) mode = (n_tiles / count >= 256) ? RT_SHARD_TILES : RT_SHARD_SAMPLES;
-    if (count == 1) mode = RT_SHARD_TILES;
-    if (mode == RT_SHARD_TILES) {
-        A.tile_stride = count;
-        A.tile_offset = rank;
-        A.n_local_tiles = (n_tiles - rank + count - 1) / count;
-        A.sample_stride = 1;
-        A.sample_offset = 0;
-        A.n_local_samples = p->samples_per_pixel;
-    } else if (mode == RT_SHARD_SAMPLES) {
-        A.tile_stride = 1;
-        A.tile_offset = 0;
-        A.n_local_tiles = n_tiles;
-        A.sample_stride = count;
-        A.sample_offset = rank;
-        A.n_local_samples = (p->samples_per_pixel - rank + count - 1) / count;
-    } else {
-        return fail(ctx, RT_ERR_INVALID, "rt_render: unknown shard_mode %d", p->shard_mode);
-    }
+    const int mode = shard_mode_of(p->width, p->height, tile_size_of(p), count, p->shard_mode);
+    if (mode != RT_SHARD_TILES && mode != RT_SHARD_SAMPLES) return fail(ctx, RT_ERR_INVALID, "rt_render: unknown shard_mode %d", p->shard_mode);
     AccumLayout L;
     L.width = p->width;
     L.height = p->height;
@@ -2226,8 +2270,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         L.compact = true;
         L.rank = rank;
         L.count = count;
-        L.tile = A.tile_size;
-        A.compact = 1;
+        L.tile = tile_size_of(p);
     }
     if ((p->flags & RT_FLAG_ACCUMULATE) && ctx->accum && !(ctx->acc == L))
         return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE onto a buffer of another frame size or tile layout");
@@ -2237,43 +2280,26 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         rc = ensure_moments(ctx, L.slots());
         if (rc != RT_OK) return rc;
     }
-    A.set_side(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
     ctx->moments_valid = moments;  // an accumulating moments pass was checked above; any pass without the flag invalidates them
     ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
-    // which instance of render_kernel_v2 runs: LITE = no triangles, no point lights, no defocus blur in this scene (see hit_prim)
-    const bool lite = ctx->scene_lite && !getenv("RT_B200_NO_LITE");
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
-    int variant = (want_nee || want_shadow) ? (lite ? 3 : 4) : (stats ? 2 : (lite ? 1 : 0));
-    if (moments) variant |= kMomentsVariant;  // the general binary-tree twins: no per-scene moments instances
-    const int width = ctx->scene.wide_width ? ctx->scene.wide_width : 2;
-    // the first compiled instance that covers the scene's features (RT_B200_GENERAL_INSTANCE=1: always a general one)
-    if (variant <= 1 && width == 2 && !getenv("RT_B200_GENERAL_INSTANCE"))
-        for (int k = 0; k < kNumInstances; k++)
-            if ((!kInstances[k].lite || lite) && (ctx->scene_feat & ~kInstances[k].feat) == 0) {
-                variant = 5 + k;
-                break;
-            }
-    int bps = 0;
-    rc = v2_blocks_per_sm(ctx, variant, width, &bps);
+    // which instance of render_kernel_v2 runs: LITE = no triangles, no point lights, no defocus blur in this scene (see
+    // hit_prim); the NEE instances count no STATS; the first per-scene instance that covers the scene's features, unless
+    // RT_B200_GENERAL_INSTANCE=1 asks for a general one
+    const V2Key req{stats && !(want_nee || want_shadow), ctx->scene_lite && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, moments,
+                    false, ctx->scene.wide_width ? ctx->scene.wide_width : 2, getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
+    const V2Instance* e = v2_select(req);
+    int grid = 0;
+    rc = v2_grid(ctx, e, &grid);
     if (rc != RT_OK) return rc;
-    const int grid = ctx->sm_count * (bps > 0 ? bps : 1);
-    // segment length: enough work items to keep every resident warp busy ~64 times over,
-    // but never shorter than 1 sample (fixed-point sums make the split result-neutral)
-    const unsigned long long pixel_blocks = (unsigned long long)A.n_local_tiles * A.blocks_per_tile_x * A.blocks_per_tile_y;
-    const unsigned long long resident_warps = (unsigned long long)grid * (RT_V2_THREADS / 32);
-    int n_seg = 1;
-    if (A.n_local_samples > 0 && pixel_blocks > 0) {
-        // >= 64 items per resident warp: the end-of-kernel tail is one item long
-        unsigned long long want = (resident_warps * 64 + pixel_blocks - 1) / pixel_blocks;
-        if (want < 1) want = 1;
-        if (want > (unsigned long long)A.n_local_samples) want = A.n_local_samples;
-        n_seg = (int)want;
-    }
-    A.seg_len = A.n_local_samples > 0 ? (A.n_local_samples + n_seg - 1) / n_seg : 1;
-    A.n_segments = A.n_local_samples > 0 ? (A.n_local_samples + A.seg_len - 1) / A.seg_len : 0;
-    A.n_items = pixel_blocks * (unsigned long long)A.n_segments;
+    RenderArgs A;
+    plan_pass(A, p, mode, rank, count, 1, grid);
+    A.compact = L.compact;
+    A.set_side(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
+    A.nee_emitters = want_nee;
+    A.shadow_point_lights = want_shadow;
     A.k0 = (uint32_t)(p->seed & 0xffffffffu);
     A.k1 = (uint32_t)(p->seed >> 32);
 
@@ -2281,7 +2307,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     auto pass_samples = [&]() -> uint64_t {
         if (!(mode == RT_SHARD_TILES && count > 1)) return (uint64_t)A.n_local_samples * (uint64_t)p->width * p->height;
         uint64_t px = 0;
-        for (int t = rank; t < n_tiles; t += count) {
+        for (int t = rank; t < A.tiles_x * A.tiles_y; t += count) {
             int tx = t % A.tiles_x, ty = t / A.tiles_x;
             int w = std::min(A.tile_size, p->width - tx * A.tile_size), h = std::min(A.tile_size, p->height - ty * A.tile_size);
             px += (uint64_t)w * h;
@@ -2311,11 +2337,8 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         }
         CU(ctx, cudaMemsetAsync(cnt, 0, 4 * sizeof(unsigned long long), ls));
         if (A.n_items > 0) {
-            A.nee_emitters = want_nee;
-            A.shadow_point_lights = want_shadow;
-            rc = launch_v2(ctx, variant, width, grid, A, ls, cnt);
+            rc = launch_v2(ctx, *e, grid, A, ctx->accum, cnt, ls);
             if (rc != RT_OK) return rc;
-            CU(ctx, cudaGetLastError());
         }
         CU(ctx, cudaEventRecord(ctx->lane_end[k], ls));
         ctx->lane_busy[k] = true;
@@ -2327,27 +2350,8 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     }
     if (!(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->accum, 0, L.slots() * 32, stream));
     if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->moments, 0, L.slots() * 48, stream));
-    CU(ctx, cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), stream));
     if (stats) CU(ctx, cudaMemsetAsync(ctx->dstats, 0, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long), stream));
-    const bool async = (p->flags & RT_FLAG_ASYNC) != 0;
-    CU(ctx, cudaEventRecord(ctx->ev0, stream));
-    ctx->stats.kernel_launches = 0;
-    if (A.n_items > 0) {
-        A.nee_emitters = want_nee;
-        A.shadow_point_lights = want_shadow;
-        rc = launch_v2(ctx, variant, width, grid, A, stream);
-        if (rc != RT_OK) return rc;
-        CU(ctx, cudaGetLastError());
-        ctx->stats.kernel_launches = 1;
-    }
-    ctx->stats.blocks = grid;
-    ctx->stats.samples = pass_samples();
-    CU(ctx, cudaEventRecord(ctx->ev1, stream));
-    ctx->pending_async = true;
-    ctx->pending_stats = stats;
-    ctx->pending_stream = stream;
-    if (async) return RT_OK;
-    return dev_wait(ctx);
+    return enqueue_pass(ctx, *e, grid, A, ctx->accum, stream, pass_samples(), stats, (p->flags & RT_FLAG_ASYNC) != 0);
 }
 
 // ---- multi-view batches (rt_render_views) ---------------------------------------------------------------------------
@@ -2357,22 +2361,15 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
 // sums are order-independent integers.
 static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_camera* cameras, const uint64_t* seeds, int32_t n_views) {
     if (!ctx) return RT_ERR_INVALID;
-    if (!p || p->struct_size != sizeof(rt_render_params)) return fail(ctx, RT_ERR_INVALID, "rt_render_views: bad params struct");
-    if (!ctx->has_scene) return fail(ctx, RT_ERR_STATE, "rt_render_views: no scene uploaded");
+    int rc = check_render_params(ctx, p, "rt_render_views");
+    if (rc != RT_OK) return rc;
     if (n_views < 1 || !cameras) return fail(ctx, RT_ERR_INVALID, "rt_render_views: needs n_views >= 1 cameras (got %d%s)", n_views, cameras ? "" : ", NULL");
-    if (p->width <= 0 || p->height <= 0 || p->samples_per_pixel <= 0 || p->max_depth < 0 || p->spp_begin < 0)
-        return fail(ctx, RT_ERR_INVALID, "rt_render_views: width/height/samples must be positive");
     const uint32_t unsupported = RT_FLAG_STATS | RT_FLAG_MOMENTS | RT_FLAG_COMPACT_TILES | RT_FLAG_OVERLAP;
     if ((p->flags & unsupported) || p->shard_count > 1)
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP and shards are not "
                                              "supported for multi-view batches (flags 0x%x, shard_count %d)", p->flags & unsupported, p->shard_count);
-    if ((long long)p->spp_begin + p->samples_per_pixel > 65536)
-        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: samples %d + %d exceed 65536 per pixel, the capacity of the 64-bit fixed-point sums",
-                    p->spp_begin, p->samples_per_pixel);
     if ((long long)n_views * p->width * p->height >= (1ll << 31))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: %d views of %dx%d are 2^31 slots or more", n_views, p->width, p->height);
-    const int tile_size = p->tile_size > 0 ? p->tile_size : 16;
-    if (tile_size % 8 != 0) return fail(ctx, RT_ERR_INVALID, "rt_render_views: tile_size must be a multiple of 8");
     bool defocus = false;
     for (int v = 0; v < n_views; v++) {
         if (std::memcmp(cameras[v].background, ctx->camera.background, sizeof ctx->camera.background) != 0)
@@ -2401,7 +2398,7 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
     // a pending asynchronous render shares the work counter and the events with this one; it may also still read the table
-    int rc = dev_wait(ctx);
+    rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
     const size_t slots = (size_t)n_views * p->width * p->height;
     if (!ctx->views_accum || slots * 32 > ctx->views_cap) {
@@ -2423,67 +2420,29 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     // the single-frame path's background, whether or not rt_render has set up the camera since the upload
     put_background(ctx->scene, ctx->camera);
 
-    RenderArgs A;
-    std::memset(&A, 0, sizeof A);
-    A.width = p->width;
-    A.height = p->height;
-    A.max_depth = p->max_depth;
-    A.spp_begin = p->spp_begin;
-    A.tile_size = tile_size;
-    A.tiles_x = (p->width + tile_size - 1) / tile_size;
-    A.tiles_y = (p->height + tile_size - 1) / tile_size;
-    A.blocks_per_tile_x = tile_size / 8;
-    A.blocks_per_tile_y = tile_size / 4;
-    // the local tiles are views x tiles, view-major; no shards
-    A.tile_stride = 1;
-    A.tile_offset = 0;
-    A.n_local_tiles = n_views * A.tiles_x * A.tiles_y;
-    A.sample_stride = 1;
-    A.sample_offset = 0;
-    A.n_local_samples = p->samples_per_pixel;
-    A.set_side(ctx->view_table);
-    // LITE only when no view needs the defocus code the LITE instance leaves out
-    const bool lite = ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE");
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
-    const int variant = kViewsVariant | ((want_nee || want_shadow) ? (lite ? 3 : 4) : (lite ? 1 : 0));
-    int bps = 0;
-    rc = v2_blocks_per_sm(ctx, variant, 2, &bps);
+    // LITE only when no view needs the defocus code the LITE instance leaves out
+    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, 2, FEAT_ALL};
+    const V2Instance* e = v2_select(req);
+    int grid = 0;
+    rc = v2_grid(ctx, e, &grid);
     if (rc != RT_OK) return rc;
-    const int grid = ctx->sm_count * (bps > 0 ? bps : 1);
-    // segment length as in dev_render, over the pixel blocks of all views
-    const unsigned long long pixel_blocks = (unsigned long long)A.n_local_tiles * A.blocks_per_tile_x * A.blocks_per_tile_y;
-    const unsigned long long resident_warps = (unsigned long long)grid * (RT_V2_THREADS / 32);
-    unsigned long long want = (resident_warps * 64 + pixel_blocks - 1) / pixel_blocks;
-    if (want < 1) want = 1;
-    if (want > (unsigned long long)A.n_local_samples) want = A.n_local_samples;
-    const int n_seg = (int)want;
-    A.seg_len = (A.n_local_samples + n_seg - 1) / n_seg;
-    A.n_segments = (A.n_local_samples + A.seg_len - 1) / A.seg_len;
-    A.n_items = pixel_blocks * (unsigned long long)A.n_segments;
+    RenderArgs A;
+    plan_pass(A, p, RT_SHARD_TILES, 0, 1, n_views, grid);
+    A.set_side(ctx->view_table);
     A.nee_emitters = want_nee;
     A.shadow_point_lights = want_shadow;
 
     CU(ctx, cudaMemcpyAsync(ctx->view_table, table.data(), table.size() * sizeof(ViewRecord), cudaMemcpyHostToDevice, stream));
     if (!accumulate) CU(ctx, cudaMemsetAsync(ctx->views_accum, 0, slots * 32, stream));
-    CU(ctx, cudaMemsetAsync(ctx->counters, 0, 4 * sizeof(unsigned long long), stream));
-    CU(ctx, cudaEventRecord(ctx->ev0, stream));
-    v2_kernel(variant, 2)<<<grid, RT_V2_THREADS, 0, stream>>>(ctx->scene, A, ctx->views_accum, ctx->counters, ctx->dstats);
-    CU(ctx, cudaGetLastError());
-    CU(ctx, cudaEventRecord(ctx->ev1, stream));
     ctx->views_n = n_views;
     ctx->views_w = p->width;
     ctx->views_h = p->height;
     ctx->views_key = key;
-    ctx->stats.kernel_launches = 1;
-    ctx->stats.blocks = grid;
-    ctx->stats.samples = (uint64_t)slots * (uint64_t)p->samples_per_pixel;
-    ctx->pending_async = true;
-    ctx->pending_stats = false;
-    ctx->pending_stream = stream;
     // `table` may go with an asynchronous pass still queued: a copy from pageable memory has been staged when it returns
-    if (p->flags & RT_FLAG_ASYNC) return RT_OK;
-    return dev_wait(ctx);
+    return enqueue_pass(ctx, *e, grid, A, ctx->views_accum, stream, (uint64_t)slots * (uint64_t)p->samples_per_pixel, false,
+                        (p->flags & RT_FLAG_ASYNC) != 0);
 }
 
 // resolve_kernel over the slots of the accumulation buffer (full frame or compact tiles) into DEVICE buffers
