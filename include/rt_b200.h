@@ -497,7 +497,9 @@ int rt_untile(rt_ctx* ctx, const void* dev_shards, size_t shard_stride_bytes, in
  *   rt_untile_begin    like rt_untile (bytes_per_pixel 3 or 12), same hand-out
  *   rt_frame_end       waits for the OLDEST outstanding begin and returns pointers into the context's pinned
  *                      buffer (NULL for a plane that was not asked for), valid until two more begins; at most two
- *                      frames may be outstanding */
+ *                      frames may be outstanding
+ * Synchronous readbacks (rt_download, rt_download_variance, rt_accum_download, ...) issued while a frame is outstanding
+ * are ordered after its copy, so rt_frame_end returns the frame as it was at its begin. */
 int rt_download_begin(rt_ctx* ctx, int32_t total_spp, int32_t want_linear, int32_t want_rgb8);
 int rt_untile_begin(rt_ctx* ctx, const void* dev_shards, size_t shard_stride_bytes, int32_t bytes_per_pixel, int32_t shard_count,
                     int32_t width, int32_t height, int32_t tile_size);

@@ -350,6 +350,38 @@ static int gather_to_dev0(rt_ctx* ctx, const std::vector<const void*>& src, cons
     return RT_OK;
 }
 
+// Every pixel of the frame lives on one device: tile shards of this context only, no restored checkpoint to add
+static bool one_device_per_pixel(const rt_ctx* ctx) {
+    return ctx->dev[0]->acc.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size();
+}
+
+// What a device contributes to a gather: its raw sums, or its slots resolved or turned into variance on the device
+enum class Plane { Sums, Rgb8, Linear, Variance };
+
+// The plane of every device's slots, produced on that device and gathered on device 0 (device d at ctx->gather + d * *stride)
+static int gather_plane(rt_ctx* ctx, Plane what, int32_t total_spp, size_t* stride) {
+    const int n = (int)ctx->dev.size();
+    const size_t bpp = what == Plane::Sums ? 32 : what == Plane::Rgb8 ? 3 : 12;
+    const bool resolve = what == Plane::Rgb8 || what == Plane::Linear;
+    std::vector<const void*> src((size_t)n);
+    std::vector<size_t> bytes((size_t)n);
+    *stride = 0;
+    for (int d = 0; d < n; d++) {
+        DevCtx* dc = ctx->dev[d];
+        const size_t slots = dc->acc.slots();
+        int rc = what == Plane::Variance ? moments_ready(dc, "rt_download_variance") : dev_wait(dc);
+        if (rc == RT_OK && what == Plane::Variance) rc = dev_variance_into(dc, total_spp);
+        if (rc == RT_OK && resolve) rc = stage_buffers(dc, slots, 0);
+        if (rc == RT_OK && resolve)
+            rc = dev_resolve_into(dc, dc->accum, slots, total_spp, what == Plane::Linear ? dc->out_lin : nullptr, what == Plane::Rgb8 ? dc->out_rgb8 : nullptr);
+        if (rc != RT_OK) return fwd(ctx, dc, rc);
+        src[d] = what == Plane::Sums ? (const void*)dc->accum : what == Plane::Rgb8 ? (const void*)dc->out_rgb8 : (const void*)dc->out_lin;
+        bytes[d] = slots * bpp;
+        *stride = std::max(*stride, (bytes[d] + 255) & ~(size_t)255);
+    }
+    return gather_to_dev0(ctx, src, bytes, *stride);
+}
+
 // The sums of all devices as ONE full row-major frame on device 0 (in d0->frame_scratch): compact tiles are
 // gathered and scattered, sample-sharded full frames are added; a restored checkpoint is added on top.
 static int gather_sums_full(rt_ctx* ctx) {
@@ -357,22 +389,11 @@ static int gather_sums_full(rt_ctx* ctx) {
     DevCtx* d0 = ctx->dev[0];
     const int w = ctx->last.width, h = ctx->last.height;
     const size_t full = (size_t)w * h * 32;
-    for (int d = 0; d < n; d++) {
-        int rc = dev_wait(ctx->dev[d]);
-        if (rc != RT_OK) return fwd(ctx, ctx->dev[d], rc);
-    }
-    std::vector<const void*> src((size_t)n);
-    std::vector<size_t> bytes((size_t)n);
     size_t stride = 0;
-    for (int d = 0; d < n; d++) {
-        src[d] = ctx->dev[d]->accum;
-        bytes[d] = ctx->dev[d]->acc.slots() * 32;
-        stride = std::max(stride, (bytes[d] + 255) & ~(size_t)255);
-    }
-    int rc = gather_to_dev0(ctx, src, bytes, stride);
+    int rc = gather_plane(ctx, Plane::Sums, 0, &stride);
     if (rc != RT_OK) return rc;
     cudaSetDevice(d0->device);
-    rc = ensure_scratch_out(d0, full);
+    rc = stage_buffers(d0, 0, full);
     if (rc != RT_OK) return fwd(ctx, d0, rc);
     if (d0->acc.compact) {
         // the devices hold shards urank * n + d of count ucount * n: inside this context they are n consecutive shards, so
@@ -404,44 +425,20 @@ extern "C" int rt_download(rt_ctx* ctx, int32_t total_spp, float* rgb_linear, ui
     if (!rgb_linear && !rgb8) return RT_OK;
     DevCtx* d0 = ctx->dev[0];
     const int w = ctx->last.width, h = ctx->last.height;
-    const size_t px = (size_t)w * h;
-    const bool fast = d0->acc.compact && !ctx->base_sums && ctx->last.shard_count == n;
-    if (!fast) {
+    if (!one_device_per_pixel(ctx)) {
         // sums first (sample-sharded frames, restored checkpoints), then one resolve of the whole frame on device 0
         int rc = gather_sums_full(ctx);
         if (rc != RT_OK) return rc;
-        rc = ensure_out(d0, px);
-        if (rc != RT_OK) return fwd(ctx, d0, rc);
-        const double inv = 1.0 / ((double)kAccumScale * (double)total_spp);
-        resolve_kernel<<<(unsigned)((px + 255) / 256), 256, 0, d0->stream>>>((const unsigned long long*)d0->frame_scratch, (int)px, inv,
-                                                                            rgb_linear ? d0->out_lin : nullptr, rgb8 ? d0->out_rgb8 : nullptr);
-        CUX(ctx, cudaGetLastError());
-        if (rgb_linear) CUX(ctx, cudaMemcpyAsync(rgb_linear, d0->out_lin, px * 12, cudaMemcpyDeviceToHost, d0->stream));
-        if (rgb8) CUX(ctx, cudaMemcpyAsync(rgb8, d0->out_rgb8, px * 3, cudaMemcpyDeviceToHost, d0->stream));
-        CUX(ctx, cudaStreamSynchronize(d0->stream));
-        return RT_OK;
+        return fwd(ctx, d0, resolve_to_host(d0, (const unsigned long long*)d0->frame_scratch, AccumLayout{w, h}, total_spp, rgb_linear, rgb8));
     }
     // tiles: resolve where they were rendered, move 3 (RGB8) or 12 (float) bytes per pixel instead of 32
     for (int pass = 0; pass < 2; pass++) {
         const bool lin = pass == 1;
         if ((lin && !rgb_linear) || (!lin && !rgb8)) continue;
-        const size_t bpp = lin ? 12 : 3;
-        std::vector<const void*> src((size_t)n);
-        std::vector<size_t> bytes((size_t)n);
         size_t stride = 0;
-        for (int d = 0; d < n; d++) {
-            DevCtx* dc = ctx->dev[d];
-            int rc = dev_wait(dc);
-            if (rc == RT_OK) rc = ensure_out(dc, dc->acc.slots());
-            if (rc == RT_OK) rc = dev_resolve_into(dc, total_spp, lin ? dc->out_lin : nullptr, lin ? nullptr : dc->out_rgb8);
-            if (rc != RT_OK) return fwd(ctx, dc, rc);
-            src[d] = lin ? (const void*)dc->out_lin : (const void*)dc->out_rgb8;
-            bytes[d] = dc->acc.slots() * bpp;
-            stride = std::max(stride, (bytes[d] + 255) & ~(size_t)255);
-        }
-        int rc = gather_to_dev0(ctx, src, bytes, stride);
+        int rc = gather_plane(ctx, lin ? Plane::Linear : Plane::Rgb8, total_spp, &stride);
         if (rc != RT_OK) return rc;
-        rc = dev_untile(d0, ctx->gather, stride, (int)bpp, n, w, h, ctx->last.tile_size, lin ? (void*)rgb_linear : (void*)rgb8);
+        rc = dev_untile(d0, ctx->gather, stride, lin ? 12 : 3, n, w, h, ctx->last.tile_size, lin ? (void*)rgb_linear : (void*)rgb8);
         if (rc != RT_OK) return fwd(ctx, d0, rc);
     }
     return RT_OK;
@@ -456,10 +453,7 @@ extern "C" int rt_accum_download(rt_ctx* ctx, uint64_t* host, size_t bytes) {
     if (bytes < full) return failx(ctx, RT_ERR_INVALID, "rt_accum_download: need %zu bytes, got %zu", full, bytes);
     int rc = gather_sums_full(ctx);
     if (rc != RT_OK) return rc;
-    DevCtx* d0 = ctx->dev[0];
-    CUX(ctx, cudaMemcpyAsync(host, d0->frame_scratch, full, cudaMemcpyDeviceToHost, d0->stream));
-    CUX(ctx, cudaStreamSynchronize(d0->stream));
-    return RT_OK;
+    return fwd(ctx, ctx->dev[0], plane_to_host(ctx->dev[0], ctx->dev[0]->frame_scratch, 32, AccumLayout{ctx->last.width, ctx->last.height}, host));
 }
 
 extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height) {
@@ -496,7 +490,7 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
 // A multi-device frame has per-device variance only when each pixel lives on one device: tiles, no restored checkpoint.
 static int multi_moments_frame(rt_ctx* ctx, const char* what) {
     if (!ctx->rendered) return failx(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
-    if (!(ctx->dev[0]->acc.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size()))
+    if (!one_device_per_pixel(ctx))
         return failx(ctx, RT_ERR_UNSUPPORTED, "%s: a multi-device context resolves tile-sharded frames without a restored checkpoint only", what);
     return RT_OK;
 }
@@ -509,20 +503,9 @@ extern "C" int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* varia
     if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
     int rc = multi_moments_frame(ctx, "rt_download_variance");
     if (rc != RT_OK) return rc;
-    // like the linear radiance of rt_download: resolved where the tiles were rendered, 12 bytes per pixel gathered
-    std::vector<const void*> src((size_t)n);
-    std::vector<size_t> bytes((size_t)n);
+    // like the linear radiance of rt_download: produced where the tiles were rendered, 12 bytes per pixel gathered
     size_t stride = 0;
-    for (int d = 0; d < n; d++) {
-        DevCtx* dc = ctx->dev[d];
-        rc = moments_ready(dc, "rt_download_variance");
-        if (rc == RT_OK) rc = dev_variance_into(dc, total_spp);
-        if (rc != RT_OK) return fwd(ctx, dc, rc);
-        src[d] = dc->out_lin;
-        bytes[d] = dc->acc.slots() * 12;
-        stride = std::max(stride, (bytes[d] + 255) & ~(size_t)255);
-    }
-    rc = gather_to_dev0(ctx, src, bytes, stride);
+    rc = gather_plane(ctx, Plane::Variance, total_spp, &stride);
     if (rc != RT_OK) return rc;
     return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 12, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, variance));
 }
@@ -580,30 +563,13 @@ extern "C" int rt_download_begin(rt_ctx* ctx, int32_t total_spp, int32_t want_li
     // several devices: the gather is synchronous (it is microseconds over NVLink), the PCIe copy is what overlaps
     if (!ctx->rendered) return failx(ctx, RT_ERR_STATE, "rt_download_begin: nothing rendered yet");
     if (total_spp <= 0 || (!!want_linear == !!want_rgb8)) return failx(ctx, RT_ERR_INVALID, "rt_download_begin: a multi-device context hands out ONE of linear / rgb8 per call");
-    DevCtx* d0 = ctx->dev[0];
-    const int w = ctx->last.width, h = ctx->last.height;
-    if (!(d0->acc.compact && !ctx->base_sums && ctx->last.shard_count == n))
+    if (!one_device_per_pixel(ctx))
         return failx(ctx, RT_ERR_UNSUPPORTED, "rt_download_begin: tile-sharded frames without a restored checkpoint only (use rt_download)");
     const bool lin = want_linear != 0;
-    const size_t bpp = lin ? 12 : 3;
-    std::vector<const void*> src((size_t)n);
-    std::vector<size_t> bytes((size_t)n);
     size_t stride = 0;
-    for (int d = 0; d < n; d++) {
-        DevCtx* dc = ctx->dev[d];
-        int rc = dev_wait(dc);
-        if (rc == RT_OK) rc = ensure_out(dc, dc->acc.slots());
-        // device 0's resolve output is also what its previous hand-out may still be copying from? no: hand-outs of a
-        // multi-device context copy from frame_scratch (the untiled frame), not from out_lin / out_rgb8
-        if (rc == RT_OK) rc = dev_resolve_into(dc, total_spp, lin ? dc->out_lin : nullptr, lin ? nullptr : dc->out_rgb8);
-        if (rc != RT_OK) return fwd(ctx, dc, rc);
-        src[d] = lin ? (const void*)dc->out_lin : (const void*)dc->out_rgb8;
-        bytes[d] = dc->acc.slots() * bpp;
-        stride = std::max(stride, (bytes[d] + 255) & ~(size_t)255);
-    }
-    int rc = gather_to_dev0(ctx, src, bytes, stride);
+    int rc = gather_plane(ctx, lin ? Plane::Linear : Plane::Rgb8, total_spp, &stride);
     if (rc != RT_OK) return rc;
-    return fwd(ctx, d0, dev_untile_begin(d0, ctx->gather, stride, (int)bpp, n, w, h, ctx->last.tile_size));
+    return fwd(ctx, ctx->dev[0], dev_untile_begin(ctx->dev[0], ctx->gather, stride, lin ? 12 : 3, n, ctx->last.width, ctx->last.height, ctx->last.tile_size));
 }
 extern "C" int rt_untile_begin(rt_ctx* ctx, const void* dev_shards, size_t shard_stride_bytes, int32_t bytes_per_pixel, int32_t shard_count,
                                int32_t width, int32_t height, int32_t tile_size) {

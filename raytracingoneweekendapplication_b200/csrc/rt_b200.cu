@@ -9,7 +9,7 @@
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
 //   variance_kernel, noise_kernel   sums + second moments -> per-pixel sample variance, frame noise partials
-//   untile_kernel, tile_pack_kernel, add_sums_kernel   shard frames: compact tiles <-> full frame, sums
+//   untile_kernel, add_sums_kernel   shard frames: compact tiles -> full frame, sums
 //   pair_nodes_kernel      device-built BVH2 nodes -> the paired layout the traversal reads
 //   probe_*_kernel         per-function known-answer probes
 //   fma_peak_kernel, l1_peak_kernel   FP32 and L1 roofline denominators
@@ -750,11 +750,6 @@ __global__ void l1_peak_kernel(const uint4* __restrict__ buf, int iters, uint4* 
 // ---------------------------------------------------------------------------------
 // context
 // ---------------------------------------------------------------------------------
-struct DevBuf {
-    void* p = nullptr;
-    size_t bytes = 0;
-};
-
 // Layout of an accumulation buffer.  Full: one 32-byte slot per pixel, row-major.  Compact
 // (RT_FLAG_COMPACT_TILES): only the tiles of one shard (tile t of the frame belongs to shard t mod count
 // and is its local tile t / count), each tile a tile_size x tile_size block of slots -- 1 / count of the
@@ -1936,20 +1931,6 @@ __global__ void untile_kernel(const unsigned char* __restrict__ shards, size_t s
         out[0] = src[0]; out[1] = src[1]; out[2] = src[2];
     }
 }
-// the inverse for the sums: gather one shard's tiles out of a full frame (restoring a checkpoint into a compact buffer)
-__global__ void tile_pack_kernel(const unsigned long long* __restrict__ full, int rank, int count, int width, int height, int tile,
-                                 unsigned long long* __restrict__ compact) {
-    const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y;
-    if (x >= width || y >= height) return;
-    const int tiles_x = (width + tile - 1) / tile;
-    const int t = (y / tile) * tiles_x + x / tile;
-    if (t % count != rank) return;
-    const size_t slot = ((size_t)(t / count) * tile + (size_t)(y % tile)) * tile + (size_t)(x % tile);
-    const uint4* s4 = reinterpret_cast<const uint4*>(full + 4 * ((size_t)y * width + x));
-    uint4* d4 = reinterpret_cast<uint4*>(compact + 4 * slot);
-    d4[0] = s4[0];
-    d4[1] = s4[1];
-}
 // a += b over n uint64 (fixed-point sums are associative: the order of the shards does not matter)
 __global__ void add_sums_kernel(unsigned long long* __restrict__ a, const unsigned long long* __restrict__ b, size_t n) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1968,15 +1949,49 @@ static cudaError_t launch_untile(int bpp, const void* shards, size_t stride, int
     return cudaGetLastError();
 }
 
-// device scratch that grows on demand (full-frame copies of compact data, gather staging)
-static int ensure_scratch_out(DevCtx* ctx, size_t bytes) {
-    if (bytes <= ctx->frame_scratch_cap) return RT_OK;
-    if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // an outstanding hand-out may still be copying from it
-    if (ctx->frame_scratch) cudaFree(ctx->frame_scratch);
-    ctx->frame_scratch = nullptr;
-    ctx->frame_scratch_cap = 0;
-    if (cudaMalloc(&ctx->frame_scratch, bytes) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of frame scratch", bytes);
-    ctx->frame_scratch_cap = bytes;
+// The one way to the staging buffers for a writer on ctx->stream: out_lin / out_rgb8 of `pixels` slots and frame_scratch
+// of `scratch_bytes` (full-frame copies of compact data, gathered sums), grown on demand.  The writer is ordered after
+// the copy of every outstanding hand-out (rt_download_begin / rt_untile_begin), which reads these buffers until its
+// rt_frame_end: a readback issued meanwhile does not change the frame the hand-out returns.
+static int stage_buffers(DevCtx* ctx, size_t pixels, size_t scratch_bytes) {
+    const bool grow_out = pixels > ctx->out_pixels, grow_scratch = scratch_bytes > ctx->frame_scratch_cap;
+    if ((grow_out || grow_scratch) && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // no free under a running copy
+    if (grow_out) {
+        if (ctx->out_lin) cudaFree(ctx->out_lin);
+        if (ctx->out_rgb8) cudaFree(ctx->out_rgb8);
+        ctx->out_lin = nullptr;
+        ctx->out_rgb8 = nullptr;
+        ctx->out_pixels = 0;
+        if (cudaMalloc(&ctx->out_lin, pixels * 3 * sizeof(float)) != cudaSuccess || cudaMalloc(&ctx->out_rgb8, pixels * 3) != cudaSuccess)
+            return fail(ctx, RT_ERR_NOMEM, "rt_download: cannot allocate the output buffers");
+        ctx->out_pixels = pixels;
+    }
+    if (grow_scratch) {
+        if (ctx->frame_scratch) cudaFree(ctx->frame_scratch);
+        ctx->frame_scratch = nullptr;
+        ctx->frame_scratch_cap = 0;
+        if (cudaMalloc(&ctx->frame_scratch, scratch_bytes) != cudaSuccess)
+            return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of frame scratch", scratch_bytes);
+        ctx->frame_scratch_cap = scratch_bytes;
+    }
+    for (const DevCtx::OutFrame& f : ctx->frames)
+        if (f.active) CU(ctx, cudaStreamWaitEvent(ctx->stream, f.done, 0));
+    return RT_OK;
+}
+
+// A plane of `bpp`-byte slots in layout L on the device -> the full row-major frame in host memory; a compact plane's
+// tiles go to their places in a zeroed frame (black elsewhere).  Returns with ctx->stream synchronised.
+static int plane_to_host(DevCtx* ctx, const void* plane, int bpp, const AccumLayout& L, void* host) {
+    const size_t full = (size_t)L.width * L.height * bpp;
+    if (L.compact) {
+        int rc = stage_buffers(ctx, 0, full);
+        if (rc != RT_OK) return rc;
+        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
+        CU(ctx, launch_untile(bpp, plane, 0, L.count, L.rank, L.width, L.height, L.tile, ctx->frame_scratch, ctx->stream));
+        plane = ctx->frame_scratch;
+    }
+    CU(ctx, cudaMemcpyAsync(host, plane, full, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
 
@@ -1994,17 +2009,7 @@ static int dev_accum_download(DevCtx* ctx, uint64_t* host, size_t bytes) {
     CU(ctx, cudaSetDevice(ctx->device));
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    const unsigned long long* src = ctx->accum;
-    if (ctx->acc.compact) {
-        rc = ensure_scratch_out(ctx, full);
-        if (rc != RT_OK) return rc;
-        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
-        CU(ctx, launch_untile(32, ctx->accum, 0, ctx->acc.count, ctx->acc.rank, ctx->acc.width, ctx->acc.height, ctx->acc.tile, ctx->frame_scratch, ctx->stream));
-        src = (const unsigned long long*)ctx->frame_scratch;
-    }
-    CU(ctx, cudaMemcpyAsync(host, src, full, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    return plane_to_host(ctx, ctx->accum, 32, ctx->acc, host);
 }
 
 static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height) {
@@ -2445,28 +2450,23 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
                         (p->flags & RT_FLAG_ASYNC) != 0);
 }
 
-// resolve_kernel over the slots of the accumulation buffer (full frame or compact tiles) into DEVICE buffers
-static int dev_resolve_into(DevCtx* ctx, int32_t total_spp, float* dev_lin, unsigned char* dev_rgb8) {
-    const size_t n = ctx->acc.slots();
+// resolve_kernel over `n` slots of sums (an accumulation buffer, a range of views, a gathered frame) into DEVICE buffers
+static int dev_resolve_into(DevCtx* ctx, const unsigned long long* sums, size_t n, int32_t total_spp, float* dev_lin, unsigned char* dev_rgb8) {
     if (n == 0 || (!dev_lin && !dev_rgb8)) return RT_OK;
     const double inv = 1.0 / ((double)kAccumScale * (double)total_spp);
-    resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, (int)n, inv, dev_lin, dev_rgb8);
+    resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(sums, (int)n, inv, dev_lin, dev_rgb8);
     CU(ctx, cudaGetLastError());
     return RT_OK;
 }
 
-static int ensure_out(DevCtx* ctx, size_t pixels) {
-    if (pixels <= ctx->out_pixels) return RT_OK;
-    if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // an outstanding hand-out may still be copying from them
-    if (ctx->out_lin) cudaFree(ctx->out_lin);
-    if (ctx->out_rgb8) cudaFree(ctx->out_rgb8);
-    ctx->out_lin = nullptr;
-    ctx->out_rgb8 = nullptr;
-    ctx->out_pixels = 0;
-    if (cudaMalloc(&ctx->out_lin, pixels * 3 * sizeof(float)) != cudaSuccess || cudaMalloc(&ctx->out_rgb8, pixels * 3) != cudaSuccess)
-        return fail(ctx, RT_ERR_NOMEM, "rt_download: cannot allocate the output buffers");
-    ctx->out_pixels = pixels;
-    return RT_OK;
+// The sums of layout L resolved into out_lin / out_rgb8 and copied to the host planes that are not null
+static int resolve_to_host(DevCtx* ctx, const unsigned long long* sums, const AccumLayout& L, int32_t total_spp, float* rgb_linear, uint8_t* rgb8) {
+    const size_t n = L.slots();
+    int rc = stage_buffers(ctx, n, 0);
+    if (rc == RT_OK) rc = dev_resolve_into(ctx, sums, n, total_spp, rgb_linear ? ctx->out_lin : nullptr, rgb8 ? ctx->out_rgb8 : nullptr);
+    if (rc == RT_OK && rgb_linear) rc = plane_to_host(ctx, ctx->out_lin, 12, L, rgb_linear);
+    if (rc == RT_OK && rgb8) rc = plane_to_host(ctx, ctx->out_rgb8, 3, L, rgb8);
+    return rc;
 }
 
 // The compact tiles of this shard resolved into caller-owned DEVICE buffers (for a gather over NCCL by the caller:
@@ -2478,7 +2478,7 @@ static int dev_resolve_tiles(DevCtx* ctx, int32_t total_spp, float* dev_rgb_line
     if (capacity_pixels < ctx->acc.slots()) return fail(ctx, RT_ERR_INVALID, "rt_resolve_tiles: the buffers hold %zu pixels, the frame has %zu", capacity_pixels, ctx->acc.slots());
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    rc = dev_resolve_into(ctx, total_spp, dev_rgb_linear, dev_rgb8);
+    rc = dev_resolve_into(ctx, ctx->accum, ctx->acc.slots(), total_spp, dev_rgb_linear, dev_rgb8);
     if (rc != RT_OK) return rc;
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return RT_OK;
@@ -2493,7 +2493,7 @@ static int dev_untile(DevCtx* ctx, const void* dev_shards, size_t shard_stride_b
         return fail(ctx, RT_ERR_INVALID, "rt_untile: bad arguments");
     CU(ctx, cudaSetDevice(ctx->device));
     const size_t full = (size_t)width * height * bytes_per_pixel;
-    int rc = ensure_scratch_out(ctx, full);
+    int rc = stage_buffers(ctx, 0, full);
     if (rc != RT_OK) return rc;
     CU(ctx, launch_untile(bytes_per_pixel, dev_shards, shard_stride_bytes, shard_count, -1, width, height, tile_size, ctx->frame_scratch, ctx->stream));
     CU(ctx, cudaMemcpyAsync(host_out, ctx->frame_scratch, full, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2526,12 +2526,6 @@ static int frame_slot(DevCtx* ctx, size_t px, bool lin, bool rgb8, DevCtx::OutFr
     *out = &f;
     return RT_OK;
 }
-// the device buffers the previous begin copied from are about to be overwritten: its copy must be through
-static int frame_wait_prev_copy(DevCtx* ctx) {
-    const DevCtx::OutFrame& prev = ctx->frames[ctx->frame_head ^ 1];
-    if (prev.active) CU(ctx, cudaStreamWaitEvent(ctx->stream, prev.done, 0));
-    return RT_OK;
-}
 static int frame_queue_copy(DevCtx* ctx, DevCtx::OutFrame* f, const void* dev_lin, const void* dev_rgb8, size_t px) {
     CU(ctx, cudaEventRecord(ctx->ev_ready, ctx->stream));
     CU(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_ready, 0));
@@ -2552,14 +2546,11 @@ static int dev_download_begin(DevCtx* ctx, int32_t total_spp, int32_t want_linea
     CU(ctx, cudaSetDevice(ctx->device));
     const size_t px = ctx->acc.slots();
     DevCtx::OutFrame* f = nullptr;
+    // stream order, no host wait: the previous copy and the pending render (on its own stream), then the resolve
     int rc = frame_slot(ctx, px, want_linear != 0, want_rgb8 != 0, &f);
-    if (rc == RT_OK) rc = ensure_out(ctx, px);
-    if (rc != RT_OK) return rc;
-    // stream order, no host wait: the pending render (on its own stream), then the previous copy, then the resolve
-    rc = dev_join(ctx, ctx->stream);
-    if (rc != RT_OK) return rc;
-    rc = frame_wait_prev_copy(ctx);
-    if (rc == RT_OK) rc = dev_resolve_into(ctx, total_spp, want_linear ? ctx->out_lin : nullptr, want_rgb8 ? ctx->out_rgb8 : nullptr);
+    if (rc == RT_OK) rc = stage_buffers(ctx, px, 0);
+    if (rc == RT_OK) rc = dev_join(ctx, ctx->stream);
+    if (rc == RT_OK) rc = dev_resolve_into(ctx, ctx->accum, px, total_spp, want_linear ? ctx->out_lin : nullptr, want_rgb8 ? ctx->out_rgb8 : nullptr);
     if (rc != RT_OK) return rc;
     return frame_queue_copy(ctx, f, ctx->out_lin, ctx->out_rgb8, px);
 }
@@ -2573,8 +2564,7 @@ static int dev_untile_begin(DevCtx* ctx, const void* dev_shards, size_t shard_st
     const size_t px = (size_t)width * height;
     DevCtx::OutFrame* f = nullptr;
     int rc = frame_slot(ctx, px, bytes_per_pixel == 12, bytes_per_pixel == 3, &f);
-    if (rc == RT_OK) rc = ensure_scratch_out(ctx, px * bytes_per_pixel);
-    if (rc == RT_OK) rc = frame_wait_prev_copy(ctx);
+    if (rc == RT_OK) rc = stage_buffers(ctx, 0, px * bytes_per_pixel);
     if (rc != RT_OK) return rc;
     CU(ctx, launch_untile(bytes_per_pixel, dev_shards, shard_stride_bytes, shard_count, -1, width, height, tile_size, ctx->frame_scratch, ctx->stream));
     return frame_queue_copy(ctx, f, ctx->frame_scratch, ctx->frame_scratch, px);
@@ -2599,33 +2589,7 @@ static int dev_download(DevCtx* ctx, int32_t total_spp, float* rgb_linear, uint8
     if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_download: total_spp must be positive");
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    const size_t n = ctx->acc.slots(), full = (size_t)ctx->acc.width * ctx->acc.height;
-    rc = ensure_out(ctx, n);
-    if (rc != RT_OK) return rc;
-    float* dlin = rgb_linear ? ctx->out_lin : nullptr;
-    unsigned char* d8 = rgb8 ? ctx->out_rgb8 : nullptr;
-    rc = dev_resolve_into(ctx, total_spp, dlin, d8);
-    if (rc != RT_OK) return rc;
-    cudaError_t e = cudaSuccess;
-    if (ctx->acc.compact) {
-        // one shard of a frame: its tiles go to their places in a zeroed full frame (black elsewhere)
-        const AccumLayout& L = ctx->acc;
-        rc = ensure_scratch_out(ctx, full * 15 + 256);
-        if (rc != RT_OK) return rc;
-        unsigned char* f8 = ctx->frame_scratch;
-        unsigned char* flin = ctx->frame_scratch + ((full * 3 + 255) & ~(size_t)255);
-        e = cudaMemsetAsync(ctx->frame_scratch, 0, ctx->frame_scratch_cap, ctx->stream);
-        if (e == cudaSuccess && rgb8) e = launch_untile(3, d8, 0, L.count, L.rank, L.width, L.height, L.tile, f8, ctx->stream);
-        if (e == cudaSuccess && rgb_linear) e = launch_untile(12, dlin, 0, L.count, L.rank, L.width, L.height, L.tile, flin, ctx->stream);
-        if (e == cudaSuccess && rgb_linear) e = cudaMemcpyAsync(rgb_linear, flin, full * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess && rgb8) e = cudaMemcpyAsync(rgb8, f8, full * 3, cudaMemcpyDeviceToHost, ctx->stream);
-    } else {
-        if (rgb_linear) e = cudaMemcpyAsync(rgb_linear, dlin, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess && rgb8) e = cudaMemcpyAsync(rgb8, d8, n * 3, cudaMemcpyDeviceToHost, ctx->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_download: %s", cudaGetErrorString(e));
-    return RT_OK;
+    return resolve_to_host(ctx, ctx->accum, ctx->acc, total_spp, rgb_linear, rgb8);
 }
 
 // views [first, first + count) of the views frame, each resolved like rt_download's planes
@@ -2638,20 +2602,9 @@ static int dev_download_views(DevCtx* ctx, int32_t total_spp, int32_t first, int
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
     if (!rgb_linear && !rgb8) return RT_OK;
-    const size_t per_view = (size_t)ctx->views_w * ctx->views_h, n = per_view * count;
-    rc = ensure_out(ctx, n);
-    if (rc != RT_OK) return rc;
-    // an outstanding rt_download_begin may still be copying out of the output buffers
-    if (ctx->copy_stream) CU(ctx, cudaStreamSynchronize(ctx->copy_stream));
-    const double inv = 1.0 / ((double)kAccumScale * (double)total_spp);
-    resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->views_accum + 4 * per_view * first, (int)n, inv,
-                                                                          rgb_linear ? ctx->out_lin : nullptr, rgb8 ? ctx->out_rgb8 : nullptr);
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess && rgb_linear) e = cudaMemcpyAsync(rgb_linear, ctx->out_lin, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && rgb8) e = cudaMemcpyAsync(rgb8, ctx->out_rgb8, n * 3, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_download_views: %s", cudaGetErrorString(e));
-    return RT_OK;
+    // consecutive views of one size are one full frame views_w x (views_h * count)
+    return resolve_to_host(ctx, ctx->views_accum + (size_t)first * ctx->views_w * ctx->views_h * 4, AccumLayout{ctx->views_w, ctx->views_h * count},
+                           total_spp, rgb_linear, rgb8);
 }
 
 // ---- second moments (RT_FLAG_MOMENTS) ------------------------------------------------------------------------------
@@ -2664,7 +2617,7 @@ static int moments_ready(DevCtx* ctx, const char* what) {
 // variance_kernel over the slots of the frame into out_lin (the buffer of the linear radiance of rt_download)
 static int dev_variance_into(DevCtx* ctx, int32_t total_spp) {
     const size_t n = ctx->acc.slots();
-    int rc = ensure_out(ctx, n);
+    int rc = stage_buffers(ctx, n, 0);
     if (rc != RT_OK) return rc;
     if (n) variance_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, ctx->moments, (int)n, total_spp, ctx->out_lin);
     CU(ctx, cudaGetLastError());
@@ -2677,20 +2630,7 @@ static int dev_download_variance(DevCtx* ctx, int32_t total_spp, float* variance
     int rc = moments_ready(ctx, "rt_download_variance");
     if (rc == RT_OK) rc = dev_variance_into(ctx, total_spp);
     if (rc != RT_OK) return rc;
-    const size_t full = (size_t)ctx->acc.width * ctx->acc.height * 12;
-    const void* src = ctx->out_lin;
-    if (ctx->acc.compact) {
-        // one shard of a frame: its tiles go to their places in a zeroed full frame
-        const AccumLayout& L = ctx->acc;
-        rc = ensure_scratch_out(ctx, full);
-        if (rc != RT_OK) return rc;
-        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
-        CU(ctx, launch_untile(12, ctx->out_lin, 0, L.count, L.rank, L.width, L.height, L.tile, ctx->frame_scratch, ctx->stream));
-        src = ctx->frame_scratch;
-    }
-    CU(ctx, cudaMemcpyAsync(variance, src, full, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    return plane_to_host(ctx, ctx->out_lin, 12, ctx->acc, variance);
 }
 
 // the 12 integer partials of noise_kernel over the slots of this device, and the frame pixels they cover
@@ -2726,17 +2666,7 @@ static int dev_moments_download(DevCtx* ctx, uint64_t* host, size_t bytes) {
     if (ctx->accum && bytes != full) return fail(ctx, RT_ERR_INVALID, "rt_moments_download: a %dx%d frame is %zu bytes, got %zu", ctx->acc.width, ctx->acc.height, full, bytes);
     int rc = moments_ready(ctx, "rt_moments_download");
     if (rc != RT_OK) return rc;
-    const unsigned long long* src = ctx->moments;
-    if (ctx->acc.compact) {
-        rc = ensure_scratch_out(ctx, full);
-        if (rc != RT_OK) return rc;
-        CU(ctx, cudaMemsetAsync(ctx->frame_scratch, 0, full, ctx->stream));
-        CU(ctx, launch_untile(48, ctx->moments, 0, ctx->acc.count, ctx->acc.rank, ctx->acc.width, ctx->acc.height, ctx->acc.tile, ctx->frame_scratch, ctx->stream));
-        src = (const unsigned long long*)ctx->frame_scratch;
-    }
-    CU(ctx, cudaMemcpyAsync(host, src, full, cudaMemcpyDeviceToHost, ctx->stream));
-    CU(ctx, cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
+    return plane_to_host(ctx, ctx->moments, 48, ctx->acc, host);
 }
 
 // the moments of the sums rt_accum_upload restored just before (same full frame)
