@@ -291,7 +291,7 @@ typedef struct rt_render_params {
 
 typedef struct rt_stats {
     double render_ms;          /* device time of the last synchronous rt_render (CUDA events) */
-    double upload_ms;          /* host time of the last rt_upload_scene (incl. BVH build) */
+    double upload_ms;          /* host time of the last rt_upload_scene or rt_refit_scene (incl. BVH build) */
     uint64_t samples;          /* camera samples traced by the last rt_render       */
     uint64_t rays;             /* world.hit root queries incl. primary (RT_FLAG_STATS) */
     uint64_t node_visits;      /* BVH nodes fetched (each holds two child boxes)    */
@@ -330,8 +330,9 @@ typedef struct rt_stats {
     /* multi-device contexts: devices of the context (counters above are summed over them, render_ms is the slowest
      * device's) and how rt_download gathers their tiles on device 0: 0 single device, 1 peer copies, 2 NCCL send/recv */
     uint32_t devices, gather_mode;
-    /* last rt_upload_scene: bytes copied to the device, and 1 when the scene was byte-identical to the one already
-     * uploaded (same builder settings), so that only the staged arena was copied again -- no validation, no BVH build */
+    /* last rt_upload_scene or rt_refit_scene: bytes copied to the device, and 1 when the scene was byte-identical to the
+     * one already uploaded (same builder settings), so that only the staged arena was copied again -- no validation, no
+     * BVH build */
     uint64_t upload_bytes;
     uint32_t scene_reused, reserved3_;
 } rt_stats;
@@ -353,6 +354,27 @@ const char* rt_last_error(const rt_ctx* ctx);
  * transforms, builds the SAH BVH on the host, converts to the device layout and
  * uploads.  Replaces main.cpp:442 (bvh_node construction). */
 int rt_upload_scene(rt_ctx* ctx, const rt_scene_desc* scene);
+
+/* Animation update: replaces the uploaded scene by `scene`, which must have the STRUCTURE of the scene last uploaded
+ * to ctx, without a tree build.  The tree keeps its topology and leaf order and its boxes are recomputed on the GPU.
+ * Structure: every count of rt_scene_desc; each mesh's n_triangles and each image's size; the device kind of every
+ * world primitive and boundary (sphere, moving sphere -- a non-zero center_vec --, quad, triangle); the quads of the
+ * next-event emitter list (a quad with an emissive material and a non-zero area), in their order; each medium's
+ * boundary class (one sphere, a six-quad box, general).  Anything else may change: transforms, centres, radii, motion,
+ * corners, mesh positions, indices and uvs (checked like an upload), materials, textures, texels, Perlin tables, point
+ * lights, media densities and the camera.
+ * Every device record and table then equals the one rt_upload_scene(ctx, scene) would make, so frames equal a fresh
+ * upload's bit for bit except for rays that hit two primitives at exactly the same t and, on a host-built scene with
+ * several emitters, RT_FLAG_NEE (the emitter list keeps the uploaded tree's leaf order).  A refitted tree loosens as
+ * objects move away from where it was built: upload again when render time grows (DESIGN.md section 10c).
+ * RT_ERR_STATE without a scene, RT_ERR_INVALID for an invalid description or another structure (the message names
+ * the first difference), RT_ERR_UNSUPPORTED when the scene is traversed as a wide tree (rt_set_bvh_width 4 / 8).
+ * A refused refit changes nothing.  A refit waits for the passes in flight and treats the frame like rt_upload_scene:
+ * a single-device context keeps its frame, moments and bound buffer; a multi-device context needs an rt_render before
+ * its next download.  bvh_nodes, bvh_depth and bvh_leaves are unchanged; upload_ms and
+ * upload_bytes report the refit.  An rt_upload_scene of the last uploaded scene afterwards may still reuse its staged
+ * arena (scene_reused). */
+int rt_refit_scene(rt_ctx* ctx, const rt_scene_desc* scene);
 
 /* Which builder rt_upload_scene uses (replaces bvh.h:13-45 either way).
  *   1 host:   transforms baked, binned-SAH BVH2 and device records built on the CPU (best tree)

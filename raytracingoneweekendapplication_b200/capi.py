@@ -151,7 +151,7 @@ EXPORTED_SYMBOLS = [
     "rt_set_bvh_width", "rt_device_count", "rt_shard_pixels", "rt_resolve_tiles", "rt_untile",
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
     "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
-    "rt_render_views", "rt_download_views",
+    "rt_render_views", "rt_download_views", "rt_refit_scene",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
@@ -193,6 +193,7 @@ def load() -> C.CDLL:
     lib.rt_last_error.argtypes = [vp]
     lib.rt_last_error.restype = C.c_char_p
     lib.rt_upload_scene.argtypes = [vp, C.POINTER(rt_scene_desc)]
+    lib.rt_refit_scene.argtypes = [vp, C.POINTER(rt_scene_desc)]
     lib.rt_render.argtypes = [vp, C.POINTER(rt_render_params)]
     lib.rt_sync.argtypes = [vp]
     lib.rt_join.argtypes = [vp, vp]
@@ -381,14 +382,22 @@ class Context:
         """2 (binary tree) | 4 | 8 (wide quantised tree) for the next upload."""
         self._check(self.lib.rt_set_bvh_width(self._h, width))
 
-    def upload(self, scene) -> None:
+    @staticmethod
+    def _desc_ptr(scene):
         if hasattr(scene, "desc_ptr"):          # capi.Scene or any object that keeps a description alive
-            ptr = scene.desc_ptr
-        elif isinstance(scene, rt_scene_desc):
-            ptr = C.pointer(scene)
-        else:
-            ptr = scene
-        self._check(self.lib.rt_upload_scene(self._h, ptr))
+            return scene.desc_ptr
+        if isinstance(scene, rt_scene_desc):
+            return C.pointer(scene)
+        return scene
+
+    def upload(self, scene) -> None:
+        self._check(self.lib.rt_upload_scene(self._h, self._desc_ptr(scene)))
+
+    def refit(self, scene) -> None:
+        """rt_refit_scene: replace the uploaded scene by `scene`, which has its structure (same counts, primitive kinds,
+        emitters and media classes) but may move, without a tree build: the tree keeps its topology, its boxes are
+        recomputed.  Takes what upload() takes."""
+        self._check(self.lib.rt_refit_scene(self._h, self._desc_ptr(scene)))
 
     def render(self, width: int, height: int, spp: int, max_depth: int = 50, seed: int = 1, spp_begin: int = 0,
                accumulate: bool = False, stats: bool = False, shard_rank: int = 0, shard_count: int = 1,

@@ -27,6 +27,7 @@
 // once, coalesced in sorted order on the write side; algorithmic bytes per primitive are listed
 // in DESIGN.md.  The result is an LBVH: built in milliseconds, traced slower than the host's
 // SAH tree (measured numbers in DESIGN.md); rt_set_bvh_builder / RT_B200_BVH choose.
+// bvh_refit.cuh refits an uploaded tree of either builder from the same inputs (rt_refit_scene).
 #pragma once
 #include <cub/cub.cuh>
 
@@ -449,10 +450,9 @@ struct Layout {
     size_t cub_temp_bytes, total;
 };
 
-// `n` primitives: the world refs with every mesh ref expanded (validate_scene counted them)
-inline Layout plan_scratch(const rt_scene_desc* sc, int n_prims) {
-    Layout L{};
-    ScratchPlan p;
+// The raw ABI arrays of `sc` and, with meshes, the primitive map: the inputs of both the build and the refit
+// (bvh_refit.cuh).  `n` primitives: the world refs with every mesh ref expanded (validate_scene counted them).
+inline void plan_inputs(ScratchPlan& p, Layout& L, const rt_scene_desc* sc, int n_prims) {
     const size_t n = (size_t)n_prims, n_world = (size_t)sc->n_world;
     L.world = p.add(n_world * sizeof(rt_prim_ref));
     L.spheres = p.add((size_t)sc->n_spheres * sizeof(rt_sphere));
@@ -493,6 +493,13 @@ inline Layout plan_scratch(const rt_scene_desc* sc, int n_prims) {
     L.ref_count = p.add(meshes ? n_world * 4 : 0);
     L.ref_first = p.add(meshes ? n_world * 4 : 0);
     L.prim_map = p.add(meshes ? n * 8 : 0);
+}
+
+inline Layout plan_scratch(const rt_scene_desc* sc, int n_prims) {
+    Layout L{};
+    ScratchPlan p;
+    const size_t n = (size_t)n_prims, n_world = (size_t)sc->n_world;
+    plan_inputs(p, L, sc, n_prims);
     L.box_lo = p.add(n * 16); L.box_hi = p.add(n * 16);
     L.key_in = p.add(n * 8); L.key_out = p.add(n * 8);
     L.val_in = p.add(n * 4); L.val_out = p.add(n * 4);
@@ -583,36 +590,26 @@ struct BuildResult {
     float ms_copy_in = 0, ms_build = 0, ms_emit = 0, ms_top = 0;
 };
 
-// Copies the raw arrays of `sc` into `scratch` and runs the build of its `n` primitives (world refs
-// with the mesh refs expanded) on `stream`.  `T` points into the scene arena.  Returns a
-// cudaError_t-compatible code (0 = success).  The mesh indices must have been checked.
-inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char* scratch, const Layout& L, const Targets& T,
-                                   cudaStream_t stream, CopyRing& ring, int device, bool hybrid_top, const int* quad_light,
-                                   BuildResult& out) {
-    const int n_world = sc->n_world;
-    const bool meshes = sc->n_meshes > 0;
-    Scratch W{};
+// Copies the raw arrays of `sc` (the plan_inputs part of `L`) into `scratch` on `stream`, adding the bytes to `bytes_in`.
+inline cudaError_t copy_inputs(const rt_scene_desc* sc, unsigned char* scratch, const Layout& L, cudaStream_t stream, CopyRing& ring,
+                               int device, size_t& bytes_in) {
     auto at = [&](size_t off) { return scratch + off; };
     cudaError_t e;
-    cudaEvent_t ev[4];
-    for (auto& v : ev) if ((e = cudaEventCreate(&v)) != cudaSuccess) return e;
-    cudaEventRecord(ev[0], stream);
 #define RT_COPY_IN(field, ptr, count, type)                                                                                   \
     if ((count) > 0) {                                                                                                        \
         if ((e = copy_in(at(L.field), ptr, (size_t)(count) * sizeof(type), stream, ring, device)) != cudaSuccess) return e;  \
-        out.bytes_in += (size_t)(count) * sizeof(type);                                                                       \
+        bytes_in += (size_t)(count) * sizeof(type);                                                                           \
     }
-    RT_COPY_IN(world, sc->world, n_world, rt_prim_ref)
+    RT_COPY_IN(world, sc->world, sc->n_world, rt_prim_ref)
     RT_COPY_IN(spheres, sc->spheres, sc->n_spheres, rt_sphere)
     RT_COPY_IN(quads, sc->quads, sc->n_quads, rt_quad)
     RT_COPY_IN(triangles, sc->triangles, sc->n_triangles, rt_triangle)
     RT_COPY_IN(xforms, sc->xforms, sc->n_xforms, rt_xform)
-    if (quad_light) { RT_COPY_IN(quad_light, quad_light, sc->n_quads, int) }
-    if (meshes) {
+    if (sc->n_meshes > 0) {
         // each distinct mesh array once, then the mesh table with its pointers moved to those copies
         for (const MeshArray& a : L.mesh_arrays) {
             if ((e = copy_in(at(a.off), a.host, a.bytes, stream, ring, device)) != cudaSuccess) return e;
-            out.bytes_in += a.bytes;
+            bytes_in += a.bytes;
         }
         std::vector<rt_mesh> table(sc->meshes, sc->meshes + sc->n_meshes);
         auto dev = [&](int slot) -> const void* { return slot < 0 ? nullptr : at(L.mesh_arrays[(size_t)slot].off); };
@@ -622,15 +619,58 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char
             table[i].uvs = (const float*)dev(L.mesh_slots[4 * i + 2]);
             table[i].uv_indices = (const uint32_t*)dev(L.mesh_slots[4 * i + 3]);
         }
+        // pageable source: cudaMemcpyAsync has staged it by the time it returns, so `table` may go
         RT_COPY_IN(meshes, table.data(), sc->n_meshes, rt_mesh)
     }
 #undef RT_COPY_IN
-    cudaEventRecord(ev[1], stream);
+    return cudaSuccess;
+}
+
+// The copied inputs as the kernels read them: world list, typed sources, primitive count and map
+inline Scratch input_view(const rt_scene_desc* sc, int n, unsigned char* scratch, const Layout& L) {
+    Scratch W{};
+    auto at = [&](size_t off) { return scratch + off; };
     W.world = (const rt_prim_ref*)at(L.world);
     W.src = Sources{(const rt_sphere*)at(L.spheres), (const rt_quad*)at(L.quads), (const rt_triangle*)at(L.triangles),
                     (const rt_xform*)at(L.xforms), (const rt_mesh*)at(L.meshes)};
     W.n = n;
-    W.prim_map = meshes ? (uint2*)at(L.prim_map) : nullptr;
+    W.prim_map = sc->n_meshes > 0 ? (uint2*)at(L.prim_map) : nullptr;
+    return W;
+}
+
+// Scenes with meshes: primitive -> (world ref, triangle of the mesh), from a scan over the per-ref primitive counts
+inline cudaError_t map_prims(const Scratch& W, int n_world, unsigned char* scratch, const Layout& L, void* cub_temp, size_t cub_temp_bytes,
+                             cudaStream_t stream) {
+    const int tpb = 256;
+    uint32_t* count = (uint32_t*)(scratch + L.ref_count);
+    uint32_t* first = (uint32_t*)(scratch + L.ref_first);
+    ref_count_kernel<<<(n_world + tpb - 1) / tpb, tpb, 0, stream>>>(W, n_world, count);
+    cudaError_t e = cub::DeviceScan::ExclusiveSum(cub_temp, cub_temp_bytes, count, first, n_world, stream);
+    if (e != cudaSuccess) return e;
+    prim_map_kernel<<<(W.n + tpb - 1) / tpb, tpb, 0, stream>>>(W, first, n_world);
+    return cudaSuccess;
+}
+
+// Copies the raw arrays of `sc` into `scratch` and runs the build of its `n` primitives (world refs
+// with the mesh refs expanded) on `stream`.  `T` points into the scene arena.  Returns a
+// cudaError_t-compatible code (0 = success).  The mesh indices must have been checked.
+inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char* scratch, const Layout& L, const Targets& T,
+                                   cudaStream_t stream, CopyRing& ring, int device, bool hybrid_top, const int* quad_light,
+                                   BuildResult& out) {
+    const int n_world = sc->n_world;
+    const bool meshes = sc->n_meshes > 0;
+    auto at = [&](size_t off) { return scratch + off; };
+    cudaError_t e;
+    cudaEvent_t ev[4];
+    for (auto& v : ev) if ((e = cudaEventCreate(&v)) != cudaSuccess) return e;
+    cudaEventRecord(ev[0], stream);
+    if ((e = copy_inputs(sc, scratch, L, stream, ring, device, out.bytes_in)) != cudaSuccess) return e;
+    if (quad_light) {
+        if ((e = copy_in(at(L.quad_light), quad_light, (size_t)sc->n_quads * sizeof(int), stream, ring, device)) != cudaSuccess) return e;
+        out.bytes_in += (size_t)sc->n_quads * sizeof(int);
+    }
+    cudaEventRecord(ev[1], stream);
+    Scratch W = input_view(sc, n, scratch, L);
     W.box_lo = (float4*)at(L.box_lo); W.box_hi = (float4*)at(L.box_hi);
     W.key_in = (unsigned long long*)at(L.key_in); W.key_out = (unsigned long long*)at(L.key_out);
     W.val_in = (uint32_t*)at(L.val_in); W.val_out = (uint32_t*)at(L.val_out);
@@ -648,11 +688,7 @@ inline cudaError_t build_on_device(const rt_scene_desc* sc, int n, unsigned char
     init_kernel<<<1, 32, 0, stream>>>(W);
     size_t tb = W.cub_temp_bytes;
     if (meshes) {
-        uint32_t* count = (uint32_t*)at(L.ref_count);
-        uint32_t* first = (uint32_t*)at(L.ref_first);
-        ref_count_kernel<<<(n_world + tpb - 1) / tpb, tpb, 0, stream>>>(W, n_world, count);
-        if ((e = cub::DeviceScan::ExclusiveSum(W.cub_temp, tb, count, first, n_world, stream)) != cudaSuccess) return e;
-        prim_map_kernel<<<gn, tpb, 0, stream>>>(W, first, n_world);
+        if ((e = map_prims(W, n_world, scratch, L, W.cub_temp, tb, stream)) != cudaSuccess) return e;
         bounds_kernel<true><<<gn, tpb, 0, stream>>>(W);
     } else {
         bounds_kernel<false><<<gn, tpb, 0, stream>>>(W);

@@ -3,8 +3,8 @@
 //
 // A context drives ONE OR SEVERAL GPUs of one box from one process (SURVEY 8b / 8e; replaces the reference's
 // row bands over CPU threads, Camera.txt:59-61, 96-100):
-//   * the scene is replicated: rt_upload_scene uploads (and, for big scenes, builds) on every device, in
-//     parallel host threads;
+//   * the scene is replicated: rt_upload_scene uploads (and, for big scenes, builds) and rt_refit_scene refits on
+//     every device, in parallel host threads;
 //   * rt_render cuts the frame into tile x tile tiles, tile t -> device t mod n (small frames: sample
 //     s -> device s mod n), every device renders into a COMPACT buffer that holds only its own tiles
 //     (1 / n of the frame), all devices run concurrently on their own streams;
@@ -162,29 +162,43 @@ extern "C" int rt_visible_devices(void) {
     if (!(ctx)) return RT_ERR_INVALID;                      \
     if ((ctx)->dev.empty()) return failx(ctx, RT_ERR_STATE, "the context was not created")
 
-extern "C" int rt_upload_scene(rt_ctx* ctx, const rt_scene_desc* sc) {
-    RT_NEED(ctx);
-    // an ABI-3 description ends where `meshes` begins: read no byte past its struct_size, upload it as a scene without meshes
-    rt_scene_desc v3;
-    if (sc && sc->abi_version == 3 && sc->struct_size == offsetof(rt_scene_desc, meshes)) {
-        std::memset(&v3, 0, sizeof v3);
-        std::memcpy(&v3, sc, offsetof(rt_scene_desc, meshes));
-        v3.struct_size = sizeof v3;
-        v3.abi_version = RT_B200_ABI_VERSION;
-        sc = &v3;
-    }
-    ctx->rendered = false;
-    if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], dev_upload_scene(ctx->dev[0], sc));
-    // replicated scene: one host thread per device (the host BVH build is repeated per device -- milliseconds for
-    // scenes below the device-build threshold; above it every device builds its own tree from the same input)
+// An ABI-3 description ends where `meshes` begins: read no byte past its struct_size, take it as a scene without meshes
+static const rt_scene_desc* widen_v3(const rt_scene_desc* sc, rt_scene_desc* v3) {
+    if (!sc || sc->abi_version != 3 || sc->struct_size != offsetof(rt_scene_desc, meshes)) return sc;
+    std::memset(v3, 0, sizeof *v3);
+    std::memcpy(v3, sc, offsetof(rt_scene_desc, meshes));
+    v3->struct_size = sizeof *v3;
+    v3->abi_version = RT_B200_ABI_VERSION;
+    return v3;
+}
+
+// The scene is replicated: one host thread per device (the host BVH build is repeated per device -- milliseconds for
+// scenes below the device-build threshold; above it every device builds its own tree from the same input)
+static int on_every_device(rt_ctx* ctx, int (*fn)(DevCtx*, const rt_scene_desc*), const rt_scene_desc* sc) {
+    if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], fn(ctx->dev[0], sc));
     std::vector<int> rcs(ctx->dev.size(), RT_OK);
     std::vector<std::thread> pool;
-    for (size_t i = 1; i < ctx->dev.size(); i++) pool.emplace_back([&, i]() { rcs[i] = dev_upload_scene(ctx->dev[i], sc); });
-    rcs[0] = dev_upload_scene(ctx->dev[0], sc);
+    for (size_t i = 1; i < ctx->dev.size(); i++) pool.emplace_back([&, i]() { rcs[i] = fn(ctx->dev[i], sc); });
+    rcs[0] = fn(ctx->dev[0], sc);
     for (auto& t : pool) t.join();
     for (size_t i = 0; i < ctx->dev.size(); i++)
         if (rcs[i] != RT_OK) return fwd(ctx, ctx->dev[i], rcs[i]);
     return RT_OK;
+}
+
+extern "C" int rt_upload_scene(rt_ctx* ctx, const rt_scene_desc* sc) {
+    RT_NEED(ctx);
+    rt_scene_desc v3;
+    ctx->rendered = false;
+    return on_every_device(ctx, dev_upload_scene, widen_v3(sc, &v3));
+}
+
+extern "C" int rt_refit_scene(rt_ctx* ctx, const rt_scene_desc* sc) {
+    RT_NEED(ctx);
+    rt_scene_desc v3;
+    const int rc = on_every_device(ctx, dev_refit_scene, widen_v3(sc, &v3));
+    if (rc == RT_OK) ctx->rendered = false;  // like an upload; a refused refit changes nothing
+    return rc;
 }
 
 extern "C" int rt_set_bvh_builder(rt_ctx* ctx, int32_t mode) {

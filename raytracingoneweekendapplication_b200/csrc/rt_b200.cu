@@ -519,6 +519,7 @@ __global__ void pair_nodes_kernel(float4* __restrict__ nodes, int n) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) pair_node(nodes + 4 * (size_t)i);
 }
+#include "bvh_refit.cuh"
 
 // Camera.txt:136-168 in double: the pixel-centre ray of pixel (i, j) is center + t * (dir00 + i du + j dv)
 struct CameraD {
@@ -863,8 +864,30 @@ struct DevCtx {
     size_t world_type_count[4] = {0, 0, 0, 0};  // primitives of each device type in the world list (validate_scene)
     int n_prims = 0;  // primitives of the world list with every mesh ref expanded to its triangles (validate_scene)
     rtlbvh::CopyRing copy_ring;        // pinned staging of the device path's raw-input copy
-    unsigned char* scratch = nullptr;  // work space of the device build, reused across uploads
+    unsigned char* scratch = nullptr;  // work space of the device build and of rt_refit_scene, reused across calls
     size_t scratch_cap = 0;
+    // the scene-side state of the scene whose arena image is in `staging`: a cache hit of rt_upload_scene restores it
+    // together with the arena (an rt_refit_scene in between changes both)
+    struct SceneState {
+        DevScene scene;
+        rt_camera camera;
+        int scene_feat;
+        bool scene_lite, geom_lite;
+    } staged_state{};
+    // what rt_refit_scene compares a description with: the structure of the uploaded scene
+    struct Shape {
+        int32_t counts[13];
+        std::vector<int32_t> mesh_tris, image_wh;
+        std::vector<uint32_t> boundary_packed;  // the boundaries' records (type << 28 | index)
+        std::vector<int8_t> media_class;        // 1 one sphere, 2 a six-quad box, 0 general
+        // the next-event emitters in list order: canonical ids of a host-built scene, source quads of a device-built one
+        std::vector<int32_t> nee_ids;
+        std::vector<unsigned char*> image_dev;  // the images' texels in the arena
+        int n_prims;                             // world primitives with the meshes expanded, and of each device type
+        size_t world_type_count[4];
+        bool device_built;                       // the tree and the world records were built on the device
+    } shape;
+    rtlbvh::RefitTree refit_tree;  // the uploaded tree in the order the refit visits it (derived on its first refit)
 };
 
 // From this many primitives on, RT_B200_BVH=auto builds on the device: the host SAH build costs
@@ -898,6 +921,7 @@ static void release_buffers(DevCtx* ctx) {
     if (ctx->arena) cudaFree(ctx->arena);
     if (ctx->scratch) cudaFree(ctx->scratch);
     ctx->copy_ring.release();
+    ctx->refit_tree.release();
     ctx->scratch = nullptr;
     ctx->scratch_cap = 0;
     if (ctx->staging) cudaFreeHost(ctx->staging);
@@ -1364,8 +1388,203 @@ static bool box_slabs(const rtprep::BakedPrim* q, float4 out[4]) {
     return true;
 }
 
+// The device records the host emits, in the typed arrays of the arena, after `base[t]` records of each type: the host
+// path emits the world primitives in leaf order and then the boundaries from base 0; the device path and
+// rt_refit_scene emit the boundaries only, after the world records the kernels write.
+struct TypedRecords {
+    size_t base[4] = {0, 0, 0, 0};
+    std::vector<float4> sph, msph, quad, tri, tri_sh;
+    std::vector<double> sph_d, msph_d, quad_d, tri_d;
+    std::vector<int4> sph_sh, msph_sh, quad_sh;
+    // appends the record of `b`; returns its packed ref type << 28 | index
+    uint32_t emit(const BakedPrim& b) {
+        auto f4 = [](rtprep::F4 v) { return make_float4(v.x, v.y, v.z, v.w); };
+        auto i4 = [](rtprep::I4 v) { return make_int4(v.x, v.y, v.z, v.w); };
+        if (b.dev_type == PT_SPHERE) {
+            const rtprep::SphereRec r = rtprep::make_sphere(b);
+            sph.push_back(f4(r.g));
+            sph_d.insert(sph_d.end(), r.d, r.d + 4);
+            sph_sh.push_back(i4(r.sh));
+            return (PT_SPHERE << 28) | (uint32_t)(base[PT_SPHERE] + sph.size() - 1);
+        } else if (b.dev_type == PT_MSPHERE) {
+            const rtprep::MSphereRec r = rtprep::make_msphere(b);
+            msph.push_back(f4(r.g0));
+            msph.push_back(f4(r.g1));
+            msph_d.insert(msph_d.end(), r.d, r.d + 8);
+            msph_sh.push_back(i4(r.sh));
+            return (PT_MSPHERE << 28) | (uint32_t)(base[PT_MSPHERE] + msph_sh.size() - 1);
+        } else if (b.dev_type == PT_QUAD) {
+            const rtprep::QuadRec r = rtprep::make_quad(b);
+            for (int k = 0; k < 3; k++) quad.push_back(f4(r.q[k]));
+            quad_d.insert(quad_d.end(), r.d, r.d + 12);
+            quad_sh.push_back(i4(r.sh));
+            return (PT_QUAD << 28) | (uint32_t)(base[PT_QUAD] + quad_sh.size() - 1);
+        } else {
+            const rtprep::TriRec r = rtprep::make_triangle(b);
+            for (int k = 0; k < 3; k++) tri.push_back(f4(r.t[k]));
+            tri_d.insert(tri_d.end(), r.d, r.d + 9);
+            for (int k = 0; k < 3; k++) tri_sh.push_back(f4(r.sh[k]));
+            return (PT_TRI << 28) | (uint32_t)(base[PT_TRI] + tri_sh.size() / 3 - 1);
+        }
+    }
+};
+
+// A quad with an emissive material and a non-zero area joins the next-event emitter list (RT_FLAG_NEE); `area` is the
+// running total, the cdf is normalised by finish_emitters.
+static bool add_emitter(const rt_scene_desc* sc, const BakedPrim& b, std::vector<DevNeeLight>& lights, double& area_sum) {
+    if (b.dev_type != PT_QUAD || b.material < 0 || b.material >= sc->n_materials) return false;
+    const rt_material& m = sc->materials[b.material];
+    if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) return false;
+    const D3 nn = dcross(b.b, b.c);
+    const double area = std::sqrt(ddot(nn, nn));
+    if (!(area > 0.0)) return false;
+    DevNeeLight lt;
+    std::memset(&lt, 0, sizeof lt);
+    lt.Q[0] = (float)b.a.x; lt.Q[1] = (float)b.a.y; lt.Q[2] = (float)b.a.z;
+    lt.u[0] = (float)b.b.x; lt.u[1] = (float)b.b.y; lt.u[2] = (float)b.b.z;
+    lt.v[0] = (float)b.c.x; lt.v[1] = (float)b.c.y; lt.v[2] = (float)b.c.z;
+    lt.n[0] = (float)(nn.x / area); lt.n[1] = (float)(nn.y / area); lt.n[2] = (float)(nn.z / area);
+    lt.area = (float)area;
+    lt.tex = m.texture;
+    area_sum += area;
+    lt.cdf = (float)area_sum;
+    lights.push_back(lt);
+    return true;
+}
+static void finish_emitters(std::vector<DevNeeLight>& lights, double area_sum) {
+    for (DevNeeLight& lt : lights) lt.cdf = (float)(lt.cdf / area_sum);
+    if (!lights.empty()) lights.back().cdf = 1.0f;
+}
+
+// which boundary class a medium has: 1 one sphere, 2 a six-quad box (box_slabs), 0 general
+static int8_t media_class(const DevMedium& d) { return d.sphere >= 0 ? 1 : (d.box >= 0 ? 2 : 0); }
+
+// The scene's tables as the render kernels read them.  `boundaries` are the baked boundary primitives and
+// `boundary_packed` their records; the image table's texel pointers are left null.
+struct SceneTables {
+    std::vector<DevMaterial> mats;
+    std::vector<DevTexture> texs;
+    std::vector<DevImage> images;
+    std::vector<float4> perlin_vec;
+    std::vector<unsigned char> perlin_perm;
+    std::vector<DevMedium> media;
+    std::vector<float4> media_box;
+    std::vector<DevLight> lights;
+    std::vector<float> xrot;
+};
+static void derive_tables(const rt_scene_desc* sc, const BakedPrim* boundaries, const std::vector<uint32_t>& boundary_packed, SceneTables& T) {
+    std::vector<DevMaterial>& mats = T.mats;
+    mats.resize((size_t)sc->n_materials);
+    for (int i = 0; i < sc->n_materials; i++) {
+        const rt_material& m = sc->materials[i];
+        DevMaterial& d = mats[i];
+        d.type = m.type;
+        d.tex = m.texture;
+        for (int k = 0; k < 3; k++) d.albedo[k] = (float)m.albedo[k];
+        d.param = (float)m.param;
+        d.needs_uv = texture_needs_uv(sc, m.texture) ? 1 : 0;
+        d.pad = 0;
+    }
+    std::vector<DevTexture>& texs = T.texs;
+    texs.resize((size_t)sc->n_textures);
+    for (int i = 0; i < sc->n_textures; i++) {
+        const rt_texture& t = sc->textures[i];
+        DevTexture& d = texs[i];
+        d.type = t.type;
+        d.a = t.type == RT_TEX_IMAGE ? t.image : (t.type == RT_TEX_NOISE ? t.perlin : t.even);
+        d.b = t.odd;
+        d.scale = (float)t.scale;
+        for (int k = 0; k < 3; k++) d.color[k] = (float)t.color[k];
+        d.pad = 0;
+    }
+    std::vector<DevImage>& images = T.images;
+    images.resize((size_t)sc->n_images);
+    for (int i = 0; i < sc->n_images; i++) {
+        images[i].rgb = nullptr;
+        images[i].w = sc->images[i].width;
+        images[i].h = sc->images[i].height;
+    }
+    std::vector<float4>& perlin_vec = T.perlin_vec;
+    std::vector<unsigned char>& perlin_perm = T.perlin_perm;
+    perlin_vec.resize((size_t)sc->n_perlins * 256);
+    perlin_perm.resize((size_t)sc->n_perlins * 768);
+    for (int i = 0; i < sc->n_perlins; i++) {
+        const rt_perlin& p = sc->perlins[i];
+        for (int k = 0; k < 256; k++) {
+            perlin_vec[(size_t)i * 256 + k] = make_float4((float)p.randvec[k][0], (float)p.randvec[k][1], (float)p.randvec[k][2], 0.0f);
+            perlin_perm[(size_t)i * 768 + k] = (unsigned char)p.perm_x[k];
+            perlin_perm[(size_t)i * 768 + 256 + k] = (unsigned char)p.perm_y[k];
+            perlin_perm[(size_t)i * 768 + 512 + k] = (unsigned char)p.perm_z[k];
+        }
+    }
+    std::vector<DevMedium>& media = T.media;
+    std::vector<float4>& media_box = T.media_box;
+    media.resize((size_t)sc->n_media);
+    for (int i = 0; i < sc->n_media; i++) {
+        const rt_medium& m = sc->media[i];
+        DevMedium& d = media[i];
+        std::memset(&d, 0, sizeof d);
+        d.bfirst = m.boundary_first;
+        d.bcount = m.boundary_count;
+        d.neg_inv_density = (float)(-1.0 / (m.density * m.multiplicity));
+        d.material = m.material;
+        D3 n = xf_dir(m.xform >= 0 ? &sc->xforms[m.xform] : nullptr, D3{1, 0, 0});
+        d.normal[0] = (float)n.x; d.normal[1] = (float)n.y; d.normal[2] = (float)n.z;
+        d.sphere = -1;
+        d.box = -1;
+        if (m.boundary_count == 1 && (boundary_packed[m.boundary_first] >> 28) == PT_SPHERE)
+            d.sphere = (int)(boundary_packed[m.boundary_first] & 0x0fffffffu);
+        float4 slabs[4];
+        if (m.boundary_count == 6 && !getenv("RT_B200_NO_BOX_MEDIA") && box_slabs(boundaries + m.boundary_first, slabs)) {
+            d.box = (int)(media_box.size() / 4);
+            media_box.insert(media_box.end(), slabs, slabs + 4);
+        }
+    }
+    std::vector<DevLight>& lights = T.lights;
+    lights.resize((size_t)sc->n_lights);
+    for (int i = 0; i < sc->n_lights; i++) {
+        const rt_point_light& l = sc->lights[i];
+        for (int k = 0; k < 3; k++) { lights[i].pos[k] = (float)l.position[k]; lights[i].intensity[k] = (float)l.intensity[k]; }
+        lights[i].size = (float)l.size;
+        lights[i].pad = 0;
+    }
+    std::vector<float>& xrot = T.xrot;
+    xrot.resize((size_t)sc->n_xforms * 9);
+    for (int i = 0; i < sc->n_xforms; i++)
+        for (int k = 0; k < 9; k++) xrot[(size_t)i * 9 + k] = (float)sc->xforms[i].r[k];
+}
+
+// FEAT_* bits and the LITE conditions of a scene: `msph` / `tri`: it has moving spheres / triangles
+static void set_features(DevCtx* ctx, const rt_scene_desc* sc, const std::vector<DevMedium>& media, bool msph, bool tri) {
+    ctx->scene_feat = 0;
+    if (sc->n_media > 0) ctx->scene_feat |= FEAT_MEDIA;
+    for (const DevMedium& d : media)
+        if (d.sphere < 0) ctx->scene_feat |= FEAT_MEDIA_GENERAL;
+    for (int i = 0; i < sc->n_materials; i++)
+        if (sc->materials[i].type == RT_MAT_SPECULAR) ctx->scene_feat |= FEAT_SPECULAR;
+    if (msph) ctx->scene_feat |= FEAT_MSPHERE;
+    if (tri) ctx->scene_feat |= FEAT_TRI;
+    if (sc->n_lights > 0) ctx->scene_feat |= FEAT_LIGHTS;
+    if (sc->camera.defocus_angle > 0) ctx->scene_feat |= FEAT_DEFOCUS;
+    ctx->geom_lite = !tri && sc->n_lights == 0;
+    ctx->scene_lite = ctx->geom_lite && !(sc->camera.defocus_angle > 0);
+}
+
+// the work space of the device build and of rt_refit_scene, grown to `bytes`
+static int ensure_scratch(DevCtx* ctx, size_t bytes, const char* entry) {
+    if (bytes <= ctx->scratch_cap) return RT_OK;
+    if (ctx->scratch) cudaFree(ctx->scratch);
+    ctx->scratch = nullptr;
+    ctx->scratch_cap = 0;
+    size_t cap = bytes + bytes / 8;
+    if (cudaMalloc(&ctx->scratch, cap) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "%s: cannot allocate %zu bytes of build work space", entry, cap);
+    ctx->scratch_cap = cap;
+    return RT_OK;
+}
+
 static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_build, bool* too_deep) {
     auto t_begin = std::chrono::steady_clock::now();
+    int rc;
     const rtprep::Sources src{sc->spheres, sc->quads, sc->triangles, sc->xforms, sc->meshes};
     const int n_prims = ctx->n_prims;      // the world list with every mesh ref expanded: canonical ids 0 .. n_prims - 1
     size_t world_count[4] = {0, 0, 0, 0};  // device path: primitives of each device type the kernels will write
@@ -1404,64 +1623,19 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     const size_t first_boundary = device_build ? 0 : (size_t)n_prims;
 
     // ---- device arrays in leaf order, boundaries appended ------------------------------
-    std::vector<float4> sph, msph, quad, tri, tri_sh;
-    std::vector<double> sph_d, msph_d, quad_d, tri_d;
-    std::vector<int4> sph_sh, msph_sh, quad_sh;
+    TypedRecords recs;
+    for (int k = 0; k < 4; k++) recs.base[k] = world_count[k];
     std::vector<uint32_t> boundary_packed((size_t)sc->n_boundary_refs);
-    auto f4 = [](rtprep::F4 v) { return make_float4(v.x, v.y, v.z, v.w); };
-    auto i4 = [](rtprep::I4 v) { return make_int4(v.x, v.y, v.z, v.w); };
-    auto emit = [&](const BakedPrim& b) -> uint32_t {
-        if (b.dev_type == PT_SPHERE) {
-            const rtprep::SphereRec r = rtprep::make_sphere(b);
-            sph.push_back(f4(r.g));
-            sph_d.insert(sph_d.end(), r.d, r.d + 4);
-            sph_sh.push_back(i4(r.sh));
-            return (PT_SPHERE << 28) | (uint32_t)(world_count[PT_SPHERE] + sph.size() - 1);
-        } else if (b.dev_type == PT_MSPHERE) {
-            const rtprep::MSphereRec r = rtprep::make_msphere(b);
-            msph.push_back(f4(r.g0));
-            msph.push_back(f4(r.g1));
-            msph_d.insert(msph_d.end(), r.d, r.d + 8);
-            msph_sh.push_back(i4(r.sh));
-            return (PT_MSPHERE << 28) | (uint32_t)(world_count[PT_MSPHERE] + msph_sh.size() - 1);
-        } else if (b.dev_type == PT_QUAD) {
-            const rtprep::QuadRec r = rtprep::make_quad(b);
-            for (int k = 0; k < 3; k++) quad.push_back(f4(r.q[k]));
-            quad_d.insert(quad_d.end(), r.d, r.d + 12);
-            quad_sh.push_back(i4(r.sh));
-            return (PT_QUAD << 28) | (uint32_t)(world_count[PT_QUAD] + quad_sh.size() - 1);
-        } else {
-            const rtprep::TriRec r = rtprep::make_triangle(b);
-            for (int k = 0; k < 3; k++) tri.push_back(f4(r.t[k]));
-            tri_d.insert(tri_d.end(), r.d, r.d + 9);
-            for (int k = 0; k < 3; k++) tri_sh.push_back(f4(r.sh[k]));
-            return (PT_TRI << 28) | (uint32_t)(world_count[PT_TRI] + tri_sh.size() / 3 - 1);
-        }
-    };
     // quads with an emissive material are also listed for the opt-in next-event estimation
     std::vector<DevNeeLight> nee_lights;
+    std::vector<int32_t> nee_ids;
     double nee_area = 0.0;
     for (uint32_t id : bvh.order) {
         const BakedPrim& b = baked[id];
-        const uint32_t packed = emit(b);
-        if (b.dev_type != PT_QUAD || b.material < 0) continue;
-        const rt_material& m = sc->materials[b.material];
-        if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) continue;
-        const D3 nn = dcross(b.b, b.c);
-        const double area = std::sqrt(ddot(nn, nn));
-        if (!(area > 0.0)) continue;
-        DevNeeLight lt;
-        std::memset(&lt, 0, sizeof lt);
-        lt.Q[0] = (float)b.a.x; lt.Q[1] = (float)b.a.y; lt.Q[2] = (float)b.a.z;
-        lt.u[0] = (float)b.b.x; lt.u[1] = (float)b.b.y; lt.u[2] = (float)b.b.z;
-        lt.v[0] = (float)b.c.x; lt.v[1] = (float)b.c.y; lt.v[2] = (float)b.c.z;
-        lt.n[0] = (float)(nn.x / area); lt.n[1] = (float)(nn.y / area); lt.n[2] = (float)(nn.z / area);
-        lt.area = (float)area;
-        lt.tex = m.texture;
-        nee_area += area;
-        lt.cdf = (float)nee_area;  // normalised below
-        nee_lights.push_back(lt);
-        quad_sh[(packed & 0x0fffffffu) - world_count[PT_QUAD]].w = (int)nee_lights.size();
+        const uint32_t packed = recs.emit(b);
+        if (!add_emitter(sc, b, nee_lights, nee_area)) continue;
+        recs.quad_sh[(packed & 0x0fffffffu) - world_count[PT_QUAD]].w = (int)nee_lights.size();
+        nee_ids.push_back((int32_t)id);
     }
     // device path: the emitters are found in the source array (one pass over the quads, not over the
     // world list); the kernels that write the quad records look the light number up by source index
@@ -1473,106 +1647,19 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         for (int i = 0; i < sc->n_world; i++)
             if (sc->world[i].type == RT_PRIM_QUAD) in_world[(size_t)sc->world[i].index] = 1;
         for (int i = 0; i < sc->n_quads; i++) {
-            const rt_quad& q = sc->quads[i];
             if (!in_world[(size_t)i]) continue;
-            if (q.material < 0 || q.material >= sc->n_materials) continue;
-            const rt_material& m = sc->materials[q.material];
-            if (m.type != RT_MAT_DIFFUSE_LIGHT && m.type != RT_MAT_EMISSIVE_LIGHT) continue;
-            const BakedPrim b = rtprep::bake_prim(src, rt_prim_ref{RT_PRIM_QUAD, i}, -1);
-            const D3 nn = dcross(b.b, b.c);
-            const double area = std::sqrt(ddot(nn, nn));
-            if (!(area > 0.0)) continue;
-            DevNeeLight lt;
-            std::memset(&lt, 0, sizeof lt);
-            lt.Q[0] = (float)b.a.x; lt.Q[1] = (float)b.a.y; lt.Q[2] = (float)b.a.z;
-            lt.u[0] = (float)b.b.x; lt.u[1] = (float)b.b.y; lt.u[2] = (float)b.b.z;
-            lt.v[0] = (float)b.c.x; lt.v[1] = (float)b.c.y; lt.v[2] = (float)b.c.z;
-            lt.n[0] = (float)(nn.x / area); lt.n[1] = (float)(nn.y / area); lt.n[2] = (float)(nn.z / area);
-            lt.area = (float)area;
-            lt.tex = m.texture;
-            nee_area += area;
-            lt.cdf = (float)nee_area;
-            nee_lights.push_back(lt);
+            if (!add_emitter(sc, rtprep::bake_prim(src, rt_prim_ref{RT_PRIM_QUAD, i}, -1), nee_lights, nee_area)) continue;
             if (quad_light.empty()) quad_light.assign((size_t)sc->n_quads, 0);
             quad_light[(size_t)i] = (int32_t)nee_lights.size();
+            nee_ids.push_back(i);
         }
     }
-    for (DevNeeLight& lt : nee_lights) lt.cdf = (float)(lt.cdf / nee_area);
-    if (!nee_lights.empty()) nee_lights.back().cdf = 1.0f;
-    for (int i = 0; i < sc->n_boundary_refs; i++) boundary_packed[i] = emit(baked[first_boundary + i]);
+    finish_emitters(nee_lights, nee_area);
+    for (int i = 0; i < sc->n_boundary_refs; i++) boundary_packed[i] = recs.emit(baked[first_boundary + i]);
 
     // ---- tables ---------------------------------------------------------------------------
-    std::vector<DevMaterial> mats((size_t)sc->n_materials);
-    for (int i = 0; i < sc->n_materials; i++) {
-        const rt_material& m = sc->materials[i];
-        DevMaterial& d = mats[i];
-        d.type = m.type;
-        d.tex = m.texture;
-        for (int k = 0; k < 3; k++) d.albedo[k] = (float)m.albedo[k];
-        d.param = (float)m.param;
-        d.needs_uv = texture_needs_uv(sc, m.texture) ? 1 : 0;
-        d.pad = 0;
-    }
-    std::vector<DevTexture> texs((size_t)sc->n_textures);
-    for (int i = 0; i < sc->n_textures; i++) {
-        const rt_texture& t = sc->textures[i];
-        DevTexture& d = texs[i];
-        d.type = t.type;
-        d.a = t.type == RT_TEX_IMAGE ? t.image : (t.type == RT_TEX_NOISE ? t.perlin : t.even);
-        d.b = t.odd;
-        d.scale = (float)t.scale;
-        for (int k = 0; k < 3; k++) d.color[k] = (float)t.color[k];
-        d.pad = 0;
-    }
-    std::vector<DevImage> images((size_t)sc->n_images);
-    for (int i = 0; i < sc->n_images; i++) {
-        images[i].rgb = nullptr;  // patched once the arena address is known
-        images[i].w = sc->images[i].width;
-        images[i].h = sc->images[i].height;
-    }
-    std::vector<float4> perlin_vec((size_t)sc->n_perlins * 256);
-    std::vector<unsigned char> perlin_perm((size_t)sc->n_perlins * 768);
-    for (int i = 0; i < sc->n_perlins; i++) {
-        const rt_perlin& p = sc->perlins[i];
-        for (int k = 0; k < 256; k++) {
-            perlin_vec[(size_t)i * 256 + k] = make_float4((float)p.randvec[k][0], (float)p.randvec[k][1], (float)p.randvec[k][2], 0.0f);
-            perlin_perm[(size_t)i * 768 + k] = (unsigned char)p.perm_x[k];
-            perlin_perm[(size_t)i * 768 + 256 + k] = (unsigned char)p.perm_y[k];
-            perlin_perm[(size_t)i * 768 + 512 + k] = (unsigned char)p.perm_z[k];
-        }
-    }
-    std::vector<DevMedium> media((size_t)sc->n_media);
-    std::vector<float4> media_box;
-    for (int i = 0; i < sc->n_media; i++) {
-        const rt_medium& m = sc->media[i];
-        DevMedium& d = media[i];
-        std::memset(&d, 0, sizeof d);
-        d.bfirst = m.boundary_first;
-        d.bcount = m.boundary_count;
-        d.neg_inv_density = (float)(-1.0 / (m.density * m.multiplicity));
-        d.material = m.material;
-        D3 n = xf_dir(m.xform >= 0 ? &sc->xforms[m.xform] : nullptr, D3{1, 0, 0});
-        d.normal[0] = (float)n.x; d.normal[1] = (float)n.y; d.normal[2] = (float)n.z;
-        d.sphere = -1;
-        d.box = -1;
-        if (m.boundary_count == 1 && (boundary_packed[m.boundary_first] >> 28) == PT_SPHERE)
-            d.sphere = (int)(boundary_packed[m.boundary_first] & 0x0fffffffu);
-        float4 slabs[4];
-        if (m.boundary_count == 6 && !getenv("RT_B200_NO_BOX_MEDIA") && box_slabs(&baked[first_boundary + (size_t)m.boundary_first], slabs)) {
-            d.box = (int)(media_box.size() / 4);
-            media_box.insert(media_box.end(), slabs, slabs + 4);
-        }
-    }
-    std::vector<DevLight> lights((size_t)sc->n_lights);
-    for (int i = 0; i < sc->n_lights; i++) {
-        const rt_point_light& l = sc->lights[i];
-        for (int k = 0; k < 3; k++) { lights[i].pos[k] = (float)l.position[k]; lights[i].intensity[k] = (float)l.intensity[k]; }
-        lights[i].size = (float)l.size;
-        lights[i].pad = 0;
-    }
-    std::vector<float> xrot((size_t)sc->n_xforms * 9);
-    for (int i = 0; i < sc->n_xforms; i++)
-        for (int k = 0; k < 9; k++) xrot[(size_t)i * 9 + k] = (float)sc->xforms[i].r[k];
+    SceneTables tables;
+    derive_tables(sc, baked.data() + first_boundary, boundary_packed, tables);
 
     std::vector<float4> nodes(bvh.nodes.size() * 4);
     static_assert(sizeof(rtbvh::Node) == 64, "node layout");
@@ -1619,7 +1706,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     // device path: n - 1 radix-tree slots + room for the SAH top tree over at most kMaxClusters clusters
     const size_t node_skip = device_build ? ((size_t)(n_prims - 1) + rtlbvh::kMaxClusters) * 64 : 0;
 #define UP(vec, field) add_block(vec.data(), vec.size() * sizeof(vec[0]), 0, (const void**)&S.field);
-#define UPW(vec, field, type, rec_bytes) add_block(vec.data(), vec.size() * sizeof(vec[0]), world_count[type] * (size_t)(rec_bytes), (const void**)&S.field);
+#define UPW(vec, field, type, rec_bytes) add_block(recs.vec.data(), recs.vec.size() * sizeof(recs.vec[0]), world_count[type] * (size_t)(rec_bytes), (const void**)&S.field);
     add_block(nodes.data(), device_build ? 0 : nodes.size() * sizeof(float4), node_skip, (const void**)&S.nodes);
     if (wide.n_nodes) {
         add_block(wide.words.data(), wide.words.size() * sizeof(uint32_t), 0, (const void**)&S.wnodes);
@@ -1628,9 +1715,9 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     UPW(sph, sph, PT_SPHERE, 16) UPW(msph, msph, PT_MSPHERE, 32) UPW(quad, quad, PT_QUAD, 48) UPW(tri, tri, PT_TRI, 48)
     UPW(sph_d, sph_d, PT_SPHERE, 32) UPW(msph_d, msph_d, PT_MSPHERE, 64) UPW(quad_d, quad_d, PT_QUAD, 96) UPW(tri_d, tri_d, PT_TRI, 72)
     UPW(sph_sh, sph_sh, PT_SPHERE, 16) UPW(msph_sh, msph_sh, PT_MSPHERE, 16) UPW(quad_sh, quad_sh, PT_QUAD, 16) UPW(tri_sh, tri_sh, PT_TRI, 48)
-    UP(xrot, xrot) UP(media, media) UP(media_box, media_box)
-    UP(boundary_packed, boundary) UP(mats, mats) UP(texs, texs) UP(images, images) UP(perlin_vec, perlin_vec)
-    UP(perlin_perm, perlin_perm) UP(lights, lights) UP(nee_lights, nee_lights)
+    UP(tables.xrot, xrot) UP(tables.media, media) UP(tables.media_box, media_box)
+    UP(boundary_packed, boundary) UP(tables.mats, mats) UP(tables.texs, texs) UP(tables.images, images) UP(tables.perlin_vec, perlin_vec)
+    UP(tables.perlin_perm, perlin_perm) UP(tables.lights, lights) UP(nee_lights, nee_lights)
 #undef UP
 #undef UPW
     if (plan.size > ctx->arena_cap) {
@@ -1652,7 +1739,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
         ctx->staging_cap = cap;
     }
     for (int i = 0; i < sc->n_images; i++) {
-        images[i].rgb = ctx->arena + img_off[i];
+        tables.images[i].rgb = ctx->arena + img_off[i];
         std::memcpy(ctx->staging + (device_build ? img_stage[i] : img_off[i]), sc->images[i].rgb, (size_t)sc->images[i].width * sc->images[i].height * 3);
     }
     for (const Block& b : blocks) {
@@ -1682,14 +1769,7 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
                 staged += b.bytes;
             }
         const rtlbvh::Layout L = rtlbvh::plan_scratch(sc, n_prims);
-        if (L.total > ctx->scratch_cap) {
-            if (ctx->scratch) cudaFree(ctx->scratch);
-            ctx->scratch = nullptr;
-            ctx->scratch_cap = 0;
-            size_t cap = L.total + L.total / 8;
-            if (cudaMalloc(&ctx->scratch, cap) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_upload_scene: cannot allocate %zu bytes of build work space", cap);
-            ctx->scratch_cap = cap;
-        }
+        if ((rc = ensure_scratch(ctx, L.total, "rt_upload_scene")) != RT_OK) return rc;
         rtlbvh::Targets T;
         T.nodes = (float4*)S.nodes;
         T.sph = (float4*)S.sph; T.msph = (float4*)S.msph; T.quad = (float4*)S.quad; T.tri = (float4*)S.tri; T.tri_sh = (float4*)S.tri_sh;
@@ -1737,20 +1817,31 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     ctx->camera = sc->camera;
     ctx->n_materials = sc->n_materials;
     ctx->n_textures = sc->n_textures;
-    ctx->scene_feat = 0;
-    if (sc->n_media > 0) ctx->scene_feat |= FEAT_MEDIA;
-    for (const DevMedium& d : media)
-        if (d.sphere < 0) ctx->scene_feat |= FEAT_MEDIA_GENERAL;
-    for (int i = 0; i < sc->n_materials; i++)
-        if (sc->materials[i].type == RT_MAT_SPECULAR) ctx->scene_feat |= FEAT_SPECULAR;
-    if (world_count[PT_MSPHERE] > 0 || !msph.empty()) ctx->scene_feat |= FEAT_MSPHERE;
-    if (!tri.empty() || world_count[PT_TRI] > 0) ctx->scene_feat |= FEAT_TRI;
-    if (sc->n_lights > 0) ctx->scene_feat |= FEAT_LIGHTS;
-    if (sc->camera.defocus_angle > 0) ctx->scene_feat |= FEAT_DEFOCUS;
-    ctx->geom_lite = tri.empty() && world_count[PT_TRI] == 0 && sc->n_lights == 0;
-    ctx->scene_lite = ctx->geom_lite && !(sc->camera.defocus_angle > 0);
+    set_features(ctx, sc, tables.media, world_count[PT_MSPHERE] > 0 || !recs.msph.empty(), !recs.tri.empty() || world_count[PT_TRI] > 0);
     ctx->cam_w = ctx->cam_h = 0;
     ctx->has_scene = true;
+    // the structure rt_refit_scene holds a description to
+    DevCtx::Shape& sh = ctx->shape;
+    const int32_t counts[13] = {sc->n_world, sc->n_boundary_refs, sc->n_spheres, sc->n_quads, sc->n_triangles, sc->n_media, sc->n_xforms,
+                                sc->n_materials, sc->n_textures, sc->n_images, sc->n_perlins, sc->n_lights, sc->n_meshes};
+    std::memcpy(sh.counts, counts, sizeof counts);
+    sh.mesh_tris.clear();
+    for (int i = 0; i < sc->n_meshes; i++) sh.mesh_tris.push_back(sc->meshes[i].n_triangles);
+    sh.image_wh.clear();
+    sh.image_dev.clear();
+    for (int i = 0; i < sc->n_images; i++) {
+        sh.image_wh.push_back(sc->images[i].width);
+        sh.image_wh.push_back(sc->images[i].height);
+        sh.image_dev.push_back(ctx->arena + img_off[i]);
+    }
+    sh.boundary_packed = boundary_packed;
+    sh.media_class.clear();
+    for (const DevMedium& d : tables.media) sh.media_class.push_back(media_class(d));
+    sh.nee_ids = nee_ids;
+    sh.n_prims = n_prims;
+    sh.device_built = device_build;
+    for (int k = 0; k < 4; k++) sh.world_type_count[k] = ctx->world_type_count[k];
+    ctx->refit_tree.levels.clear();
     ctx->stats.bvh_nodes = n_nodes;
     ctx->stats.bvh_depth = depth;
     ctx->stats.bvh_leaves = leaves;
@@ -1780,6 +1871,13 @@ static int dev_upload_scene(DevCtx* ctx, const rt_scene_desc* sc) {
     if (key && ctx->has_scene && ctx->staged_key == key && ctx->staged_bytes > 0) {
         CU(ctx, cudaMemcpyAsync(ctx->arena, ctx->staging, ctx->staged_bytes, cudaMemcpyHostToDevice, ctx->stream));
         CU(ctx, cudaStreamSynchronize(ctx->stream));
+        const DevCtx::SceneState& st = ctx->staged_state;
+        ctx->scene = st.scene;
+        ctx->camera = st.camera;
+        ctx->scene_feat = st.scene_feat;
+        ctx->scene_lite = st.scene_lite;
+        ctx->geom_lite = st.geom_lite;
+        ctx->cam_w = ctx->cam_h = 0;
         ctx->stats.scene_reused = 1;
         ctx->stats.upload_bytes = ctx->staged_bytes;
         ctx->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
@@ -1798,9 +1896,210 @@ static int dev_upload_scene(DevCtx* ctx, const rt_scene_desc* sc) {
         rc = upload_scene_impl(ctx, sc, false, &too_deep);  // degenerate input: the SAH tree is shallow
         if (cache) key = scene_key(ctx, sc);
     }
-    if (rc == RT_OK && ctx->staged_bytes > 0) ctx->staged_key = key;  // host path: the whole arena sits in the pinned staging buffer
+    if (rc == RT_OK && ctx->staged_bytes > 0) {  // host path: the whole arena sits in the pinned staging buffer
+        ctx->staged_key = key;
+        ctx->staged_state = DevCtx::SceneState{ctx->scene, ctx->camera, ctx->scene_feat, ctx->scene_lite, ctx->geom_lite};
+    }
     if (rc == RT_OK) ctx->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
     return rc;
+}
+
+// rt_refit_scene (bvh_refit.cuh): `sc` has the structure of the uploaded scene; its records, boxes and tables replace
+// the uploaded ones, the tree keeps its topology and leaf order.  Everything is checked before the arena is written:
+// a refused refit leaves the uploaded scene as it was.
+static int dev_refit_scene(DevCtx* ctx, const rt_scene_desc* sc) {
+    if (!ctx) return RT_ERR_INVALID;
+    auto t_begin = std::chrono::steady_clock::now();
+    if (!ctx->has_scene) return fail(ctx, RT_ERR_STATE, "rt_refit_scene: no scene uploaded (rt_upload_scene first)");
+    DevScene& S = ctx->scene;
+    if (S.wide_width)
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_refit_scene: the uploaded scene is traversed as a %d-wide tree; only the binary tree "
+                    "is refitted (rt_set_bvh_width(2) and rt_upload_scene)", S.wide_width);
+    // validated like an upload; the counts validate_scene leaves in ctx are the new description's, the uploaded
+    // scene's are kept with its structure
+    const DevCtx::Shape& sh = ctx->shape;
+    const int n_prims = sh.n_prims;
+    const size_t* type_count = sh.world_type_count;
+    size_t new_count[4];
+    int rc = validate_scene(ctx, sc, /*shallow=*/false);
+    const int new_prims = ctx->n_prims;
+    std::memcpy(new_count, ctx->world_type_count, sizeof new_count);
+    if (rc != RT_OK) {
+        if (ctx->error.rfind("rt_upload_scene", 0) == 0) ctx->error.replace(0, 15, "rt_refit_scene");
+        return rc;
+    }
+    // ---- the structure, on the host: counts, meshes, images, boundaries, emitters, media -----------------
+    static const char* kHint = "; a scene of another structure needs rt_upload_scene";
+    static const char* kKind[4] = {"sphere", "moving sphere", "quad", "triangle"};
+    static const char* kCountName[13] = {"n_world", "n_boundary_refs", "n_spheres", "n_quads", "n_triangles", "n_media", "n_xforms",
+                                         "n_materials", "n_textures", "n_images", "n_perlins", "n_lights", "n_meshes"};
+    const int32_t counts[13] = {sc->n_world, sc->n_boundary_refs, sc->n_spheres, sc->n_quads, sc->n_triangles, sc->n_media, sc->n_xforms,
+                                sc->n_materials, sc->n_textures, sc->n_images, sc->n_perlins, sc->n_lights, sc->n_meshes};
+    for (int k = 0; k < 13; k++)
+        if (counts[k] != sh.counts[k])
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: %s is %d, the uploaded scene's %d%s", kCountName[k], counts[k], sh.counts[k], kHint);
+    for (int i = 0; i < sc->n_meshes; i++)
+        if (sc->meshes[i].n_triangles != sh.mesh_tris[(size_t)i])
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: meshes[%d] has %d triangles, the uploaded scene's %d%s", i, sc->meshes[i].n_triangles,
+                        sh.mesh_tris[(size_t)i], kHint);
+    for (int i = 0; i < sc->n_images; i++)
+        if (sc->images[i].width != sh.image_wh[2 * (size_t)i] || sc->images[i].height != sh.image_wh[2 * (size_t)i + 1])
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: images[%d] is %dx%d, the uploaded scene's %dx%d%s", i, sc->images[i].width,
+                        sc->images[i].height, sh.image_wh[2 * (size_t)i], sh.image_wh[2 * (size_t)i + 1], kHint);
+    if (new_prims != n_prims)
+        return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: the world list has %d primitives, the uploaded scene %d%s", new_prims, n_prims, kHint);
+    for (int t = 0; t < 4; t++)
+        if (new_count[t] != type_count[t])
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: the world list has %zu primitives of kind %s, the uploaded scene %zu%s", new_count[t],
+                        kKind[t], type_count[t], kHint);
+    const rtprep::Sources src{sc->spheres, sc->quads, sc->triangles, sc->xforms, sc->meshes};
+    std::vector<BakedPrim> boundaries;
+    for (int i = 0; i < sc->n_boundary_refs; i++) {
+        boundaries.push_back(rtprep::bake_prim(src, sc->boundary_refs[i], -1));
+        const uint32_t was = sh.boundary_packed[(size_t)i] >> 28;
+        if (boundaries.back().dev_type != was)
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: boundary_refs[%d] changes kind (%s, the uploaded scene's %s)%s", i,
+                        kKind[boundaries.back().dev_type], kKind[was], kHint);
+    }
+    // the emitters of `sc` by the rule of the upload that built the tree, keyed like shape.nee_ids (ascending)
+    std::vector<std::pair<int32_t, BakedPrim>> emitters;
+    {
+        std::vector<DevNeeLight> probe;
+        double area = 0.0;
+        if (sh.device_built) {
+            std::vector<char> in_world((size_t)sc->n_quads, 0);
+            for (int i = 0; i < sc->n_world; i++)
+                if (sc->world[i].type == RT_PRIM_QUAD) in_world[(size_t)sc->world[i].index] = 1;
+            for (int i = 0; i < sc->n_quads; i++) {
+                if (!in_world[(size_t)i]) continue;
+                const BakedPrim b = rtprep::bake_prim(src, rt_prim_ref{RT_PRIM_QUAD, i}, -1);
+                if (add_emitter(sc, b, probe, area)) emitters.emplace_back(i, b);
+            }
+        } else {
+            int32_t id = 0;
+            for (int i = 0; i < sc->n_world; i++) {
+                const rt_prim_ref r = sc->world[i];
+                if (r.type == RT_PRIM_MESH) {
+                    id += sc->meshes[r.index].n_triangles;
+                    continue;
+                }
+                if (r.type == RT_PRIM_QUAD) {
+                    const BakedPrim b = rtprep::bake_prim(src, r, id);
+                    if (add_emitter(sc, b, probe, area)) emitters.emplace_back(id, b);
+                }
+                id++;
+            }
+        }
+    }
+    std::vector<int32_t> listed = sh.nee_ids;
+    std::sort(listed.begin(), listed.end());
+    for (size_t i = 0; i < std::max(listed.size(), emitters.size()); i++) {
+        const int32_t was = i < listed.size() ? listed[i] : INT32_MAX, now = i < emitters.size() ? emitters[i].first : INT32_MAX;
+        if (was != now)
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: %s %d %s the next-event emitter list (an emissive material and a non-zero area "
+                        "make a quad an emitter)%s", sh.device_built ? "source quad" : "primitive", std::min(was, now),
+                        was < now ? "leaves" : "joins", kHint);
+    }
+    std::vector<DevNeeLight> nee_lights;
+    double nee_area = 0.0;
+    for (int32_t id : sh.nee_ids) {
+        auto it = std::lower_bound(emitters.begin(), emitters.end(), id, [](const std::pair<int32_t, BakedPrim>& e, int32_t v) { return e.first < v; });
+        add_emitter(sc, it->second, nee_lights, nee_area);
+    }
+    finish_emitters(nee_lights, nee_area);
+    SceneTables tables;
+    derive_tables(sc, boundaries.data(), sh.boundary_packed, tables);
+    static const char* kClass[3] = {"general", "one sphere", "a six-quad box"};
+    for (int i = 0; i < sc->n_media; i++) {
+        const int8_t now = media_class(tables.media[(size_t)i]), was = sh.media_class[(size_t)i];
+        if (now != was)
+            return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: media[%d] changes its boundary class (%s, the uploaded scene's %s)%s", i, kClass[now],
+                        kClass[was], kHint);
+    }
+
+    // ---- the inputs on the device, and the kind of every world record slot's primitive -------------------
+    CU(ctx, cudaSetDevice(ctx->device));
+    const rtlbvh::Layout L = rtlbvh::plan_refit(sc, n_prims);
+    if ((rc = ensure_scratch(ctx, L.total, "rt_refit_scene")) != RT_OK) return rc;
+    if (L.largest_input >= 4 * rtlbvh::kCopyChunk) CU(ctx, ctx->copy_ring.init());
+    size_t bytes_in = 0;
+    CU(ctx, rtlbvh::copy_inputs(sc, ctx->scratch, L, ctx->stream, ctx->copy_ring, ctx->device, bytes_in));
+    rtlbvh::Scratch W = rtlbvh::input_view(sc, n_prims, ctx->scratch, L);
+    W.box_lo = (float4*)(ctx->scratch + L.box_lo);
+    W.box_hi = (float4*)(ctx->scratch + L.box_hi);
+    W.counters = (unsigned*)(ctx->scratch + L.counters);
+    const bool meshes = sc->n_meshes > 0;
+    if (meshes && n_prims > 0) CU(ctx, rtlbvh::map_prims(W, sc->n_world, ctx->scratch, L, ctx->scratch + L.cub_temp, L.cub_temp_bytes, ctx->stream));
+    rtlbvh::RefitSlots R;
+    R.T.nodes = (float4*)S.nodes;
+    R.T.sph = (float4*)S.sph; R.T.msph = (float4*)S.msph; R.T.quad = (float4*)S.quad; R.T.tri = (float4*)S.tri; R.T.tri_sh = (float4*)S.tri_sh;
+    R.T.sph_d = (double*)S.sph_d; R.T.msph_d = (double*)S.msph_d; R.T.quad_d = (double*)S.quad_d; R.T.tri_d = (double*)S.tri_d;
+    R.T.sph_sh = (int4*)S.sph_sh; R.T.msph_sh = (int4*)S.msph_sh; R.T.quad_sh = (int4*)S.quad_sh;
+    R.base[0] = 0;
+    for (int t = 0; t < 4; t++) R.base[t + 1] = R.base[t] + (unsigned)type_count[t];
+    // a device-built tree numbers its emitters by source quad, and a world quad may now name another source quad: the
+    // emitter number of each slot follows its quad, as prims_kernel sets it at upload
+    R.quad_light = nullptr;
+    if (sh.device_built && !sh.nee_ids.empty()) {
+        std::vector<int32_t> quad_light((size_t)sc->n_quads, 0);
+        for (size_t k = 0; k < sh.nee_ids.size(); k++) quad_light[(size_t)sh.nee_ids[k]] = (int32_t)(k + 1);
+        CU(ctx, rtlbvh::copy_in(ctx->scratch + L.quad_light, quad_light.data(), quad_light.size() * sizeof(int32_t), ctx->stream, ctx->copy_ring,
+                                ctx->device));
+        bytes_in += quad_light.size() * sizeof(int32_t);
+        R.quad_light = (const int*)(ctx->scratch + L.quad_light);
+    }
+    unsigned bad = ~0u;
+    if (n_prims > 0) {
+        CU(ctx, cudaMemsetAsync(W.counters, 0xff, sizeof bad, ctx->stream));
+        if (meshes) rtlbvh::refit_check_kernel<true><<<(n_prims + 255) / 256, 256, 0, ctx->stream>>>(W, R, W.counters);
+        else rtlbvh::refit_check_kernel<false><<<(n_prims + 255) / 256, 256, 0, ctx->stream>>>(W, R, W.counters);
+        CU(ctx, cudaGetLastError());
+        CU(ctx, cudaMemcpyAsync(&bad, W.counters, sizeof bad, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    if (bad != ~0u)
+        return fail(ctx, RT_ERR_INVALID, "rt_refit_scene: world primitive %u changes kind (%s, the uploaded scene's %s)%s", bad >> 4, kKind[bad & 3u],
+                    kKind[(bad >> 2) & 3u], kHint);
+    // the uploaded tree in breadth-first order, once per upload (n_world == 0: the root is never followed)
+    const bool has_tree = S.n_world > 0 && S.root >= 0;
+    if (has_tree && ctx->refit_tree.levels.empty()) {
+        bool ok = false;
+        CU(ctx, rtlbvh::derive_refit_tree(ctx->refit_tree, S.nodes, S.root, S.n_nodes, STACK_SIZE, ctx->sm_count, ctx->stream, ok));
+        if (!ok) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_refit_scene: the uploaded tree has more than %d levels", STACK_SIZE);
+    }
+
+    // ---- from here on the arena is written: wait for the passes that read it, like an upload ---------------
+    rc = dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    CU(ctx, rtlbvh::refit_on_device(W, R, meshes, (float4*)S.nodes, ctx->refit_tree, ctx->stream));
+    TypedRecords recs;
+    for (int k = 0; k < 4; k++) recs.base[k] = type_count[k];
+    for (const BakedPrim& b : boundaries) recs.emit(b);
+    auto put = [&](const void* dst, const void* host, size_t bytes) -> cudaError_t {
+        if (!bytes) return cudaSuccess;
+        bytes_in += bytes;
+        return cudaMemcpyAsync((void*)dst, host, bytes, cudaMemcpyHostToDevice, ctx->stream);
+    };
+#define PUT(vec, field) CU(ctx, put(S.field, vec.data(), vec.size() * sizeof(vec[0])));
+#define PUTW(vec, field, type, rec_bytes) \
+    CU(ctx, put((const unsigned char*)S.field + type_count[type] * (size_t)(rec_bytes), recs.vec.data(), recs.vec.size() * sizeof(recs.vec[0])));
+    PUTW(sph, sph, PT_SPHERE, 16) PUTW(msph, msph, PT_MSPHERE, 32) PUTW(quad, quad, PT_QUAD, 48) PUTW(tri, tri, PT_TRI, 48)
+    PUTW(sph_d, sph_d, PT_SPHERE, 32) PUTW(msph_d, msph_d, PT_MSPHERE, 64) PUTW(quad_d, quad_d, PT_QUAD, 96) PUTW(tri_d, tri_d, PT_TRI, 72)
+    PUTW(sph_sh, sph_sh, PT_SPHERE, 16) PUTW(msph_sh, msph_sh, PT_MSPHERE, 16) PUTW(quad_sh, quad_sh, PT_QUAD, 16) PUTW(tri_sh, tri_sh, PT_TRI, 48)
+    PUT(tables.xrot, xrot) PUT(tables.media, media) PUT(tables.media_box, media_box) PUT(tables.mats, mats) PUT(tables.texs, texs)
+    PUT(tables.perlin_vec, perlin_vec) PUT(tables.perlin_perm, perlin_perm) PUT(tables.lights, lights) PUT(nee_lights, nee_lights)
+#undef PUT
+#undef PUTW
+    for (int i = 0; i < sc->n_images; i++) CU(ctx, put(sh.image_dev[(size_t)i], sc->images[i].rgb, (size_t)sc->images[i].width * sc->images[i].height * 3));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    S.nee_total_area = (float)nee_area;
+    ctx->camera = sc->camera;
+    ctx->cam_w = ctx->cam_h = 0;
+    set_features(ctx, sc, tables.media, type_count[PT_MSPHERE] > 0 || !recs.msph.empty(), !recs.tri.empty() || type_count[PT_TRI] > 0);
+    ctx->stats.scene_reused = 0;
+    ctx->stats.upload_bytes = bytes_in;
+    ctx->stats.upload_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
+    return RT_OK;
 }
 
 // 0 auto, 1 host SAH, 2 device LBVH: which builder the next rt_upload_scene uses
