@@ -41,6 +41,8 @@ int main(int argc, char** argv) {
     //            --noise X [--noise-every N]  stop once the relative frame noise is <= X, checked every N samples (default 256)
     //            --variance FILE.exr|.pfm     also write the per-pixel sample variance
     //            --turntable N                N views around lookat in one batch, written to <stem>_000<ext> ...
+    //            --aov FILE.exr|.pfm          also write the antialiased first-hit albedo, normal and depth to
+    //                                         <stem>_albedo<ext>, <stem>_normal<ext>, <stem>_depth<ext>
     for (int i = 7; i + 1 < argc; i += 2) {
         std::string k = argv[i];
         if (k == "--checkpoint") cam.checkpoint_path = argv[i + 1];
@@ -52,6 +54,7 @@ int main(int argc, char** argv) {
         else if (k == "--noise-every") cam.noise_check_every_spp = std::atoi(argv[i + 1]);
         else if (k == "--variance") cam.variance_name = argv[i + 1];
         else if (k == "--turntable") cam.turntable_frames = std::atoi(argv[i + 1]);
+        else if (k == "--aov") cam.aov_name = argv[i + 1];
         else if (k == "--shadowed-point-lights") cam.shadowed_point_lights = std::atoi(argv[i + 1]) != 0;
         else if (k == "--devices") {
             std::string v = argv[i + 1];

@@ -270,6 +270,13 @@ typedef enum rt_shard_mode {
                                  whose moments describe its sums (RT_ERR_STATE otherwise), and one without it leaves the
                                  frame without moments.  Runs the general kernel instances (plain / NEE); with RT_FLAG_STATS
                                  it is RT_ERR_UNSUPPORTED.  The image is the same as without the flag. */
+#define RT_FLAG_AOV 256u      /* also add each camera sample's first-vertex albedo, normal, depth and hit to AOV sums of the
+                                 context (64 bytes per pixel, the layout of the sums), read with rt_download_aov.  The
+                                 state rules are those of RT_FLAG_MOMENTS: a pass without RT_FLAG_ACCUMULATE starts them;
+                                 an accumulating pass with the flag needs a frame whose AOV sums describe its sums
+                                 (RT_ERR_STATE otherwise); a pass without it, and rt_accum_upload, leave the frame without
+                                 them.  Runs the general kernel instances (plain / NEE); with RT_FLAG_STATS or
+                                 RT_FLAG_MOMENTS it is RT_ERR_UNSUPPORTED.  The image is the same as without the flag. */
 
 typedef struct rt_render_params {
     uint32_t struct_size;
@@ -425,7 +432,7 @@ int rt_download(rt_ctx* ctx, int32_t total_spp, float* rgb_linear, uint8_t* rgb8
  * and seed (seeds[v] when seeds != NULL).  cameras[v].background must equal the uploaded camera's (RT_ERR_INVALID
  * otherwise), as must n_views >= 1 and cameras != NULL.
  *   - flags: RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_NEE and RT_FLAG_SHADOWED_POINT_LIGHTS; params->stream is honoured.
- *     RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, shard_count > 1 and multi-device contexts are
+ *     RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_AOV, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, shard_count > 1 and multi-device contexts are
  *     RT_ERR_UNSUPPORTED, and so is a frame of n_views x width x height >= 2^31 slots.
  *   - the views frame is a buffer of its own: a views render does not touch the frame, moments or bound buffer of
  *     rt_render, and rt_render does not touch the views frame.
@@ -498,6 +505,29 @@ int rt_moments_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, int32_t w
  * (saturating at 2^64 - 1), then divided once on the host.  Covers the pixels the context holds (a compact shard: its
  * own tiles).  Multi-device contexts: as rt_download_variance. */
 int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double* rms_std_error);
+
+/* Auxiliary outputs of a frame rendered with RT_FLAG_AOV: the standard inputs of an external denoiser (albedo, normal)
+ * and the depth of compositing, antialiased like the radiance because they come from the same camera samples.  They are
+ * taken at the first event of each camera sample, with values the path computes there and no random number of its own:
+ *   surface that scatters   albedo = the attenuation of the bounce (texture value for lambertian and isotropic, albedo for
+ *                           metal -- also a sample the metal absorbs -- and specular, 1 for dielectric); normal = the
+ *                           shading normal facing the ray (world space); depth = t |d|, the distance from the camera
+ *                           ray's origin (on the lens when defocused); a hit
+ *   light                   albedo = the emitted radiance clamped to [0, 1]; normal and depth as above; a hit
+ *   medium scatter event    albedo = the isotropic attenuation; normal 0; depth = the distance to the event; a hit
+ *   miss                    albedo = the background clamped to [0, 1]; normal 0; no depth; no hit
+ * The sums are 8 uint64 per pixel: albedo x3 and depth unsigned, clamped to [0, 2^20], normal x3 signed (two's
+ * complement), clamped to [-1, 1], all in 2^-RT_ACCUM_FRAC_BITS units, then the hit count.  A sample adds at most 2^48 to a
+ * word (2^28 in magnitude to a normal word), so with at most 65536 samples per pixel no word overflows however the
+ * samples are split -- save for 65536 samples all saturated at 2^20, the edge the radiance words share -- and, like the
+ * radiance sums, they are bit-identical for any device count, shard, pass split, overlap or resume.
+ * rt_download_aov writes width*height*8 floats, row-major and full-frame like rgb_linear (a compact shard: its own tiles,
+ * zero elsewhere); per pixel albedo r, g, b, normal x, y, z, depth, coverage, each computed in double and rounded once to
+ * float: albedo and normal sum / (2^28 n) with n = total_spp, depth sum / (2^28 hits) (0 without a hit), coverage hits / n.
+ * So the albedo and the normal average over all n samples, misses included, and the depth over the samples that hit.
+ * total_spp <= 0 is RT_ERR_INVALID, a frame without valid AOV sums RT_ERR_STATE.  Multi-device contexts: tile-sharded
+ * frames without a restored checkpoint (else RT_ERR_UNSUPPORTED).  Ordered after outstanding hand-outs like rt_download. */
+int rt_download_aov(rt_ctx* ctx, int32_t total_spp, float* aov);
 
 /* Compact tile buffers across processes (one process per GPU, e.g. under torchrun; single-device contexts):
  *   rt_shard_pixels   slots of the compact buffer of shard (rank, count): its tiles x tile_size^2 (edge tiles padded)

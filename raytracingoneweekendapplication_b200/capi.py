@@ -25,6 +25,7 @@ RT_SHARD_AUTO, RT_SHARD_TILES, RT_SHARD_SAMPLES = range(3)
 RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_STATS, RT_FLAG_NEE, RT_FLAG_SHADOWED_POINT_LIGHTS, RT_FLAG_COMPACT_TILES = 1, 2, 4, 8, 16, 32
 RT_FLAG_OVERLAP = 64
 RT_FLAG_MOMENTS = 128
+RT_FLAG_AOV = 256
 
 d3 = C.c_double * 3
 
@@ -151,7 +152,7 @@ EXPORTED_SYMBOLS = [
     "rt_set_bvh_width", "rt_device_count", "rt_shard_pixels", "rt_resolve_tiles", "rt_untile",
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
     "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
-    "rt_render_views", "rt_download_views", "rt_refit_scene",
+    "rt_render_views", "rt_download_views", "rt_refit_scene", "rt_download_aov",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
@@ -218,6 +219,7 @@ def load() -> C.CDLL:
     lib.rt_moments_download.argtypes = [vp, vp, C.c_size_t]
     lib.rt_moments_upload.argtypes = [vp, vp, C.c_size_t, i32, i32]
     lib.rt_frame_noise.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    lib.rt_download_aov.argtypes = [vp, i32, vp]
     lib.rt_render_views.argtypes = [vp, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.POINTER(C.c_uint64), i32]
     lib.rt_download_views.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double)]
@@ -403,7 +405,7 @@ class Context:
                accumulate: bool = False, stats: bool = False, shard_rank: int = 0, shard_count: int = 1,
                shard_mode: int = RT_SHARD_AUTO, tile_size: int = 0, stream: Optional[int] = None, blocking: bool = True,
                nee: bool = False, shadowed_point_lights: bool = False, compact: bool = False, overlap: bool = False,
-               moments: bool = False) -> None:
+               moments: bool = False, aov: bool = False) -> None:
         p = rt_render_params()
         p.struct_size = C.sizeof(rt_render_params)
         p.width, p.height, p.samples_per_pixel, p.max_depth = width, height, spp, max_depth
@@ -411,7 +413,8 @@ class Context:
         p.shard_mode, p.shard_rank, p.shard_count = shard_mode, shard_rank, shard_count
         p.flags = ((RT_FLAG_ACCUMULATE if accumulate else 0) | (RT_FLAG_STATS if stats else 0) | (0 if blocking else RT_FLAG_ASYNC) |
                    (RT_FLAG_NEE if nee else 0) | (RT_FLAG_SHADOWED_POINT_LIGHTS if shadowed_point_lights else 0) |
-                   (RT_FLAG_COMPACT_TILES if compact else 0) | (RT_FLAG_OVERLAP if overlap else 0) | (RT_FLAG_MOMENTS if moments else 0))
+                   (RT_FLAG_COMPACT_TILES if compact else 0) | (RT_FLAG_OVERLAP if overlap else 0) | (RT_FLAG_MOMENTS if moments else 0) |
+                   (RT_FLAG_AOV if aov else 0))
         p.stream = stream
         self._check(self.lib.rt_render(self._h, C.byref(p)))
         self.width, self.height = width, height
@@ -563,6 +566,13 @@ class Context:
         mean, rms = C.c_double(), C.c_double()
         self._check(self.lib.rt_frame_noise(self._h, total_spp, C.byref(mean), C.byref(rms)))
         return mean.value, rms.value
+
+    def download_aov(self, total_spp: int) -> dict:
+        """The auxiliary outputs of a frame rendered with aov=True: `albedo` (H, W, 3), `normal` (H, W, 3), `depth` (H, W)
+        and `coverage` (H, W) float32, views of one (H, W, 8) array (their `.base`)."""
+        out = np.empty((self.height, self.width, 8), dtype=np.float32)
+        self._check(self.lib.rt_download_aov(self._h, total_spp, out.ctypes.data))
+        return {"albedo": out[..., 0:3], "normal": out[..., 3:6], "depth": out[..., 6], "coverage": out[..., 7]}
 
     def stats(self) -> dict:
         st = rt_stats()

@@ -369,13 +369,14 @@ static bool one_device_per_pixel(const rt_ctx* ctx) {
     return ctx->dev[0]->acc.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size();
 }
 
-// What a device contributes to a gather: its raw sums, or its slots resolved or turned into variance on the device
-enum class Plane { Sums, Rgb8, Linear, Variance };
+// What a device contributes to a gather: its raw sums, or its slots resolved, turned into variance or its AOV sums
+// resolved on the device
+enum class Plane { Sums, Rgb8, Linear, Variance, Aov };
 
 // The plane of every device's slots, produced on that device and gathered on device 0 (device d at ctx->gather + d * *stride)
 static int gather_plane(rt_ctx* ctx, Plane what, int32_t total_spp, size_t* stride) {
     const int n = (int)ctx->dev.size();
-    const size_t bpp = what == Plane::Sums ? 32 : what == Plane::Rgb8 ? 3 : 12;
+    const size_t bpp = what == Plane::Sums || what == Plane::Aov ? 32 : what == Plane::Rgb8 ? 3 : 12;
     const bool resolve = what == Plane::Rgb8 || what == Plane::Linear;
     std::vector<const void*> src((size_t)n);
     std::vector<size_t> bytes((size_t)n);
@@ -383,13 +384,15 @@ static int gather_plane(rt_ctx* ctx, Plane what, int32_t total_spp, size_t* stri
     for (int d = 0; d < n; d++) {
         DevCtx* dc = ctx->dev[d];
         const size_t slots = dc->acc.slots();
-        int rc = what == Plane::Variance ? moments_ready(dc, "rt_download_variance") : dev_wait(dc);
+        int rc = what == Plane::Variance ? moments_ready(dc, "rt_download_variance") : what == Plane::Aov ? aov_ready(dc, "rt_download_aov") : dev_wait(dc);
         if (rc == RT_OK && what == Plane::Variance) rc = dev_variance_into(dc, total_spp);
+        const void* aov_plane = nullptr;
+        if (rc == RT_OK && what == Plane::Aov) rc = dev_aov_into(dc, total_spp, 0, &aov_plane);
         if (rc == RT_OK && resolve) rc = stage_buffers(dc, slots, 0);
         if (rc == RT_OK && resolve)
             rc = dev_resolve_into(dc, dc->accum, slots, total_spp, what == Plane::Linear ? dc->out_lin : nullptr, what == Plane::Rgb8 ? dc->out_rgb8 : nullptr);
         if (rc != RT_OK) return fwd(ctx, dc, rc);
-        src[d] = what == Plane::Sums ? (const void*)dc->accum : what == Plane::Rgb8 ? (const void*)dc->out_rgb8 : (const void*)dc->out_lin;
+        src[d] = what == Plane::Sums ? (const void*)dc->accum : what == Plane::Aov ? aov_plane : what == Plane::Rgb8 ? (const void*)dc->out_rgb8 : (const void*)dc->out_lin;
         bytes[d] = slots * bpp;
         *stride = std::max(*stride, (bytes[d] + 255) & ~(size_t)255);
     }
@@ -488,6 +491,7 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
         if (d->accum && !d->accum_external) CUX(ctx, cudaMemsetAsync(d->accum, 0, d->accum_bytes, d->stream));
         CUX(ctx, cudaStreamSynchronize(d->stream));
         d->moments_valid = false;  // moments are not restored across devices (rt_moments_upload is single-device)
+        d->aov_valid = false;      // nor are the AOV sums
     }
     cudaSetDevice(d0->device);
     if (ctx->base_sums) cudaFree(ctx->base_sums);
@@ -500,9 +504,10 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
     return RT_OK;
 }
 
-// ---- second moments (RT_FLAG_MOMENTS) ------------------------------------------------------------------------------
-// A multi-device frame has per-device variance only when each pixel lives on one device: tiles, no restored checkpoint.
-static int multi_moments_frame(rt_ctx* ctx, const char* what) {
+// ---- second moments (RT_FLAG_MOMENTS) and auxiliary outputs (RT_FLAG_AOV) --------------------------------------------
+// A multi-device frame has per-device variance and AOVs only when each pixel lives on one device: tiles, no restored
+// checkpoint.
+static int multi_per_pixel_frame(rt_ctx* ctx, const char* what) {
     if (!ctx->rendered) return failx(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
     if (!one_device_per_pixel(ctx))
         return failx(ctx, RT_ERR_UNSUPPORTED, "%s: a multi-device context resolves tile-sharded frames without a restored checkpoint only", what);
@@ -515,7 +520,7 @@ extern "C" int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* varia
     if (n == 1) return fwd(ctx, ctx->dev[0], dev_download_variance(ctx->dev[0], total_spp, variance));
     if (!variance) return RT_ERR_INVALID;
     if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
-    int rc = multi_moments_frame(ctx, "rt_download_variance");
+    int rc = multi_per_pixel_frame(ctx, "rt_download_variance");
     if (rc != RT_OK) return rc;
     // like the linear radiance of rt_download: produced where the tiles were rendered, 12 bytes per pixel gathered
     size_t stride = 0;
@@ -524,12 +529,27 @@ extern "C" int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* varia
     return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 12, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, variance));
 }
 
+extern "C" int rt_download_aov(rt_ctx* ctx, int32_t total_spp, float* aov) {
+    RT_NEED(ctx);
+    const int n = (int)ctx->dev.size();
+    if (n == 1) return fwd(ctx, ctx->dev[0], dev_download_aov(ctx->dev[0], total_spp, aov));
+    if (!aov) return RT_ERR_INVALID;
+    if (total_spp <= 0) return failx(ctx, RT_ERR_INVALID, "rt_download_aov: total_spp must be positive");
+    int rc = multi_per_pixel_frame(ctx, "rt_download_aov");
+    if (rc != RT_OK) return rc;
+    // resolved where the tiles were rendered, 32 bytes per pixel gathered
+    size_t stride = 0;
+    rc = gather_plane(ctx, Plane::Aov, total_spp, &stride);
+    if (rc != RT_OK) return rc;
+    return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 32, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, aov));
+}
+
 extern "C" int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double* rms_std_error) {
     RT_NEED(ctx);
     if (!mean_radiance || !rms_std_error) return RT_ERR_INVALID;
     if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_frame_noise: total_spp must be at least 2");
     if (ctx->dev.size() > 1) {
-        int rc = multi_moments_frame(ctx, "rt_frame_noise");
+        int rc = multi_per_pixel_frame(ctx, "rt_frame_noise");
         if (rc != RT_OK) return rc;
     }
     // integer partials of every device added on the host: the same words whatever the device count

@@ -2,13 +2,14 @@
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
 // Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
-//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS>
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS, AOV>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
 //                          fixed-point accumulation.  Its compiled instances are the rows of kV2Instances
 //   aov_kernel             deterministic primary hits (parity tests)
 //   resolve_kernel         accumulation buffer -> float radiance + RGB8 (Camera.txt:74-89)
 //   variance_kernel, noise_kernel   sums + second moments -> per-pixel sample variance, frame noise partials
+//   aov_resolve_kernel     AOV sums -> albedo, normal, depth, coverage (RT_FLAG_AOV)
 //   untile_kernel, add_sums_kernel   shard frames: compact tiles -> full frame, sums
 //   pair_nodes_kernel      device-built BVH2 nodes -> the paired layout the traversal reads
 //   probe_*_kernel         per-function known-answer probes
@@ -54,7 +55,9 @@ struct RenderArgs {
     uint32_t side_lo;        // the side pointer, its two 32-bit halves in the struct's two alignment holes (here and after
                              // shadow_point_lights), so that no offset of a field or a kernel parameter moves.  It serves the
                              // instances that need it, which are never the same: MOMENTS, the moments buffer (unsigned long
-                             // long); VIEWS, the view table (ViewRecord)
+                             // long); VIEWS, the view table (ViewRecord).  The AOV sums of RT_FLAG_AOV, which MOMENTS
+                             // excludes too, go in the kernel's gstats parameter instead: only STATS instances read that
+                             // one, and AOV excludes STATS
     unsigned long long n_items;
     uint32_t k0, k1;
     int compact;             // RT_FLAG_COMPACT_TILES: `accum` holds only this shard's tiles, tile-major: slot = local_tile * tile_size^2 + y_in_tile * tile_size + x_in_tile
@@ -81,6 +84,29 @@ __device__ __forceinline__ void add_square(unsigned long long* m, unsigned long 
     if (l0) atomicAdd(m, l0);
     if (l1) atomicAdd(m + 1, l1);
 }
+
+// RT_FLAG_AOV: one camera sample's first-vertex outputs added to the 8 words of its slot -- albedo x3 and depth unsigned,
+// clamped like radiance to [0, 2^20]; the normal x3 signed (two's complement), clamped to [-1, 1]; all in 2^-28 units;
+// then the hit count.  The exactness argument of the radiance words holds word for word: at most 2^16 samples of at most
+// 2^48 each (|x| <= 2^28 for the normal).  A zero word (two normal components of every axis-aligned wall) costs no atomic.
+// Out of line, and |d| in double: inlined, or with float arithmetic on values the path also uses, it changed how the
+// compiler restructured and contracted the path's own arithmetic in the AOV instances, and so the image.
+__device__ __noinline__ void add_aov(unsigned long long* a, V3 albedo, V3 n, float t, V3 d, bool hit) {
+    const double dx = d.x, dy = d.y, dz = d.z;
+    const float depth = (float)(t * sqrt(dx * dx + dy * dy + dz * dz));
+    const float al[3] = {albedo.x, albedo.y, albedo.z}, nn[3] = {n.x, n.y, n.z};
+#pragma unroll
+    for (int c = 0; c < 3; c++) {
+        const unsigned long long x = __float2ull_rn(fminf(fmaxf(al[c], 0.0f), kSampleClamp) * kAccumScale);
+        if (x) atomicAdd(a + c, x);
+        const long long s = __float2ll_rn(fminf(fmaxf(nn[c], -1.0f), 1.0f) * kAccumScale);
+        if (s) atomicAdd(a + 3 + c, (unsigned long long)s);
+    }
+    const unsigned long long x = __float2ull_rn(fminf(fmaxf(depth, 0.0f), kSampleClamp) * kAccumScale);
+    if (x) atomicAdd(a + 6, x);
+    if (hit) atomicAdd(a + 7, 1ull);
+}
+__device__ __forceinline__ V3 clamp01(V3 c) { return v3(__saturatef(c.x), __saturatef(c.y), __saturatef(c.z)); }
 
 // ---------------------------------------------------------------------------------
 // render_kernel_v2 — the production megakernel.
@@ -162,7 +188,11 @@ struct LocalSlot {
 // (item / items_per_view = tile / (tiles_x * tiles_y) is the view); each lane takes camera and Philox key from its view's
 // record in A.side() and accumulates into slot view * width * height + pixel of `accum`, kept in lane_slot like a
 // compact tile slot.  Never with STATS, MOMENTS, compact tiles or shards.
-template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false, bool VIEWS = false>
+// AOV: also add each camera sample's first-vertex albedo, normal, depth and hit (add_aov) to the AOV sums, 8 words per
+// slot of `accum`'s layout, passed in the gstats parameter (only STATS instances read that one, and AOV is never STATS).
+// Never with STATS, MOMENTS or VIEWS.
+template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false, bool VIEWS = false,
+          bool AOV = false>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
                                                         unsigned long long* __restrict__ counters, Stats* __restrict__ gstats) {
@@ -347,6 +377,11 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                 load_path();
                 L = L + T * v3(S.background);
                 done = true;
+                if constexpr (AOV) {
+                    if (bounce == 0)
+                        add_aov(reinterpret_cast<unsigned long long*>(gstats) + 8ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel),
+                                clamp01(v3(S.background)), v3(0, 0, 0), 0.0f, v3(0, 0, 0), false);
+                }
             } else {
                 Surface sf;
                 if (medium >= 0) {  // constant_medium.h:45-50
@@ -369,6 +404,15 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                 Ray next;
                 const bool scattered = shade_surface<(FEAT & FEAT_SPECULAR) != 0>(S, m, ray, sf, [&] { return rng.draw(bounce, RS_SCATTER); },
                                                                                   emitted, att, next);
+                if constexpr (AOV) {
+                    // the first event of the camera ray: a light reports what it emits (clamped), anything else the
+                    // attenuation it returned -- also a metal sample absorbed at a grazing angle; a medium has no normal
+                    if (bounce == 0) {
+                        const bool light = m.type == RT_MAT_DIFFUSE_LIGHT || m.type == RT_MAT_EMISSIVE_LIGHT;
+                        add_aov(reinterpret_cast<unsigned long long*>(gstats) + 8ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel),
+                                light ? clamp01(emitted) : att, medium >= 0 ? v3(0, 0, 0) : sf.normal, sf.t, ray.d, true);
+                    }
+                }
                 // NEE: a listed emitter reached from a vertex that also sampled the emitters directly shares the
                 // estimate with that sample (balance heuristic)
                 if (NEE && nee_pdf > 0.0f && medium < 0 && sf.nee_light > 0) {
@@ -443,55 +487,59 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
 
 // Every compiled instance of render_kernel_v2, by its template parameters.  A request runs the first entry that covers it
 // (v2_select), so the order is the preference: the per-scene feature instances of the plain binary-tree kernel (see FEAT_*
-// above), then the general ones, LITE before plain.  NEE, MOMENTS and VIEWS exist for the binary tree only (every scene
+// above), then the general ones, LITE before plain.  NEE, MOMENTS, VIEWS and AOV exist for the binary tree only (every scene
 // has one; shadow rays and paths then both go through it), and only as general instances.
 typedef void (*RenderKernel)(const DevScene, const RenderArgs, unsigned long long*, unsigned long long*, Stats*);
 struct V2Instance {
-    bool stats, lite, nee, moments, views;  // lite: the scene must be LITE (no triangles, point lights, defocus)
+    bool stats, lite, nee, moments, views, aov;  // lite: the scene must be LITE (no triangles, point lights, defocus)
     int width;
     int feat;  // FEAT_* bits the instance carries
     RenderKernel kernel;
 };
-#define RT_V2(S, L, N, M, V, W, F) {S, L, N, M, V, W, F, render_kernel_v2<S, L, N, W, F, M, V>}
+#define RT_V2(S, L, N, M, V, W, F, AV) {S, L, N, M, V, AV, W, F, render_kernel_v2<S, L, N, W, F, M, V, AV>}
 static const V2Instance kV2Instances[] = {
-    RT_V2(false, true, false, false, false, 2, 0),                                  // C2: quads, nothing else
-    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MSPHERE),          // C5: media bounded by spheres, a moving sphere
-    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MEDIA_GENERAL),    // C3: media bounded by boxes
-    RT_V2(false, false, false, false, false, 2, FEAT_DEFOCUS),                      // C1: defocus blur, nothing else
-    RT_V2(false, false, false, false, false, 2, FEAT_TRI | FEAT_LIGHTS),            // C4: triangles and point lights
-    RT_V2(false, true, false, false, false, 2, FEAT_ALL),                           // LITE
-    RT_V2(false, false, false, false, false, 2, FEAT_ALL),                          // plain
-    RT_V2(true, false, false, false, false, 2, FEAT_ALL),                           // STATS
-    RT_V2(false, true, false, false, false, 4, FEAT_ALL),
-    RT_V2(false, false, false, false, false, 4, FEAT_ALL),
-    RT_V2(true, false, false, false, false, 4, FEAT_ALL),
-    RT_V2(false, true, false, false, false, 8, FEAT_ALL),
-    RT_V2(false, false, false, false, false, 8, FEAT_ALL),
-    RT_V2(true, false, false, false, false, 8, FEAT_ALL),
-    RT_V2(false, true, true, false, false, 2, FEAT_ALL),                            // NEE + LITE
-    RT_V2(false, false, true, false, false, 2, FEAT_ALL),                           // NEE
-    RT_V2(false, true, false, true, false, 2, FEAT_ALL),                            // MOMENTS twins
-    RT_V2(false, false, false, true, false, 2, FEAT_ALL),
-    RT_V2(false, true, true, true, false, 2, FEAT_ALL),
-    RT_V2(false, false, true, true, false, 2, FEAT_ALL),
-    RT_V2(false, true, false, false, true, 2, FEAT_ALL),                            // VIEWS twins (rt_render_views)
-    RT_V2(false, false, false, false, true, 2, FEAT_ALL),
-    RT_V2(false, true, true, false, true, 2, FEAT_ALL),
-    RT_V2(false, false, true, false, true, 2, FEAT_ALL),
+    RT_V2(false, true, false, false, false, 2, 0, false),                                  // C2: quads, nothing else
+    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MSPHERE, false),          // C5: media bounded by spheres, a moving sphere
+    RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MEDIA_GENERAL, false),    // C3: media bounded by boxes
+    RT_V2(false, false, false, false, false, 2, FEAT_DEFOCUS, false),                      // C1: defocus blur, nothing else
+    RT_V2(false, false, false, false, false, 2, FEAT_TRI | FEAT_LIGHTS, false),            // C4: triangles and point lights
+    RT_V2(false, true, false, false, false, 2, FEAT_ALL, false),                           // LITE
+    RT_V2(false, false, false, false, false, 2, FEAT_ALL, false),                          // plain
+    RT_V2(true, false, false, false, false, 2, FEAT_ALL, false),                           // STATS
+    RT_V2(false, true, false, false, false, 4, FEAT_ALL, false),
+    RT_V2(false, false, false, false, false, 4, FEAT_ALL, false),
+    RT_V2(true, false, false, false, false, 4, FEAT_ALL, false),
+    RT_V2(false, true, false, false, false, 8, FEAT_ALL, false),
+    RT_V2(false, false, false, false, false, 8, FEAT_ALL, false),
+    RT_V2(true, false, false, false, false, 8, FEAT_ALL, false),
+    RT_V2(false, true, true, false, false, 2, FEAT_ALL, false),                            // NEE + LITE
+    RT_V2(false, false, true, false, false, 2, FEAT_ALL, false),                           // NEE
+    RT_V2(false, true, false, true, false, 2, FEAT_ALL, false),                            // MOMENTS twins
+    RT_V2(false, false, false, true, false, 2, FEAT_ALL, false),
+    RT_V2(false, true, true, true, false, 2, FEAT_ALL, false),
+    RT_V2(false, false, true, true, false, 2, FEAT_ALL, false),
+    RT_V2(false, true, false, false, true, 2, FEAT_ALL, false),                            // VIEWS twins (rt_render_views)
+    RT_V2(false, false, false, false, true, 2, FEAT_ALL, false),
+    RT_V2(false, true, true, false, true, 2, FEAT_ALL, false),
+    RT_V2(false, false, true, false, true, 2, FEAT_ALL, false),
+    RT_V2(false, true, false, false, false, 2, FEAT_ALL, true),                            // AOV twins (RT_FLAG_AOV)
+    RT_V2(false, false, false, false, false, 2, FEAT_ALL, true),
+    RT_V2(false, true, true, false, false, 2, FEAT_ALL, true),
+    RT_V2(false, false, true, false, false, 2, FEAT_ALL, true),
 };
 #undef RT_V2
 
 // What a pass asks of the kernel: nee = NEE or shadowed point lights; lite = the scene (and every view) allows LITE;
 // width = the uploaded tree; feat = the FEAT_* bits the scene needs (FEAT_ALL: a general instance)
 struct V2Key {
-    bool stats, lite, nee, moments, views;
+    bool stats, lite, nee, moments, views, aov;
     int width;
     int feat;
 };
 static const V2Instance* v2_select(const V2Key& k) {
-    const int width = (k.nee || k.moments || k.views) ? 2 : k.width;  // binary tree only
+    const int width = (k.nee || k.moments || k.views || k.aov) ? 2 : k.width;  // binary tree only
     for (const V2Instance& e : kV2Instances)
-        if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.width == width &&
+        if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.aov == k.aov && e.width == width &&
             (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
             return &e;
     return nullptr;
@@ -655,6 +703,20 @@ __global__ void noise_kernel(const unsigned long long* __restrict__ accum, const
     if (threadIdx.x < 12 && part[threadIdx.x]) atomicAdd(out + threadIdx.x, part[threadIdx.x]);
 }
 
+// RT_FLAG_AOV resolve: the 8 sums of a slot (add_aov) -> albedo r, g, b, normal x, y, z, depth, coverage, each computed in
+// double and rounded once to float.  With n = total_spp: albedo and normal sum / (2^28 n), depth sum / (2^28 hits) (0
+// without a hit), coverage hits / n.
+__global__ void aov_resolve_kernel(const unsigned long long* __restrict__ aov, int n_slots, int n, float4* __restrict__ out) {
+    const int px = blockIdx.x * blockDim.x + threadIdx.x;
+    if (px >= n_slots) return;
+    const unsigned long long* a = aov + 8ull * px;
+    const double scale = (double)kAccumScale * (double)n, hits = (double)a[7];
+    out[2ull * px] = make_float4((float)((double)a[0] / scale), (float)((double)a[1] / scale), (float)((double)a[2] / scale),
+                                 (float)((double)(long long)a[3] / scale));
+    out[2ull * px + 1] = make_float4((float)((double)(long long)a[4] / scale), (float)((double)(long long)a[5] / scale),
+                                     a[7] ? (float)((double)a[6] / ((double)kAccumScale * hits)) : 0.0f, (float)(hits / (double)n));
+}
+
 __global__ void probe_texture_kernel(const __grid_constant__ DevScene S, int tex, int n, const float* __restrict__ uvp,
                                      float* __restrict__ rgb) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -812,6 +874,12 @@ struct DevCtx {
     bool moments_valid = false;
     bool sums_uploaded = false;              // the frame is an rt_accum_upload, not rendered onto since (rt_moments_upload)
     unsigned long long* noise_sums = nullptr;  // rt_frame_noise: the 12 partial words of noise_kernel
+    // RT_FLAG_AOV: 8 words per slot of `acc` (add_aov), allocated by the first AOV render; valid when they describe the
+    // same samples as the sums (set by a non-accumulating AOV pass, cleared by a pass without the flag and wherever the
+    // moments are cleared)
+    unsigned long long* aov = nullptr;
+    size_t aov_cap = 0;
+    bool aov_valid = false;
     // rt_render_views: the views frame (views_n x views_h x views_w slots of 32 B, view-major; no other call touches it),
     // the view table on the device, and what an accumulating views pass must match: the frame's shape and a
     // fingerprint of the cameras and seeds (views_n == 0: no views render yet)
@@ -1000,6 +1068,7 @@ static void dev_destroy(DevCtx* ctx) {
     if (ctx->accum && !ctx->accum_external) cudaFree(ctx->accum);
     if (ctx->moments) cudaFree(ctx->moments);
     if (ctx->noise_sums) cudaFree(ctx->noise_sums);
+    if (ctx->aov) cudaFree(ctx->aov);
     if (ctx->views_accum) cudaFree(ctx->views_accum);
     if (ctx->view_table) cudaFree(ctx->view_table);
     if (ctx->counters) cudaFree(ctx->counters);
@@ -2137,7 +2206,7 @@ static int ensure_accum(DevCtx* ctx, const AccumLayout& L) {
         return RT_OK;
     }
     if (ctx->accum && ctx->acc == L) return RT_OK;
-    ctx->moments_valid = false;
+    ctx->moments_valid = ctx->aov_valid = false;
     if (!ctx->accum || need > ctx->accum_cap) {
         if (ctx->accum) cudaFree(ctx->accum);
         ctx->accum = nullptr;
@@ -2164,6 +2233,18 @@ static int ensure_moments(DevCtx* ctx, size_t slots) {
     return RT_OK;
 }
 
+// the AOV sums of RT_FLAG_AOV: 64 bytes per slot, same layout as `accum` (its contents are set by the caller)
+static int ensure_aov(DevCtx* ctx, size_t slots) {
+    const size_t need = std::max<size_t>(slots, 1) * 8 * sizeof(unsigned long long);
+    if (ctx->aov && need <= ctx->aov_cap) return RT_OK;
+    if (ctx->aov) cudaFree(ctx->aov);
+    ctx->aov = nullptr;
+    ctx->aov_cap = 0;
+    if (cudaMalloc(&ctx->aov, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes for the AOV sums", need);
+    ctx->aov_cap = need;
+    return RT_OK;
+}
+
 static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t width, int32_t height) {
     if (!ctx) return RT_ERR_INVALID;
     CU(ctx, cudaSetDevice(ctx->device));
@@ -2175,7 +2256,7 @@ static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t w
     ctx->accum_external = false;
     ctx->acc = AccumLayout();
     ctx->accum_bytes = ctx->accum_cap = 0;
-    ctx->moments_valid = ctx->sums_uploaded = false;
+    ctx->moments_valid = ctx->aov_valid = ctx->sums_uploaded = false;
     if (!device_ptr) return RT_OK;
     size_t need = (size_t)width * height * 4 * sizeof(unsigned long long);
     if (width <= 0 || height <= 0 || bytes < need) return fail(ctx, RT_ERR_INVALID, "rt_bind_accum: need %zu bytes for %dx%d, got %zu", need, width, height, bytes);
@@ -2330,6 +2411,7 @@ static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int
     CU(ctx, cudaMemcpyAsync(ctx->accum, host, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->moments_valid = false;  // until rt_moments_upload restores the moments of the same samples
+    ctx->aov_valid = false;      // the AOV sums are not restored
     ctx->sums_uploaded = true;
     return RT_OK;
 }
@@ -2438,7 +2520,9 @@ static int v2_grid(DevCtx* ctx, const V2Instance* e, int* grid) {
 
 static int launch_v2(DevCtx* ctx, const V2Instance& e, int grid, const RenderArgs& A, unsigned long long* accum,
                      unsigned long long* counters, cudaStream_t stream) {
-    e.kernel<<<grid, RT_V2_THREADS, v2_smem(ctx, e.width), stream>>>(ctx->scene, A, accum, counters, ctx->dstats);
+    // an AOV instance takes its sums in the gstats parameter (it never counts stats; RenderArgs has no free hole left)
+    Stats* side = e.aov ? reinterpret_cast<Stats*>(ctx->aov) : ctx->dstats;
+    e.kernel<<<grid, RT_V2_THREADS, v2_smem(ctx, e.width), stream>>>(ctx->scene, A, accum, counters, side);
     CU(ctx, cudaGetLastError());
     return RT_OK;
 }
@@ -2550,6 +2634,12 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     if (moments && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->moments_valid)
         return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_MOMENTS | RT_FLAG_ACCUMULATE onto a frame whose sums have no moments "
                                        "(start it with a non-accumulating moments pass, or restore both with rt_accum_upload + rt_moments_upload)");
+    const bool aov = (p->flags & RT_FLAG_AOV) != 0;
+    if (aov && (p->flags & (RT_FLAG_STATS | RT_FLAG_MOMENTS)))
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_AOV has no RT_FLAG_STATS or RT_FLAG_MOMENTS instance");
+    if (aov && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->aov_valid)
+        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_AOV | RT_FLAG_ACCUMULATE onto a frame whose sums have no AOV sums "
+                                       "(start it with a non-accumulating AOV pass)");
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
     // RT_FLAG_OVERLAP: this pass goes to one of the two lane streams with its own work counter and waits for nothing on
@@ -2585,6 +2675,11 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         if (rc != RT_OK) return rc;
     }
     ctx->moments_valid = moments;  // an accumulating moments pass was checked above; any pass without the flag invalidates them
+    if (aov && !(p->flags & RT_FLAG_ACCUMULATE)) {
+        rc = ensure_aov(ctx, L.slots());
+        if (rc != RT_OK) return rc;
+    }
+    ctx->aov_valid = aov;  // the same rule
     ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
@@ -2593,7 +2688,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     // hit_prim); the NEE instances count no STATS; the first per-scene instance that covers the scene's features, unless
     // RT_B200_GENERAL_INSTANCE=1 asks for a general one
     const V2Key req{stats && !(want_nee || want_shadow), ctx->scene_lite && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, moments,
-                    false, ctx->scene.wide_width ? ctx->scene.wide_width : 2, getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
+                    false, aov, ctx->scene.wide_width ? ctx->scene.wide_width : 2, getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
     const V2Instance* e = v2_select(req);
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
@@ -2654,6 +2749,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     }
     if (!(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->accum, 0, L.slots() * 32, stream));
     if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->moments, 0, L.slots() * 48, stream));
+    if (aov && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->aov, 0, L.slots() * 64, stream));
     if (stats) CU(ctx, cudaMemsetAsync(ctx->dstats, 0, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long), stream));
     return enqueue_pass(ctx, *e, grid, A, ctx->accum, stream, pass_samples(), stats, (p->flags & RT_FLAG_ASYNC) != 0);
 }
@@ -2668,9 +2764,9 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     int rc = check_render_params(ctx, p, "rt_render_views");
     if (rc != RT_OK) return rc;
     if (n_views < 1 || !cameras) return fail(ctx, RT_ERR_INVALID, "rt_render_views: needs n_views >= 1 cameras (got %d%s)", n_views, cameras ? "" : ", NULL");
-    const uint32_t unsupported = RT_FLAG_STATS | RT_FLAG_MOMENTS | RT_FLAG_COMPACT_TILES | RT_FLAG_OVERLAP;
+    const uint32_t unsupported = RT_FLAG_STATS | RT_FLAG_MOMENTS | RT_FLAG_COMPACT_TILES | RT_FLAG_OVERLAP | RT_FLAG_AOV;
     if ((p->flags & unsupported) || p->shard_count > 1)
-        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP and shards are not "
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, RT_FLAG_AOV and shards are not "
                                              "supported for multi-view batches (flags 0x%x, shard_count %d)", p->flags & unsupported, p->shard_count);
     if ((long long)n_views * p->width * p->height >= (1ll << 31))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: %d views of %dx%d are 2^31 slots or more", n_views, p->width, p->height);
@@ -2727,7 +2823,7 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
     // LITE only when no view needs the defocus code the LITE instance leaves out
-    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, 2, FEAT_ALL};
+    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, false, 2, FEAT_ALL};
     const V2Instance* e = v2_select(req);
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
@@ -2984,6 +3080,36 @@ static int dev_moments_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, i
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->moments_valid = true;
     return RT_OK;
+}
+
+// ---- auxiliary outputs (RT_FLAG_AOV) ---------------------------------------------------------------------------------
+static int aov_ready(DevCtx* ctx, const char* what) {
+    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
+    if (!ctx->aov_valid) return fail(ctx, RT_ERR_STATE, "%s: the frame has no AOV sums (render it with RT_FLAG_AOV)", what);
+    return dev_wait(ctx);
+}
+
+// aov_resolve_kernel over the slots of the frame into frame_scratch, `offset` bytes in (8 floats per slot)
+static int dev_aov_into(DevCtx* ctx, int32_t total_spp, size_t offset, const void** plane) {
+    const size_t n = ctx->acc.slots();
+    int rc = stage_buffers(ctx, 0, offset + n * 32);
+    if (rc != RT_OK) return rc;
+    *plane = ctx->frame_scratch + offset;
+    if (n) aov_resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->aov, (int)n, total_spp, (float4*)(ctx->frame_scratch + offset));
+    CU(ctx, cudaGetLastError());
+    return RT_OK;
+}
+
+static int dev_download_aov(DevCtx* ctx, int32_t total_spp, float* aov) {
+    if (!ctx || !aov) return RT_ERR_INVALID;
+    if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_download_aov: total_spp must be positive");
+    int rc = aov_ready(ctx, "rt_download_aov");
+    // a compact plane is untiled into the front of frame_scratch (plane_to_host): resolve it behind that room
+    const size_t room = ctx->acc.compact ? (size_t)ctx->acc.width * ctx->acc.height * 32 : 0;
+    const void* plane = nullptr;
+    if (rc == RT_OK) rc = dev_aov_into(ctx, total_spp, room, &plane);
+    if (rc != RT_OK) return rc;
+    return plane_to_host(ctx, plane, 32, ctx->acc, aov);
 }
 
 static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* prim_id, float* t, float* normal, float* point,

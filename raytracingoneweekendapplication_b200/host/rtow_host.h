@@ -1741,6 +1741,11 @@ class camera {
     // frame with `seed`; frame k is written to <stem>_<k:03d><ext> and last_rgb8 holds all frames, frame-major.  Not
     // combined with a checkpoint, a noise target, variance output or several devices.  0 or 1: off.
     int turntable_frames = 0;
+    // auxiliary outputs (RT_FLAG_AOV): aov_name "x.exr" / "x.pfm" also writes the antialiased first-hit albedo, normal
+    // and depth of the same samples to x_albedo.exr, x_normal.exr and x_depth.exr (depth in all three channels) -- the
+    // inputs of an external denoiser and of compositing.  Not combined with a turntable, a checkpoint, a noise target
+    // or variance output.  Empty: off.
+    std::string aov_name;
 
     int image_height() const {
         int h = int(image_width / aspect_ratio);  // Camera.txt:137-138
@@ -1772,13 +1777,17 @@ class camera {
         return c;
     }
 
-    // <stem>_<k:03d><ext> of a turntable frame (the extension is what follows the last '.' of the file name)
-    static std::string frame_name(const std::string& name, int k) {
+    // <stem><suffix><ext> (the extension is what follows the last '.' of the file name)
+    static std::string suffixed_name(const std::string& name, const char* suffix) {
         const size_t slash = name.find_last_of("/\\"), dot = name.find_last_of('.');
         const bool ext = dot != std::string::npos && (slash == std::string::npos || dot > slash);
+        return ext ? name.substr(0, dot) + suffix + name.substr(dot) : name + suffix;
+    }
+    // <stem>_<k:03d><ext> of a turntable frame
+    static std::string frame_name(const std::string& name, int k) {
         char num[16];
         std::snprintf(num, sizeof num, "_%03d", k);
-        return ext ? name.substr(0, dot) + num + name.substr(dot) : name + num;
+        return suffixed_name(name, num);
     }
 
     // Same signature as Camera.txt:54.  Fails loudly (message + exit code 2) when the
@@ -1796,8 +1805,12 @@ class camera {
             if (ctx) rt_destroy(ctx);
             std::exit(2);
         };
-        if (turntable_frames > 1 && (!checkpoint_path.empty() || noise_target > 0 || !variance_name.empty() || devs.size() > 1)) {
-            std::cerr << "rt_b200: a turntable renders on one device without a checkpoint, a noise target or variance output" << std::endl;
+        if (turntable_frames > 1 && (!checkpoint_path.empty() || noise_target > 0 || !variance_name.empty() || !aov_name.empty() || devs.size() > 1)) {
+            std::cerr << "rt_b200: a turntable renders on one device without a checkpoint, a noise target, variance or AOV output" << std::endl;
+            std::exit(2);
+        }
+        if (!aov_name.empty() && (!checkpoint_path.empty() || noise_target > 0 || !variance_name.empty())) {
+            std::cerr << "rt_b200: AOV output is not combined with a checkpoint, a noise target or variance output" << std::endl;
             std::exit(2);
         }
         if (rt_create(&ctx, devs.data(), (int)devs.size()) != RT_OK) fail("rt_create");
@@ -1839,6 +1852,8 @@ class camera {
             }
             p.shard_mode = RT_SHARD_TILES;  // a multi-device context resolves the noise of tile-sharded frames
         }
+        const bool aov = !aov_name.empty();
+        if (aov && devs.size() > 1) p.shard_mode = RT_SHARD_TILES;  // and the AOVs
         std::vector<uint64_t> sums, msums;
         if (!checkpoint_path.empty()) {
             rtb200::checkpoint_header old;
@@ -1889,7 +1904,8 @@ class camera {
             // longest paths of one pass run while the next fills the freed SMs; integer sums, same frame).  Every eighth
             // pass is waited for, so that the progress line below stays within eight passes of the truth; checkpoints
             // and the download wait for everything by themselves.
-            p.flags = (fresh ? 0 : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC | RT_FLAG_OVERLAP)) | estimator_flags | (moments ? RT_FLAG_MOMENTS : 0u);
+            p.flags = (fresh ? 0 : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC | RT_FLAG_OVERLAP)) | estimator_flags | (moments ? RT_FLAG_MOMENTS : 0u) |
+                      (aov ? RT_FLAG_AOV : 0u);
             fresh = false;
             if (rt_render(ctx, &p) != RT_OK) fail("rt_render");
             if (++passes % 8 == 0 && rt_sync(ctx) != RT_OK) fail("rt_sync");
@@ -1922,6 +1938,11 @@ class camera {
             variance.assign((size_t)p.width * p.height * 3, 0.0f);
             if (rt_download_variance(ctx, done, variance.data()) != RT_OK) fail("rt_download_variance");
         }
+        std::vector<float> aovs;
+        if (aov && done > 0) {
+            aovs.assign((size_t)p.width * p.height * 8, 0.0f);
+            if (rt_download_aov(ctx, done, aovs.data()) != RT_OK) fail("rt_download_aov");
+        }
         rt_get_stats(ctx, &last_stats);
         rt_destroy(ctx);
         std::cout << "\nDone rendering " << image_name << std::endl;
@@ -1937,6 +1958,24 @@ class camera {
             bool ok = pfm ? rtb200::write_pfm(variance_name.c_str(), p.width, p.height, variance.data())
                           : rtb200::write_exr(variance_name.c_str(), p.width, p.height, variance.data());
             if (!ok) std::cerr << "rt_b200: cannot write " << variance_name << std::endl;
+        }
+        if (!aovs.empty()) {
+            // per pixel albedo r g b, normal x y z, depth, coverage -> three RGB planes
+            const size_t n = (size_t)p.width * p.height;
+            std::vector<float> albedo(n * 3), normal(n * 3), depth(n * 3);
+            for (size_t i = 0; i < n; i++)
+                for (int c = 0; c < 3; c++) {
+                    albedo[3 * i + c] = aovs[8 * i + c];
+                    normal[3 * i + c] = aovs[8 * i + 3 + c];
+                    depth[3 * i + c] = aovs[8 * i + 6];
+                }
+            const bool pfm = aov_name.size() >= 4 && aov_name.compare(aov_name.size() - 4, 4, ".pfm") == 0;
+            for (const auto& plane : {std::make_pair("_albedo", &albedo), std::make_pair("_normal", &normal), std::make_pair("_depth", &depth)}) {
+                const std::string name = suffixed_name(aov_name, plane.first);
+                bool ok = pfm ? rtb200::write_pfm(name.c_str(), p.width, p.height, plane.second->data())
+                              : rtb200::write_exr(name.c_str(), p.width, p.height, plane.second->data());
+                if (!ok) std::cerr << "rt_b200: cannot write " << name << std::endl;
+            }
         }
     }
 
