@@ -43,8 +43,15 @@ int main(int argc, char** argv) {
     //            --turntable N                N views around lookat in one batch, written to <stem>_000<ext> ...
     //            --aov FILE.exr|.pfm          also write the antialiased first-hit albedo, normal and depth to
     //                                         <stem>_albedo<ext>, <stem>_normal<ext>, <stem>_depth<ext>
-    for (int i = 7; i + 1 < argc; i += 2) {
+    //            --panorama                   a 360-degree equirectangular view around lookfrom (takes no value)
+    for (int i = 7; i < argc; i += 2) {
         std::string k = argv[i];
+        if (k == "--panorama") {
+            cam.panorama = true;
+            i--;
+            continue;
+        }
+        if (i + 1 >= argc) break;
         if (k == "--checkpoint") cam.checkpoint_path = argv[i + 1];
         else if (k == "--every") cam.checkpoint_every_spp = std::atoi(argv[i + 1]);
         else if (k == "--stop-after") cam.stop_after_spp = std::atoi(argv[i + 1]);

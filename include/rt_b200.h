@@ -277,6 +277,10 @@ typedef enum rt_shard_mode {
                                  (RT_ERR_STATE otherwise); a pass without it, and rt_accum_upload, leave the frame without
                                  them.  Runs the general kernel instances (plain / NEE); with RT_FLAG_STATS or
                                  RT_FLAG_MOMENTS it is RT_ERR_UNSUPPORTED.  The image is the same as without the flag. */
+#define RT_FLAG_CAMERA_RAYS 512u /* the primary rays come from the records of rt_set_camera_rays instead of the uploaded
+                                 camera (see there).  RT_ERR_STATE without rays, RT_ERR_INVALID when width / height are
+                                 not those of the rays; with RT_FLAG_STATS or RT_FLAG_MOMENTS, and in rt_render_views,
+                                 RT_ERR_UNSUPPORTED.  Every other flag, shards and multi-device contexts work with it. */
 
 typedef struct rt_render_params {
     uint32_t struct_size;
@@ -432,7 +436,7 @@ int rt_download(rt_ctx* ctx, int32_t total_spp, float* rgb_linear, uint8_t* rgb8
  * and seed (seeds[v] when seeds != NULL).  cameras[v].background must equal the uploaded camera's (RT_ERR_INVALID
  * otherwise), as must n_views >= 1 and cameras != NULL.
  *   - flags: RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_NEE and RT_FLAG_SHADOWED_POINT_LIGHTS; params->stream is honoured.
- *     RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_AOV, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, shard_count > 1 and multi-device contexts are
+ *     RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_AOV, RT_FLAG_CAMERA_RAYS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, shard_count > 1 and multi-device contexts are
  *     RT_ERR_UNSUPPORTED, and so is a frame of n_views x width x height >= 2^31 slots.
  *   - the views frame is a buffer of its own: a views render does not touch the frame, moments or bound buffer of
  *     rt_render, and rt_render does not touch the views frame.
@@ -529,6 +533,32 @@ int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double
  * frames without a restored checkpoint (else RT_ERR_UNSUPPORTED).  Ordered after outstanding hand-outs like rt_download. */
 int rt_download_aov(rt_ctx* ctx, int32_t total_spp, float* aov);
 
+/* Caller-defined cameras: one primary ray record per pixel, for camera models the uploaded pinhole cannot express
+ * (fisheye and calibrated lenses, 360-degree panoramas, stereo rigs, the rays of a dataset).  A record holds the ray's
+ * origin, its direction through the pixel centre (any non-zero length, like the rays of Camera.txt) and the change of
+ * that direction per pixel in x and in y: the footprint the antialiasing jitter spans. */
+typedef struct rt_camera_ray {
+    float origin[3];
+    float direction[3];
+    float dx[3], dy[3];
+} rt_camera_ray; /* 48 bytes; rt_struct_size(16) */
+
+/* rt_set_camera_rays copies width*height records (row-major, top-down: rays[j*width + i] is pixel (i, j)) from host
+ * memory into a buffer the context owns on each of its devices; the caller may free its copy when the call returns.
+ * It waits for the passes in flight first.  rays == NULL frees the buffer.  RT_ERR_INVALID for width or height <= 0,
+ * width*height >= 2^31, or a record with a non-finite value or a zero direction (the message names the first); a
+ * refused call changes nothing.  rt_upload_scene and rt_refit_scene leave the rays as they are.
+ * With RT_FLAG_CAMERA_RAYS, sample s of pixel (i, j) draws the camera uniforms u of Camera.txt:177-200 as rt_render does
+ * and traces origin, direction + (u.x - 0.5) dx + (u.y - 0.5) dy (two FMAs per component, dy first) at time u.z, with no
+ * defocus; a miss sees the uploaded camera's background.  Everything after the primary ray is unchanged, so a frame
+ * rendered from the pinhole rays of the uploaded camera (origin = lookfrom, direction = pixel00 + i du + j dv - lookfrom,
+ * dx = du, dy = dv) has the expectation of rt_render's, though not its bits.  The frame is the ordinary frame: every
+ * download, checkpoint, shard and AOV call takes it as it is.
+ * A frame accumulates passes of one source: the uploaded camera, or one rt_set_camera_rays call.  An RT_FLAG_ACCUMULATE
+ * pass of the other source, or a rays pass after the rays were set again, is RT_ERR_STATE.  A frame restored with
+ * rt_accum_upload (or bound with rt_bind_accum) accepts either, which is how a checkpointed rays render resumes. */
+int rt_set_camera_rays(rt_ctx* ctx, const rt_camera_ray* rays, int32_t width, int32_t height);
+
 /* Compact tile buffers across processes (one process per GPU, e.g. under torchrun; single-device contexts):
  *   rt_shard_pixels   slots of the compact buffer of shard (rank, count): its tiles x tile_size^2 (edge tiles padded)
  *   rt_resolve_tiles  the compact sums of the last RT_FLAG_COMPACT_TILES render -> averaged radiance (3 floats per slot)
@@ -563,7 +593,7 @@ int rt_get_stats(rt_ctx* ctx, rt_stats* out);
  * binding (ctypes, cgo, JNI ...) can verify its own declarations at load time.
  * which: 0 rt_scene_desc, 1 rt_render_params, 2 rt_stats, 3 rt_sphere, 4 rt_quad,
  * 5 rt_triangle, 6 rt_medium, 7 rt_material, 8 rt_texture, 9 rt_image, 10 rt_perlin,
- * 11 rt_point_light, 12 rt_camera, 13 rt_xform, 14 rt_prim_ref, 15 rt_mesh; 0 for anything else. */
+ * 11 rt_point_light, 12 rt_camera, 13 rt_xform, 14 rt_prim_ref, 15 rt_mesh, 16 rt_camera_ray; 0 for anything else. */
 size_t rt_struct_size(int which);
 
 /* FP32 FMA issue-rate microbenchmark on the context's device, for the FP32

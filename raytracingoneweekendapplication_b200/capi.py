@@ -26,6 +26,7 @@ RT_FLAG_ACCUMULATE, RT_FLAG_ASYNC, RT_FLAG_STATS, RT_FLAG_NEE, RT_FLAG_SHADOWED_
 RT_FLAG_OVERLAP = 64
 RT_FLAG_MOMENTS = 128
 RT_FLAG_AOV = 256
+RT_FLAG_CAMERA_RAYS = 512
 
 d3 = C.c_double * 3
 
@@ -87,6 +88,10 @@ class rt_point_light(C.Structure):
 class rt_camera(C.Structure):
     _fields_ = [("lookfrom", d3), ("lookat", d3), ("vup", d3), ("vfov", C.c_double), ("defocus_angle", C.c_double),
                 ("focus_dist", C.c_double), ("background", d3)]
+
+
+class rt_camera_ray(C.Structure):
+    _fields_ = [("origin", C.c_float * 3), ("direction", C.c_float * 3), ("dx", C.c_float * 3), ("dy", C.c_float * 3)]
 
 
 class rt_scene_desc(C.Structure):
@@ -152,11 +157,11 @@ EXPORTED_SYMBOLS = [
     "rt_set_bvh_width", "rt_device_count", "rt_shard_pixels", "rt_resolve_tiles", "rt_untile",
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
     "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
-    "rt_render_views", "rt_download_views", "rt_refit_scene", "rt_download_aov",
+    "rt_render_views", "rt_download_views", "rt_refit_scene", "rt_download_aov", "rt_set_camera_rays",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
-               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref, rt_mesh]
+               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref, rt_mesh, rt_camera_ray]
 
 _lib = None
 _scenes = None
@@ -220,6 +225,7 @@ def load() -> C.CDLL:
     lib.rt_moments_upload.argtypes = [vp, vp, C.c_size_t, i32, i32]
     lib.rt_frame_noise.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.rt_download_aov.argtypes = [vp, i32, vp]
+    lib.rt_set_camera_rays.argtypes = [vp, vp, i32, i32]
     lib.rt_render_views.argtypes = [vp, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.POINTER(C.c_uint64), i32]
     lib.rt_download_views.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double)]
@@ -265,6 +271,7 @@ def load_scenes() -> C.CDLL:
     s.rtsc_render_turntable.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_char_p, C.c_int,
                                         C.c_int, C.c_int]
     s.rtsc_turntable_camera.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.POINTER(rt_camera)]
+    s.rtsc_panorama_rays.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.POINTER(rt_camera_ray)]
     s.rtsc_write_exr.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
     s.rtsc_write_pfm.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
     s.rtsc_load_obj.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_double)]
@@ -405,7 +412,8 @@ class Context:
                accumulate: bool = False, stats: bool = False, shard_rank: int = 0, shard_count: int = 1,
                shard_mode: int = RT_SHARD_AUTO, tile_size: int = 0, stream: Optional[int] = None, blocking: bool = True,
                nee: bool = False, shadowed_point_lights: bool = False, compact: bool = False, overlap: bool = False,
-               moments: bool = False, aov: bool = False) -> None:
+               moments: bool = False, aov: bool = False, camera_rays: bool = False) -> None:
+        """camera_rays=True traces the primary rays set with set_camera_rays() instead of the uploaded camera's."""
         p = rt_render_params()
         p.struct_size = C.sizeof(rt_render_params)
         p.width, p.height, p.samples_per_pixel, p.max_depth = width, height, spp, max_depth
@@ -414,10 +422,27 @@ class Context:
         p.flags = ((RT_FLAG_ACCUMULATE if accumulate else 0) | (RT_FLAG_STATS if stats else 0) | (0 if blocking else RT_FLAG_ASYNC) |
                    (RT_FLAG_NEE if nee else 0) | (RT_FLAG_SHADOWED_POINT_LIGHTS if shadowed_point_lights else 0) |
                    (RT_FLAG_COMPACT_TILES if compact else 0) | (RT_FLAG_OVERLAP if overlap else 0) | (RT_FLAG_MOMENTS if moments else 0) |
-                   (RT_FLAG_AOV if aov else 0))
+                   (RT_FLAG_AOV if aov else 0) | (RT_FLAG_CAMERA_RAYS if camera_rays else 0))
         p.stream = stream
         self._check(self.lib.rt_render(self._h, C.byref(p)))
         self.width, self.height = width, height
+
+    def set_camera_rays(self, rays) -> None:
+        """rt_set_camera_rays: one primary ray per pixel for render(..., camera_rays=True), an (H, W, 12) float32 array
+        (numpy, or a contiguous CPU tensor) of rt_camera_ray records: origin, direction through the pixel centre, and the
+        change of the direction per pixel in x and in y.  None frees them."""
+        if rays is None:
+            self._check(self.lib.rt_set_camera_rays(self._h, None, 0, 0))
+            return
+        if hasattr(rays, "numpy"):  # a torch tensor: its CPU memory as it is
+            if rays.device.type != "cpu" or not rays.is_contiguous():
+                raise ValueError("camera rays must be a contiguous CPU tensor")
+            rays = rays.numpy()
+        a = np.asarray(rays)
+        if a.dtype != np.float32 or a.ndim != 3 or a.shape[2] != 12:
+            raise ValueError(f"camera rays must be an (H, W, 12) float32 array, got {a.dtype} {a.shape}")
+        a = np.ascontiguousarray(a)
+        self._check(self.lib.rt_set_camera_rays(self._h, a.ctypes.data, a.shape[1], a.shape[0]))
 
     def render_views(self, cameras, width: int, height: int, spp: int, max_depth: int = 50, seed: int = 1, seeds=None,
                      spp_begin: int = 0, accumulate: bool = False, blocking: bool = True, nee: bool = False,

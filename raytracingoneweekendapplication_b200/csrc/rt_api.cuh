@@ -229,6 +229,34 @@ extern "C" int rt_accum_buffer(rt_ctx* ctx, void** device_ptr, size_t* bytes) {
     return fwd(ctx, ctx->dev[0], dev_accum_buffer(ctx->dev[0], device_ptr, bytes));
 }
 
+// ---- caller-defined cameras ----------------------------------------------------------------------------------------
+extern "C" int rt_set_camera_rays(rt_ctx* ctx, const rt_camera_ray* rays, int32_t width, int32_t height) {
+    RT_NEED(ctx);
+    if (rays) {  // everything is checked before any device changes
+        if (width <= 0 || height <= 0 || (long long)width * height >= (1ll << 31))
+            return failx(ctx, RT_ERR_INVALID, "rt_set_camera_rays: bad frame size %dx%d", width, height);
+        const size_t n = (size_t)width * height;
+        auto finite = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
+        for (size_t k = 0; k < n; k++) {
+            const rt_camera_ray& r = rays[k];
+            const char* bad = !(finite(r.origin) && finite(r.direction) && finite(r.dx) && finite(r.dy)) ? "a non-finite value"
+                              : (r.direction[0] == 0.0f && r.direction[1] == 0.0f && r.direction[2] == 0.0f) ? "a zero direction"
+                                                                                                            : nullptr;
+            if (bad)
+                return failx(ctx, RT_ERR_INVALID, "rt_set_camera_rays: record %zu (pixel %d, %d) has %s", k, (int)(k % (size_t)width),
+                             (int)(k / (size_t)width), bad);
+        }
+    }
+    for (DevCtx* d : ctx->dev) {
+        const int rc = dev_set_camera_rays(d, rays, width, height);
+        if (rc == RT_OK) continue;
+        fwd(ctx, d, rc);
+        for (DevCtx* e : ctx->dev) dev_set_camera_rays(e, nullptr, 0, 0);  // no device keeps rays the others lack
+        return rc;
+    }
+    return RT_OK;
+}
+
 // ---- multi-device render ----------------------------------------------------------------------------------------
 static bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
 
@@ -492,6 +520,7 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
         CUX(ctx, cudaStreamSynchronize(d->stream));
         d->moments_valid = false;  // moments are not restored across devices (rt_moments_upload is single-device)
         d->aov_valid = false;      // nor are the AOV sums
+        d->frame_src = -1;         // a checkpoint resumes with either source
     }
     cudaSetDevice(d0->device);
     if (ctx->base_sums) cudaFree(ctx->base_sums);

@@ -2,7 +2,7 @@
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
 // Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
-//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS, AOV>
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS, AOV, RAYS>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
 //                          fixed-point accumulation.  Its compiled instances are the rows of kV2Instances
@@ -108,6 +108,19 @@ __device__ __noinline__ void add_aov(unsigned long long* a, V3 albedo, V3 n, flo
 }
 __device__ __forceinline__ V3 clamp01(V3 c) { return v3(__saturatef(c.x), __saturatef(c.y), __saturatef(c.z)); }
 
+// RT_FLAG_CAMERA_RAYS: the primary ray of a sample from its pixel's rt_camera_ray record, 3 float4 on the device
+// (o.xyz d.x | d.yz dx.xy | dx.z dy.xyz: the record's 12 floats in order).  The uniforms are camera_ray's, drawn the same
+// way, and the jitter is its two FMAs with the record's direction for dir00 + i du + j dv; there is no lens.
+__device__ __forceinline__ Ray record_ray(const float4* __restrict__ rec, const Rng& rng) {
+    const float4 a = __ldg(rec), b = __ldg(rec + 1), c = __ldg(rec + 2);
+    const float4 u = rng.draw(0, RS_CAMERA);
+    Ray r;
+    r.o = v3(a.x, a.y, a.z);
+    r.d = fma3(u.x - 0.5f, v3(b.z, b.w, c.x), fma3(u.y - 0.5f, v3(c.y, c.z, c.w), v3(a.w, b.x, b.y)));
+    r.time = u.z;
+    return r;
+}
+
 // ---------------------------------------------------------------------------------
 // render_kernel_v2 — the production megakernel.
 //
@@ -191,8 +204,10 @@ struct LocalSlot {
 // AOV: also add each camera sample's first-vertex albedo, normal, depth and hit (add_aov) to the AOV sums, 8 words per
 // slot of `accum`'s layout, passed in the gstats parameter (only STATS instances read that one, and AOV is never STATS).
 // Never with STATS, MOMENTS or VIEWS.
+// RAYS: the primary ray of a sample comes from its pixel's record of rt_set_camera_rays (record_ray), 3 float4 per pixel
+// at A.side(), instead of the uploaded camera.  Never with STATS, MOMENTS or VIEWS, the other users of A.side().
 template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false, bool VIEWS = false,
-          bool AOV = false>
+          bool AOV = false, bool RAYS = false>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
                                                         unsigned long long* __restrict__ counters, Stats* __restrict__ gstats) {
@@ -284,6 +299,8 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
                         rng.k0 = V.k0;
                         rng.k1 = V.k1;
                         ray = camera_ray<NO_DEFOCUS>(V, px, py, rng);
+                    } else if constexpr (RAYS) {
+                        ray = record_ray(A.side<const float4>() + 3ull * rng.pixel, rng);
                     } else {
                         ray = camera_ray<NO_DEFOCUS>(S, px, py, rng);
                     }
@@ -487,16 +504,17 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
 
 // Every compiled instance of render_kernel_v2, by its template parameters.  A request runs the first entry that covers it
 // (v2_select), so the order is the preference: the per-scene feature instances of the plain binary-tree kernel (see FEAT_*
-// above), then the general ones, LITE before plain.  NEE, MOMENTS, VIEWS and AOV exist for the binary tree only (every scene
-// has one; shadow rays and paths then both go through it), and only as general instances.
+// above), then the general ones, LITE before plain.  NEE, MOMENTS, VIEWS, AOV and RAYS exist for the binary tree only (every
+// scene has one; shadow rays and paths then both go through it), and only as general instances.
 typedef void (*RenderKernel)(const DevScene, const RenderArgs, unsigned long long*, unsigned long long*, Stats*);
 struct V2Instance {
-    bool stats, lite, nee, moments, views, aov;  // lite: the scene must be LITE (no triangles, point lights, defocus)
+    bool stats, lite, nee, moments, views, aov, rays;  // lite: the scene must be LITE (no triangles, point lights, defocus)
     int width;
     int feat;  // FEAT_* bits the instance carries
     RenderKernel kernel;
 };
-#define RT_V2(S, L, N, M, V, W, F, AV) {S, L, N, M, V, AV, W, F, render_kernel_v2<S, L, N, W, F, M, V, AV>}
+#define RT_V2(S, L, N, M, V, W, F, AV) {S, L, N, M, V, AV, false, W, F, render_kernel_v2<S, L, N, W, F, M, V, AV>}
+#define RT_V2_RAYS(L, N, AV) {false, L, N, false, false, AV, true, 2, FEAT_ALL, render_kernel_v2<false, L, N, 2, FEAT_ALL, false, false, AV, true>}
 static const V2Instance kV2Instances[] = {
     RT_V2(false, true, false, false, false, 2, 0, false),                                  // C2: quads, nothing else
     RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MSPHERE, false),          // C5: media bounded by spheres, a moving sphere
@@ -526,21 +544,30 @@ static const V2Instance kV2Instances[] = {
     RT_V2(false, false, false, false, false, 2, FEAT_ALL, true),
     RT_V2(false, true, true, false, false, 2, FEAT_ALL, true),
     RT_V2(false, false, true, false, false, 2, FEAT_ALL, true),
+    RT_V2_RAYS(true, false, false),                                                        // RAYS twins (RT_FLAG_CAMERA_RAYS)
+    RT_V2_RAYS(false, false, false),
+    RT_V2_RAYS(true, true, false),
+    RT_V2_RAYS(false, true, false),
+    RT_V2_RAYS(true, false, true),                                                         // RAYS + AOV
+    RT_V2_RAYS(false, false, true),
+    RT_V2_RAYS(true, true, true),
+    RT_V2_RAYS(false, true, true),
 };
 #undef RT_V2
+#undef RT_V2_RAYS
 
 // What a pass asks of the kernel: nee = NEE or shadowed point lights; lite = the scene (and every view) allows LITE;
 // width = the uploaded tree; feat = the FEAT_* bits the scene needs (FEAT_ALL: a general instance)
 struct V2Key {
-    bool stats, lite, nee, moments, views, aov;
+    bool stats, lite, nee, moments, views, aov, rays;
     int width;
     int feat;
 };
 static const V2Instance* v2_select(const V2Key& k) {
-    const int width = (k.nee || k.moments || k.views || k.aov) ? 2 : k.width;  // binary tree only
+    const int width = (k.nee || k.moments || k.views || k.aov || k.rays) ? 2 : k.width;  // binary tree only
     for (const V2Instance& e : kV2Instances)
-        if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.aov == k.aov && e.width == width &&
-            (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
+        if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.aov == k.aov && e.rays == k.rays &&
+            e.width == width && (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
             return &e;
     return nullptr;
 }
@@ -880,6 +907,13 @@ struct DevCtx {
     unsigned long long* aov = nullptr;
     size_t aov_cap = 0;
     bool aov_valid = false;
+    // rt_set_camera_rays: 3 float4 per pixel (record_ray) of a rays_w x rays_h frame, and the number of the call that set
+    // them.  frame_src is the source of the passes the frame holds: 0 the uploaded camera, rays_gen for those rays, -1 a
+    // cleared, bound or restored frame that takes either (RT_FLAG_ACCUMULATE must not mix sources)
+    float4* rays = nullptr;
+    size_t rays_cap = 0;
+    int rays_w = 0, rays_h = 0;
+    int64_t rays_gen = 0, frame_src = -1;
     // rt_render_views: the views frame (views_n x views_h x views_w slots of 32 B, view-major; no other call touches it),
     // the view table on the device, and what an accumulating views pass must match: the frame's shape and a
     // fingerprint of the cameras and seeds (views_n == 0: no views render yet)
@@ -1069,6 +1103,7 @@ static void dev_destroy(DevCtx* ctx) {
     if (ctx->moments) cudaFree(ctx->moments);
     if (ctx->noise_sums) cudaFree(ctx->noise_sums);
     if (ctx->aov) cudaFree(ctx->aov);
+    if (ctx->rays) cudaFree(ctx->rays);
     if (ctx->views_accum) cudaFree(ctx->views_accum);
     if (ctx->view_table) cudaFree(ctx->view_table);
     if (ctx->counters) cudaFree(ctx->counters);
@@ -2216,6 +2251,7 @@ static int ensure_accum(DevCtx* ctx, const AccumLayout& L) {
     }
     ctx->accum_bytes = need;
     ctx->acc = L;
+    ctx->frame_src = -1;
     cudaMemsetAsync(ctx->accum, 0, need, ctx->stream);
     cudaStreamSynchronize(ctx->stream);
     return RT_OK;
@@ -2257,6 +2293,7 @@ static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t w
     ctx->acc = AccumLayout();
     ctx->accum_bytes = ctx->accum_cap = 0;
     ctx->moments_valid = ctx->aov_valid = ctx->sums_uploaded = false;
+    ctx->frame_src = -1;
     if (!device_ptr) return RT_OK;
     size_t need = (size_t)width * height * 4 * sizeof(unsigned long long);
     if (width <= 0 || height <= 0 || bytes < need) return fail(ctx, RT_ERR_INVALID, "rt_bind_accum: need %zu bytes for %dx%d, got %zu", need, width, height, bytes);
@@ -2413,6 +2450,7 @@ static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int
     ctx->moments_valid = false;  // until rt_moments_upload restores the moments of the same samples
     ctx->aov_valid = false;      // the AOV sums are not restored
     ctx->sums_uploaded = true;
+    ctx->frame_src = -1;         // a checkpoint resumes with either source
     return RT_OK;
 }
 
@@ -2640,6 +2678,17 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     if (aov && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->aov_valid)
         return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_AOV | RT_FLAG_ACCUMULATE onto a frame whose sums have no AOV sums "
                                        "(start it with a non-accumulating AOV pass)");
+    const bool rays = (p->flags & RT_FLAG_CAMERA_RAYS) != 0;
+    if (rays && (p->flags & (RT_FLAG_STATS | RT_FLAG_MOMENTS)))
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_CAMERA_RAYS has no RT_FLAG_STATS or RT_FLAG_MOMENTS instance");
+    if (rays && !ctx->rays_w) return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_CAMERA_RAYS without rays (set them with rt_set_camera_rays)");
+    if (rays && (p->width != ctx->rays_w || p->height != ctx->rays_h))
+        return fail(ctx, RT_ERR_INVALID, "rt_render: RT_FLAG_CAMERA_RAYS for a %dx%d frame, the rays are %dx%d", p->width, p->height,
+                    ctx->rays_w, ctx->rays_h);
+    const int64_t src = rays ? ctx->rays_gen : 0;
+    if ((p->flags & RT_FLAG_ACCUMULATE) && ctx->frame_src >= 0 && ctx->frame_src != src)
+        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE %s onto a frame of %s", rays ? "with RT_FLAG_CAMERA_RAYS" : "from the camera",
+                    ctx->frame_src == 0 ? "the camera" : "other rays (rt_set_camera_rays was called since it started)");
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
     // RT_FLAG_OVERLAP: this pass goes to one of the two lane streams with its own work counter and waits for nothing on
@@ -2680,15 +2729,17 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         if (rc != RT_OK) return rc;
     }
     ctx->aov_valid = aov;  // the same rule
+    ctx->frame_src = src;  // an accumulating pass of another source was refused above
     ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
     // which instance of render_kernel_v2 runs: LITE = no triangles, no point lights, no defocus blur in this scene (see
     // hit_prim); the NEE instances count no STATS; the first per-scene instance that covers the scene's features, unless
-    // RT_B200_GENERAL_INSTANCE=1 asks for a general one
-    const V2Key req{stats && !(want_nee || want_shadow), ctx->scene_lite && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, moments,
-                    false, aov, ctx->scene.wide_width ? ctx->scene.wide_width : 2, getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
+    // RT_B200_GENERAL_INSTANCE=1 asks for a general one.  A rays pass never defocuses: LITE up to the camera is enough
+    const V2Key req{stats && !(want_nee || want_shadow), (rays ? ctx->geom_lite : ctx->scene_lite) && !getenv("RT_B200_NO_LITE"),
+                    want_nee || want_shadow, moments, false, aov, rays, ctx->scene.wide_width ? ctx->scene.wide_width : 2,
+                    getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
     const V2Instance* e = v2_select(req);
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
@@ -2696,7 +2747,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     RenderArgs A;
     plan_pass(A, p, mode, rank, count, 1, grid);
     A.compact = L.compact;
-    A.set_side(ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
+    A.set_side(rays ? (const void*)ctx->rays : (const void*)ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
     A.nee_emitters = want_nee;
     A.shadow_point_lights = want_shadow;
     A.k0 = (uint32_t)(p->seed & 0xffffffffu);
@@ -2768,6 +2819,7 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     if ((p->flags & unsupported) || p->shard_count > 1)
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_STATS, RT_FLAG_MOMENTS, RT_FLAG_COMPACT_TILES, RT_FLAG_OVERLAP, RT_FLAG_AOV and shards are not "
                                              "supported for multi-view batches (flags 0x%x, shard_count %d)", p->flags & unsupported, p->shard_count);
+    if (p->flags & RT_FLAG_CAMERA_RAYS) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: RT_FLAG_CAMERA_RAYS is for rt_render (a views batch has cameras)");
     if ((long long)n_views * p->width * p->height >= (1ll << 31))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views: %d views of %dx%d are 2^31 slots or more", n_views, p->width, p->height);
     bool defocus = false;
@@ -2823,7 +2875,7 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
     // LITE only when no view needs the defocus code the LITE instance leaves out
-    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, false, 2, FEAT_ALL};
+    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, false, false, 2, FEAT_ALL};
     const V2Instance* e = v2_select(req);
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
@@ -3112,6 +3164,35 @@ static int dev_download_aov(DevCtx* ctx, int32_t total_spp, float* aov) {
     return plane_to_host(ctx, plane, 32, ctx->acc, aov);
 }
 
+// ---- caller-defined cameras (rt_set_camera_rays, RT_FLAG_CAMERA_RAYS) ----------------------------------------------
+static_assert(sizeof(rt_camera_ray) == 3 * sizeof(float4), "a record is the 3 float4 record_ray loads, in the same order");
+
+// The records (checked by rt_set_camera_rays) copied to the device as they are, after the passes in flight, which may
+// still read the previous ones.  NULL frees them.  Every call is a new source of frames (frame_src).
+static int dev_set_camera_rays(DevCtx* ctx, const rt_camera_ray* rays, int32_t width, int32_t height) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    int rc = dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    ctx->rays_gen++;
+    ctx->rays_w = ctx->rays_h = 0;
+    const size_t need = rays ? (size_t)width * height * sizeof(rt_camera_ray) : 0;
+    if (ctx->rays && (!rays || need > ctx->rays_cap)) {
+        cudaFree(ctx->rays);
+        ctx->rays = nullptr;
+        ctx->rays_cap = 0;
+    }
+    if (!rays) return RT_OK;
+    if (!ctx->rays) {
+        if (cudaMalloc(&ctx->rays, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_camera_rays: cannot allocate %zu bytes for the rays", need);
+        ctx->rays_cap = need;
+    }
+    CU(ctx, cudaMemcpyAsync(ctx->rays, rays, need, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    ctx->rays_w = width;
+    ctx->rays_h = height;
+    return RT_OK;
+}
+
 static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* prim_id, float* t, float* normal, float* point,
                              float* uv) {
     if (!ctx) return RT_ERR_INVALID;
@@ -3160,7 +3241,7 @@ extern "C" size_t rt_struct_size(int which) {
     static const size_t sizes[] = {sizeof(rt_scene_desc), sizeof(rt_render_params), sizeof(rt_stats), sizeof(rt_sphere), sizeof(rt_quad),
                                    sizeof(rt_triangle), sizeof(rt_medium), sizeof(rt_material), sizeof(rt_texture), sizeof(rt_image),
                                    sizeof(rt_perlin), sizeof(rt_point_light), sizeof(rt_camera), sizeof(rt_xform), sizeof(rt_prim_ref),
-                                   sizeof(rt_mesh)};
+                                   sizeof(rt_mesh), sizeof(rt_camera_ray)};
     return (which >= 0 && which < (int)(sizeof(sizes) / sizeof(sizes[0]))) ? sizes[which] : 0;
 }
 

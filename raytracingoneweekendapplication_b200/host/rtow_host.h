@@ -1746,6 +1746,10 @@ class camera {
     // inputs of an external denoiser and of compositing.  Not combined with a turntable, a checkpoint, a noise target
     // or variance output.  Empty: off.
     std::string aov_name;
+    // panorama (RT_FLAG_CAMERA_RAYS): a 360-degree equirectangular view around lookfrom with vup up and lookat - lookfrom
+    // at the image centre (panorama_rays), instead of the pinhole.  Combines with AOV output and several devices; not
+    // with a turntable, a checkpoint, a noise target or variance output.
+    bool panorama = false;
 
     int image_height() const {
         int h = int(image_width / aspect_ratio);  // Camera.txt:137-138
@@ -1777,6 +1781,44 @@ class camera {
         return c;
     }
 
+    // The rt_camera_ray records of the panorama for a width x height frame, row-major.  Pixel (i, j) looks at longitude
+    // phi = 2 pi ((i + 0.5) / width - 0.5) to the right of the forward direction f and latitude
+    // theta = pi (0.5 - (j + 0.5) / height) above it: d = cos theta (sin phi r + cos phi f) + sin theta up, with
+    // r = f x vup and up = r x f normalised.  dx and dy are its exact derivatives per pixel, 2 pi / width dd/dphi and
+    // -pi / height dd/dtheta.  Everything in double, each value rounded once to float.
+    std::vector<rt_camera_ray> panorama_rays(int width, int height) const {
+        const double pi = 3.1415926535897932385;
+        auto unit = [](double v[3]) {
+            const double l = std::sqrt(v[0] * v[0] + v[1] * v[1] + v[2] * v[2]);
+            for (int k = 0; k < 3; k++) v[k] /= l;
+        };
+        double f[3] = {lookat[0] - lookfrom[0], lookat[1] - lookfrom[1], lookat[2] - lookfrom[2]}, r[3], up[3];
+        unit(f);
+        r[0] = f[1] * vup[2] - f[2] * vup[1];
+        r[1] = f[2] * vup[0] - f[0] * vup[2];
+        r[2] = f[0] * vup[1] - f[1] * vup[0];
+        unit(r);
+        up[0] = r[1] * f[2] - r[2] * f[1];
+        up[1] = r[2] * f[0] - r[0] * f[2];
+        up[2] = r[0] * f[1] - r[1] * f[0];
+        std::vector<rt_camera_ray> rays((size_t)width * height);
+        for (int j = 0; j < height; j++) {
+            const double theta = pi * (0.5 - (j + 0.5) / height), ct = std::cos(theta), st = std::sin(theta);
+            for (int i = 0; i < width; i++) {
+                const double phi = 2.0 * pi * ((i + 0.5) / width - 0.5), cp = std::cos(phi), sp = std::sin(phi);
+                rt_camera_ray& R = rays[(size_t)j * width + i];
+                for (int k = 0; k < 3; k++) {
+                    const double side = sp * r[k] + cp * f[k];  // the horizontal direction at longitude phi
+                    R.origin[k] = (float)lookfrom[k];
+                    R.direction[k] = (float)(ct * side + st * up[k]);
+                    R.dx[k] = (float)(2.0 * pi / width * ct * (cp * r[k] - sp * f[k]));
+                    R.dy[k] = (float)(-pi / height * (ct * up[k] - st * side));
+                }
+            }
+        }
+        return rays;
+    }
+
     // <stem><suffix><ext> (the extension is what follows the last '.' of the file name)
     static std::string suffixed_name(const std::string& name, const char* suffix) {
         const size_t slash = name.find_last_of("/\\"), dot = name.find_last_of('.');
@@ -1805,6 +1847,10 @@ class camera {
             if (ctx) rt_destroy(ctx);
             std::exit(2);
         };
+        if (panorama && (turntable_frames > 1 || !checkpoint_path.empty() || noise_target > 0 || !variance_name.empty())) {
+            std::cerr << "rt_b200: a panorama is not combined with a turntable, a checkpoint, a noise target or variance output" << std::endl;
+            std::exit(2);
+        }
         if (turntable_frames > 1 && (!checkpoint_path.empty() || noise_target > 0 || !variance_name.empty() || !aov_name.empty() || devs.size() > 1)) {
             std::cerr << "rt_b200: a turntable renders on one device without a checkpoint, a noise target, variance or AOV output" << std::endl;
             std::exit(2);
@@ -1854,6 +1900,10 @@ class camera {
         }
         const bool aov = !aov_name.empty();
         if (aov && devs.size() > 1) p.shard_mode = RT_SHARD_TILES;  // and the AOVs
+        if (panorama) {
+            const std::vector<rt_camera_ray> rays = panorama_rays(p.width, p.height);
+            if (rt_set_camera_rays(ctx, rays.data(), p.width, p.height) != RT_OK) fail("rt_set_camera_rays");
+        }
         std::vector<uint64_t> sums, msums;
         if (!checkpoint_path.empty()) {
             rtb200::checkpoint_header old;
@@ -1905,7 +1955,7 @@ class camera {
             // pass is waited for, so that the progress line below stays within eight passes of the truth; checkpoints
             // and the download wait for everything by themselves.
             p.flags = (fresh ? 0 : (RT_FLAG_ACCUMULATE | RT_FLAG_ASYNC | RT_FLAG_OVERLAP)) | estimator_flags | (moments ? RT_FLAG_MOMENTS : 0u) |
-                      (aov ? RT_FLAG_AOV : 0u);
+                      (aov ? RT_FLAG_AOV : 0u) | (panorama ? RT_FLAG_CAMERA_RAYS : 0u);
             fresh = false;
             if (rt_render(ctx, &p) != RT_OK) fail("rt_render");
             if (++passes % 8 == 0 && rt_sync(ctx) != RT_OK) fail("rt_sync");

@@ -146,6 +146,19 @@ int rtsc_turntable_camera(const char* name, unsigned seed, const char* asset_dir
     return 0;
 }
 
+// The rt_camera_ray records camera::panorama_rays makes for a BASELINE scene at width x height (out: width * height).
+int rtsc_panorama_rays(const char* name, unsigned seed, const char* asset_dir, int width, int height, rt_camera_ray* out) {
+    scene_config cfg;
+    if (asset_dir) cfg.asset_dir = asset_dir;
+    hittable_list world;
+    camera cam;
+    std::vector<point_light> lights;
+    if (!out || width <= 0 || height <= 0 || !build_scene(name, seed, world, cam, lights, cfg)) return 1;
+    const std::vector<rt_camera_ray> rays = cam.panorama_rays(width, height);
+    std::copy(rays.begin(), rays.end(), out);
+    return 0;
+}
+
 // mesh::loadObj on its own (SURVEY 8f rank 2).  loader = 1 selects the reference's structure
 // (one shared_ptr<triangle> per face, mesh.h:22-121), 0 the fast path (parallel parse, one
 // triangle_soup), 2 the fast path into one indexed_mesh (rt_mesh).  with_media adds three constant_medium spheres next to the mesh and wraps the list
