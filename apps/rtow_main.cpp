@@ -44,6 +44,8 @@ int main(int argc, char** argv) {
     //            --aov FILE.exr|.pfm          also write the antialiased first-hit albedo, normal and depth to
     //                                         <stem>_albedo<ext>, <stem>_normal<ext>, <stem>_depth<ext>
     //            --panorama                   a 360-degree equirectangular view around lookfrom (takes no value)
+    //            --env FILE.pfm [--env-rotate DEG]  light the scene with an equirectangular HDR map instead of the
+    //                                         background, turned DEG degrees about +y
     for (int i = 7; i < argc; i += 2) {
         std::string k = argv[i];
         if (k == "--panorama") {
@@ -62,6 +64,8 @@ int main(int argc, char** argv) {
         else if (k == "--variance") cam.variance_name = argv[i + 1];
         else if (k == "--turntable") cam.turntable_frames = std::atoi(argv[i + 1]);
         else if (k == "--aov") cam.aov_name = argv[i + 1];
+        else if (k == "--env") cam.environment_map = argv[i + 1];
+        else if (k == "--env-rotate") cam.environment_rotation_y = std::atof(argv[i + 1]);
         else if (k == "--shadowed-point-lights") cam.shadowed_point_lights = std::atoi(argv[i + 1]) != 0;
         else if (k == "--devices") {
             std::string v = argv[i + 1];

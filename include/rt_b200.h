@@ -519,7 +519,8 @@ int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double
  *                           ray's origin (on the lens when defocused); a hit
  *   light                   albedo = the emitted radiance clamped to [0, 1]; normal and depth as above; a hit
  *   medium scatter event    albedo = the isotropic attenuation; normal 0; depth = the distance to the event; a hit
- *   miss                    albedo = the background clamped to [0, 1]; normal 0; no depth; no hit
+ *   miss                    albedo = the background (rt_set_environment: the environment) clamped to [0, 1]; normal 0;
+ *                           no depth; no hit
  * The sums are 8 uint64 per pixel: albedo x3 and depth unsigned, clamped to [0, 2^20], normal x3 signed (two's
  * complement), clamped to [-1, 1], all in 2^-RT_ACCUM_FRAC_BITS units, then the hit count.  A sample adds at most 2^48 to a
  * word (2^28 in magnitude to a normal word), so with at most 65536 samples per pixel no word overflows however the
@@ -559,6 +560,37 @@ typedef struct rt_camera_ray {
  * rt_accum_upload (or bound with rt_bind_accum) accepts either, which is how a checkpointed rays render resumes. */
 int rt_set_camera_rays(rt_ctx* ctx, const rt_camera_ray* rays, int32_t width, int32_t height);
 
+/* Environment lighting: an equirectangular map of linear radiance that every ray leaving the scene sees, instead of the
+ * camera's constant background -- image-based lighting, sky backgrounds, random HDRIs for synthetic data.
+ * The map frame has +y up, -z at the image centre and +x to the right (camera::panorama_rays with lookfrom 0, lookat
+ * (0, 0, -1) and vup +y, so pixel (i, j) of a width x height panorama looks at the centre of texel (i, j)).  rgb holds
+ * width*height*3 floats, row-major, row 0 at the +y pole; rotation takes map directions to world directions (row-major). */
+typedef struct rt_environment {
+    const float* rgb;
+    int32_t width, height;
+    double rotation[9];
+} rt_environment; /* rt_struct_size(17) */
+
+/* rt_set_environment copies the map to every device of the context (the caller may free its texels when the call
+ * returns), after the passes in flight, overlapped ones included.  env == NULL goes back to the camera's background.
+ * RT_ERR_INVALID for rgb == NULL, width or height < 1, width*height >= 2^31, a texel that is negative or not finite, or a
+ * rotation that is not orthonormal with determinant +1 within 1e-6 (the message names the first); a refused call changes
+ * nothing.  rt_upload_scene and rt_refit_scene keep the environment, and setting it does not touch the frame.
+ * The radiance of a ray with direction d that leaves the scene (in FP32):
+ *   1. m = R^T d, R = rotation
+ *   2. phi = atan2(m.x, -m.z), theta = atan2(m.y, sqrt(m.x^2 + m.z^2))
+ *   3. tx = (phi / (2 pi) + 1/2) width - 1/2, ty = (1/2 - theta / pi) height - 1/2
+ *   4. bilinear between texels floor(tx), floor(tx) + 1 (columns modulo width) and floor(ty), floor(ty) + 1 (rows
+ *      clamped to [0, height - 1]), each lerp a + t (b - a), so that a uniform map returns its texel exactly: a map of
+ *      texels equal to the background renders the frame of the background bit for bit.
+ * While an environment is set it replaces the background in every render: rt_render with any flags, shards, compact
+ * tiles, overlapped passes and multi-device contexts, and rt_render_views (whose rule on cameras[v].background stays).
+ * With RT_FLAG_AOV a miss reports the environment clamped to [0, 1] as its albedo.  With RT_FLAG_NEE the environment is
+ * gathered only by the paths whose BSDF-sampled direction leaves the scene, at full weight: NEE samples the listed quad
+ * emitters only, so no other technique covers those directions and the estimate stays unbiased.  RT_FLAG_STATS is
+ * RT_ERR_UNSUPPORTED while an environment is set, and a wide tree (rt_set_bvh_width) is traversed as the binary tree. */
+int rt_set_environment(rt_ctx* ctx, const rt_environment* env);
+
 /* Compact tile buffers across processes (one process per GPU, e.g. under torchrun; single-device contexts):
  *   rt_shard_pixels   slots of the compact buffer of shard (rank, count): its tiles x tile_size^2 (edge tiles padded)
  *   rt_resolve_tiles  the compact sums of the last RT_FLAG_COMPACT_TILES render -> averaged radiance (3 floats per slot)
@@ -593,7 +625,8 @@ int rt_get_stats(rt_ctx* ctx, rt_stats* out);
  * binding (ctypes, cgo, JNI ...) can verify its own declarations at load time.
  * which: 0 rt_scene_desc, 1 rt_render_params, 2 rt_stats, 3 rt_sphere, 4 rt_quad,
  * 5 rt_triangle, 6 rt_medium, 7 rt_material, 8 rt_texture, 9 rt_image, 10 rt_perlin,
- * 11 rt_point_light, 12 rt_camera, 13 rt_xform, 14 rt_prim_ref, 15 rt_mesh, 16 rt_camera_ray; 0 for anything else. */
+ * 11 rt_point_light, 12 rt_camera, 13 rt_xform, 14 rt_prim_ref, 15 rt_mesh, 16 rt_camera_ray, 17 rt_environment;
+ * 0 for anything else. */
 size_t rt_struct_size(int which);
 
 /* FP32 FMA issue-rate microbenchmark on the context's device, for the FP32

@@ -94,6 +94,10 @@ class rt_camera_ray(C.Structure):
     _fields_ = [("origin", C.c_float * 3), ("direction", C.c_float * 3), ("dx", C.c_float * 3), ("dy", C.c_float * 3)]
 
 
+class rt_environment(C.Structure):
+    _fields_ = [("rgb", C.c_void_p), ("width", C.c_int32), ("height", C.c_int32), ("rotation", C.c_double * 9)]
+
+
 class rt_scene_desc(C.Structure):
     _fields_ = [
         ("struct_size", C.c_uint32), ("abi_version", C.c_uint32),
@@ -158,10 +162,12 @@ EXPORTED_SYMBOLS = [
     "rt_download_begin", "rt_untile_begin", "rt_frame_end", "rt_measure_l1_peak", "rt_visible_devices", "rt_join",
     "rt_download_variance", "rt_moments_download", "rt_moments_upload", "rt_frame_noise",
     "rt_render_views", "rt_download_views", "rt_refit_scene", "rt_download_aov", "rt_set_camera_rays",
+    "rt_set_environment",
 ]
 
 ABI_STRUCTS = [rt_scene_desc, rt_render_params, rt_stats, rt_sphere, rt_quad, rt_triangle, rt_medium, rt_material, rt_texture,
-               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref, rt_mesh, rt_camera_ray]
+               rt_image, rt_perlin, rt_point_light, rt_camera, rt_xform, rt_prim_ref, rt_mesh, rt_camera_ray,
+               rt_environment]
 
 _lib = None
 _scenes = None
@@ -226,6 +232,7 @@ def load() -> C.CDLL:
     lib.rt_frame_noise.argtypes = [vp, i32, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.rt_download_aov.argtypes = [vp, i32, vp]
     lib.rt_set_camera_rays.argtypes = [vp, vp, i32, i32]
+    lib.rt_set_environment.argtypes = [vp, C.POINTER(rt_environment)]
     lib.rt_render_views.argtypes = [vp, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.POINTER(C.c_uint64), i32]
     lib.rt_download_views.argtypes = [vp, i32, i32, i32, vp, vp]
     lib.rt_measure_fp32_peak.argtypes = [vp, C.POINTER(C.c_double)]
@@ -274,6 +281,7 @@ def load_scenes() -> C.CDLL:
     s.rtsc_panorama_rays.argtypes = [C.c_char_p, C.c_uint, C.c_char_p, C.c_int, C.c_int, C.POINTER(rt_camera_ray)]
     s.rtsc_write_exr.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
     s.rtsc_write_pfm.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_void_p]
+    s.rtsc_read_pfm.argtypes = [C.c_char_p, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p, C.c_size_t]
     s.rtsc_load_obj.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_float, C.POINTER(C.c_double)]
     s.rtsc_load_obj.restype = C.c_void_p
     s.rtsc_scene_hash.argtypes = [C.c_void_p]
@@ -443,6 +451,30 @@ class Context:
             raise ValueError(f"camera rays must be an (H, W, 12) float32 array, got {a.dtype} {a.shape}")
         a = np.ascontiguousarray(a)
         self._check(self.lib.rt_set_camera_rays(self._h, a.ctypes.data, a.shape[1], a.shape[0]))
+
+    def set_environment(self, rgb, rotation=None) -> None:
+        """rt_set_environment: an equirectangular map of linear radiance seen by every ray that leaves the scene, an
+        (H, W, 3) float32 array (numpy, or a contiguous CPU tensor), row 0 at the +y pole; rotation: the 3x3 rotation from
+        the map frame to the world (identity by default).  None goes back to the camera's background."""
+        if rgb is None:
+            self._check(self.lib.rt_set_environment(self._h, None))
+            return
+        if hasattr(rgb, "numpy"):  # a torch tensor: its CPU memory as it is
+            if rgb.device.type != "cpu" or not rgb.is_contiguous():
+                raise ValueError("an environment map must be a contiguous CPU tensor")
+            rgb = rgb.numpy()
+        a = np.asarray(rgb)
+        if a.dtype != np.float32 or a.ndim != 3 or a.shape[2] != 3:
+            raise ValueError(f"an environment map must be an (H, W, 3) float32 array, got {a.dtype} {a.shape}")
+        a = np.ascontiguousarray(a)
+        r = np.eye(3) if rotation is None else np.asarray(rotation, dtype=np.float64)
+        if r.shape != (3, 3):
+            raise ValueError(f"the rotation must be 3x3, got {r.shape}")
+        e = rt_environment()
+        e.rgb = a.ctypes.data
+        e.width, e.height = a.shape[1], a.shape[0]
+        e.rotation = (C.c_double * 9)(*r.reshape(9).tolist())
+        self._check(self.lib.rt_set_environment(self._h, C.byref(e)))
 
     def render_views(self, cameras, width: int, height: int, spp: int, max_depth: int = 50, seed: int = 1, seeds=None,
                      spp_begin: int = 0, accumulate: bool = False, blocking: bool = True, nee: bool = False,

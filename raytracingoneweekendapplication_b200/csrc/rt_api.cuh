@@ -257,6 +257,49 @@ extern "C" int rt_set_camera_rays(rt_ctx* ctx, const rt_camera_ray* rays, int32_
     return RT_OK;
 }
 
+// ---- environment lighting ----------------------------------------------------------------------------------------
+extern "C" int rt_set_environment(rt_ctx* ctx, const rt_environment* env) {
+    RT_NEED(ctx);
+    std::vector<float4> map;
+    if (env) {  // everything is checked before any device changes
+        if (!env->rgb) return failx(ctx, RT_ERR_INVALID, "rt_set_environment: rgb is NULL");
+        if (env->width < 1 || env->height < 1 || (long long)env->width * env->height >= (1ll << 31))
+            return failx(ctx, RT_ERR_INVALID, "rt_set_environment: bad map size %dx%d", env->width, env->height);
+        const double* R = env->rotation;
+        for (int i = 0; i < 9; i++)
+            if (!std::isfinite(R[i])) return failx(ctx, RT_ERR_INVALID, "rt_set_environment: rotation[%d] is not finite", i);
+        for (int i = 0; i < 3; i++)
+            for (int j = i; j < 3; j++) {
+                const double dot = R[3 * i] * R[3 * j] + R[3 * i + 1] * R[3 * j + 1] + R[3 * i + 2] * R[3 * j + 2];
+                if (std::fabs(dot - (i == j ? 1.0 : 0.0)) > 1e-6)
+                    return failx(ctx, RT_ERR_INVALID, "rt_set_environment: the rotation is not orthonormal (rows %d and %d: dot %.9g)", i, j, dot);
+            }
+        const double det = R[0] * (R[4] * R[8] - R[5] * R[7]) - R[1] * (R[3] * R[8] - R[5] * R[6]) + R[2] * (R[3] * R[7] - R[4] * R[6]);
+        if (std::fabs(det - 1.0) > 1e-6) return failx(ctx, RT_ERR_INVALID, "rt_set_environment: the rotation has determinant %.9g, not +1", det);
+        const size_t n = (size_t)env->width * env->height;
+        map.resize(kEnvHeader + n);
+        for (size_t k = 0; k < n; k++) {
+            const float* c = env->rgb + 3 * k;
+            for (int i = 0; i < 3; i++)
+                if (!(std::isfinite(c[i]) && c[i] >= 0.0f))
+                    return failx(ctx, RT_ERR_INVALID, "rt_set_environment: texel %zu (%d, %d) channel %d is %g (texels are finite and >= 0)", k,
+                                 (int)(k % (size_t)env->width), (int)(k / (size_t)env->width), i, (double)c[i]);
+            map[kEnvHeader + k] = make_float4(c[0], c[1], c[2], 0.0f);
+        }
+        for (int i = 0; i < 3; i++) map[i] = make_float4((float)R[3 * i], (float)R[3 * i + 1], (float)R[3 * i + 2], 0.0f);
+        std::memcpy(&map[0].w, &env->width, 4);
+        std::memcpy(&map[1].w, &env->height, 4);
+    }
+    for (DevCtx* d : ctx->dev) {
+        const int rc = dev_set_environment(d, env ? map.data() : nullptr, map.size());
+        if (rc == RT_OK) continue;
+        fwd(ctx, d, rc);
+        for (DevCtx* e : ctx->dev) dev_set_environment(e, nullptr, 0);  // no device keeps a map the others lack
+        return rc;
+    }
+    return RT_OK;
+}
+
 // ---- multi-device render ----------------------------------------------------------------------------------------
 static bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
 

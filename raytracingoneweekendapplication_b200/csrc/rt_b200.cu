@@ -2,7 +2,7 @@
 // device layout) and the sm_100a kernels of the path-tracing hot path.
 //
 // Kernel inventory (hand-written; the device builder of bvh_device.cuh also runs cub's sort and scan):
-//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS, AOV, RAYS>
+//   render_kernel_v2<STATS, LITE, NEE, WIDTH, FEAT, MOMENTS, VIEWS, AOV, RAYS, ENV>
 //                          the persistent megakernel that renders: raygen -> traverse -> media ->
 //                          shade -> accumulate, per-warp streams of (pixel, sample) pairs and 64-bit
 //                          fixed-point accumulation.  Its compiled instances are the rows of kV2Instances
@@ -121,6 +121,39 @@ __device__ __forceinline__ Ray record_ray(const float4* __restrict__ rec, const 
     return r;
 }
 
+// rt_set_environment: the radiance of the map along direction d, the lookup of include/rt_b200.h.  The map is 3 float4 of
+// header (rotation rows 0, 1, 2 in .xyz; width and height as ints in .w of the first two) and then one float4 per texel,
+// row-major.  Out of line for the reason add_aov is: the ENV instances keep the arithmetic of their twins' paths.
+constexpr int kEnvHeader = 3;
+__device__ __noinline__ V3 env_radiance(const DevScene& S, V3 d) {
+    const float4* __restrict__ e = S.env();
+    const float4 r0 = __ldg(e), r1 = __ldg(e + 1), r2 = __ldg(e + 2);
+    const int w = __float_as_int(r0.w), h = __float_as_int(r1.w);
+    // m = R^T d: the direction in the map frame
+    const float mx = fmaf(d.x, r0.x, fmaf(d.y, r1.x, d.z * r2.x));
+    const float my = fmaf(d.x, r0.y, fmaf(d.y, r1.y, d.z * r2.y));
+    const float mz = fmaf(d.x, r0.z, fmaf(d.y, r1.z, d.z * r2.z));
+    const float phi = atan2f(mx, -mz), theta = atan2f(my, sqrtf(fmaf(mx, mx, mz * mz)));
+    const float tx = fmaf(phi, 0.15915494309189535f, 0.5f) * (float)w - 0.5f;  // 1 / (2 pi)
+    const float ty = fmaf(-theta, 0.31830988618379067f, 0.5f) * (float)h - 0.5f;  // 1 / pi
+    const float fx0 = floorf(tx), fy0 = floorf(ty);
+    // clamped, so that a non-finite direction still reads texels inside the map
+    const float fx = fminf(fmaxf(tx - fx0, 0.0f), 1.0f), fy = fminf(fmaxf(ty - fy0, 0.0f), 1.0f);
+    int x0 = min(max((int)fx0, -1), w - 1), y0 = min(max((int)fy0, -1), h - 1);
+    int x1 = x0 + 1, y1 = y0 + 1;
+    if (x0 < 0) x0 += w;
+    if (x1 >= w) x1 -= w;
+    y0 = max(y0, 0);
+    y1 = min(y1, h - 1);
+    const float4* __restrict__ t = e + kEnvHeader;
+    const float4 a = __ldg(t + (size_t)y0 * w + x0), b = __ldg(t + (size_t)y0 * w + x1);
+    const float4 c = __ldg(t + (size_t)y1 * w + x0), q = __ldg(t + (size_t)y1 * w + x1);
+    auto lerp = [](float u, float v, float s) { return fmaf(s, v - u, u); };  // u + s (v - u): exact for u == v
+    const V3 top = v3(lerp(a.x, b.x, fx), lerp(a.y, b.y, fx), lerp(a.z, b.z, fx));
+    const V3 bot = v3(lerp(c.x, q.x, fx), lerp(c.y, q.y, fx), lerp(c.z, q.z, fx));
+    return v3(lerp(top.x, bot.x, fy), lerp(top.y, bot.y, fy), lerp(top.z, bot.z, fy));
+}
+
 // ---------------------------------------------------------------------------------
 // render_kernel_v2 — the production megakernel.
 //
@@ -206,8 +239,10 @@ struct LocalSlot {
 // Never with STATS, MOMENTS or VIEWS.
 // RAYS: the primary ray of a sample comes from its pixel's record of rt_set_camera_rays (record_ray), 3 float4 per pixel
 // at A.side(), instead of the uploaded camera.  Never with STATS, MOMENTS or VIEWS, the other users of A.side().
+// ENV: a ray that leaves the scene sees the environment map of rt_set_environment (env_radiance, at S.env()) instead of
+// S.background, in its radiance and in its AOV albedo.  Never with STATS, and on the binary tree only.
 template <bool STATS, bool LITE, bool NEE = false, int WIDTH = 2, int FEAT = FEAT_ALL, bool MOMENTS = false, bool VIEWS = false,
-          bool AOV = false, bool RAYS = false>
+          bool AOV = false, bool RAYS = false, bool ENV = false>
 __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT_WIDE_MIN_BLOCKS) render_kernel_v2(const __grid_constant__ DevScene S, const __grid_constant__ RenderArgs A,
                                                         unsigned long long* __restrict__ accum,
                                                         unsigned long long* __restrict__ counters, Stats* __restrict__ gstats) {
@@ -391,13 +426,16 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
             if ((FEAT & FEAT_MEDIA) && S.n_media > 0) medium = media_hit<STATS, (FEAT & FEAT_MEDIA_GENERAL) != 0>(S, ray, 0.001f, hit.t, rng, bounce, &st);
             bool done = false;
             if (medium < 0 && hit.prim == PRIM_NONE) {
+                V3 sky = v3(0, 0, 0);  // ENV: looked up before the path is loaded, so that L and T are not live across the call
+                if constexpr (ENV) sky = env_radiance(S, ray.d);
                 load_path();
-                L = L + T * v3(S.background);
+                if constexpr (ENV) L = L + T * sky;
+                else L = L + T * v3(S.background);
                 done = true;
                 if constexpr (AOV) {
                     if (bounce == 0)
                         add_aov(reinterpret_cast<unsigned long long*>(gstats) + 8ull * (A.compact ? lane_slot[threadIdx.x] : rng.pixel),
-                                clamp01(v3(S.background)), v3(0, 0, 0), 0.0f, v3(0, 0, 0), false);
+                                clamp01(ENV ? sky : v3(S.background)), v3(0, 0, 0), 0.0f, v3(0, 0, 0), false);
                 }
             } else {
                 Surface sf;
@@ -504,17 +542,20 @@ __global__ void __launch_bounds__(RT_V2_THREADS, WIDTH == 2 ? RT_MIN_BLOCKS : RT
 
 // Every compiled instance of render_kernel_v2, by its template parameters.  A request runs the first entry that covers it
 // (v2_select), so the order is the preference: the per-scene feature instances of the plain binary-tree kernel (see FEAT_*
-// above), then the general ones, LITE before plain.  NEE, MOMENTS, VIEWS, AOV and RAYS exist for the binary tree only (every
-// scene has one; shadow rays and paths then both go through it), and only as general instances.
+// above), then the general ones, LITE before plain.  NEE, MOMENTS, VIEWS, AOV, RAYS and ENV exist for the binary tree only
+// (every scene has one; shadow rays and paths then both go through it), and only as general instances.  ENV has no LITE
+// instances: its non-LITE ones cover every scene, and LITE twins would gain about 4.5 % on LITE scenes for six more
+// instances of build time and code size (DESIGN §11g).
 typedef void (*RenderKernel)(const DevScene, const RenderArgs, unsigned long long*, unsigned long long*, Stats*);
 struct V2Instance {
-    bool stats, lite, nee, moments, views, aov, rays;  // lite: the scene must be LITE (no triangles, point lights, defocus)
+    bool stats, lite, nee, moments, views, aov, rays, env;  // lite: the scene must be LITE (no triangles, point lights, defocus)
     int width;
     int feat;  // FEAT_* bits the instance carries
     RenderKernel kernel;
 };
-#define RT_V2(S, L, N, M, V, W, F, AV) {S, L, N, M, V, AV, false, W, F, render_kernel_v2<S, L, N, W, F, M, V, AV>}
-#define RT_V2_RAYS(L, N, AV) {false, L, N, false, false, AV, true, 2, FEAT_ALL, render_kernel_v2<false, L, N, 2, FEAT_ALL, false, false, AV, true>}
+#define RT_V2(S, L, N, M, V, W, F, AV) {S, L, N, M, V, AV, false, false, W, F, render_kernel_v2<S, L, N, W, F, M, V, AV>}
+#define RT_V2_RAYS(L, N, AV) {false, L, N, false, false, AV, true, false, 2, FEAT_ALL, render_kernel_v2<false, L, N, 2, FEAT_ALL, false, false, AV, true>}
+#define RT_V2_ENV(N, M, V, AV, R) {false, false, N, M, V, AV, R, true, 2, FEAT_ALL, render_kernel_v2<false, false, N, 2, FEAT_ALL, M, V, AV, R, true>}
 static const V2Instance kV2Instances[] = {
     RT_V2(false, true, false, false, false, 2, 0, false),                                  // C2: quads, nothing else
     RT_V2(false, true, false, false, false, 2, FEAT_MEDIA | FEAT_MSPHERE, false),          // C5: media bounded by spheres, a moving sphere
@@ -552,22 +593,36 @@ static const V2Instance kV2Instances[] = {
     RT_V2_RAYS(false, false, true),
     RT_V2_RAYS(true, true, true),
     RT_V2_RAYS(false, true, true),
+    RT_V2_ENV(false, false, false, false, false),                                          // ENV twins (rt_set_environment)
+    RT_V2_ENV(true, false, false, false, false),
+    RT_V2_ENV(false, true, false, false, false),                                           // + MOMENTS
+    RT_V2_ENV(true, true, false, false, false),
+    RT_V2_ENV(false, false, true, false, false),                                           // + VIEWS
+    RT_V2_ENV(true, false, true, false, false),
+    RT_V2_ENV(false, false, false, true, false),                                           // + AOV
+    RT_V2_ENV(true, false, false, true, false),
+    RT_V2_ENV(false, false, false, false, true),                                           // + RAYS
+    RT_V2_ENV(true, false, false, false, true),
+    RT_V2_ENV(false, false, false, true, true),                                            // + RAYS + AOV
+    RT_V2_ENV(true, false, false, true, true),
 };
 #undef RT_V2
 #undef RT_V2_RAYS
+#undef RT_V2_ENV
 
 // What a pass asks of the kernel: nee = NEE or shadowed point lights; lite = the scene (and every view) allows LITE;
-// width = the uploaded tree; feat = the FEAT_* bits the scene needs (FEAT_ALL: a general instance)
+// width = the uploaded tree; feat = the FEAT_* bits the scene needs (FEAT_ALL: a general instance); env = an environment
+// map is set
 struct V2Key {
-    bool stats, lite, nee, moments, views, aov, rays;
+    bool stats, lite, nee, moments, views, aov, rays, env;
     int width;
     int feat;
 };
 static const V2Instance* v2_select(const V2Key& k) {
-    const int width = (k.nee || k.moments || k.views || k.aov || k.rays) ? 2 : k.width;  // binary tree only
+    const int width = (k.nee || k.moments || k.views || k.aov || k.rays || k.env) ? 2 : k.width;  // binary tree only
     for (const V2Instance& e : kV2Instances)
         if (e.stats == k.stats && e.nee == k.nee && e.moments == k.moments && e.views == k.views && e.aov == k.aov && e.rays == k.rays &&
-            e.width == width && (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
+            e.env == k.env && e.width == width && (!e.lite || k.lite) && (k.feat & ~e.feat) == 0)
             return &e;
     return nullptr;
 }
@@ -914,6 +969,9 @@ struct DevCtx {
     size_t rays_cap = 0;
     int rays_w = 0, rays_h = 0;
     int64_t rays_gen = 0, frame_src = -1;
+    // rt_set_environment: the map as env_radiance reads it (kEnvHeader float4, then the texels); null: the background
+    float4* env = nullptr;
+    size_t env_cap = 0;
     // rt_render_views: the views frame (views_n x views_h x views_w slots of 32 B, view-major; no other call touches it),
     // the view table on the device, and what an accumulating views pass must match: the frame's shape and a
     // fingerprint of the cameras and seeds (views_n == 0: no views render yet)
@@ -1104,6 +1162,7 @@ static void dev_destroy(DevCtx* ctx) {
     if (ctx->noise_sums) cudaFree(ctx->noise_sums);
     if (ctx->aov) cudaFree(ctx->aov);
     if (ctx->rays) cudaFree(ctx->rays);
+    if (ctx->env) cudaFree(ctx->env);
     if (ctx->views_accum) cudaFree(ctx->views_accum);
     if (ctx->view_table) cudaFree(ctx->view_table);
     if (ctx->counters) cudaFree(ctx->counters);
@@ -2560,7 +2619,11 @@ static int launch_v2(DevCtx* ctx, const V2Instance& e, int grid, const RenderArg
                      unsigned long long* counters, cudaStream_t stream) {
     // an AOV instance takes its sums in the gstats parameter (it never counts stats; RenderArgs has no free hole left)
     Stats* side = e.aov ? reinterpret_cast<Stats*>(ctx->aov) : ctx->dstats;
-    e.kernel<<<grid, RT_V2_THREADS, v2_smem(ctx, e.width), stream>>>(ctx->scene, A, accum, counters, side);
+    // the environment pointer goes on this launch's copy of the scene, so whatever rebuilds or restores ctx->scene (an
+    // upload, the staged-scene cache, a refit) needs not know of it
+    DevScene S = ctx->scene;
+    if (e.env) S.set_env(ctx->env);
+    e.kernel<<<grid, RT_V2_THREADS, v2_smem(ctx, e.width), stream>>>(S, A, accum, counters, side);
     CU(ctx, cudaGetLastError());
     return RT_OK;
 }
@@ -2685,6 +2748,9 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     if (rays && (p->width != ctx->rays_w || p->height != ctx->rays_h))
         return fail(ctx, RT_ERR_INVALID, "rt_render: RT_FLAG_CAMERA_RAYS for a %dx%d frame, the rays are %dx%d", p->width, p->height,
                     ctx->rays_w, ctx->rays_h);
+    const bool env = ctx->env != nullptr;
+    if (env && (p->flags & RT_FLAG_STATS))
+        return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_STATS has no instance with an environment (rt_set_environment)");
     const int64_t src = rays ? ctx->rays_gen : 0;
     if ((p->flags & RT_FLAG_ACCUMULATE) && ctx->frame_src >= 0 && ctx->frame_src != src)
         return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE %s onto a frame of %s", rays ? "with RT_FLAG_CAMERA_RAYS" : "from the camera",
@@ -2738,7 +2804,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     // hit_prim); the NEE instances count no STATS; the first per-scene instance that covers the scene's features, unless
     // RT_B200_GENERAL_INSTANCE=1 asks for a general one.  A rays pass never defocuses: LITE up to the camera is enough
     const V2Key req{stats && !(want_nee || want_shadow), (rays ? ctx->geom_lite : ctx->scene_lite) && !getenv("RT_B200_NO_LITE"),
-                    want_nee || want_shadow, moments, false, aov, rays, ctx->scene.wide_width ? ctx->scene.wide_width : 2,
+                    want_nee || want_shadow, moments, false, aov, rays, env, ctx->scene.wide_width ? ctx->scene.wide_width : 2,
                     getenv("RT_B200_GENERAL_INSTANCE") ? FEAT_ALL : ctx->scene_feat};
     const V2Instance* e = v2_select(req);
     int grid = 0;
@@ -2875,7 +2941,8 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
     // LITE only when no view needs the defocus code the LITE instance leaves out
-    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, false, false, 2, FEAT_ALL};
+    const V2Key req{false, ctx->geom_lite && !defocus && !getenv("RT_B200_NO_LITE"), want_nee || want_shadow, false, true, false, false,
+                    ctx->env != nullptr, 2, FEAT_ALL};
     const V2Instance* e = v2_select(req);
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
@@ -3193,6 +3260,31 @@ static int dev_set_camera_rays(DevCtx* ctx, const rt_camera_ray* rays, int32_t w
     return RT_OK;
 }
 
+// ---- environment lighting (rt_set_environment) ----------------------------------------------------------------------
+// The map as env_radiance reads it (packed and checked by rt_set_environment: n float4), copied after the passes in
+// flight, which may still read the previous one.  NULL frees it.
+static int dev_set_environment(DevCtx* ctx, const float4* map, size_t n) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    int rc = dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    const size_t need = map ? n * sizeof(float4) : 0;
+    if (ctx->env && (!map || need > ctx->env_cap)) {
+        cudaFree(ctx->env);
+        ctx->env = nullptr;
+        ctx->env_cap = 0;
+    }
+    if (!map) return RT_OK;
+    float4* buf = ctx->env;
+    if (!buf) {
+        if (cudaMalloc(&buf, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_environment: cannot allocate %zu bytes for the map", need);
+        ctx->env_cap = need;
+    }
+    ctx->env = buf;
+    CU(ctx, cudaMemcpyAsync(buf, map, need, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return RT_OK;
+}
+
 static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* prim_id, float* t, float* normal, float* point,
                              float* uv) {
     if (!ctx) return RT_ERR_INVALID;
@@ -3241,7 +3333,7 @@ extern "C" size_t rt_struct_size(int which) {
     static const size_t sizes[] = {sizeof(rt_scene_desc), sizeof(rt_render_params), sizeof(rt_stats), sizeof(rt_sphere), sizeof(rt_quad),
                                    sizeof(rt_triangle), sizeof(rt_medium), sizeof(rt_material), sizeof(rt_texture), sizeof(rt_image),
                                    sizeof(rt_perlin), sizeof(rt_point_light), sizeof(rt_camera), sizeof(rt_xform), sizeof(rt_prim_ref),
-                                   sizeof(rt_mesh), sizeof(rt_camera_ray)};
+                                   sizeof(rt_mesh), sizeof(rt_camera_ray), sizeof(rt_environment)};
     return (which >= 0 && which < (int)(sizeof(sizes) / sizeof(sizes[0]))) ? sizes[which] : 0;
 }
 

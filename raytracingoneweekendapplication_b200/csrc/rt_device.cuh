@@ -19,6 +19,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <stddef.h>
 #include <stdint.h>
 #include "rt_b200.h"
 
@@ -81,6 +82,9 @@ struct DevScene {
     int root;
     int n_nodes;
     int n_world;  // 0: every ray misses (the root link is not followed)
+    uint32_t env_lo;  // the environment map of rt_set_environment (env_radiance), its two 32-bit halves in two alignment
+                      // holes (here and after n_media), so that no field or kernel parameter offset moves; only the ENV
+                      // instances read them.  Stamped on the launch's copy of the scene (launch_v2)
     // the W-wide quantised BVH collapsed from `nodes` (bvh_wide.h; null when the scene has none):
     // W = 8: 5 uint4 per node, W = 4: 3; wrefs[W * node + slot] = BVH2 leaf link of a leaf child
     const void* wnodes;
@@ -103,6 +107,7 @@ struct DevScene {
     const DevMedium* media;
     const float4* media_box;  // per box-bounded medium: {axis0, lo0} {axis1, lo1} {axis2, lo2} {hi0, hi1, hi2, -}
     int n_media;
+    uint32_t env_hi;
     const uint32_t* boundary;  // packed prim refs type<<28 | index
     const DevMaterial* mats;
     const DevTexture* texs;
@@ -118,7 +123,12 @@ struct DevScene {
     float center[3], dir00[3], du[3], dv[3], disk_u[3], disk_v[3];
     float background[3];
     int defocus;
+    __host__ __device__ const float4* env() const { return (const float4*)(((uint64_t)env_hi << 32) | env_lo); }
+    void set_env(const void* p) { env_lo = (uint32_t)(uintptr_t)p; env_hi = (uint32_t)((uint64_t)(uintptr_t)p >> 32); }
 };
+static_assert(sizeof(DevScene) == 344 && offsetof(DevScene, env_lo) == 20 && offsetof(DevScene, wnodes) == 24 &&
+                  offsetof(DevScene, env_hi) == 172 && offsetof(DevScene, boundary) == 176,
+              "the environment pointer fills alignment holes only");
 
 // One camera of a multi-view batch (rt_render_views): the camera block of DevScene for that view's camera and frame,
 // and the Philox key of its seed.  96 B.

@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace rtb200 {
@@ -24,6 +25,35 @@ inline bool write_pfm(const char* path, int w, int h, const float* rgb) {
     std::fprintf(f, "PF\n%d %d\n-1.0\n", w, h);
     for (int y = h - 1; y >= 0; y--) std::fwrite(rgb + (size_t)y * w * 3, sizeof(float), (size_t)w * 3, f);
     return std::fclose(f) == 0;
+}
+
+// A colour PFM ("PF") into rgb, w*h*3 floats, rows TOP-DOWN.  The header is "PF", the width, the height and the scale,
+// separated by whitespace, with one whitespace byte before the data; a negative scale means little-endian floats, a
+// positive one big-endian.  false for anything else, or a file shorter than its header says.
+inline bool read_pfm(const char* path, int& w, int& h, std::vector<float>& rgb) {
+    std::FILE* f = std::fopen(path, "rb");
+    if (!f) return false;
+    char magic[3] = {0, 0, 0};
+    double scale = 0;
+    bool ok = std::fread(magic, 1, 2, f) == 2 && magic[0] == 'P' && magic[1] == 'F' && std::fscanf(f, "%d %d %lf", &w, &h, &scale) == 3 &&
+              std::fgetc(f) != EOF && w > 0 && h > 0 && scale != 0 && (long long)w * h < (1ll << 31);
+    if (ok) {
+        const size_t row = (size_t)w * 3;
+        rgb.resize(row * h);
+        for (int y = h - 1; y >= 0 && ok; y--) ok = std::fread(rgb.data() + (size_t)y * row, sizeof(float), row, f) == row;
+        const uint32_t one = 1;
+        const bool host_little = *(const uint8_t*)&one == 1;
+        if (ok && (scale < 0) != host_little)
+            for (float& v : rgb) {
+                uint8_t b[4];
+                std::memcpy(b, &v, 4);
+                std::swap(b[0], b[3]);
+                std::swap(b[1], b[2]);
+                std::memcpy(&v, b, 4);
+            }
+    }
+    std::fclose(f);
+    return ok;
 }
 
 namespace exr_detail {

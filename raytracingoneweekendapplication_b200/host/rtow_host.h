@@ -1750,6 +1750,12 @@ class camera {
     // at the image centre (panorama_rays), instead of the pinhole.  Combines with AOV output and several devices; not
     // with a turntable, a checkpoint, a noise target or variance output.
     bool panorama = false;
+    // environment lighting (rt_set_environment): environment_map "sky.pfm" is an equirectangular map of linear radiance
+    // that every ray leaving the scene sees instead of the background, turned by environment_rotation_y degrees about
+    // +y (environment_rotation).  Combines with everything else; a checkpoint resumes only under the same map and turn.
+    // Empty: off.
+    std::string environment_map;
+    double environment_rotation_y = 0;
 
     int image_height() const {
         int h = int(image_width / aspect_ratio);  // Camera.txt:137-138
@@ -1819,6 +1825,13 @@ class camera {
         return rays;
     }
 
+    // rt_environment::rotation for environment_rotation_y: a turn of that many degrees about +y, row-major
+    void environment_rotation(double R[9]) const {
+        const double a = environment_rotation_y * 3.1415926535897932385 / 180.0, c = std::cos(a), s = std::sin(a);
+        const double r[9] = {c, 0, s, 0, 1, 0, -s, 0, c};
+        std::copy(r, r + 9, R);
+    }
+
     // <stem><suffix><ext> (the extension is what follows the last '.' of the file name)
     static std::string suffixed_name(const std::string& name, const char* suffix) {
         const size_t slash = name.find_last_of("/\\"), dot = name.find_last_of('.');
@@ -1859,8 +1872,19 @@ class camera {
             std::cerr << "rt_b200: AOV output is not combined with a checkpoint, a noise target or variance output" << std::endl;
             std::exit(2);
         }
+        rt_environment env{};
+        std::vector<float> env_rgb;
+        if (!environment_map.empty()) {
+            if (!rtb200::read_pfm(environment_map.c_str(), env.width, env.height, env_rgb)) {
+                std::cerr << "rt_b200: cannot read the environment map " << environment_map << " (a colour PFM)" << std::endl;
+                std::exit(2);
+            }
+            env.rgb = env_rgb.data();
+            environment_rotation(env.rotation);
+        }
         if (rt_create(&ctx, devs.data(), (int)devs.size()) != RT_OK) fail("rt_create");
         if (rt_upload_scene(ctx, &d) != RT_OK) fail("rt_upload_scene");
+        if (env.rgb && rt_set_environment(ctx, &env) != RT_OK) fail("rt_set_environment");
         if (turntable_frames > 1) {
             render_turntable(ctx, fail);
             return;
@@ -1882,6 +1906,12 @@ class camera {
         ck.version = moments ? 2 : 1;  // 2: the second moments follow the sums
         ck.width = p.width; ck.height = p.height; ck.max_depth = max_depth; ck.seed = seed;
         ck.scene_hash = checkpoint_path.empty() ? 0 : fs.hash();
+        if (ck.scene_hash && env.rgb) {  // the environment lights the frame too
+            ck.scene_hash = rtb200::fnv1a(&env.width, sizeof env.width, ck.scene_hash);
+            ck.scene_hash = rtb200::fnv1a(&env.height, sizeof env.height, ck.scene_hash);
+            ck.scene_hash = rtb200::fnv1a(env.rotation, sizeof env.rotation, ck.scene_hash);
+            ck.scene_hash = rtb200::fnv1a(env_rgb.data(), env_rgb.size() * sizeof(float), ck.scene_hash);
+        }
         const uint32_t estimator_flags = (next_event_estimation ? RT_FLAG_NEE : 0u) | (shadowed_point_lights ? RT_FLAG_SHADOWED_POINT_LIGHTS : 0u);
         ck.flags = estimator_flags;
         // a sample is clamped to 2^20 and stored in 2^-28 units: 2^16 samples of a saturated channel fill the 64-bit sum
@@ -1917,7 +1947,7 @@ class camera {
                     done = old.spp_done;
                     std::cerr << "Resuming " << image_name << " at sample " << done << " from " << checkpoint_path << std::endl;
                 } else {
-                    std::cerr << "Ignoring " << checkpoint_path << ": it belongs to a different scene, frame, depth, seed or estimator (NEE / shadowed lights)" << std::endl;
+                    std::cerr << "Ignoring " << checkpoint_path << ": it belongs to a different scene, environment, frame, depth, seed or estimator (NEE / shadowed lights)" << std::endl;
                 }
             }
         }

@@ -210,6 +210,18 @@ rtsc_scene* rtsc_load_obj(const char* path, int loader, int with_media, float sc
 // The writers on their own (CPU tests): frame of w*h*3 floats -> file.
 int rtsc_write_exr(const char* path, int w, int h, const float* rgb) { return rtb200::write_exr(path, w, h, rgb) ? 0 : 1; }
 int rtsc_write_pfm(const char* path, int w, int h, const float* rgb) { return rtb200::write_pfm(path, w, h, rgb) ? 0 : 1; }
+// The PFM reader on its own: a colour PFM -> w, h and, when capacity >= w*h*3, its floats top-down in rgb.  0 when read,
+// 2 when rgb is NULL or too small (w and h are set), 1 when the file is not a readable PFM.
+int rtsc_read_pfm(const char* path, int* w, int* h, float* rgb, size_t capacity) {
+    std::vector<float> px;
+    int pw = 0, ph = 0;
+    if (!path || !w || !h || !rtb200::read_pfm(path, pw, ph, px)) return 1;
+    *w = pw;
+    *h = ph;
+    if (!rgb || capacity < px.size()) return 2;
+    std::copy(px.begin(), px.end(), rgb);
+    return 0;
+}
 uint64_t rtsc_scene_hash(const rtsc_scene* s) { return s ? s->fs.hash() : 0; }
 // 1 when this library decodes JPEG / PNG textures (built with the user's stb_image.h), 0 when only PPM / PGM
 int rtsc_has_stb() {
