@@ -17,6 +17,7 @@
 //
 // Included by rt_b200.cu after pair_node.
 #pragma once
+#include "buffer.h"
 #include "bvh_device.cuh"
 
 namespace rtlbvh {
@@ -201,17 +202,12 @@ inline Layout plan_refit(const rt_scene_desc* sc, int n_prims) {
 // breadth-first order of the reachable nodes, where each one's child nodes sit in that order, a union box per
 // position, and the nodes per level.
 struct RefitTree {
-    unsigned char* mem = nullptr;
-    size_t cap = 0;
+    DeviceBuffer<unsigned char> mem;
     int* order = nullptr;
     int2* kids = nullptr;
     float4 *box_lo = nullptr, *box_hi = nullptr;
     int* count = nullptr;        // device: nodes per level
     std::vector<int> levels;     // nodes per level (empty: not derived for the uploaded tree)
-    void release() {
-        if (mem) cudaFree(mem);
-        *this = RefitTree();
-    }
 };
 
 // Walks the `n_nodes`-slot tree from `root` (a node) on `stream`; at most `max_levels` levels.  Returns false in
@@ -225,13 +221,7 @@ inline cudaError_t derive_refit_tree(RefitTree& RT, const float4* nodes, int roo
     const size_t o_order = p.add(n * 4), o_kids = p.add(n * 8), o_lo = p.add(n * 16), o_hi = p.add(n * 16),
                  o_count = p.add((size_t)(max_levels + 1) * 4);
     cudaError_t e;
-    if (p.size > RT.cap) {
-        if (RT.mem) cudaFree(RT.mem);
-        RT.mem = nullptr;
-        RT.cap = 0;
-        if ((e = cudaMalloc(&RT.mem, p.size)) != cudaSuccess) return e;
-        RT.cap = p.size;
-    }
+    if ((e = RT.mem.reserve(p.size)) != cudaSuccess) return e;
     RT.order = (int*)(RT.mem + o_order);
     RT.kids = (int2*)(RT.mem + o_kids);
     RT.box_lo = (float4*)(RT.mem + o_lo);

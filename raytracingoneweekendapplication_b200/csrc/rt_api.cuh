@@ -55,9 +55,8 @@ struct rt_ctx {
     // multi-device state
     bool rendered = false;
     rt_render_params last{};      // the frame the devices hold (resolved shard mode and tile size)
-    unsigned char* gather = nullptr;  // device 0: the shards' data side by side, shard d at d * gather_stride
-    size_t gather_cap = 0;
-    unsigned long long* base_sums = nullptr;  // device 0: a restored checkpoint (full frame), added to what the devices render
+    DeviceBuffer<unsigned char> gather;           // device 0: the shards' data side by side, shard d at d * gather_stride
+    DeviceBuffer<unsigned long long> base_sums;  // device 0: a restored checkpoint (full frame), added to what the devices render
     int base_w = 0, base_h = 0;
     NcclApi nccl;
     std::vector<NcclApi::comm_t> comms;
@@ -140,8 +139,8 @@ extern "C" void rt_destroy(rt_ctx* ctx) {
     if (!ctx->dev.empty()) {
         cudaSetDevice(ctx->dev[0]->device);
         cudaDeviceSynchronize();
-        if (ctx->gather) cudaFree(ctx->gather);
-        if (ctx->base_sums) cudaFree(ctx->base_sums);
+        ctx->gather.release();
+        ctx->base_sums.release();
     }
     for (auto c : ctx->comms)
         if (c) ctx->nccl.CommDestroy(c);
@@ -330,8 +329,7 @@ extern "C" int rt_render(rt_ctx* ctx, const rt_render_params* p) {
         return failx(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE onto a frame of another size or sharding");
     if (!(p->flags & RT_FLAG_ACCUMULATE) && ctx->base_sums) {  // a fresh frame forgets the restored checkpoint
         cudaSetDevice(ctx->dev[0]->device);
-        cudaFree(ctx->base_sums);
-        ctx->base_sums = nullptr;
+        ctx->base_sums.release();
     }
     // every device gets its shard and starts; nothing waits until all are running
     for (int d = 0; d < n; d++) {
@@ -382,24 +380,14 @@ extern "C" int rt_sync(rt_ctx* ctx) {
     return RT_OK;
 }
 
-static int ensure_gather(rt_ctx* ctx, size_t bytes) {
-    if (bytes <= ctx->gather_cap) return RT_OK;
-    cudaSetDevice(ctx->dev[0]->device);
-    if (ctx->gather) cudaFree(ctx->gather);
-    ctx->gather = nullptr;
-    ctx->gather_cap = 0;
-    if (cudaMalloc(&ctx->gather, bytes) != cudaSuccess) return failx(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of gather staging on device %d", bytes, ctx->dev[0]->device);
-    ctx->gather_cap = bytes;
-    return RT_OK;
-}
-
 // src[d] (on device d, `bytes[d]` bytes, produced on that device's stream) -> gather + d * stride on device 0.
 // NCCL: one group of n - 1 send/recv pairs over NVLink; otherwise peer copies on the source devices' streams.
 static int gather_to_dev0(rt_ctx* ctx, const std::vector<const void*>& src, const std::vector<size_t>& bytes, size_t stride) {
     const int n = (int)ctx->dev.size();
-    int rc = ensure_gather(ctx, stride * n);
-    if (rc != RT_OK) return rc;
     DevCtx* d0 = ctx->dev[0];
+    cudaSetDevice(d0->device);
+    if (ctx->gather.reserve(stride * n) != cudaSuccess)
+        return failx(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of gather staging on device %d", stride * n, d0->device);
     ctx->gathers++;
     if (ctx->gather_mode == 1) {
         // device 0's own part is a local copy; the others travel as send/recv pairs
@@ -437,7 +425,7 @@ static int gather_to_dev0(rt_ctx* ctx, const std::vector<const void*>& src, cons
 
 // Every pixel of the frame lives on one device: tile shards of this context only, no restored checkpoint to add
 static bool one_device_per_pixel(const rt_ctx* ctx) {
-    return ctx->dev[0]->acc.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size();
+    return ctx->dev[0]->frame.layout.compact && !ctx->base_sums && ctx->last.shard_count == (int)ctx->dev.size();
 }
 
 // What a device contributes to a gather: its raw sums, or its slots resolved, turned into variance or its AOV sums
@@ -454,16 +442,18 @@ static int gather_plane(rt_ctx* ctx, Plane what, int32_t total_spp, size_t* stri
     *stride = 0;
     for (int d = 0; d < n; d++) {
         DevCtx* dc = ctx->dev[d];
-        const size_t slots = dc->acc.slots();
-        int rc = what == Plane::Variance ? moments_ready(dc, "rt_download_variance") : what == Plane::Aov ? aov_ready(dc, "rt_download_aov") : dev_wait(dc);
+        const size_t slots = dc->frame.layout.slots();
+        int rc = what == Plane::Variance ? companion_ready(dc, kMoments, "rt_download_variance")
+                 : what == Plane::Aov    ? companion_ready(dc, kAov, "rt_download_aov")
+                                         : dev_wait(dc);
         if (rc == RT_OK && what == Plane::Variance) rc = dev_variance_into(dc, total_spp);
         const void* aov_plane = nullptr;
         if (rc == RT_OK && what == Plane::Aov) rc = dev_aov_into(dc, total_spp, 0, &aov_plane);
         if (rc == RT_OK && resolve) rc = stage_buffers(dc, slots, 0);
         if (rc == RT_OK && resolve)
-            rc = dev_resolve_into(dc, dc->accum, slots, total_spp, what == Plane::Linear ? dc->out_lin : nullptr, what == Plane::Rgb8 ? dc->out_rgb8 : nullptr);
+            rc = dev_resolve_into(dc, dc->frame.sums, slots, total_spp, what == Plane::Linear ? dc->out_lin.get() : nullptr, what == Plane::Rgb8 ? dc->out_rgb8.get() : nullptr);
         if (rc != RT_OK) return fwd(ctx, dc, rc);
-        src[d] = what == Plane::Sums ? (const void*)dc->accum : what == Plane::Aov ? aov_plane : what == Plane::Rgb8 ? (const void*)dc->out_rgb8 : (const void*)dc->out_lin;
+        src[d] = what == Plane::Sums ? (const void*)dc->frame.sums : what == Plane::Aov ? aov_plane : what == Plane::Rgb8 ? (const void*)dc->out_rgb8 : (const void*)dc->out_lin;
         bytes[d] = slots * bpp;
         *stride = std::max(*stride, (bytes[d] + 255) & ~(size_t)255);
     }
@@ -483,7 +473,7 @@ static int gather_sums_full(rt_ctx* ctx) {
     cudaSetDevice(d0->device);
     rc = stage_buffers(d0, 0, full);
     if (rc != RT_OK) return fwd(ctx, d0, rc);
-    if (d0->acc.compact) {
+    if (d0->frame.layout.compact) {
         // the devices hold shards urank * n + d of count ucount * n: inside this context they are n consecutive shards, so
         // the scatter works on the sub-frame "tiles with t mod count in [urank * n, urank * n + n)"; with ucount == 1
         // (the only case a single box needs) that is every tile
@@ -493,12 +483,12 @@ static int gather_sums_full(rt_ctx* ctx) {
         CUX(ctx, cudaMemcpyAsync(d0->frame_scratch, ctx->gather, full, cudaMemcpyDeviceToDevice, d0->stream));
         const size_t words = full / 8;
         for (int d = 1; d < n; d++)
-            add_sums_kernel<<<(unsigned)((words + 255) / 256), 256, 0, d0->stream>>>((unsigned long long*)d0->frame_scratch,
+            add_sums_kernel<<<(unsigned)((words + 255) / 256), 256, 0, d0->stream>>>((unsigned long long*)d0->frame_scratch.get(),
                                                                                      (const unsigned long long*)(ctx->gather + d * stride), words);
     }
     if (ctx->base_sums && ctx->base_w == w && ctx->base_h == h) {
         const size_t words = full / 8;
-        add_sums_kernel<<<(unsigned)((words + 255) / 256), 256, 0, d0->stream>>>((unsigned long long*)d0->frame_scratch, ctx->base_sums, words);
+        add_sums_kernel<<<(unsigned)((words + 255) / 256), 256, 0, d0->stream>>>((unsigned long long*)d0->frame_scratch.get(), ctx->base_sums, words);
     }
     CUX(ctx, cudaGetLastError());
     return RT_OK;
@@ -517,7 +507,7 @@ extern "C" int rt_download(rt_ctx* ctx, int32_t total_spp, float* rgb_linear, ui
         // sums first (sample-sharded frames, restored checkpoints), then one resolve of the whole frame on device 0
         int rc = gather_sums_full(ctx);
         if (rc != RT_OK) return rc;
-        return fwd(ctx, d0, resolve_to_host(d0, (const unsigned long long*)d0->frame_scratch, AccumLayout{w, h}, total_spp, rgb_linear, rgb8));
+        return fwd(ctx, d0, resolve_to_host(d0, (const unsigned long long*)d0->frame_scratch.get(), AccumLayout{w, h}, total_spp, rgb_linear, rgb8));
     }
     // tiles: resolve where they were rendered, move 3 (RGB8) or 12 (float) bytes per pixel instead of 32
     for (int pass = 0; pass < 2; pass++) {
@@ -559,16 +549,13 @@ extern "C" int rt_accum_upload(rt_ctx* ctx, const uint64_t* host, size_t bytes, 
         if (rc != RT_OK) return fwd(ctx, d, rc);
         // forget what the devices hold: the next RT_FLAG_ACCUMULATE render starts from cleared buffers
         cudaSetDevice(d->device);
-        if (d->accum && !d->accum_external) CUX(ctx, cudaMemsetAsync(d->accum, 0, d->accum_bytes, d->stream));
+        if (d->frame.sums) CUX(ctx, cudaMemsetAsync(d->frame.sums, 0, d->frame.sums_bytes(), d->stream));
         CUX(ctx, cudaStreamSynchronize(d->stream));
-        d->moments_valid = false;  // moments are not restored across devices (rt_moments_upload is single-device)
-        d->aov_valid = false;      // nor are the AOV sums
-        d->frame_src = -1;         // a checkpoint resumes with either source
+        frame_forget(d);  // companions are not restored across devices (rt_moments_upload is single-device)
     }
     cudaSetDevice(d0->device);
-    if (ctx->base_sums) cudaFree(ctx->base_sums);
-    ctx->base_sums = nullptr;
-    if (cudaMalloc(&ctx->base_sums, need) != cudaSuccess) return failx(ctx, RT_ERR_NOMEM, "rt_accum_upload: cannot allocate %zu bytes", need);
+    ctx->base_sums.release();  // allocated for exactly this frame
+    if (ctx->base_sums.reserve(need) != cudaSuccess) return failx(ctx, RT_ERR_NOMEM, "rt_accum_upload: cannot allocate %zu bytes", need);
     ctx->base_w = width;
     ctx->base_h = height;
     CUX(ctx, cudaMemcpyAsync(ctx->base_sums, host, need, cudaMemcpyHostToDevice, d0->stream));
@@ -586,34 +573,31 @@ static int multi_per_pixel_frame(rt_ctx* ctx, const char* what) {
     return RT_OK;
 }
 
+// A companion's plane of a multi-device frame (`what` names the entry point), produced where the tiles were rendered and
+// gathered at `bpp` bytes per pixel: the variance like the linear radiance of rt_download, the AOVs resolved
+static int download_companion(rt_ctx* ctx, Plane plane, int bpp, const char* what, int32_t total_spp, float* host) {
+    int rc = multi_per_pixel_frame(ctx, what);
+    if (rc != RT_OK) return rc;
+    size_t stride = 0;
+    rc = gather_plane(ctx, plane, total_spp, &stride);
+    if (rc != RT_OK) return rc;
+    return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, bpp, (int)ctx->dev.size(), ctx->last.width, ctx->last.height, ctx->last.tile_size, host));
+}
+
 extern "C" int rt_download_variance(rt_ctx* ctx, int32_t total_spp, float* variance) {
     RT_NEED(ctx);
-    const int n = (int)ctx->dev.size();
-    if (n == 1) return fwd(ctx, ctx->dev[0], dev_download_variance(ctx->dev[0], total_spp, variance));
+    if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], dev_download_variance(ctx->dev[0], total_spp, variance));
     if (!variance) return RT_ERR_INVALID;
     if (total_spp < 2) return failx(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
-    int rc = multi_per_pixel_frame(ctx, "rt_download_variance");
-    if (rc != RT_OK) return rc;
-    // like the linear radiance of rt_download: produced where the tiles were rendered, 12 bytes per pixel gathered
-    size_t stride = 0;
-    rc = gather_plane(ctx, Plane::Variance, total_spp, &stride);
-    if (rc != RT_OK) return rc;
-    return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 12, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, variance));
+    return download_companion(ctx, Plane::Variance, 12, "rt_download_variance", total_spp, variance);
 }
 
 extern "C" int rt_download_aov(rt_ctx* ctx, int32_t total_spp, float* aov) {
     RT_NEED(ctx);
-    const int n = (int)ctx->dev.size();
-    if (n == 1) return fwd(ctx, ctx->dev[0], dev_download_aov(ctx->dev[0], total_spp, aov));
+    if (ctx->dev.size() == 1) return fwd(ctx, ctx->dev[0], dev_download_aov(ctx->dev[0], total_spp, aov));
     if (!aov) return RT_ERR_INVALID;
     if (total_spp <= 0) return failx(ctx, RT_ERR_INVALID, "rt_download_aov: total_spp must be positive");
-    int rc = multi_per_pixel_frame(ctx, "rt_download_aov");
-    if (rc != RT_OK) return rc;
-    // resolved where the tiles were rendered, 32 bytes per pixel gathered
-    size_t stride = 0;
-    rc = gather_plane(ctx, Plane::Aov, total_spp, &stride);
-    if (rc != RT_OK) return rc;
-    return fwd(ctx, ctx->dev[0], dev_untile(ctx->dev[0], ctx->gather, stride, 32, n, ctx->last.width, ctx->last.height, ctx->last.tile_size, aov));
+    return download_companion(ctx, Plane::Aov, 32, "rt_download_aov", total_spp, aov);
 }
 
 extern "C" int rt_frame_noise(rt_ctx* ctx, int32_t total_spp, double* mean_radiance, double* rms_std_error) {

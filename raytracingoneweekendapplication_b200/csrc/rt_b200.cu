@@ -27,6 +27,7 @@
 #include <thread>
 #include <vector>
 
+#include "buffer.h"
 #include "bvh_build.h"
 #include "bvh_wide.h"
 #include "prim_derive.h"
@@ -922,6 +923,35 @@ struct AccumLayout {
     }
 };
 
+// The planes that carry per-slot data of the same samples as the sums, in the layout of the sums: the second moments
+// of RT_FLAG_MOMENTS (add_square) and the AOV sums of RT_FLAG_AOV (add_aov)
+enum { kMoments, kAov, kCompanions };
+struct CompanionKind {
+    int words;  // uint64 per slot
+    const char *flag, *noun, *buffer, *start;  // what the messages call the flag, the data and the buffer, how to start it
+};
+static const CompanionKind kCompanionKinds[kCompanions] = {
+    {6, "RT_FLAG_MOMENTS", "moments", "moments buffer",
+     "start it with a non-accumulating moments pass, or restore both with rt_accum_upload + rt_moments_upload"},
+    {8, "RT_FLAG_AOV", "AOV sums", "AOV sums", "start it with a non-accumulating AOV pass"}};
+
+// What a context knows of its accumulated frame.  A companion is valid only while it describes the same samples as the
+// sums, and an accumulating pass continues the source of the passes the frame holds.  Only frame_forget, ensure_accum,
+// dev_bind_accum, dev_accum_upload, the pass path of dev_render and dev_moments_upload write this record.
+struct FrameRecord {
+    unsigned long long* sums = nullptr;      // `owned`, or the caller's buffer of rt_bind_accum; null: nothing rendered or bound
+    DeviceBuffer<unsigned long long> owned;  // never holds a bound frame
+    bool bound = false;
+    AccumLayout layout;                      // of `sums`
+    struct Companion {
+        DeviceBuffer<unsigned long long> buf;  // allocated by the first pass that wants it
+        bool valid = false;
+    } companion[kCompanions];
+    int64_t src = -1;       // 0 the uploaded camera, rays_gen for those rays, -1 a cleared, bound or restored frame: either
+    bool uploaded = false;  // the sums are an rt_accum_upload, not rendered onto since (what rt_moments_upload completes)
+    size_t sums_bytes() const { return std::max<size_t>(layout.slots(), 1) * 4 * sizeof(unsigned long long); }
+};
+
 struct DevCtx {
     int device = 0;
     std::string error;
@@ -929,62 +959,35 @@ struct DevCtx {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     // the whole device scene lives in ONE arena, staged in pinned host memory and moved with
     // one copy per rt_upload_scene; both grow on demand and are reused across uploads
-    unsigned char* arena = nullptr;
-    size_t arena_cap = 0;
-    unsigned char* staging = nullptr;
-    size_t staging_cap = 0;
+    DeviceBuffer<unsigned char> arena;
+    PinnedBuffer<unsigned char> staging;
     // persistent output buffers of rt_download
-    float* out_lin = nullptr;
-    unsigned char* out_rgb8 = nullptr;
-    size_t out_pixels = 0;
+    DeviceBuffer<float> out_lin;
+    DeviceBuffer<unsigned char> out_rgb8;
     DevScene scene{};
     bool has_scene = false;
     bool scene_lite = false;  // no triangles, no point lights, no defocus: the LITE kernel instance applies
     bool geom_lite = false;   // no triangles, no point lights: LITE up to the camera (rt_render_views checks its views)
     rt_camera camera{};
-    // accumulation
-    unsigned long long* accum = nullptr;
-    size_t accum_bytes = 0, accum_cap = 0;
-    bool accum_external = false;
-    AccumLayout acc;                        // layout of `accum`
-    // RT_FLAG_MOMENTS: 6 words per slot of `acc` (add_square), allocated by the first moments render; valid when they
-    // describe the same samples as the sums (set by a non-accumulating moments pass or rt_moments_upload, cleared by
-    // an accumulating pass without the flag, a pass that replaces the frame without it, a layout change, rt_bind_accum
-    // and rt_accum_upload)
-    unsigned long long* moments = nullptr;
-    size_t moments_cap = 0;
-    bool moments_valid = false;
-    bool sums_uploaded = false;              // the frame is an rt_accum_upload, not rendered onto since (rt_moments_upload)
-    unsigned long long* noise_sums = nullptr;  // rt_frame_noise: the 12 partial words of noise_kernel
-    // RT_FLAG_AOV: 8 words per slot of `acc` (add_aov), allocated by the first AOV render; valid when they describe the
-    // same samples as the sums (set by a non-accumulating AOV pass, cleared by a pass without the flag and wherever the
-    // moments are cleared)
-    unsigned long long* aov = nullptr;
-    size_t aov_cap = 0;
-    bool aov_valid = false;
+    FrameRecord frame;
+    DeviceBuffer<unsigned long long> noise_sums;  // rt_frame_noise: the 12 partial words of noise_kernel
     // rt_set_camera_rays: 3 float4 per pixel (record_ray) of a rays_w x rays_h frame, and the number of the call that set
-    // them.  frame_src is the source of the passes the frame holds: 0 the uploaded camera, rays_gen for those rays, -1 a
-    // cleared, bound or restored frame that takes either (RT_FLAG_ACCUMULATE must not mix sources)
-    float4* rays = nullptr;
-    size_t rays_cap = 0;
+    // them (the source of the frames they render)
+    DeviceBuffer<float4> rays;
     int rays_w = 0, rays_h = 0;
-    int64_t rays_gen = 0, frame_src = -1;
+    int64_t rays_gen = 0;
     // rt_set_environment: the map as env_radiance reads it (kEnvHeader float4, then the texels); null: the background
-    float4* env = nullptr;
-    size_t env_cap = 0;
+    DeviceBuffer<float4> env;
     // rt_render_views: the views frame (views_n x views_h x views_w slots of 32 B, view-major; no other call touches it),
     // the view table on the device, and what an accumulating views pass must match: the frame's shape and a
     // fingerprint of the cameras and seeds (views_n == 0: no views render yet)
-    unsigned long long* views_accum = nullptr;
-    size_t views_cap = 0;
-    ViewRecord* view_table = nullptr;
-    size_t view_table_cap = 0;
+    DeviceBuffer<unsigned long long> views_accum;
+    DeviceBuffer<ViewRecord> view_table;
     int views_n = 0, views_w = 0, views_h = 0;
     uint64_t views_key = 0;
-    unsigned char* frame_scratch = nullptr;  // full-frame copies of compact data (checkpoints, single-shard downloads)
-    size_t frame_scratch_cap = 0;
-    unsigned long long* counters = nullptr;  // [0] work counter, [1..3] unused
-    Stats* dstats = nullptr;
+    DeviceBuffer<unsigned char> frame_scratch;  // full-frame copies of compact data (checkpoints, single-shard downloads)
+    DeviceBuffer<unsigned long long> counters;  // [0] work counter, [1..3] unused
+    DeviceBuffer<Stats> dstats;
     rt_stats stats{};
     int cam_w = 0, cam_h = 0;  // frame the device camera block was computed for
     CameraD camera_d{};        // the same camera in double (deterministic pixel-centre rays of the AOV)
@@ -995,8 +998,8 @@ struct DevCtx {
     // its own stream into pinned double buffers while the next pass renders
     struct OutFrame {
         cudaEvent_t done = nullptr;
-        unsigned char* pinned = nullptr;
-        size_t cap = 0, off_lin = 0, off_rgb8 = 0;
+        PinnedBuffer<unsigned char> pinned;
+        size_t off_lin = 0, off_rgb8 = 0;
         bool has_lin = false, has_rgb8 = false, active = false;
     };
     OutFrame frames[2];
@@ -1024,8 +1027,7 @@ struct DevCtx {
     size_t world_type_count[4] = {0, 0, 0, 0};  // primitives of each device type in the world list (validate_scene)
     int n_prims = 0;  // primitives of the world list with every mesh ref expanded to its triangles (validate_scene)
     rtlbvh::CopyRing copy_ring;        // pinned staging of the device path's raw-input copy
-    unsigned char* scratch = nullptr;  // work space of the device build and of rt_refit_scene, reused across calls
-    size_t scratch_cap = 0;
+    DeviceBuffer<unsigned char> scratch;  // work space of the device build and of rt_refit_scene, reused across calls
     // the scene-side state of the scene whose arena image is in `staging`: a cache hit of rt_upload_scene restores it
     // together with the arena (an rt_refit_scene in between changes both)
     struct SceneState {
@@ -1077,24 +1079,6 @@ static int fail(DevCtx* ctx, int code, const char* fmt, ...) {
 
 static void free_scene(DevCtx* ctx) { ctx->has_scene = false; }
 
-static void release_buffers(DevCtx* ctx) {
-    if (ctx->arena) cudaFree(ctx->arena);
-    if (ctx->scratch) cudaFree(ctx->scratch);
-    ctx->copy_ring.release();
-    ctx->refit_tree.release();
-    ctx->scratch = nullptr;
-    ctx->scratch_cap = 0;
-    if (ctx->staging) cudaFreeHost(ctx->staging);
-    if (ctx->out_lin) cudaFree(ctx->out_lin);
-    if (ctx->out_rgb8) cudaFree(ctx->out_rgb8);
-    if (ctx->frame_scratch) cudaFree(ctx->frame_scratch);
-    ctx->frame_scratch = nullptr;
-    ctx->frame_scratch_cap = 0;
-    ctx->arena = ctx->staging = ctx->out_rgb8 = nullptr;
-    ctx->out_lin = nullptr;
-    ctx->arena_cap = ctx->staging_cap = ctx->out_pixels = 0;
-}
-
 // layout of the scene arena: every block 256-byte aligned
 struct ArenaPlan {
     size_t size = 0;
@@ -1127,8 +1111,8 @@ static int dev_create(DevCtx** out, const int* device_ids, int n_devices) {
     CU(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     CU(ctx, cudaEventCreate(&ctx->ev0));
     CU(ctx, cudaEventCreate(&ctx->ev1));
-    CU(ctx, cudaMalloc(&ctx->counters, 12 * sizeof(unsigned long long)));  // {work counter, -, -, -} x (plain, overlap lane 0, lane 1)
-    CU(ctx, cudaMalloc(&ctx->dstats, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long)));
+    CU(ctx, ctx->counters.reserve(12 * sizeof(unsigned long long)));  // {work counter, -, -, -} x (plain, overlap lane 0, lane 1)
+    CU(ctx, ctx->dstats.reserve(sizeof(Stats) + kTravHistBins * sizeof(unsigned long long)));
     // local-memory traversal stacks live in L1: prefer L1 over shared memory (the wide instances
     // get their carve-out per launch, from the depth of the uploaded tree)
     for (const V2Instance& e : kV2Instances)
@@ -1156,17 +1140,7 @@ static void dev_destroy(DevCtx* ctx) {
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     free_scene(ctx);
-    release_buffers(ctx);
-    if (ctx->accum && !ctx->accum_external) cudaFree(ctx->accum);
-    if (ctx->moments) cudaFree(ctx->moments);
-    if (ctx->noise_sums) cudaFree(ctx->noise_sums);
-    if (ctx->aov) cudaFree(ctx->aov);
-    if (ctx->rays) cudaFree(ctx->rays);
-    if (ctx->env) cudaFree(ctx->env);
-    if (ctx->views_accum) cudaFree(ctx->views_accum);
-    if (ctx->view_table) cudaFree(ctx->view_table);
-    if (ctx->counters) cudaFree(ctx->counters);
-    if (ctx->dstats) cudaFree(ctx->dstats);
+    ctx->copy_ring.release();
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
     for (int k = 0; k < 2; k++) {
@@ -1177,12 +1151,10 @@ static void dev_destroy(DevCtx* ctx) {
     if (ctx->ov_begin) cudaEventDestroy(ctx->ov_begin);
     if (ctx->copy_stream) { cudaStreamSynchronize(ctx->copy_stream); cudaStreamDestroy(ctx->copy_stream); }
     if (ctx->ev_ready) cudaEventDestroy(ctx->ev_ready);
-    for (auto& f : ctx->frames) {
+    for (auto& f : ctx->frames)
         if (f.done) cudaEventDestroy(f.done);
-        if (f.pinned) cudaFreeHost(f.pinned);
-    }
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;  // frees the buffers, on this device
 }
 
 
@@ -1735,13 +1707,8 @@ static void set_features(DevCtx* ctx, const rt_scene_desc* sc, const std::vector
 
 // the work space of the device build and of rt_refit_scene, grown to `bytes`
 static int ensure_scratch(DevCtx* ctx, size_t bytes, const char* entry) {
-    if (bytes <= ctx->scratch_cap) return RT_OK;
-    if (ctx->scratch) cudaFree(ctx->scratch);
-    ctx->scratch = nullptr;
-    ctx->scratch_cap = 0;
-    size_t cap = bytes + bytes / 8;
-    if (cudaMalloc(&ctx->scratch, cap) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "%s: cannot allocate %zu bytes of build work space", entry, cap);
-    ctx->scratch_cap = cap;
+    const size_t alloc = bytes + bytes / 8;
+    if (ctx->scratch.reserve(bytes, alloc) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "%s: cannot allocate %zu bytes of build work space", entry, alloc);
     return RT_OK;
 }
 
@@ -1883,24 +1850,12 @@ static int upload_scene_impl(DevCtx* ctx, const rt_scene_desc* sc, bool device_b
     UP(tables.perlin_perm, perlin_perm) UP(tables.lights, lights) UP(nee_lights, nee_lights)
 #undef UP
 #undef UPW
-    if (plan.size > ctx->arena_cap) {
-        if (ctx->arena) cudaFree(ctx->arena);
-        ctx->arena = nullptr;
-        ctx->arena_cap = 0;
-        size_t cap = plan.size + plan.size / 4;
-        if (cudaMalloc(&ctx->arena, cap) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_upload_scene: cannot allocate %zu bytes of device memory", cap);
-        ctx->arena_cap = cap;
-    }
-    const size_t stage_need = device_build ? stage.size : plan.size;
-    if (stage_need > ctx->staging_cap) {
-        if (ctx->staging) cudaFreeHost(ctx->staging);
-        ctx->staging = nullptr;
-        ctx->staging_cap = 0;
-        size_t cap = stage_need + stage_need / 4;
-        if (cudaHostAlloc(&ctx->staging, cap, cudaHostAllocDefault) != cudaSuccess)
-            return fail(ctx, RT_ERR_NOMEM, "rt_upload_scene: cannot allocate %zu bytes of pinned host memory", cap);
-        ctx->staging_cap = cap;
-    }
+    const size_t arena_alloc = plan.size + plan.size / 4;
+    if (ctx->arena.reserve(plan.size, arena_alloc) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_upload_scene: cannot allocate %zu bytes of device memory", arena_alloc);
+    const size_t stage_need = device_build ? stage.size : plan.size, stage_alloc = stage_need + stage_need / 4;
+    if (ctx->staging.reserve(stage_need, stage_alloc) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_upload_scene: cannot allocate %zu bytes of pinned host memory", stage_alloc);
     for (int i = 0; i < sc->n_images; i++) {
         tables.images[i].rgb = ctx->arena + img_off[i];
         std::memcpy(ctx->staging + (device_build ? img_stage[i] : img_off[i]), sc->images[i].rgb, (size_t)sc->images[i].width * sc->images[i].height * 3);
@@ -2291,52 +2246,39 @@ extern "C" size_t rt_shard_pixels(int32_t width, int32_t height, int32_t tile_si
     return L.slots();
 }
 
+// The sums changed under the companions (a new layout, a binding, a restored checkpoint): no companion describes them,
+// and the next accumulating pass may come from either source
+static void frame_forget(DevCtx* ctx) {
+    for (FrameRecord::Companion& c : ctx->frame.companion) c.valid = false;
+    ctx->frame.src = -1;
+    ctx->frame.uploaded = false;
+}
+
 static int ensure_accum(DevCtx* ctx, const AccumLayout& L) {
-    const size_t need = std::max<size_t>(L.slots(), 1) * 4 * sizeof(unsigned long long);
-    if (ctx->accum_external) {
-        if (L.compact || ctx->acc.width != L.width || ctx->acc.height != L.height)
-            return fail(ctx, RT_ERR_STATE, "rt_render: the bound accumulation buffer is a full %dx%d frame, this render needs %s%dx%d", ctx->acc.width,
-                        ctx->acc.height, L.compact ? "compact tiles of " : "", L.width, L.height);
+    FrameRecord& F = ctx->frame;
+    if (F.bound) {
+        if (L.compact || F.layout.width != L.width || F.layout.height != L.height)
+            return fail(ctx, RT_ERR_STATE, "rt_render: the bound accumulation buffer is a full %dx%d frame, this render needs %s%dx%d", F.layout.width,
+                        F.layout.height, L.compact ? "compact tiles of " : "", L.width, L.height);
         return RT_OK;
     }
-    if (ctx->accum && ctx->acc == L) return RT_OK;
-    ctx->moments_valid = ctx->aov_valid = false;
-    if (!ctx->accum || need > ctx->accum_cap) {
-        if (ctx->accum) cudaFree(ctx->accum);
-        ctx->accum = nullptr;
-        ctx->accum_cap = 0;
-        if (cudaMalloc(&ctx->accum, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render: cannot allocate %zu bytes for the accumulation buffer", need);
-        ctx->accum_cap = need;
-    }
-    ctx->accum_bytes = need;
-    ctx->acc = L;
-    ctx->frame_src = -1;
-    cudaMemsetAsync(ctx->accum, 0, need, ctx->stream);
+    if (F.sums && F.layout == L) return RT_OK;
+    frame_forget(ctx);
+    F.layout = L;
+    const size_t need = F.sums_bytes();
+    const cudaError_t e = F.owned.reserve(need);
+    F.sums = F.owned;
+    if (e != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render: cannot allocate %zu bytes for the accumulation buffer", need);
+    cudaMemsetAsync(F.sums, 0, need, ctx->stream);
     cudaStreamSynchronize(ctx->stream);
     return RT_OK;
 }
 
-// the moments buffer of RT_FLAG_MOMENTS: 48 bytes per slot, same layout as `accum` (its contents are set by the caller)
-static int ensure_moments(DevCtx* ctx, size_t slots) {
-    const size_t need = std::max<size_t>(slots, 1) * 6 * sizeof(unsigned long long);
-    if (ctx->moments && need <= ctx->moments_cap) return RT_OK;
-    if (ctx->moments) cudaFree(ctx->moments);
-    ctx->moments = nullptr;
-    ctx->moments_cap = 0;
-    if (cudaMalloc(&ctx->moments, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes for the moments buffer", need);
-    ctx->moments_cap = need;
-    return RT_OK;
-}
-
-// the AOV sums of RT_FLAG_AOV: 64 bytes per slot, same layout as `accum` (its contents are set by the caller)
-static int ensure_aov(DevCtx* ctx, size_t slots) {
-    const size_t need = std::max<size_t>(slots, 1) * 8 * sizeof(unsigned long long);
-    if (ctx->aov && need <= ctx->aov_cap) return RT_OK;
-    if (ctx->aov) cudaFree(ctx->aov);
-    ctx->aov = nullptr;
-    ctx->aov_cap = 0;
-    if (cudaMalloc(&ctx->aov, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes for the AOV sums", need);
-    ctx->aov_cap = need;
+// the buffer of companion k for `slots` slots (its contents are set by the caller)
+static int companion_reserve(DevCtx* ctx, int k, size_t slots) {
+    const size_t need = std::max<size_t>(slots, 1) * kCompanionKinds[k].words * sizeof(unsigned long long);
+    if (ctx->frame.companion[k].buf.reserve(need) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes for the %s", need, kCompanionKinds[k].buffer);
     return RT_OK;
 }
 
@@ -2346,29 +2288,27 @@ static int dev_bind_accum(DevCtx* ctx, void* device_ptr, size_t bytes, int32_t w
     // passes still in flight (asynchronous, overlapped) write into the buffer that is about to be replaced
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    if (ctx->accum && !ctx->accum_external) cudaFree(ctx->accum);
-    ctx->accum = nullptr;
-    ctx->accum_external = false;
-    ctx->acc = AccumLayout();
-    ctx->accum_bytes = ctx->accum_cap = 0;
-    ctx->moments_valid = ctx->aov_valid = ctx->sums_uploaded = false;
-    ctx->frame_src = -1;
+    FrameRecord& F = ctx->frame;
+    F.owned.release();
+    F.sums = nullptr;
+    F.bound = false;
+    F.layout = AccumLayout();
+    frame_forget(ctx);
     if (!device_ptr) return RT_OK;
     size_t need = (size_t)width * height * 4 * sizeof(unsigned long long);
     if (width <= 0 || height <= 0 || bytes < need) return fail(ctx, RT_ERR_INVALID, "rt_bind_accum: need %zu bytes for %dx%d, got %zu", need, width, height, bytes);
-    ctx->accum = (unsigned long long*)device_ptr;
-    ctx->accum_external = true;
-    ctx->accum_bytes = need;
-    ctx->acc.width = width;
-    ctx->acc.height = height;
+    F.sums = (unsigned long long*)device_ptr;
+    F.bound = true;
+    F.layout.width = width;
+    F.layout.height = height;
     return RT_OK;
 }
 
 static int dev_accum_buffer(DevCtx* ctx, void** device_ptr, size_t* bytes) {
     if (!ctx || !device_ptr || !bytes) return RT_ERR_INVALID;
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "rt_accum_buffer: nothing rendered or bound yet");
-    *device_ptr = ctx->accum;
-    *bytes = ctx->accum_bytes;
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "rt_accum_buffer: nothing rendered or bound yet");
+    *device_ptr = ctx->frame.sums;
+    *bytes = ctx->frame.sums_bytes();
     return RT_OK;
 }
 
@@ -2430,26 +2370,13 @@ static cudaError_t launch_untile(int bpp, const void* shards, size_t stride, int
 // the copy of every outstanding hand-out (rt_download_begin / rt_untile_begin), which reads these buffers until its
 // rt_frame_end: a readback issued meanwhile does not change the frame the hand-out returns.
 static int stage_buffers(DevCtx* ctx, size_t pixels, size_t scratch_bytes) {
-    const bool grow_out = pixels > ctx->out_pixels, grow_scratch = scratch_bytes > ctx->frame_scratch_cap;
-    if ((grow_out || grow_scratch) && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // no free under a running copy
-    if (grow_out) {
-        if (ctx->out_lin) cudaFree(ctx->out_lin);
-        if (ctx->out_rgb8) cudaFree(ctx->out_rgb8);
-        ctx->out_lin = nullptr;
-        ctx->out_rgb8 = nullptr;
-        ctx->out_pixels = 0;
-        if (cudaMalloc(&ctx->out_lin, pixels * 3 * sizeof(float)) != cudaSuccess || cudaMalloc(&ctx->out_rgb8, pixels * 3) != cudaSuccess)
-            return fail(ctx, RT_ERR_NOMEM, "rt_download: cannot allocate the output buffers");
-        ctx->out_pixels = pixels;
-    }
-    if (grow_scratch) {
-        if (ctx->frame_scratch) cudaFree(ctx->frame_scratch);
-        ctx->frame_scratch = nullptr;
-        ctx->frame_scratch_cap = 0;
-        if (cudaMalloc(&ctx->frame_scratch, scratch_bytes) != cudaSuccess)
-            return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of frame scratch", scratch_bytes);
-        ctx->frame_scratch_cap = scratch_bytes;
-    }
+    const size_t lin = pixels * 3 * sizeof(float), rgb8 = pixels * 3;
+    const bool grow = lin > ctx->out_lin.capacity() || rgb8 > ctx->out_rgb8.capacity() || scratch_bytes > ctx->frame_scratch.capacity();
+    if (grow && ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);  // no free under a running copy
+    if (ctx->out_lin.reserve(lin) != cudaSuccess || ctx->out_rgb8.reserve(rgb8) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_download: cannot allocate the output buffers");
+    if (ctx->frame_scratch.reserve(scratch_bytes) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of frame scratch", scratch_bytes);
     for (const DevCtx::OutFrame& f : ctx->frames)
         if (f.active) CU(ctx, cudaStreamWaitEvent(ctx->stream, f.done, 0));
     return RT_OK;
@@ -2479,13 +2406,13 @@ static int dev_wait(DevCtx* ctx);
 // FULL row-major frame on the host side: a compact buffer is scattered into a zeroed frame first.
 static int dev_accum_download(DevCtx* ctx, uint64_t* host, size_t bytes) {
     if (!ctx || !host) return RT_ERR_INVALID;
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "rt_accum_download: nothing rendered or bound yet");
-    const size_t full = (size_t)ctx->acc.width * ctx->acc.height * 32;
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "rt_accum_download: nothing rendered or bound yet");
+    const size_t full = (size_t)ctx->frame.layout.width * ctx->frame.layout.height * 32;
     if (bytes < full) return fail(ctx, RT_ERR_INVALID, "rt_accum_download: need %zu bytes, got %zu", full, bytes);
     CU(ctx, cudaSetDevice(ctx->device));
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    return plane_to_host(ctx, ctx->accum, 32, ctx->acc, host);
+    return plane_to_host(ctx, ctx->frame.sums, 32, ctx->frame.layout, host);
 }
 
 static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int32_t width, int32_t height) {
@@ -2504,12 +2431,10 @@ static int dev_accum_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, int
     // on the context's stream (cudaMemcpy from pageable memory returns once the data is STAGED; the DMA itself is
     // ordered only against the legacy stream, and ctx->stream is non-blocking: a render enqueued right after could
     // start before the sums have landed)
-    CU(ctx, cudaMemcpyAsync(ctx->accum, host, need, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(ctx->frame.sums, host, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->moments_valid = false;  // until rt_moments_upload restores the moments of the same samples
-    ctx->aov_valid = false;      // the AOV sums are not restored
-    ctx->sums_uploaded = true;
-    ctx->frame_src = -1;         // a checkpoint resumes with either source
+    frame_forget(ctx);  // until rt_moments_upload restores the moments of the same samples; the AOV sums are not restored
+    ctx->frame.uploaded = true;
     return RT_OK;
 }
 
@@ -2618,7 +2543,7 @@ static int v2_grid(DevCtx* ctx, const V2Instance* e, int* grid) {
 static int launch_v2(DevCtx* ctx, const V2Instance& e, int grid, const RenderArgs& A, unsigned long long* accum,
                      unsigned long long* counters, cudaStream_t stream) {
     // an AOV instance takes its sums in the gstats parameter (it never counts stats; RenderArgs has no free hole left)
-    Stats* side = e.aov ? reinterpret_cast<Stats*>(ctx->aov) : ctx->dstats;
+    Stats* side = e.aov ? reinterpret_cast<Stats*>(ctx->frame.companion[kAov].buf.get()) : ctx->dstats;
     // the environment pointer goes on this launch's copy of the scene, so whatever rebuilds or restores ctx->scene (an
     // upload, the staged-scene cache, a refit) needs not know of it
     DevScene S = ctx->scene;
@@ -2730,17 +2655,12 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     const int count = p->shard_count <= 1 ? 1 : p->shard_count;
     const int rank = count == 1 ? 0 : p->shard_rank;
     if (rank < 0 || rank >= count) return fail(ctx, RT_ERR_INVALID, "rt_render: shard_rank %d outside [0,%d)", rank, count);
+    const bool accumulate = (p->flags & RT_FLAG_ACCUMULATE) != 0;
     const bool moments = (p->flags & RT_FLAG_MOMENTS) != 0;
     if (moments && (p->flags & RT_FLAG_STATS)) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_MOMENTS has no RT_FLAG_STATS instance");
-    if (moments && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->moments_valid)
-        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_MOMENTS | RT_FLAG_ACCUMULATE onto a frame whose sums have no moments "
-                                       "(start it with a non-accumulating moments pass, or restore both with rt_accum_upload + rt_moments_upload)");
     const bool aov = (p->flags & RT_FLAG_AOV) != 0;
     if (aov && (p->flags & (RT_FLAG_STATS | RT_FLAG_MOMENTS)))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_AOV has no RT_FLAG_STATS or RT_FLAG_MOMENTS instance");
-    if (aov && (p->flags & RT_FLAG_ACCUMULATE) && !ctx->aov_valid)
-        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_AOV | RT_FLAG_ACCUMULATE onto a frame whose sums have no AOV sums "
-                                       "(start it with a non-accumulating AOV pass)");
     const bool rays = (p->flags & RT_FLAG_CAMERA_RAYS) != 0;
     if (rays && (p->flags & (RT_FLAG_STATS | RT_FLAG_MOMENTS)))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_CAMERA_RAYS has no RT_FLAG_STATS or RT_FLAG_MOMENTS instance");
@@ -2751,24 +2671,6 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     const bool env = ctx->env != nullptr;
     if (env && (p->flags & RT_FLAG_STATS))
         return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render: RT_FLAG_STATS has no instance with an environment (rt_set_environment)");
-    const int64_t src = rays ? ctx->rays_gen : 0;
-    if ((p->flags & RT_FLAG_ACCUMULATE) && ctx->frame_src >= 0 && ctx->frame_src != src)
-        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE %s onto a frame of %s", rays ? "with RT_FLAG_CAMERA_RAYS" : "from the camera",
-                    ctx->frame_src == 0 ? "the camera" : "other rays (rt_set_camera_rays was called since it started)");
-    CU(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
-    // RT_FLAG_OVERLAP: this pass goes to one of the two lane streams with its own work counter and waits for nothing on
-    // the host; it needs the frame the passes before it render into, unchanged
-    // (the camera of this frame size must be set up already: the first pass onto a restored checkpoint is a plain one)
-    const bool overlap = (p->flags & RT_FLAG_OVERLAP) && (p->flags & RT_FLAG_ASYNC) && (p->flags & RT_FLAG_ACCUMULATE) &&
-                         !(p->flags & RT_FLAG_STATS) && ctx->accum != nullptr &&
-                         ctx->cam_w == p->width && ctx->cam_h == p->height;
-    // a pending asynchronous render (possibly on another stream) shares the work counter, the guard flags and the
-    // stats block with this one: finish it first
-    rc = overlap ? RT_OK : dev_wait(ctx);
-    if (rc != RT_OK) return rc;
-    if (ctx->cam_w != p->width || ctx->cam_h != p->height) setup_camera(ctx, p->width, p->height);
-
     const int mode = shard_mode_of(p->width, p->height, tile_size_of(p), count, p->shard_mode);
     if (mode != RT_SHARD_TILES && mode != RT_SHARD_SAMPLES) return fail(ctx, RT_ERR_INVALID, "rt_render: unknown shard_mode %d", p->shard_mode);
     AccumLayout L;
@@ -2781,22 +2683,35 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         L.count = count;
         L.tile = tile_size_of(p);
     }
-    if ((p->flags & RT_FLAG_ACCUMULATE) && ctx->accum && !(ctx->acc == L))
-        return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE onto a buffer of another frame size or tile layout");
+    // an accumulating pass continues the frame: every companion it adds to, the source of its rays and its layout
+    const int64_t src = rays ? ctx->rays_gen : 0;
+    const bool want[kCompanions] = {moments, aov};
+    const FrameRecord& F = ctx->frame;
+    if (accumulate) {
+        for (int k = 0; k < kCompanions; k++)
+            if (want[k] && !F.companion[k].valid)
+                return fail(ctx, RT_ERR_STATE, "rt_render: %s | RT_FLAG_ACCUMULATE onto a frame whose sums have no %s (%s)", kCompanionKinds[k].flag,
+                            kCompanionKinds[k].noun, kCompanionKinds[k].start);
+        if (F.src >= 0 && F.src != src)
+            return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE %s onto a frame of %s", rays ? "with RT_FLAG_CAMERA_RAYS" : "from the camera",
+                        F.src == 0 ? "the camera" : "other rays (rt_set_camera_rays was called since it started)");
+        if (F.sums && !(F.layout == L))
+            return fail(ctx, RT_ERR_STATE, "rt_render: RT_FLAG_ACCUMULATE onto a buffer of another frame size or tile layout");
+    }
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t stream = p->stream ? (cudaStream_t)p->stream : ctx->stream;
+    // RT_FLAG_OVERLAP: this pass goes to one of the two lane streams with its own work counter and waits for nothing on
+    // the host; it needs the frame the passes before it render into, unchanged
+    // (the camera of this frame size must be set up already: the first pass onto a restored checkpoint is a plain one)
+    const bool overlap = (p->flags & RT_FLAG_OVERLAP) && (p->flags & RT_FLAG_ASYNC) && accumulate && !(p->flags & RT_FLAG_STATS) && F.sums &&
+                         ctx->cam_w == p->width && ctx->cam_h == p->height;
+    // a pending asynchronous render (possibly on another stream) shares the work counter, the guard flags and the
+    // stats block with this one: finish it first
+    rc = overlap ? RT_OK : dev_wait(ctx);
+    if (rc != RT_OK) return rc;
+    if (ctx->cam_w != p->width || ctx->cam_h != p->height) setup_camera(ctx, p->width, p->height);
     rc = ensure_accum(ctx, L);
     if (rc != RT_OK) return rc;
-    if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) {
-        rc = ensure_moments(ctx, L.slots());
-        if (rc != RT_OK) return rc;
-    }
-    ctx->moments_valid = moments;  // an accumulating moments pass was checked above; any pass without the flag invalidates them
-    if (aov && !(p->flags & RT_FLAG_ACCUMULATE)) {
-        rc = ensure_aov(ctx, L.slots());
-        if (rc != RT_OK) return rc;
-    }
-    ctx->aov_valid = aov;  // the same rule
-    ctx->frame_src = src;  // an accumulating pass of another source was refused above
-    ctx->sums_uploaded = false;
     const bool stats = (p->flags & RT_FLAG_STATS) != 0;
     const bool want_nee = (p->flags & RT_FLAG_NEE) != 0 && ctx->scene.n_nee_lights > 0;
     const bool want_shadow = (p->flags & RT_FLAG_SHADOWED_POINT_LIGHTS) != 0 && ctx->scene.n_lights > 0;
@@ -2810,10 +2725,21 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
     int grid = 0;
     rc = v2_grid(ctx, e, &grid);
     if (rc != RT_OK) return rc;
+    // the pass is taken: a fresh pass clears the companions it starts, and the record describes the frame it leaves (a
+    // pass without a companion's flag leaves the frame without that companion)
+    for (int k = 0; k < kCompanions; k++) {
+        if (!want[k] || accumulate) continue;
+        rc = companion_reserve(ctx, k, L.slots());
+        if (rc != RT_OK) return rc;
+        CU(ctx, cudaMemsetAsync(ctx->frame.companion[k].buf, 0, L.slots() * kCompanionKinds[k].words * sizeof(unsigned long long), stream));
+    }
+    for (int k = 0; k < kCompanions; k++) ctx->frame.companion[k].valid = want[k];
+    ctx->frame.src = src;
+    ctx->frame.uploaded = false;
     RenderArgs A;
     plan_pass(A, p, mode, rank, count, 1, grid);
     A.compact = L.compact;
-    A.set_side(rays ? (const void*)ctx->rays : (const void*)ctx->moments);  // after ensure_moments: the first moments pass allocates the buffer
+    A.set_side(rays ? (const void*)ctx->rays : (const void*)ctx->frame.companion[kMoments].buf);  // after companion_reserve
     A.nee_emitters = want_nee;
     A.shadow_point_lights = want_shadow;
     A.k0 = (uint32_t)(p->seed & 0xffffffffu);
@@ -2853,7 +2779,7 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         }
         CU(ctx, cudaMemsetAsync(cnt, 0, 4 * sizeof(unsigned long long), ls));
         if (A.n_items > 0) {
-            rc = launch_v2(ctx, *e, grid, A, ctx->accum, cnt, ls);
+            rc = launch_v2(ctx, *e, grid, A, ctx->frame.sums, cnt, ls);
             if (rc != RT_OK) return rc;
         }
         CU(ctx, cudaEventRecord(ctx->lane_end[k], ls));
@@ -2864,11 +2790,9 @@ static int dev_render(DevCtx* ctx, const rt_render_params* p) {
         ctx->stats.samples = pass_samples();
         return RT_OK;
     }
-    if (!(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->accum, 0, L.slots() * 32, stream));
-    if (moments && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->moments, 0, L.slots() * 48, stream));
-    if (aov && !(p->flags & RT_FLAG_ACCUMULATE)) CU(ctx, cudaMemsetAsync(ctx->aov, 0, L.slots() * 64, stream));
+    if (!accumulate) CU(ctx, cudaMemsetAsync(ctx->frame.sums, 0, L.slots() * 32, stream));
     if (stats) CU(ctx, cudaMemsetAsync(ctx->dstats, 0, sizeof(Stats) + kTravHistBins * sizeof(unsigned long long), stream));
-    return enqueue_pass(ctx, *e, grid, A, ctx->accum, stream, pass_samples(), stats, (p->flags & RT_FLAG_ASYNC) != 0);
+    return enqueue_pass(ctx, *e, grid, A, ctx->frame.sums, stream, pass_samples(), stats, (p->flags & RT_FLAG_ASYNC) != 0);
 }
 
 // ---- multi-view batches (rt_render_views) ---------------------------------------------------------------------------
@@ -2919,22 +2843,10 @@ static int dev_render_views(DevCtx* ctx, const rt_render_params* p, const rt_cam
     rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
     const size_t slots = (size_t)n_views * p->width * p->height;
-    if (!ctx->views_accum || slots * 32 > ctx->views_cap) {
-        if (ctx->views_accum) cudaFree(ctx->views_accum);
-        ctx->views_accum = nullptr;
-        ctx->views_cap = 0;
-        ctx->views_n = 0;
-        if (cudaMalloc(&ctx->views_accum, slots * 32) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate %zu bytes for the views frame", slots * 32);
-        ctx->views_cap = slots * 32;
-    }
-    if ((size_t)n_views * sizeof(ViewRecord) > ctx->view_table_cap) {
-        if (ctx->view_table) cudaFree(ctx->view_table);
-        ctx->view_table = nullptr;
-        ctx->view_table_cap = 0;
-        if (cudaMalloc(&ctx->view_table, (size_t)n_views * sizeof(ViewRecord)) != cudaSuccess)
-            return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate the table of %d views", n_views);
-        ctx->view_table_cap = (size_t)n_views * sizeof(ViewRecord);
-    }
+    if (slots * 32 > ctx->views_accum.capacity()) ctx->views_n = 0;  // a regrown views frame has lost its contents
+    if (ctx->views_accum.reserve(slots * 32) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate %zu bytes for the views frame", slots * 32);
+    if (ctx->view_table.reserve((size_t)n_views * sizeof(ViewRecord)) != cudaSuccess)
+        return fail(ctx, RT_ERR_NOMEM, "rt_render_views: cannot allocate the table of %d views", n_views);
     // the single-frame path's background, whether or not rt_render has set up the camera since the upload
     put_background(ctx->scene, ctx->camera);
 
@@ -2977,7 +2889,7 @@ static int dev_resolve_into(DevCtx* ctx, const unsigned long long* sums, size_t 
 static int resolve_to_host(DevCtx* ctx, const unsigned long long* sums, const AccumLayout& L, int32_t total_spp, float* rgb_linear, uint8_t* rgb8) {
     const size_t n = L.slots();
     int rc = stage_buffers(ctx, n, 0);
-    if (rc == RT_OK) rc = dev_resolve_into(ctx, sums, n, total_spp, rgb_linear ? ctx->out_lin : nullptr, rgb8 ? ctx->out_rgb8 : nullptr);
+    if (rc == RT_OK) rc = dev_resolve_into(ctx, sums, n, total_spp, rgb_linear ? ctx->out_lin.get() : nullptr, rgb8 ? ctx->out_rgb8.get() : nullptr);
     if (rc == RT_OK && rgb_linear) rc = plane_to_host(ctx, ctx->out_lin, 12, L, rgb_linear);
     if (rc == RT_OK && rgb8) rc = plane_to_host(ctx, ctx->out_rgb8, 3, L, rgb8);
     return rc;
@@ -2987,12 +2899,12 @@ static int resolve_to_host(DevCtx* ctx, const unsigned long long* sums, const Ac
 // one process per GPU).  capacity_pixels >= rt_shard_pixels(...) of the rendered layout.
 static int dev_resolve_tiles(DevCtx* ctx, int32_t total_spp, float* dev_rgb_linear, uint8_t* dev_rgb8, size_t capacity_pixels) {
     if (!ctx) return RT_ERR_INVALID;
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "rt_resolve_tiles: nothing rendered yet");
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "rt_resolve_tiles: nothing rendered yet");
     if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_resolve_tiles: total_spp must be positive");
-    if (capacity_pixels < ctx->acc.slots()) return fail(ctx, RT_ERR_INVALID, "rt_resolve_tiles: the buffers hold %zu pixels, the frame has %zu", capacity_pixels, ctx->acc.slots());
+    if (capacity_pixels < ctx->frame.layout.slots()) return fail(ctx, RT_ERR_INVALID, "rt_resolve_tiles: the buffers hold %zu pixels, the frame has %zu", capacity_pixels, ctx->frame.layout.slots());
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    rc = dev_resolve_into(ctx, ctx->accum, ctx->acc.slots(), total_spp, dev_rgb_linear, dev_rgb8);
+    rc = dev_resolve_into(ctx, ctx->frame.sums, ctx->frame.layout.slots(), total_spp, dev_rgb_linear, dev_rgb8);
     if (rc != RT_OK) return rc;
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return RT_OK;
@@ -3026,13 +2938,7 @@ static int frame_slot(DevCtx* ctx, size_t px, bool lin, bool rgb8, DevCtx::OutFr
     DevCtx::OutFrame& f = ctx->frames[ctx->frame_head];
     if (!f.done) CU(ctx, cudaEventCreateWithFlags(&f.done, cudaEventDisableTiming));
     const size_t need = (lin ? px * 12 : 0) + 256 + (rgb8 ? px * 3 : 0);
-    if (need > f.cap) {
-        if (f.pinned) cudaFreeHost(f.pinned);
-        f.pinned = nullptr;
-        f.cap = 0;
-        if (cudaHostAlloc(&f.pinned, need, cudaHostAllocDefault) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of pinned host memory", need);
-        f.cap = need;
-    }
+    if (f.pinned.reserve(need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "cannot allocate %zu bytes of pinned host memory", need);
     f.has_lin = lin;
     f.has_rgb8 = rgb8;
     f.off_lin = 0;
@@ -3054,17 +2960,17 @@ static int frame_queue_copy(DevCtx* ctx, DevCtx::OutFrame* f, const void* dev_li
 
 static int dev_download_begin(DevCtx* ctx, int32_t total_spp, int32_t want_linear, int32_t want_rgb8) {
     if (!ctx) return RT_ERR_INVALID;
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "rt_download_begin: nothing rendered yet");
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "rt_download_begin: nothing rendered yet");
     if (total_spp <= 0 || (!want_linear && !want_rgb8)) return fail(ctx, RT_ERR_INVALID, "rt_download_begin: bad arguments");
-    if (ctx->acc.compact) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_download_begin: compact tile buffers go through rt_resolve_tiles / rt_untile_begin");
+    if (ctx->frame.layout.compact) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_download_begin: compact tile buffers go through rt_resolve_tiles / rt_untile_begin");
     CU(ctx, cudaSetDevice(ctx->device));
-    const size_t px = ctx->acc.slots();
+    const size_t px = ctx->frame.layout.slots();
     DevCtx::OutFrame* f = nullptr;
     // stream order, no host wait: the previous copy and the pending render (on its own stream), then the resolve
     int rc = frame_slot(ctx, px, want_linear != 0, want_rgb8 != 0, &f);
     if (rc == RT_OK) rc = stage_buffers(ctx, px, 0);
     if (rc == RT_OK) rc = dev_join(ctx, ctx->stream);
-    if (rc == RT_OK) rc = dev_resolve_into(ctx, ctx->accum, px, total_spp, want_linear ? ctx->out_lin : nullptr, want_rgb8 ? ctx->out_rgb8 : nullptr);
+    if (rc == RT_OK) rc = dev_resolve_into(ctx, ctx->frame.sums, px, total_spp, want_linear ? ctx->out_lin.get() : nullptr, want_rgb8 ? ctx->out_rgb8.get() : nullptr);
     if (rc != RT_OK) return rc;
     return frame_queue_copy(ctx, f, ctx->out_lin, ctx->out_rgb8, px);
 }
@@ -3099,11 +3005,11 @@ static int dev_frame_end(DevCtx* ctx, const float** rgb_linear, const uint8_t** 
 
 static int dev_download(DevCtx* ctx, int32_t total_spp, float* rgb_linear, uint8_t* rgb8) {
     if (!ctx) return RT_ERR_INVALID;
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "rt_download: nothing rendered yet");
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "rt_download: nothing rendered yet");
     if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_download: total_spp must be positive");
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    return resolve_to_host(ctx, ctx->accum, ctx->acc, total_spp, rgb_linear, rgb8);
+    return resolve_to_host(ctx, ctx->frame.sums, ctx->frame.layout, total_spp, rgb_linear, rgb8);
 }
 
 // views [first, first + count) of the views frame, each resolved like rt_download's planes
@@ -3121,19 +3027,21 @@ static int dev_download_views(DevCtx* ctx, int32_t total_spp, int32_t first, int
                            total_spp, rgb_linear, rgb8);
 }
 
-// ---- second moments (RT_FLAG_MOMENTS) ------------------------------------------------------------------------------
-static int moments_ready(DevCtx* ctx, const char* what) {
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
-    if (!ctx->moments_valid) return fail(ctx, RT_ERR_STATE, "%s: the frame has no moments (render it with RT_FLAG_MOMENTS)", what);
+// ---- second moments (RT_FLAG_MOMENTS) and auxiliary outputs (RT_FLAG_AOV) --------------------------------------------
+// The companion k of the frame, for a readback named `what`, after the passes in flight
+static int companion_ready(DevCtx* ctx, int k, const char* what) {
+    if (!ctx->frame.sums) return fail(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
+    if (!ctx->frame.companion[k].valid)
+        return fail(ctx, RT_ERR_STATE, "%s: the frame has no %s (render it with %s)", what, kCompanionKinds[k].noun, kCompanionKinds[k].flag);
     return dev_wait(ctx);
 }
 
 // variance_kernel over the slots of the frame into out_lin (the buffer of the linear radiance of rt_download)
 static int dev_variance_into(DevCtx* ctx, int32_t total_spp) {
-    const size_t n = ctx->acc.slots();
+    const size_t n = ctx->frame.layout.slots();
     int rc = stage_buffers(ctx, n, 0);
     if (rc != RT_OK) return rc;
-    if (n) variance_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, ctx->moments, (int)n, total_spp, ctx->out_lin);
+    if (n) variance_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->frame.sums, ctx->frame.companion[kMoments].buf, (int)n, total_spp, ctx->out_lin);
     CU(ctx, cudaGetLastError());
     return RT_OK;
 }
@@ -3141,24 +3049,24 @@ static int dev_variance_into(DevCtx* ctx, int32_t total_spp) {
 static int dev_download_variance(DevCtx* ctx, int32_t total_spp, float* variance) {
     if (!ctx || !variance) return RT_ERR_INVALID;
     if (total_spp < 2) return fail(ctx, RT_ERR_INVALID, "rt_download_variance: total_spp must be at least 2");
-    int rc = moments_ready(ctx, "rt_download_variance");
+    int rc = companion_ready(ctx, kMoments, "rt_download_variance");
     if (rc == RT_OK) rc = dev_variance_into(ctx, total_spp);
     if (rc != RT_OK) return rc;
-    return plane_to_host(ctx, ctx->out_lin, 12, ctx->acc, variance);
+    return plane_to_host(ctx, ctx->out_lin, 12, ctx->frame.layout, variance);
 }
 
 // the 12 integer partials of noise_kernel over the slots of this device, and the frame pixels they cover
 static int dev_noise_partials(DevCtx* ctx, int32_t total_spp, uint64_t* partials, uint64_t* pixels) {
-    int rc = moments_ready(ctx, "rt_frame_noise");
+    int rc = companion_ready(ctx, kMoments, "rt_frame_noise");
     if (rc != RT_OK) return rc;
-    if (!ctx->noise_sums) CU(ctx, cudaMalloc(&ctx->noise_sums, 12 * sizeof(unsigned long long)));
+    CU(ctx, ctx->noise_sums.reserve(12 * sizeof(unsigned long long)));
     CU(ctx, cudaMemsetAsync(ctx->noise_sums, 0, 12 * sizeof(unsigned long long), ctx->stream));
-    const size_t n = ctx->acc.slots();
-    if (n) noise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->accum, ctx->moments, (int)n, total_spp, ctx->noise_sums);
+    const size_t n = ctx->frame.layout.slots();
+    if (n) noise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->frame.sums, ctx->frame.companion[kMoments].buf, (int)n, total_spp, ctx->noise_sums);
     CU(ctx, cudaGetLastError());
     CU(ctx, cudaMemcpyAsync(partials, ctx->noise_sums, 12 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    *pixels = ctx->acc.pixels();
+    *pixels = ctx->frame.layout.pixels();
     return RT_OK;
 }
 
@@ -3176,11 +3084,11 @@ static void noise_from_partials(const uint64_t* w, uint64_t pixels, int32_t tota
 
 static int dev_moments_download(DevCtx* ctx, uint64_t* host, size_t bytes) {
     if (!ctx || !host) return RT_ERR_INVALID;
-    const size_t full = (size_t)ctx->acc.width * ctx->acc.height * 48;
-    if (ctx->accum && bytes != full) return fail(ctx, RT_ERR_INVALID, "rt_moments_download: a %dx%d frame is %zu bytes, got %zu", ctx->acc.width, ctx->acc.height, full, bytes);
-    int rc = moments_ready(ctx, "rt_moments_download");
+    const size_t full = (size_t)ctx->frame.layout.width * ctx->frame.layout.height * 48;
+    if (ctx->frame.sums && bytes != full) return fail(ctx, RT_ERR_INVALID, "rt_moments_download: a %dx%d frame is %zu bytes, got %zu", ctx->frame.layout.width, ctx->frame.layout.height, full, bytes);
+    int rc = companion_ready(ctx, kMoments, "rt_moments_download");
     if (rc != RT_OK) return rc;
-    return plane_to_host(ctx, ctx->moments, 48, ctx->acc, host);
+    return plane_to_host(ctx, ctx->frame.companion[kMoments].buf, 48, ctx->frame.layout, host);
 }
 
 // the moments of the sums rt_accum_upload restored just before (same full frame)
@@ -3189,32 +3097,25 @@ static int dev_moments_upload(DevCtx* ctx, const uint64_t* host, size_t bytes, i
     if (width <= 0 || height <= 0 || (long long)width * height >= (1ll << 31)) return fail(ctx, RT_ERR_INVALID, "rt_moments_upload: bad frame size %dx%d", width, height);
     const size_t need = (size_t)width * height * 48;
     if (bytes != need) return fail(ctx, RT_ERR_INVALID, "rt_moments_upload: a %dx%d frame is %zu bytes, got %zu", width, height, need, bytes);
-    if (!ctx->sums_uploaded || ctx->acc.compact || ctx->acc.width != width || ctx->acc.height != height)
+    if (!ctx->frame.uploaded || ctx->frame.layout.compact || ctx->frame.layout.width != width || ctx->frame.layout.height != height)
         return fail(ctx, RT_ERR_STATE, "rt_moments_upload: follows rt_accum_upload of the same %dx%d frame", width, height);
     CU(ctx, cudaSetDevice(ctx->device));
     int rc = dev_wait(ctx);
-    if (rc == RT_OK) rc = ensure_moments(ctx, (size_t)width * height);
+    if (rc == RT_OK) rc = companion_reserve(ctx, kMoments, (size_t)width * height);
     if (rc != RT_OK) return rc;
-    CU(ctx, cudaMemcpyAsync(ctx->moments, host, need, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(ctx->frame.companion[kMoments].buf, host, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
-    ctx->moments_valid = true;
+    ctx->frame.companion[kMoments].valid = true;
     return RT_OK;
-}
-
-// ---- auxiliary outputs (RT_FLAG_AOV) ---------------------------------------------------------------------------------
-static int aov_ready(DevCtx* ctx, const char* what) {
-    if (!ctx->accum) return fail(ctx, RT_ERR_STATE, "%s: nothing rendered yet", what);
-    if (!ctx->aov_valid) return fail(ctx, RT_ERR_STATE, "%s: the frame has no AOV sums (render it with RT_FLAG_AOV)", what);
-    return dev_wait(ctx);
 }
 
 // aov_resolve_kernel over the slots of the frame into frame_scratch, `offset` bytes in (8 floats per slot)
 static int dev_aov_into(DevCtx* ctx, int32_t total_spp, size_t offset, const void** plane) {
-    const size_t n = ctx->acc.slots();
+    const size_t n = ctx->frame.layout.slots();
     int rc = stage_buffers(ctx, 0, offset + n * 32);
     if (rc != RT_OK) return rc;
     *plane = ctx->frame_scratch + offset;
-    if (n) aov_resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->aov, (int)n, total_spp, (float4*)(ctx->frame_scratch + offset));
+    if (n) aov_resolve_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->frame.companion[kAov].buf, (int)n, total_spp, (float4*)(ctx->frame_scratch + offset));
     CU(ctx, cudaGetLastError());
     return RT_OK;
 }
@@ -3222,13 +3123,13 @@ static int dev_aov_into(DevCtx* ctx, int32_t total_spp, size_t offset, const voi
 static int dev_download_aov(DevCtx* ctx, int32_t total_spp, float* aov) {
     if (!ctx || !aov) return RT_ERR_INVALID;
     if (total_spp <= 0) return fail(ctx, RT_ERR_INVALID, "rt_download_aov: total_spp must be positive");
-    int rc = aov_ready(ctx, "rt_download_aov");
+    int rc = companion_ready(ctx, kAov, "rt_download_aov");
     // a compact plane is untiled into the front of frame_scratch (plane_to_host): resolve it behind that room
-    const size_t room = ctx->acc.compact ? (size_t)ctx->acc.width * ctx->acc.height * 32 : 0;
+    const size_t room = ctx->frame.layout.compact ? (size_t)ctx->frame.layout.width * ctx->frame.layout.height * 32 : 0;
     const void* plane = nullptr;
     if (rc == RT_OK) rc = dev_aov_into(ctx, total_spp, room, &plane);
     if (rc != RT_OK) return rc;
-    return plane_to_host(ctx, plane, 32, ctx->acc, aov);
+    return plane_to_host(ctx, plane, 32, ctx->frame.layout, aov);
 }
 
 // ---- caller-defined cameras (rt_set_camera_rays, RT_FLAG_CAMERA_RAYS) ----------------------------------------------
@@ -3242,17 +3143,12 @@ static int dev_set_camera_rays(DevCtx* ctx, const rt_camera_ray* rays, int32_t w
     if (rc != RT_OK) return rc;
     ctx->rays_gen++;
     ctx->rays_w = ctx->rays_h = 0;
-    const size_t need = rays ? (size_t)width * height * sizeof(rt_camera_ray) : 0;
-    if (ctx->rays && (!rays || need > ctx->rays_cap)) {
-        cudaFree(ctx->rays);
-        ctx->rays = nullptr;
-        ctx->rays_cap = 0;
+    if (!rays) {
+        ctx->rays.release();
+        return RT_OK;
     }
-    if (!rays) return RT_OK;
-    if (!ctx->rays) {
-        if (cudaMalloc(&ctx->rays, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_camera_rays: cannot allocate %zu bytes for the rays", need);
-        ctx->rays_cap = need;
-    }
+    const size_t need = (size_t)width * height * sizeof(rt_camera_ray);
+    if (ctx->rays.reserve(need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_camera_rays: cannot allocate %zu bytes for the rays", need);
     CU(ctx, cudaMemcpyAsync(ctx->rays, rays, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->rays_w = width;
@@ -3267,20 +3163,13 @@ static int dev_set_environment(DevCtx* ctx, const float4* map, size_t n) {
     CU(ctx, cudaSetDevice(ctx->device));
     int rc = dev_wait(ctx);
     if (rc != RT_OK) return rc;
-    const size_t need = map ? n * sizeof(float4) : 0;
-    if (ctx->env && (!map || need > ctx->env_cap)) {
-        cudaFree(ctx->env);
-        ctx->env = nullptr;
-        ctx->env_cap = 0;
+    if (!map) {
+        ctx->env.release();
+        return RT_OK;
     }
-    if (!map) return RT_OK;
-    float4* buf = ctx->env;
-    if (!buf) {
-        if (cudaMalloc(&buf, need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_environment: cannot allocate %zu bytes for the map", need);
-        ctx->env_cap = need;
-    }
-    ctx->env = buf;
-    CU(ctx, cudaMemcpyAsync(buf, map, need, cudaMemcpyHostToDevice, ctx->stream));
+    const size_t need = n * sizeof(float4);
+    if (ctx->env.reserve(need) != cudaSuccess) return fail(ctx, RT_ERR_NOMEM, "rt_set_environment: cannot allocate %zu bytes for the map", need);
+    CU(ctx, cudaMemcpyAsync(ctx->env, map, need, cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return RT_OK;
 }
@@ -3293,17 +3182,17 @@ static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* p
     CU(ctx, cudaSetDevice(ctx->device));
     if (ctx->cam_w != width || ctx->cam_h != height) setup_camera(ctx, width, height);
     const size_t n = (size_t)width * height;
-    int* d_id = nullptr;
-    float *d_t = nullptr, *d_n = nullptr, *d_p = nullptr, *d_uv = nullptr;
+    DeviceBuffer<int> d_id;
+    DeviceBuffer<float> d_t, d_n, d_p, d_uv;
     cudaError_t e = cudaSuccess;
-    auto alloc = [&](void** p, size_t bytes, const void* want) {
-        if (want && e == cudaSuccess) e = cudaMalloc(p, bytes);
+    auto alloc = [&](auto& buf, size_t bytes, const void* want) {
+        if (want && e == cudaSuccess) e = buf.reserve(bytes);
     };
-    alloc((void**)&d_id, n * 4, prim_id);
-    alloc((void**)&d_t, n * 4, t);
-    alloc((void**)&d_n, n * 12, normal);
-    alloc((void**)&d_p, n * 12, point);
-    alloc((void**)&d_uv, n * 8, uv);
+    alloc(d_id, n * 4, prim_id);
+    alloc(d_t, n * 4, t);
+    alloc(d_n, n * 12, normal);
+    alloc(d_p, n * 12, point);
+    alloc(d_uv, n * 8, uv);
     if (e == cudaSuccess) {
         dim3 block(8, 8), grid((width + 7) / 8, (height + 7) / 8);
         aov_kernel<<<grid, block, 0, ctx->stream>>>(ctx->scene, ctx->camera_d, width, height, d_id, d_t, d_n, d_p, d_uv);
@@ -3318,7 +3207,6 @@ static int dev_render_aov(DevCtx* ctx, int32_t width, int32_t height, int32_t* p
     fetch(normal, d_n, n * 12);
     fetch(point, d_p, n * 12);
     fetch(uv, d_uv, n * 8);
-    cudaFree(d_id); cudaFree(d_t); cudaFree(d_n); cudaFree(d_p); cudaFree(d_uv);
     if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_render_aov: %s", cudaGetErrorString(e));
     return RT_OK;
 }
@@ -3340,8 +3228,8 @@ extern "C" size_t rt_struct_size(int which) {
 static int dev_measure_fp32_peak(DevCtx* ctx, double* tflops) {
     if (!ctx || !tflops) return RT_ERR_INVALID;
     CU(ctx, cudaSetDevice(ctx->device));
-    float* d = nullptr;
-    CU(ctx, cudaMalloc(&d, 16));
+    DeviceBuffer<float> d;
+    CU(ctx, d.reserve(16));
     const int iters = 1 << 16, threads = 1024, blocks = ctx->sm_count * 2;
     double best = 0;
     for (int rep = 0; rep < 5; rep++) {
@@ -3349,13 +3237,12 @@ static int dev_measure_fp32_peak(DevCtx* ctx, double* tflops) {
         fma_peak_kernel<<<blocks, threads, 0, ctx->stream>>>(d, iters, 1.0000001f, 1e-7f);
         cudaEventRecord(ctx->ev1, ctx->stream);
         cudaError_t e = cudaEventSynchronize(ctx->ev1);
-        if (e != cudaSuccess) { cudaFree(d); return fail(ctx, RT_ERR_CUDA, "rt_measure_fp32_peak: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_measure_fp32_peak: %s", cudaGetErrorString(e));
         float ms = 0;
         cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         double flops = 2.0 * 8.0 * iters * (double)threads * blocks;
         if (rep > 0) best = std::max(best, flops / (ms * 1e-3) * 1e-12);
     }
-    cudaFree(d);
     *tflops = best;
     return RT_OK;
 }
@@ -3364,9 +3251,9 @@ static int dev_measure_l1_peak(DevCtx* ctx, double* gbs) {
     if (!ctx || !gbs) return RT_ERR_INVALID;
     CU(ctx, cudaSetDevice(ctx->device));
     const int blocks = ctx->sm_count * 2, threads = 256, iters = 1 << 13;
-    uint4* d = nullptr;
+    DeviceBuffer<uint4> d;
     const size_t bytes = (size_t)blocks * 2048 * sizeof(uint4);
-    CU(ctx, cudaMalloc(&d, bytes + 64));
+    CU(ctx, d.reserve(bytes + 64));
     cudaMemsetAsync(d, 1, bytes + 64, ctx->stream);
     cudaFuncSetAttribute(l1_peak_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 0);
     double best = 0;
@@ -3375,13 +3262,12 @@ static int dev_measure_l1_peak(DevCtx* ctx, double* gbs) {
         l1_peak_kernel<<<blocks, threads, 0, ctx->stream>>>(d, iters, d + (bytes / sizeof(uint4)));
         cudaEventRecord(ctx->ev1, ctx->stream);
         cudaError_t e = cudaEventSynchronize(ctx->ev1);
-        if (e != cudaSuccess) { cudaFree(d); return fail(ctx, RT_ERR_CUDA, "rt_measure_l1_peak: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "rt_measure_l1_peak: %s", cudaGetErrorString(e));
         float ms = 0;
         cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
         const double moved = 16.0 * 8.0 * iters * (double)threads * blocks;
         if (rep > 0) best = std::max(best, moved / (ms * 1e-3) * 1e-9);
     }
-    cudaFree(d);
     *gbs = best;
     return RT_OK;
 }
@@ -3391,16 +3277,16 @@ template <class Launch>
 static int run_probe(DevCtx* ctx, const char* name, const std::vector<std::pair<const void*, size_t>>& inputs,
                      const std::vector<std::pair<void*, size_t>>& outputs, Launch launch) {
     CU(ctx, cudaSetDevice(ctx->device));
-    std::vector<void*> din(inputs.size(), nullptr), dout(outputs.size(), nullptr);
+    std::vector<DeviceBuffer<void>> din(inputs.size()), dout(outputs.size());
     cudaError_t e = cudaSuccess;
     for (size_t i = 0; i < inputs.size() && e == cudaSuccess; i++) {
-        e = cudaMalloc(&din[i], std::max<size_t>(inputs[i].second, 16));
+        e = din[i].reserve(std::max<size_t>(inputs[i].second, 16));
         // stream-ordered with the probe kernel (a plain cudaMemcpy from pageable memory only guarantees staging:
         // the kernel on the non-blocking ctx->stream could read the buffer before the DMA lands)
         if (e == cudaSuccess && inputs[i].second) e = cudaMemcpyAsync(din[i], inputs[i].first, inputs[i].second, cudaMemcpyHostToDevice, ctx->stream);
     }
     for (size_t i = 0; i < outputs.size() && e == cudaSuccess; i++)
-        if (outputs[i].first) e = cudaMalloc(&dout[i], std::max<size_t>(outputs[i].second, 16));
+        if (outputs[i].first) e = dout[i].reserve(std::max<size_t>(outputs[i].second, 16));
     if (e == cudaSuccess) {
         launch(din, dout);
         e = cudaGetLastError();
@@ -3408,8 +3294,6 @@ static int run_probe(DevCtx* ctx, const char* name, const std::vector<std::pair<
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     for (size_t i = 0; i < outputs.size() && e == cudaSuccess; i++)
         if (outputs[i].first) e = cudaMemcpy(outputs[i].first, dout[i], outputs[i].second, cudaMemcpyDeviceToHost);
-    for (void* p : din) cudaFree(p);
-    for (void* p : dout) cudaFree(p);
     if (e != cudaSuccess) return fail(ctx, RT_ERR_CUDA, "%s: %s", name, cudaGetErrorString(e));
     return RT_OK;
 }
@@ -3420,8 +3304,8 @@ static int dev_probe_texture(DevCtx* ctx, int32_t texture, int32_t n, const floa
     if (n <= 0 || !uvp || !rgb) return fail(ctx, RT_ERR_INVALID, "rt_probe_texture: bad arguments");
     if (texture < 0 || texture >= ctx->n_textures) return fail(ctx, RT_ERR_INVALID, "rt_probe_texture: texture %d outside [0,%d)", texture, ctx->n_textures);
     return run_probe(ctx, "rt_probe_texture", {{uvp, (size_t)n * 20}}, {{rgb, (size_t)n * 12}},
-                     [&](std::vector<void*>& in, std::vector<void*>& out) {
-                         probe_texture_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, texture, n, (const float*)in[0], (float*)out[0]);
+                     [&](std::vector<DeviceBuffer<void>>& in, std::vector<DeviceBuffer<void>>& out) {
+                         probe_texture_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, texture, n, (const float*)in[0].get(), (float*)out[0].get());
                      });
 }
 
@@ -3431,9 +3315,9 @@ static int dev_probe_scatter(DevCtx* ctx, int32_t material, int32_t n, const flo
     if (n <= 0 || !in_rec || !uniforms || !out_rec) return fail(ctx, RT_ERR_INVALID, "rt_probe_scatter: bad arguments");
     if (material < 0 || material >= ctx->n_materials) return fail(ctx, RT_ERR_INVALID, "rt_probe_scatter: material %d outside [0,%d)", material, ctx->n_materials);
     return run_probe(ctx, "rt_probe_scatter", {{in_rec, (size_t)n * 64}, {uniforms, (size_t)n * 16}}, {{out_rec, (size_t)n * 64}},
-                     [&](std::vector<void*>& in, std::vector<void*>& out) {
-                         probe_scatter_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, material, n, (const float*)in[0],
-                                                                                         (const float*)in[1], (float*)out[0]);
+                     [&](std::vector<DeviceBuffer<void>>& in, std::vector<DeviceBuffer<void>>& out) {
+                         probe_scatter_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, material, n, (const float*)in[0].get(),
+                                                                                         (const float*)in[1].get(), (float*)out[0].get());
                      });
 }
 
@@ -3443,9 +3327,9 @@ static int dev_probe_hit(DevCtx* ctx, int32_t n, const float* rays, int32_t* pri
     if (n <= 0 || !rays) return fail(ctx, RT_ERR_INVALID, "rt_probe_hit: bad arguments");
     int rc = run_probe(ctx, "rt_probe_hit", {{rays, (size_t)n * 36}},
                        {{prim_id, (size_t)n * 4}, {t, (size_t)n * 4}, {normal, (size_t)n * 12}, {uv, (size_t)n * 8}},
-                       [&](std::vector<void*>& in, std::vector<void*>& out) {
-                           probe_hit_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, n, (const float*)in[0], (int*)out[0],
-                                                                                       (float*)out[1], (float*)out[2], (float*)out[3]);
+                       [&](std::vector<DeviceBuffer<void>>& in, std::vector<DeviceBuffer<void>>& out) {
+                           probe_hit_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->scene, n, (const float*)in[0].get(), (int*)out[0].get(),
+                                                                                       (float*)out[1].get(), (float*)out[2].get(), (float*)out[3].get());
                        });
     return rc;
 }
